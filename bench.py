@@ -59,7 +59,40 @@ def parse_args():
                     help="N>1: the panel is replicated over NVLink in this many pieces (0 = every rank uploads all "
                          "of it; default max(2, 16 // N): ~40 MB per rank and piece at C3; measured at N=2: "
                          "0 -> 12.8 ms, 1 -> 15.6, 4 -> 11.6, 8 -> 10.7, 16 -> 12.1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's results of the last timed step as DIR/<name>.npy "
+                         "(targets, n_windows, and w_start, w_end, w_nsites, w_loglik of every window, target after "
+                         "target); under 64 MB in all, larger results keep a fixed seeded sample of the targets")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 60_000_000  # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(path, targets, n_windows, w_start, w_end, w_nsites, w_loglik):
+    """Writes the window scores a caller of the --LD scoring path receives, one float64 .npy file per
+    array.  Only a target's first n_windows slots hold results, so the per-window arrays keep just those,
+    target after target ([sum of n_windows] and [sum of n_windows, 3]); n_windows splits them again.
+    When all of it could exceed DUMP_LIMIT_BYTES, a fixed seeded sample of the targets is kept, in target order."""
+    T, maxW = w_loglik.shape[:2]
+    per_target = 8 * (1 + 1 + maxW * (3 + 3))  # targets, n_windows, w_start/w_end/w_nsites, w_loglik
+    rows = np.arange(T)
+    if T * per_target > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(T, DUMP_LIMIT_BYTES // per_target, replace=False))
+    nw = n_windows[rows].astype(np.int64)
+    valid = np.arange(maxW)[None, :] < nw[:, None]
+
+    def windows(a):
+        return a[rows][valid].astype(np.float64)
+
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("targets", targets[rows].astype(np.float64)), ("n_windows", nw.astype(np.float64)),
+                    ("w_start", windows(w_start)), ("w_end", windows(w_end)), ("w_nsites", windows(w_nsites)),
+                    ("w_loglik", windows(w_loglik))):
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -430,6 +463,9 @@ def main():
     ms_total = timed(score, args.steps)
     rank_ms = getattr(timed, "per_rank", None)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # the e2e steps below overwrite the same host buffers, so the last timed step's results are saved now
+        dump_outputs(args.dump_outputs, targets, o_nw.numpy(), o_ws.numpy(), o_we.numpy(), o_wn.numpy(), o_ll.numpy())
     stats = eng.kernel_stats()
     ld_path = eng.last_ld_path()
     ms_step = ms_total / args.steps
