@@ -57,6 +57,8 @@ enum KernelId {
     K_V_EXPAND_B,       // column operand slabs (r0, r1, r0 & r1)
     K_LD_VMMA,          // tcgen05 GEMM over per-target windows + fused log-sum-exp -> LIBD0, LIBD1
     K_WINDOW_LINEAR,    // the reference's own running fp64 products per window (ibdgem_scores.w_lik_linear)
+    K_POSTERIOR_FWD,    // hiddengem posterior: forward pass, alpha checkpoints per 16-bin chunk
+    K_POSTERIOR_BWD,    // hiddengem posterior: backward pass, posteriors + expected occupancy
     K_COUNT
 };
 
@@ -194,7 +196,7 @@ enum ScratchSlot {
     SC_WN, SC_WS, SC_WE, SC_COUNTERS, SC_SITE_STATUS, SC_SITE_LIK, SC_LD_PART, SC_NREFPANEL,
     SC_HG_LIK, SC_HG_OFF, SC_HG_STATE, SC_HG_SCORE, SC_HG_COUNTS, SC_HG_NRMT, SC_HG_SCORET, SC_HG_FROMT, SC_HG_LAST,
     SC_MMA_TGT, SC_MMA_BG, SC_MMA_ROWLSE, SC_MMA_BGIDX, SC_MMA_MISC, SC_MMA_UNIT,
-    SC_WLIN, SC_WLL_PACK, SC_V_KS, SC_V_KE, SC_V_TWBASE, SC_V_TWI, SC_V_TWD, SC_V_ORDER, SC_V_HIST, SC_V_TILES, SC_V_MISC, SC_SLOTS
+    SC_WLIN, SC_WLL_PACK, SC_V_KS, SC_V_KE, SC_V_TWBASE, SC_V_TWI, SC_V_TWD, SC_V_ORDER, SC_V_HIST, SC_V_TILES, SC_V_MISC, SC_HG_CKPT, SC_SLOTS
 };
 int scratch(ibdgem_engine *e, int slot, size_t bytes, void **out);
 

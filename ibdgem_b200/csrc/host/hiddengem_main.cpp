@@ -3,7 +3,8 @@
 // The recursion runs on the GPU in log space (hiddengem_viterbi_batch); the reference's x87
 // long-double running products are re-synthesised for printing from their logarithms.
 // Additive: -s may be given several times; the tables are read in parallel, scored in one batch and
-// printed in order (formatted in parallel).
+// printed in order (formatted in parallel).  --posterior (additive) also prints each bin's posterior state
+// probabilities (hiddengem_posterior_batch) and the expected state fractions.
 #include <getopt.h>
 
 #include <cmath>
@@ -30,6 +31,8 @@ void print_help(int code) {
           "--p01  FLOAT             Penalty for switching between states IBD0 and IBD1 (default: 1e-3)\n"
           "--p02  FLOAT             Penalty for switching between states IBD0 and IBD2 (default: 1e-6)\n"
           "--p12  FLOAT             Penalty for switching between states IBD1 and IBD2 (default: 1e-3)\n"
+          "--posterior              Also print each segment's posterior probability of every state (columns\n"
+          "                            P_IBD0, P_IBD1, P_IBD2) and the expected share of segments per state\n"
           "--help                   Show this help message and exit\n\n"
           "Format of output table is tab-delimited with columns:\n"
           "Segment, IBD0_Score, IBD1_Score, IBD2_Score, Inferred_State\n",
@@ -106,8 +109,10 @@ int read_summary(const std::string &fn, std::vector<double> *lik) {
 int main(int argc, char *argv[]) {
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
     std::vector<std::string> files;
+    bool posterior = false;
     static struct option longopts[] = {{"summary", required_argument, 0, 's'}, {"p01", required_argument, 0, 1},
                                        {"p02", required_argument, 0, 2},       {"p12", required_argument, 0, 3},
+                                       {"posterior", no_argument, 0, 4},       // additive
                                        {"help", no_argument, 0, 'h'},          {0, 0, 0, 0}};
     if (argc == 1) print_help(0);
     int option;
@@ -117,6 +122,7 @@ int main(int argc, char *argv[]) {
             case 1: p01 = atof(optarg); break;
             case 2: p02 = atof(optarg); break;
             case 3: p12 = atof(optarg); break;
+            case 4: posterior = true; break;
             case 'h': print_help(0); break;
             case ':':
                 fprintf(stderr, "Option -%c missing required argument.\n", optopt);
@@ -155,9 +161,12 @@ int main(int argc, char *argv[]) {
     std::vector<uint8_t> state(nb);
     std::vector<double> score(nb * 3);
     std::vector<int64_t> counts((off.size() - 1) * 3);
+    std::vector<double> post(posterior ? nb * 3 : 0), expected(posterior ? (off.size() - 1) * 3 : 0);
     if (ibdgem_engine_create(&prm, &e) ||
         hiddengem_viterbi_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, state.data(), score.data(),
-                                counts.data())) {
+                                counts.data()) ||
+        (posterior && hiddengem_posterior_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, post.data(),
+                                                expected.data()))) {
         fprintf(stderr, "%s\n", ibdgem_last_error());
         exit(1);
     }
@@ -174,19 +183,29 @@ int main(int argc, char *argv[]) {
             const double n = (double)(b - a);
             std::string &out = text[k];
             out.clear();
-            out.reserve((size_t)(b - a) * 48 + 256);
-            out += "Segment\tIBD0_Score\tIBD1_Score\tIBD2_Score\tInferred_State\n";
+            out.reserve((size_t)(b - a) * (posterior ? 80 : 48) + 512);
+            out += posterior ? "Segment\tIBD0_Score\tIBD1_Score\tIBD2_Score\tInferred_State\tP_IBD0\tP_IBD1\tP_IBD2\n"
+                             : "Segment\tIBD0_Score\tIBD1_Score\tIBD2_Score\tInferred_State\n";
             char s0[48], s1[48], s2[48], row[192];
             for (int64_t i = a; i < b; i++) {
                 put_score(s0, score[(size_t)i * 3]);
                 put_score(s1, score[(size_t)i * 3 + 1]);
                 put_score(s2, score[(size_t)i * 3 + 2]);
-                out.append(row, (size_t)snprintf(row, sizeof row, "%d\t%s\t%s\t%s\t%d\n", (int)(i - a + 1), s0, s1, s2, (int)state[(size_t)i]));
+                if (posterior)
+                    out.append(row, (size_t)snprintf(row, sizeof row, "%d\t%s\t%s\t%s\t%d\t%.6f\t%.6f\t%.6f\n", (int)(i - a + 1), s0, s1, s2,
+                                                     (int)state[(size_t)i], post[(size_t)i * 3], post[(size_t)i * 3 + 1], post[(size_t)i * 3 + 2]));
+                else
+                    out.append(row, (size_t)snprintf(row, sizeof row, "%d\t%s\t%s\t%s\t%d\n", (int)(i - a + 1), s0, s1, s2, (int)state[(size_t)i]));
             }
             const double c0 = (double)counts[t * 3], c1 = (double)counts[t * 3 + 1], c2 = (double)counts[t * 3 + 2];
             out.append(row, (size_t)snprintf(row, sizeof row, "#%% IBD0 (n = %.0f): %.2f\n", c0, (c0 / n) * 100));
             out.append(row, (size_t)snprintf(row, sizeof row, "#%% IBD1 (n = %.0f): %.2f\n", c1, (c1 / n) * 100));
             out.append(row, (size_t)snprintf(row, sizeof row, "#%% IBD2 (n = %.0f): %.2f\n", c2, (c2 / n) * 100));
+            if (posterior)  // expected bins per state: the sum of the posteriors
+                for (int k = 0; k < 3; k++) {
+                    const double x = expected[t * 3 + (size_t)k];
+                    out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d (n = %.2f): %.2f\n", k, x, (x / n) * 100));
+                }
         });
         for (size_t k = 0; k < nt; k++) fwrite(text[k].data(), 1, text[k].size(), stdout);
     }

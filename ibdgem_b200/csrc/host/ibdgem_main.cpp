@@ -41,6 +41,7 @@ struct Options {
     const char *uchr = nullptr;
     int gpus = 1, batch = 0, no_tab = 0;
     int hiddengem = 0;  // --hiddengem: also write <pileup>.<target>.hiddengem.txt from the window scores
+    int posterior = 0;  // --posterior (with --hiddengem): posterior state probabilities in those files
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
 };
 
@@ -87,6 +88,10 @@ void print_help(int code) {
         "-e, --error-rate  FLOAT         Error rate of sequencing platform (default: 0.02)\n"
         "-v, --variable-sites-only       If set, make output only for sites that are not\n"
         "                                   homozygous reference in the genotype file for this sample\n"
+        "--hiddengem                     Also infer IBD states from each target's window scores: writes\n"
+        "                                   <pileup-name>.<target>.hiddengem.txt (penalties --p01, --p02, --p12)\n"
+        "--posterior                     With --hiddengem: add each segment's posterior state probabilities\n"
+        "                                   (P_IBD0, P_IBD1, P_IBD2) and the expected share of segments per state\n"
         "-h, --help                      Show this help message and exit\n\n"
         "Format of likelihood table is tab-delimited with columns:\n"
         "CHR, rsID, POS, REF, ALT, AF, DP, SQ_NREF, SQ_NALT, GT_A0, GT_A1, LIBD0, LIBD1, LIBD2\n\n"
@@ -343,6 +348,7 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
         std::vector<uint8_t> hg_state;
         std::vector<double> hg_score;
         std::vector<int64_t> hg_counts, hg_off;
+        std::vector<double> hg_post, hg_expected;
         if (o.hiddengem) {
             std::vector<double> packed;
             hg_off.assign(1, 0);
@@ -357,6 +363,13 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
             if (nbins && hiddengem_viterbi_batch(e, (int32_t)T, hg_off.data(), packed.data(), 1, o.p01, o.p02, o.p12, hg_state.data(),
                                                  hg_score.data(), hg_counts.data()))
                 return fail_engine();
+            if (o.posterior) {  // the same packed natural-log scores
+                hg_post.resize(nbins * 3);
+                hg_expected.resize(T * 3);
+                if (nbins && hiddengem_posterior_batch(e, (int32_t)T, hg_off.data(), packed.data(), 1, o.p01, o.p02, o.p12, hg_post.data(),
+                                                       hg_expected.data()))
+                    return fail_engine();
+            }
         }
 
         // one target = two files: independent, so the batch is written by a few threads
@@ -445,18 +458,26 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
                     fprintf(stderr, "[::] ERROR: Cannot open '%s' for writing.\n", hg_fn.c_str());
                     return 1;
                 }
-                fprintf(hg, "Segment\tIBD0_Score\tIBD1_Score\tIBD2_Score\tInferred_State\n");
+                fprintf(hg, o.posterior ? "Segment\tIBD0_Score\tIBD1_Score\tIBD2_Score\tInferred_State\tP_IBD0\tP_IBD1\tP_IBD2\n"
+                                        : "Segment\tIBD0_Score\tIBD1_Score\tIBD2_Score\tInferred_State\n");
                 const int64_t a = hg_off[k], b = hg_off[k + 1];
                 char s0[48], s1[48], s2[48];
                 for (int64_t i = a; i < b; i++) {
                     put_score_log(s0, hg_score[(size_t)i * 3]);
                     put_score_log(s1, hg_score[(size_t)i * 3 + 1]);
                     put_score_log(s2, hg_score[(size_t)i * 3 + 2]);
-                    fprintf(hg, "%d\t%s\t%s\t%s\t%d\n", (int)(i - a + 1), s0, s1, s2, (int)hg_state[(size_t)i]);
+                    if (o.posterior)
+                        fprintf(hg, "%d\t%s\t%s\t%s\t%d\t%.6f\t%.6f\t%.6f\n", (int)(i - a + 1), s0, s1, s2, (int)hg_state[(size_t)i],
+                                hg_post[(size_t)i * 3], hg_post[(size_t)i * 3 + 1], hg_post[(size_t)i * 3 + 2]);
+                    else
+                        fprintf(hg, "%d\t%s\t%s\t%s\t%d\n", (int)(i - a + 1), s0, s1, s2, (int)hg_state[(size_t)i]);
                 }
                 const double n = (double)(b - a);
                 for (int c = 0; c < 3; c++)
                     fprintf(hg, "#%% IBD%d (n = %.0f): %.2f\n", c, (double)hg_counts[k * 3 + (size_t)c], ((double)hg_counts[k * 3 + (size_t)c] / n) * 100);
+                if (o.posterior)
+                    for (int c = 0; c < 3; c++)
+                        fprintf(hg, "#%% posterior IBD%d (n = %.2f): %.2f\n", c, hg_expected[k * 3 + (size_t)c], (hg_expected[k * 3 + (size_t)c] / n) * 100);
                 fclose(hg);
             }
             return 0;
@@ -489,7 +510,7 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
 int main(int argc, char *argv[]) {
     const clock_t start = clock();
     Options o;
-    static int ld_flag = 0, no_tab_flag = 0, hg_flag = 0;
+    static int ld_flag = 0, no_tab_flag = 0, hg_flag = 0, post_flag = 0;
     static struct option longopts[] = {{"LD", no_argument, &ld_flag, 1},
                                        {"vcf", required_argument, 0, 'V'},
                                        {"hap", required_argument, 0, 'H'},
@@ -518,6 +539,7 @@ int main(int argc, char *argv[]) {
                                        {"panel-cache", required_argument, 0, 1003},  // additive
                                        {"no-tab", no_argument, &no_tab_flag, 1},  // additive
                                        {"hiddengem", no_argument, &hg_flag, 1},   // additive: chain the Viterbi pass
+                                       {"posterior", no_argument, &post_flag, 1},  // additive: posteriors in the hiddengem files
                                        {"p01", required_argument, 0, 1004},
                                        {"p02", required_argument, 0, 1005},
                                        {"p12", required_argument, 0, 1006},
@@ -572,6 +594,7 @@ int main(int argc, char *argv[]) {
     o.ld = ld_flag;
     o.no_tab = no_tab_flag;
     o.hiddengem = hg_flag;
+    o.posterior = post_flag;
     for (int i = optind; i < argc; i++) fprintf(stderr, "Given extra argument %s.\n", argv[i]);
     // validation: the reference exits with status 0 on invalid values (src/ibdgem.c:966-989)
     if (o.opt_d && o.target_dp <= 0) {
@@ -596,6 +619,10 @@ int main(int argc, char *argv[]) {
     }
     if (o.window < 2) {
         fprintf(stderr, "[::] ERROR: Invalid window size (-w) of %d (must be >= 2).\n", o.window);
+        exit(0);
+    }
+    if (o.posterior && !o.hiddengem) {
+        fprintf(stderr, "[::] ERROR: --posterior needs --hiddengem (the posteriors are written to the hiddengem files).\n");
         exit(0);
     }
     if (o.max_cov > IBDGEM_MAX_COV_LIMIT) o.max_cov = IBDGEM_MAX_COV_LIMIT;  // pileup lines with cov >= 128 never load

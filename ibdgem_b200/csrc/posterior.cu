@@ -1,0 +1,455 @@
+// posterior.cu — batched hiddengem posterior: per-bin IBD-state probabilities by forward-backward over the same path
+// weights the Viterbi pass (hidden.cu) maximises,
+//   W(x) = prod_i nrm[i][x_i] * prod_{i>0} pen(x_{i-1}, x_i),   gamma[i][s] = sum_{x : x_i = s} W(x) / sum_x W(x),
+// with pen = 1 on the diagonal and p01 / p02 / p12 off it (symmetric), and no prior on bin 0.  The penalties are the
+// reference's weights, not transition probabilities; the posterior is the marginal of those weights, so the Viterbi
+// path is its mode.
+//
+// Scaled forward-backward in fp64 linear space.  Only the direction of a row of alpha or beta matters, so every row is
+// rescaled by the power of two that brings its sum into [1, 2): an exact multiplication, no division on the solver's
+// critical path, and no under- or overflow however long the table (every emission row has max >= 1/3 of its sum).
+//
+// Two kernels, each the structure of viterbi_fused_kernel: a block takes 32 tables, worker warps stage 16-bin chunks
+// with coalesced loads and compute the emissions in shared memory, ONE solver warp (lane = table) walks the chunk,
+// chunks are double buffered.
+//   forward   walks the chunks in order and stores only alpha of each chunk's last bin (a checkpoint, 24 B per table
+//             per 16 bins);
+//   backward  walks the chunks in reverse; per chunk the solver recomputes alpha from the previous chunk's checkpoint
+//             (the same operations, hence the same doubles), then walks beta down the chunk; the workers form
+//             gamma = alpha * beta / sum, write it and accumulate the expected occupancy.
+// Bytes per bin: 24 read by each pass, 24 written once, plus the checkpoints (3 B): ~75 B, against ~120 B for a
+// design that stores alpha of every bin and reads it back.
+//
+// Emissions (nrm; any positive per-bin factor cancels in gamma, so only the direction is needed):
+//   is_log = 0  l_s / ((l0 + l1) + l2) as hiddengem normalises summary-file likelihoods, with the division replaced
+//               by the exact power-of-two scaling that brings the total into [1, 2);
+//   is_log = 1  exp(L_s - max_k L_k).
+// A bin whose normalised row is undefined (text: a total that is not a positive finite number, e.g. all three 0 or a
+// NaN; log: a NaN score, or a row maximum that is not finite) carries no information and gets the uniform emission (1, 1, 1).  A table whose total weight is
+// 0 (possible only with zero penalties) has NaN posteriors and NaN expected counts.
+#include <math.h>
+#include <stdlib.h>
+
+#include <algorithm>
+#include <cmath>
+#include <vector>
+
+#include "engine.h"
+#include "tc_common.cuh"
+
+namespace ibdgem {
+
+constexpr int PB_TABLES = 32, PB_BINS = 16, PB_ROW = PB_BINS * 3 + 1;  // padded row: lanes hit distinct banks
+constexpr int PB_WORKERS = 256, PB_THREADS = PB_WORKERS + 32;
+constexpr int PB_NLD = PB_TABLES * PB_BINS * 3 / PB_WORKERS;  // doubles of a chunk each worker loads
+constexpr int PB_NBIN = PB_TABLES * PB_BINS / PB_WORKERS;     // bins of a chunk each worker normalises
+constexpr int PB_FWD_SMEM = 2 * PB_TABLES * PB_ROW * 8 + 2 * PB_TABLES * 8;
+constexpr int PB_BWD_SMEM = 4 * PB_TABLES * PB_ROW * 8 + 2 * PB_TABLES * 8 + PB_TABLES * 4;
+static_assert(PB_TABLES * PB_BINS * 3 <= PB_TABLES * PB_ROW, "expected-count partials fit in one staging buffer");
+
+// 2^-floor(log2 s) for s >= 0: multiplying by it is exact and brings s into [1, 2) (0 stays 0)
+__device__ __forceinline__ double pow2_recip(double s) {
+    const int ex = min(max((__double2hiint(s) >> 20) & 0x7ff, 1), 2045);
+    return __hiloint2double((2046 - ex) << 20, 0);
+}
+
+// 1 / s for a positive normal s: hardware estimate and two Newton steps on s scaled into [1, 2) (no slow-path call)
+__device__ __forceinline__ double recip(double s) {
+    const double k = pow2_recip(s), m = s * k;
+    double y;
+    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(m));
+    y = fma(y, fma(-m, y, 1.0), y);
+    y = fma(y, fma(-m, y, 1.0), y);
+    return y * k;
+}
+
+// emission row of one bin, in place
+__device__ __forceinline__ void emission(double *L, int is_log) {
+    double e0, e1, e2;
+    bool bad;
+    if (is_log) {
+        const double m = fmax(L[0], fmax(L[1], L[2]));
+        bad = isnan(L[0]) || isnan(L[1]) || isnan(L[2]) || !isfinite(m);
+        e0 = exp_nonpos(L[0] - m);
+        e1 = exp_nonpos(L[1] - m);
+        e2 = exp_nonpos(L[2] - m);
+    } else {  // l_s / tot up to a power of two (exact, and no division)
+        const double tot = __dadd_rn(__dadd_rn(L[0], L[1]), L[2]);
+        bad = !(tot > 0) || !isfinite(tot);
+        const double sc = pow2_recip(tot);
+        e0 = L[0] * sc;
+        e1 = L[1] * sc;
+        e2 = L[2] * sc;
+    }
+    L[0] = bad ? 1.0 : e0;
+    L[1] = bad ? 1.0 : e1;
+    L[2] = bad ? 1.0 : e2;
+}
+
+// one forward step: alpha[i] from alpha[i - 1] (or nothing, on bin 0) and the emission of bin i
+__device__ __forceinline__ void fwd_step(double &a0, double &a1, double &a2, double e0, double e1, double e2, bool first, bool live,
+                                         double p01, double p02, double p12) {
+    const double t0 = first ? 1.0 : fma(a2, p02, fma(a1, p01, a0));
+    const double t1 = first ? 1.0 : fma(a2, p12, fma(a0, p01, a1));
+    const double t2 = first ? 1.0 : fma(a1, p12, fma(a0, p02, a2));
+    const double u0 = e0 * t0, u1 = e1 * t1, u2 = e2 * t2;
+    const double sc = pow2_recip(u0 + u1 + u2);
+    a0 = live ? u0 * sc : a0;
+    a1 = live ? u1 * sc : a1;
+    a2 = live ? u2 * sc : a2;
+}
+
+// Workers: raw likelihoods of chunk c of the block's tables into registers (coalesced: a table's chunk is 384
+// contiguous bytes), rows past a table's end read as 0.
+struct ChunkLoader {
+    const double *lik;
+    const int64_t *s_start, *s_len;
+    int w;
+    __device__ __forceinline__ void fetch(int c, double (&pre)[PB_NLD]) const {
+        const int64_t i0 = (int64_t)c * PB_BINS;
+#pragma unroll
+        for (int k = 0; k < PB_NLD; k++) {
+            const int idx = k * PB_WORKERS + w;
+            const int t = idx / (PB_BINS * 3), d = idx % (PB_BINS * 3);
+            pre[k] = (i0 + d / 3 < s_len[t]) ? __ldcs(lik + (s_start[t] + i0) * 3 + d) : 0.0;
+        }
+    }
+    __device__ __forceinline__ void store(const double (&pre)[PB_NLD], double (*buf)[PB_ROW]) const {
+#pragma unroll
+        for (int k = 0; k < PB_NLD; k++) {
+            const int idx = k * PB_WORKERS + w;
+            buf[idx / (PB_BINS * 3)][idx % (PB_BINS * 3)] = pre[k];
+        }
+    }
+    // emissions of chunk c in place, once every worker has stored its part (workers' barrier)
+    __device__ __forceinline__ void emit(int c, double (*buf)[PB_ROW], int is_log) const {
+        asm volatile("bar.sync 5, %0;" ::"n"(PB_WORKERS) : "memory");
+        const int64_t i0 = (int64_t)c * PB_BINS;
+#pragma unroll 1  // unrolled, the two bins need more registers than three blocks per SM leave
+        for (int k = 0; k < PB_NBIN; k++) {
+            const int idx = k * PB_WORKERS + w;
+            const int t = idx / PB_BINS, i = idx % PB_BINS;
+            if (i0 + i < s_len[t]) emission(&buf[t][i * 3], is_log);
+        }
+        __threadfence_block();
+    }
+};
+
+// Named barriers: 1 + b = chunk in buffer b has its emissions (workers arrive, solver syncs);
+//                 3 + b = chunk in buffer b is solved (solver arrives, workers sync); 5 = workers only.
+__device__ __forceinline__ void arrive_ready(int b) {
+    if (b == 0) asm volatile("bar.arrive 1, %0;" ::"n"(PB_THREADS) : "memory");
+    else asm volatile("bar.arrive 2, %0;" ::"n"(PB_THREADS) : "memory");
+}
+__device__ __forceinline__ void sync_ready(int b) {
+    if (b == 0) asm volatile("bar.sync 1, %0;" ::"n"(PB_THREADS) : "memory");
+    else asm volatile("bar.sync 2, %0;" ::"n"(PB_THREADS) : "memory");
+}
+__device__ __forceinline__ void arrive_solved(int b) {
+    if (b == 0) asm volatile("bar.arrive 3, %0;" ::"n"(PB_THREADS) : "memory");
+    else asm volatile("bar.arrive 4, %0;" ::"n"(PB_THREADS) : "memory");
+}
+__device__ __forceinline__ void sync_solved(int b) {
+    if (b == 0) asm volatile("bar.sync 3, %0;" ::"n"(PB_THREADS) : "memory");
+    else asm volatile("bar.sync 4, %0;" ::"n"(PB_THREADS) : "memory");
+}
+
+// Forward pass: alpha of each chunk's last bin -> ckpt[chunk][n_tables][3]; the final alpha's sum -> expected[t][0]
+// (0 exactly when the table's total weight is 0: scaled rows never return from 0).
+__global__ void __launch_bounds__(PB_THREADS, 3)
+posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
+                     int is_log, double p01, double p02, double p12, double *__restrict__ ckpt, double *__restrict__ expected) {
+    extern __shared__ double pb_smem[];
+    double (*em)[PB_TABLES][PB_ROW] = reinterpret_cast<double (*)[PB_TABLES][PB_ROW]>(pb_smem);
+    int64_t *s_start = reinterpret_cast<int64_t *>(pb_smem + 2 * PB_TABLES * PB_ROW), *s_len = s_start + PB_TABLES;
+    const int tb0 = blockIdx.x * PB_TABLES;
+    if (threadIdx.x < PB_TABLES) {
+        const int tb = tb0 + threadIdx.x;
+        s_start[threadIdx.x] = tb < n_tables ? start[tb] : 0;
+        s_len[threadIdx.x] = tb < n_tables ? len[tb] : 0;
+    }
+    __syncthreads();
+    int64_t blk_bins = 0;
+    for (int k = 0; k < PB_TABLES; k++) blk_bins = max(blk_bins, s_len[k]);
+    const int nchunk = (int)((blk_bins + PB_BINS - 1) / PB_BINS);
+    if (threadIdx.x >= 32) {
+        const ChunkLoader ld{lik, s_start, s_len, (int)threadIdx.x - 32};
+        double pre[PB_NLD];
+        if (nchunk > 0) ld.fetch(0, pre);
+        for (int c = 0; c <= nchunk; c++) {
+            if (c < nchunk) {
+                const int b = c & 1;
+                if (c >= 2) sync_solved(b);  // the solver is done with chunk c - 2 in this buffer
+                ld.store(pre, em[b]);
+                if (c + 1 < nchunk) ld.fetch(c + 1, pre);  // in flight under this chunk's work
+                ld.emit(c, em[b], is_log);
+                arrive_ready(b);
+            } else {
+                for (int k = max(0, nchunk - 2); k < nchunk; k++) sync_solved(k & 1);  // every arrival is consumed
+            }
+        }
+    } else {
+        const int lane = threadIdx.x;
+        const int64_t n = s_len[lane];
+        const int tb = tb0 + lane;
+        double a0 = 1, a1 = 1, a2 = 1;
+        for (int c = 0; c < nchunk; c++) {
+            const int b = c & 1;
+            sync_ready(b);
+            const int64_t i0 = (int64_t)c * PB_BINS;
+            const double *nr = &em[b][lane][0];
+#pragma unroll 4
+            for (int q = 0; q < PB_BINS; q++)
+                fwd_step(a0, a1, a2, nr[q * 3], nr[q * 3 + 1], nr[q * 3 + 2], i0 + q == 0, i0 + q < n, p01, p02, p12);
+            if (tb < n_tables) {
+                double *o = ckpt + ((size_t)c * n_tables + tb) * 3;
+                o[0] = a0; o[1] = a1; o[2] = a2;
+            }
+            __threadfence_block();
+            arrive_solved(b);
+        }
+        if (tb < n_tables) expected[(size_t)tb * 3] = a0 + a1 + a2;
+    }
+}
+
+// Backward pass: gamma -> posterior (the caller's layout), expected occupancy -> expected[t][3].
+__global__ void __launch_bounds__(PB_THREADS, 3)
+posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
+                     int is_log, double p01, double p02, double p12, const double *__restrict__ ckpt, double *__restrict__ posterior,
+                     double *__restrict__ expected) {
+    extern __shared__ double pb_smem[];
+    double (*em)[PB_TABLES][PB_ROW] = reinterpret_cast<double (*)[PB_TABLES][PB_ROW]>(pb_smem);  // emissions, then beta
+    double (*al)[PB_TABLES][PB_ROW] = reinterpret_cast<double (*)[PB_TABLES][PB_ROW]>(pb_smem + 2 * PB_TABLES * PB_ROW);
+    int64_t *s_start = reinterpret_cast<int64_t *>(pb_smem + 4 * PB_TABLES * PB_ROW), *s_len = s_start + PB_TABLES;
+    int *s_dead = reinterpret_cast<int *>(s_len + PB_TABLES);
+    const int tb0 = blockIdx.x * PB_TABLES;
+    if (threadIdx.x < PB_TABLES) {
+        const int tb = tb0 + threadIdx.x;
+        const int64_t n = tb < n_tables ? len[tb] : 0;
+        s_start[threadIdx.x] = tb < n_tables ? start[tb] : 0;
+        s_len[threadIdx.x] = n;
+        s_dead[threadIdx.x] = n > 0 && !(expected[(size_t)tb * 3] > 0);  // total weight 0
+    }
+    __syncthreads();
+    int64_t blk_bins = 0;
+    for (int k = 0; k < PB_TABLES; k++) blk_bins = max(blk_bins, s_len[k]);
+    const int nchunk = (int)((blk_bins + PB_BINS - 1) / PB_BINS);
+    const int w = (int)threadIdx.x - 32;
+    double E[PB_NBIN][3] = {};  // a worker's share of the expected counts: the same (table, bin slot) every chunk
+    if (threadIdx.x >= 32) {
+        const ChunkLoader ld{lik, s_start, s_len, w};
+        double pre[PB_NLD];
+        if (nchunk > 0) ld.fetch(nchunk - 1, pre);
+        for (int r = 0; r <= nchunk; r++) {  // r-th chunk from the end
+            if (r < nchunk) {
+                const int c = nchunk - 1 - r, b = r & 1;
+                ld.store(pre, em[b]);
+                if (c >= 1) ld.fetch(c - 1, pre);  // in flight under this chunk's work
+                ld.emit(c, em[b], is_log);
+                arrive_ready(b);
+            }
+            if (r >= 1) {  // gamma of the chunk the solver has just finished
+                const int c = nchunk - r, pb = (r - 1) & 1;
+                sync_solved(pb);
+                const int64_t i0 = (int64_t)c * PB_BINS;
+#pragma unroll
+                for (int k = 0; k < PB_NBIN; k++) {
+                    const int idx = k * PB_WORKERS + w;
+                    const int t = idx / PB_BINS, i = idx % PB_BINS;
+                    if (i0 + i < s_len[t]) {
+                        const double *A = &al[pb][t][i * 3], *B = &em[pb][t][i * 3];
+                        const double g0 = A[0] * B[0], g1 = A[1] * B[1], g2 = A[2] * B[2];
+                        const double inv = s_dead[t] ? __longlong_as_double(0x7ff8000000000000LL) : recip(g0 + g1 + g2);
+                        const double y0 = g0 * inv, y1 = g1 * inv, y2 = g2 * inv;
+                        double *o = posterior + (s_start[t] + i0 + i) * 3;
+                        __stcs(o, y0);
+                        __stcs(o + 1, y1);
+                        __stcs(o + 2, y2);
+                        E[k][0] += y0;
+                        E[k][1] += y1;
+                        E[k][2] += y2;
+                    }
+                }
+                asm volatile("bar.sync 5, %0;" ::"n"(PB_WORKERS) : "memory");  // buffer pb is free for the next chunk
+            }
+        }
+    } else {
+        const int lane = threadIdx.x;
+        const int64_t n = s_len[lane];
+        const int tb = tb0 + lane;
+        double b0 = 1, b1 = 1, b2 = 1;
+        for (int r = 0; r < nchunk; r++) {
+            const int c = nchunk - 1 - r, b = r & 1;
+            double a0 = 1, a1 = 1, a2 = 1;  // alpha entering the chunk: the previous chunk's checkpoint
+            if (c >= 1 && tb < n_tables) {
+                const double *ck = ckpt + ((size_t)(c - 1) * n_tables + tb) * 3;
+                a0 = ck[0]; a1 = ck[1]; a2 = ck[2];
+            }
+            sync_ready(b);
+            const int64_t i0 = (int64_t)c * PB_BINS;
+            double *nr = &em[b][lane][0], *ao = &al[b][lane][0];
+#pragma unroll 4
+            for (int q = 0; q < PB_BINS; q++) {
+                fwd_step(a0, a1, a2, nr[q * 3], nr[q * 3 + 1], nr[q * 3 + 2], i0 + q == 0, i0 + q < n, p01, p02, p12);
+                ao[q * 3] = a0; ao[q * 3 + 1] = a1; ao[q * 3 + 2] = a2;
+            }
+            // beta down the chunk: the slot of bin i trades its emission for beta[i], then beta[i - 1] =
+            // sum_k pen(s, k) nrm[i][k] beta[i][k], rescaled
+#pragma unroll 4
+            for (int q = PB_BINS - 1; q >= 0; q--) {
+                const double e0 = nr[q * 3], e1 = nr[q * 3 + 1], e2 = nr[q * 3 + 2];
+                nr[q * 3] = b0; nr[q * 3 + 1] = b1; nr[q * 3 + 2] = b2;
+                const double v0 = e0 * b0, v1 = e1 * b1, v2 = e2 * b2;
+                const double t0 = fma(v2, p02, fma(v1, p01, v0));
+                const double t1 = fma(v2, p12, fma(v0, p01, v1));
+                const double t2 = fma(v1, p12, fma(v0, p02, v2));
+                const double sc = pow2_recip(t0 + t1 + t2);
+                const bool live = i0 + q < n;
+                b0 = live ? t0 * sc : b0;
+                b1 = live ? t1 * sc : b1;
+                b2 = live ? t2 * sc : b2;
+            }
+            __threadfence_block();
+            arrive_solved(b);
+        }
+    }
+    __syncthreads();
+    // expected[t] = the 16 bin slots' partial sums of table t, added in a fixed order (reproducible)
+    double *part = &em[0][0][0];  // [PB_TABLES][PB_BINS][3]
+    if (threadIdx.x >= 32) {
+#pragma unroll
+        for (int k = 0; k < PB_NBIN; k++) {
+            const int idx = k * PB_WORKERS + w;
+            const int t = idx / PB_BINS, i = idx % PB_BINS;
+#pragma unroll
+            for (int s = 0; s < 3; s++) part[(t * PB_BINS + i) * 3 + s] = E[k][s];
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < PB_TABLES) {
+        const int tb = tb0 + threadIdx.x;
+        if (tb < n_tables) {
+            double x[3] = {0, 0, 0};
+            for (int i = 0; i < PB_BINS; i++)
+                for (int s = 0; s < 3; s++) x[s] += part[(threadIdx.x * PB_BINS + i) * 3 + s];
+            const double nan = __longlong_as_double(0x7ff8000000000000LL);
+            for (int s = 0; s < 3; s++) expected[(size_t)tb * 3 + s] = s_dead[threadIdx.x] ? nan : x[s];
+        }
+    }
+}
+
+}  // namespace ibdgem
+
+using namespace ibdgem;
+
+namespace {
+
+bool bad_penalties(const char *fn, double p01, double p02, double p12) {
+    const bool ok = std::isfinite(p01) && std::isfinite(p02) && std::isfinite(p12) && p01 >= 0 && p02 >= 0 && p12 >= 0;
+    if (!ok) set_error("[::] ERROR in %s(): penalties must be finite and >= 0 (p01 = %g, p02 = %g, p12 = %g).", fn, p01, p02, p12);
+    return !ok;
+}
+
+// One batch of tables, everything in device memory (start / len per table); kernels only, no host synchronisation.
+int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
+                        int is_log, double p01, double p02, double p12, double *d_post, double *d_expected) {
+    const int64_t nck = (maxbins + PB_BINS - 1) / PB_BINS;
+    if (nck == 0) {  // only empty tables: no bins, expected occupancy 0
+        IBD_CUDA(cudaMemsetAsync(d_expected, 0, (size_t)n_tables * 24, e->stream));
+        return 0;
+    }
+    double *d_ckpt;
+    if (scratch(e, SC_HG_CKPT, (size_t)nck * n_tables * 24, (void **)&d_ckpt)) return 1;
+    const unsigned grid = (unsigned)((n_tables + PB_TABLES - 1) / PB_TABLES);
+    {
+        LaunchScope ls(e, K_POSTERIOR_FWD);
+        posterior_fwd_kernel<<<grid, PB_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt,
+                                                                           d_expected);
+    }
+    {
+        LaunchScope ls(e, K_POSTERIOR_BWD);
+        IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
+        posterior_bwd_kernel<<<grid, PB_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt,
+                                                                           d_post, d_expected);
+    }
+    IBD_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// host start / length of every table; 1 (error set) on a negative length or one past the stride
+int table_layout(const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, std::vector<int64_t> *sl, int64_t *maxbins,
+                 int64_t *total) {
+    sl->assign((size_t)n_tables * 2, 0);
+    *maxbins = *total = 0;
+    for (int t = 0; t < n_tables; t++) {
+        const int64_t n = bin_offsets[t + 1] - bin_offsets[t];
+        if (n < 0 || (table_stride > 0 && n > table_stride)) {
+            set_error("[::] ERROR in %s(): table %d has %lld bins (stride %lld).", fn, t, (long long)n, (long long)table_stride);
+            return 1;
+        }
+        (*sl)[(size_t)t] = table_stride > 0 ? (int64_t)t * table_stride : bin_offsets[t];
+        (*sl)[(size_t)n_tables + t] = n;
+        *maxbins = std::max(*maxbins, n);
+        *total += n;
+    }
+    return 0;
+}
+
+}  // namespace
+
+// Host buffers in, host buffers out: the likelihoods go up, both passes run, posteriors and expected counts come down.
+extern "C" int hiddengem_posterior_batch(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, const double *lik, int32_t is_log,
+                                         double p01, double p02, double p12, double *posterior, double *expected) {
+    if (!e || n_tables <= 0 || !bin_offsets || !expected) {
+        set_error("[::] ERROR in hiddengem_posterior_batch(): bad arguments.");
+        return 1;
+    }
+    if (bad_penalties("hiddengem_posterior_batch", p01, p02, p12)) return 1;
+    std::vector<int64_t> h_sl;
+    int64_t maxbins, total;
+    if (table_layout("hiddengem_posterior_batch", n_tables, bin_offsets, 0, &h_sl, &maxbins, &total)) return 1;
+    const int64_t nb = total > 0 ? bin_offsets[n_tables] : 0;  // bins of lik / posterior
+    if (nb > 0 && (!lik || !posterior)) {
+        set_error("[::] ERROR in hiddengem_posterior_batch(): bad arguments.");
+        return 1;
+    }
+    IBD_CUDA(cudaSetDevice(e->device));
+    double *d_lik = nullptr, *d_post = nullptr, *d_expected;
+    int64_t *d_start;
+    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start) || scratch(e, SC_HG_COUNTS, (size_t)n_tables * 24, (void **)&d_expected))
+        return 1;
+    if (nb > 0 && (scratch(e, SC_HG_LIK, (size_t)nb * 24, (void **)&d_lik) || scratch(e, SC_HG_SCORE, (size_t)nb * 24, (void **)&d_post)))
+        return 1;
+    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
+    if (nb > 0) IBD_CUDA(cudaMemcpyAsync(d_lik, lik, (size_t)nb * 24, cudaMemcpyHostToDevice, e->stream));
+    if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_post, d_expected)) return 1;
+    if (nb > 0) IBD_CUDA(cudaMemcpyAsync(posterior, d_post, (size_t)nb * 24, cudaMemcpyDeviceToHost, e->stream));
+    IBD_CUDA(cudaMemcpyAsync(expected, d_expected, (size_t)n_tables * 24, cudaMemcpyDeviceToHost, e->stream));
+    IBD_CUDA(cudaStreamSynchronize(e->stream));
+    settle_timers(e);
+    return 0;
+}
+
+// Device buffers in, device buffers out; bin_offsets is a HOST array.  table_stride > 0: table t starts at bin
+// t * table_stride (ibdgem_scores.w_loglik_device with table_stride = max_windows), and its posteriors are written at
+// the same positions.
+extern "C" int hiddengem_posterior_batch_device(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, int64_t table_stride,
+                                                const double *d_lik, int32_t is_log, double p01, double p02, double p12, double *d_posterior,
+                                                double *d_expected) {
+    if (!e || n_tables <= 0 || !bin_offsets || !d_lik || !d_posterior || !d_expected || table_stride < 0) {
+        set_error("[::] ERROR in hiddengem_posterior_batch_device(): bad arguments.");
+        return 1;
+    }
+    if (bad_penalties("hiddengem_posterior_batch_device", p01, p02, p12)) return 1;
+    std::vector<int64_t> h_sl;
+    int64_t maxbins, total;
+    if (table_layout("hiddengem_posterior_batch_device", n_tables, bin_offsets, table_stride, &h_sl, &maxbins, &total)) return 1;
+    IBD_CUDA(cudaSetDevice(e->device));
+    int64_t *d_start;
+    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start)) return 1;
+    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
+    if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_posterior, d_expected)) return 1;
+    IBD_CUDA(cudaStreamSynchronize(e->stream));  // h_sl is read by the copy above
+    settle_timers(e);
+    return 0;
+}

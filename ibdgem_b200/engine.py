@@ -252,6 +252,28 @@ class Engine:
             C.c_int32(1 if is_log else 0), C.c_double(p01), C.c_double(p02), C.c_double(p12), C.c_void_p(d_state_ptr),
             C.c_void_p(d_score_ptr), C.c_void_p(d_counts_ptr)))
 
+    def posterior_batch(self, lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-3):
+        """Per-bin posterior IBD-state probabilities over the path weights hiddengem maximises
+        (hiddengem_posterior_batch): (posterior [n_bins, 3], expected [n_tables, 3])."""
+        lik = np.ascontiguousarray(lik, np.float64)
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        nt = len(off) - 1
+        post = np.zeros((int(off[-1]), 3))
+        expected = np.zeros((nt, 3))
+        self._check(self._lib.hiddengem_posterior_batch(self._h, C.c_int32(nt), _ptr(off), _ptr(lik),
+                                                        C.c_int32(1 if is_log else 0), C.c_double(p01),
+                                                        C.c_double(p02), C.c_double(p12), _ptr(post), _ptr(expected)))
+        return post, expected
+
+    def posterior_batch_device(self, d_lik_ptr: int, bin_offsets: np.ndarray, is_log: bool, d_posterior_ptr: int,
+                               d_expected_ptr: int, table_stride: int = 0, p01=1e-3, p02=1e-6, p12=1e-3):
+        """Device buffers in, device buffers out (hiddengem_posterior_batch_device); bin_offsets stays on the host."""
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        self._check(self._lib.hiddengem_posterior_batch_device(
+            self._h, C.c_int32(len(off) - 1), _ptr(off), C.c_int64(table_stride), C.c_void_p(d_lik_ptr),
+            C.c_int32(1 if is_log else 0), C.c_double(p01), C.c_double(p02), C.c_double(p12),
+            C.c_void_p(d_posterior_ptr), C.c_void_p(d_expected_ptr)))
+
     def viterbi_last_flagged(self) -> int:
         """Tables of the last hiddengem call re-evaluated on the host in long double (near-tie guard)."""
         return int(self._lib.hiddengem_last_flagged(self._h))

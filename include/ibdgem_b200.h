@@ -239,6 +239,33 @@ int hiddengem_viterbi_batch_device(ibdgem_engine *e, int32_t n_tables, const int
  * on the host with the reference's own long double recurrence.  Returns how many tables of the last call were. */
 int64_t hiddengem_last_flagged(ibdgem_engine *e);
 
+/* Posterior IBD-state probabilities of every bin, by forward-backward over the SAME path weights the Viterbi entries
+ * maximise (src/hiddengem.c:108-147): for one table of n bins and a state path x,
+ *     W(x) = prod_{i<n} nrm[i][x_i] * prod_{0<i<n} pen(x_{i-1}, x_i),    posterior[i][s] = sum_{x: x_i = s} W(x) / sum_x W(x)
+ * with pen = 1 on the diagonal and p01 / p02 / p12 off it (symmetric), no prior on bin 0, and nrm the per-bin
+ * normalisation hiddengem applies: l_s / ((l0 + l1) + l2) for is_log = 0, exp(L_s - m) / sum_k exp(L_k - m) with m the
+ * row maximum for is_log = 1.  The penalties are weights, not transition probabilities: this is the marginal of the
+ * weights hiddengem already uses, and the Viterbi path is its mode.
+ *   - A bin whose normalised row is undefined (all three likelihoods 0 or a NaN total; a NaN score, or a row maximum
+ *     that is not finite) gets the uniform emission (1, 1, 1): it carries no information.  (The Viterbi entries
+ *     propagate such a bin as the reference does.)
+ *   - Penalties may be any finite value >= 0, above 1 included; anything else is an error.  A table whose total
+ *     weight is 0 (possible only with zero penalties) gets NaN posteriors and NaN expected counts.
+ *   - An empty table has no posterior rows and expected counts 0; one bin has posterior = nrm.
+ *   lik / bin_offsets   as for the Viterbi entry (host arrays)
+ *   posterior           [sum(n_bins)][3], rows sum to 1
+ *   expected            [n_tables][3] expected bins per state, sum over the table's bins of posterior */
+int hiddengem_posterior_batch(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, const double *lik,
+                              int32_t is_log, double p01, double p02, double p12,
+                              double *posterior, double *expected);
+/* The same on DEVICE buffers of the engine's GPU (bin_offsets stays a HOST array), with the layouts of the Viterbi
+ * device entry: table_stride = 0 for packed tables; table_stride > 0 for table t at bin t * table_stride, which with
+ * table_stride = max_windows and is_log = 1 consumes ibdgem_scores.w_loglik_device as is.  Posteriors are written at
+ * the positions of the inputs; nothing past a table's bins is written. */
+int hiddengem_posterior_batch_device(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, int64_t table_stride,
+                                     const double *d_lik, int32_t is_log, double p01, double p02, double p12,
+                                     double *d_posterior, double *d_expected);
+
 /* ---- instrumentation --------------------------------------------------------------------- */
 
 /* When enabled every kernel launch is bracketed by CUDA events on the engine stream. */
