@@ -30,7 +30,7 @@ static const char *const kKernelNameList[] = {
     "ld_stage",       "ld_expand_bg",  "ld_expand_tgt", "ld_windows",   "ld_ibd0",
     "ld_mma",         "viterbi",       "viterbi_norm",  "viterbi_back", "viterbi_out", "fill",
     "v_slots",        "v_wmap",        "v_tw",          "v_sort",       "v_expand_a",  "v_expand_b",   "ld_vmma",
-    "window_linear",  "posterior_fwd", "posterior_bwd",
+    "window_linear",  "posterior_fwd", "posterior_bwd", "posterior_fwd_log", "posterior_bwd_log",
 };
 static_assert(sizeof(kKernelNameList) / sizeof(kKernelNameList[0]) == K_COUNT, "one name per KernelId, in enum order");
 const char *const *const kKernelNames = kKernelNameList;

@@ -59,6 +59,8 @@ enum KernelId {
     K_WINDOW_LINEAR,    // the reference's own running fp64 products per window (ibdgem_scores.w_lik_linear)
     K_POSTERIOR_FWD,    // hiddengem posterior: forward pass, alpha checkpoints per 16-bin chunk
     K_POSTERIOR_BWD,    // hiddengem posterior: backward pass, posteriors + expected occupancy
+    K_POSTERIOR_FWD_LOG,  // of the posterior_fwd / _bwd launches, those in natural-log arithmetic (zero or widely
+    K_POSTERIOR_BWD_LOG,  // spread penalties); counted only, their time is in posterior_fwd / _bwd
     K_COUNT
 };
 

@@ -7,7 +7,12 @@
 //
 // Scaled forward-backward in fp64 linear space.  Only the direction of a row of alpha or beta matters, so every row is
 // rescaled by the power of two that brings its sum into [1, 2): an exact multiplication, no division on the solver's
-// critical path, and no under- or overflow however long the table (every emission row has max >= 1/3 of its sum).
+// critical path, and the row's sum cannot under- or overflow however long the table.  The entries inside a row can:
+// a state more than 700 nats behind in one bin gets emission 0, and an entry below 2^-1074 of its row is flushed.
+// That is harmless while every penalty keeps all states within reach of each other (linear_penalties below); with a
+// zero penalty, or penalties spread wider than 2^400, the only paths between two states can run through such
+// entries.  Those calls run the same two kernels in natural-log arithmetic (LG = true: log-sum-exp mixing, rows
+// shifted to maximum 0), which has no range limit; they cost more fp64 work on the solver lane.
 //
 // Two kernels, each the structure of viterbi_fused_kernel: a block takes 32 tables, worker warps stage 16-bin chunks
 // with coalesced loads and compute the emissions in shared memory, ONE solver warp (lane = table) walks the chunk,
@@ -26,7 +31,8 @@
 //   is_log = 1  exp(L_s - max_k L_k).
 // A bin whose normalised row is undefined (text: a total that is not a positive finite number, e.g. all three 0 or a
 // NaN; log: a NaN score, or a row maximum that is not finite) carries no information and gets the uniform emission (1, 1, 1).  A table whose total weight is
-// 0 (possible only with zero penalties) has NaN posteriors and NaN expected counts.
+// 0 as a real number (possible only with zero penalties, so decided in log arithmetic, where it is exact) has NaN
+// posteriors and NaN expected counts.
 #include <math.h>
 #include <stdlib.h>
 
@@ -63,32 +69,75 @@ __device__ __forceinline__ double recip(double s) {
     return y * k;
 }
 
-// emission row of one bin, in place
+// log(exp(x) + exp(y) + exp(z)) for x, y, z < +inf; -inf when all three are -inf.  Terms more than 700 below the
+// largest are dropped (relative weight < 1e-304).
+__device__ __forceinline__ double lse3(double x, double y, double z) {
+    const double m = fmax(x, fmax(y, z)), ms = m > -INFINITY ? m : 0.0;
+    return ms + log(exp_nonpos(x - ms) + exp_nonpos(y - ms) + exp_nonpos(z - ms));
+}
+
+// shift a row of log weights so its maximum is 0 (a row of -inf stays -inf)
+__device__ __forceinline__ void shift_max0(double &u0, double &u1, double &u2) {
+    const double m = fmax(u0, fmax(u1, u2)), ms = m > -INFINITY ? m : 0.0;
+    u0 -= ms;
+    u1 -= ms;
+    u2 -= ms;
+}
+
+// Emission row of one bin, in place: linear (LG = false) or natural log (LG = true, no range limit).
+template <bool LG>
 __device__ __forceinline__ void emission(double *L, int is_log) {
     double e0, e1, e2;
     bool bad;
     if (is_log) {
         const double m = fmax(L[0], fmax(L[1], L[2]));
         bad = isnan(L[0]) || isnan(L[1]) || isnan(L[2]) || !isfinite(m);
-        e0 = exp_nonpos(L[0] - m);
-        e1 = exp_nonpos(L[1] - m);
-        e2 = exp_nonpos(L[2] - m);
-    } else {  // l_s / tot up to a power of two (exact, and no division)
+        if (LG) {
+            e0 = L[0] - m;
+            e1 = L[1] - m;
+            e2 = L[2] - m;
+        } else {
+            e0 = exp_nonpos(L[0] - m);
+            e1 = exp_nonpos(L[1] - m);
+            e2 = exp_nonpos(L[2] - m);
+        }
+    } else {  // l_s / tot up to a power of two (exact, and no division); in log space log l_s - log tot, which
+              // keeps a ratio l_s / tot below the double range
         const double tot = __dadd_rn(__dadd_rn(L[0], L[1]), L[2]);
         bad = !(tot > 0) || !isfinite(tot);
-        const double sc = pow2_recip(tot);
-        e0 = L[0] * sc;
-        e1 = L[1] * sc;
-        e2 = L[2] * sc;
+        if (LG) {
+            const double lt = log(tot);
+            e0 = log(L[0]) - lt;
+            e1 = log(L[1]) - lt;
+            e2 = log(L[2]) - lt;
+        } else {
+            const double sc = pow2_recip(tot);
+            e0 = L[0] * sc;
+            e1 = L[1] * sc;
+            e2 = L[2] * sc;
+        }
     }
-    L[0] = bad ? 1.0 : e0;
-    L[1] = bad ? 1.0 : e1;
-    L[2] = bad ? 1.0 : e2;
+    const double one = LG ? 0.0 : 1.0;
+    L[0] = bad ? one : e0;
+    L[1] = bad ? one : e1;
+    L[2] = bad ? one : e2;
 }
 
-// one forward step: alpha[i] from alpha[i - 1] (or nothing, on bin 0) and the emission of bin i
+// one forward step: alpha[i] from alpha[i - 1] (or nothing, on bin 0) and the emission of bin i; LG: every value a
+// natural log, p01 / p02 / p12 the logs of the penalties
+template <bool LG>
 __device__ __forceinline__ void fwd_step(double &a0, double &a1, double &a2, double e0, double e1, double e2, bool first, bool live,
                                          double p01, double p02, double p12) {
+    if (LG) {
+        double u0 = e0 + (first ? 0.0 : lse3(a0, a1 + p01, a2 + p02));
+        double u1 = e1 + (first ? 0.0 : lse3(a0 + p01, a1, a2 + p12));
+        double u2 = e2 + (first ? 0.0 : lse3(a0 + p02, a1 + p12, a2));
+        shift_max0(u0, u1, u2);
+        a0 = live ? u0 : a0;
+        a1 = live ? u1 : a1;
+        a2 = live ? u2 : a2;
+        return;
+    }
     const double t0 = first ? 1.0 : fma(a2, p02, fma(a1, p01, a0));
     const double t1 = first ? 1.0 : fma(a2, p12, fma(a0, p01, a1));
     const double t2 = first ? 1.0 : fma(a1, p12, fma(a0, p02, a2));
@@ -97,6 +146,54 @@ __device__ __forceinline__ void fwd_step(double &a0, double &a1, double &a2, dou
     a0 = live ? u0 * sc : a0;
     a1 = live ? u1 * sc : a1;
     a2 = live ? u2 * sc : a2;
+}
+
+// one backward step: beta[i - 1] = sum_k pen(s, k) nrm[i][k] beta[i][k], rescaled (LG: in logs)
+template <bool LG>
+__device__ __forceinline__ void bwd_step(double &b0, double &b1, double &b2, double e0, double e1, double e2, bool live, double p01,
+                                         double p02, double p12) {
+    if (LG) {
+        const double v0 = e0 + b0, v1 = e1 + b1, v2 = e2 + b2;
+        double t0 = lse3(v0, v1 + p01, v2 + p02);
+        double t1 = lse3(v0 + p01, v1, v2 + p12);
+        double t2 = lse3(v0 + p02, v1 + p12, v2);
+        shift_max0(t0, t1, t2);
+        b0 = live ? t0 : b0;
+        b1 = live ? t1 : b1;
+        b2 = live ? t2 : b2;
+        return;
+    }
+    const double v0 = e0 * b0, v1 = e1 * b1, v2 = e2 * b2;
+    const double t0 = fma(v2, p02, fma(v1, p01, v0));
+    const double t1 = fma(v2, p12, fma(v0, p01, v1));
+    const double t2 = fma(v1, p12, fma(v0, p02, v2));
+    const double sc = pow2_recip(t0 + t1 + t2);
+    b0 = live ? t0 * sc : b0;
+    b1 = live ? t1 * sc : b1;
+    b2 = live ? t2 * sc : b2;
+}
+
+// gamma of one bin from alpha and beta (NaN for a table of total weight 0)
+template <bool LG>
+__device__ __forceinline__ void gamma(const double *A, const double *B, bool dead, double &y0, double &y1, double &y2) {
+    double g0, g1, g2;
+    if (LG) {  // a live table has a finite maximum in every bin
+        g0 = A[0] + B[0];
+        g1 = A[1] + B[1];
+        g2 = A[2] + B[2];
+        shift_max0(g0, g1, g2);
+        g0 = exp_nonpos(g0);
+        g1 = exp_nonpos(g1);
+        g2 = exp_nonpos(g2);
+    } else {
+        g0 = A[0] * B[0];
+        g1 = A[1] * B[1];
+        g2 = A[2] * B[2];
+    }
+    const double inv = dead ? __longlong_as_double(0x7ff8000000000000LL) : recip(g0 + g1 + g2);
+    y0 = g0 * inv;
+    y1 = g1 * inv;
+    y2 = g2 * inv;
 }
 
 // Workers: raw likelihoods of chunk c of the block's tables into registers (coalesced: a table's chunk is 384
@@ -122,6 +219,7 @@ struct ChunkLoader {
         }
     }
     // emissions of chunk c in place, once every worker has stored its part (workers' barrier)
+    template <bool LG>
     __device__ __forceinline__ void emit(int c, double (*buf)[PB_ROW], int is_log) const {
         asm volatile("bar.sync 5, %0;" ::"n"(PB_WORKERS) : "memory");
         const int64_t i0 = (int64_t)c * PB_BINS;
@@ -129,7 +227,7 @@ struct ChunkLoader {
         for (int k = 0; k < PB_NBIN; k++) {
             const int idx = k * PB_WORKERS + w;
             const int t = idx / PB_BINS, i = idx % PB_BINS;
-            if (i0 + i < s_len[t]) emission(&buf[t][i * 3], is_log);
+            if (i0 + i < s_len[t]) emission<LG>(&buf[t][i * 3], is_log);
         }
         __threadfence_block();
     }
@@ -154,8 +252,9 @@ __device__ __forceinline__ void sync_solved(int b) {
     else asm volatile("bar.sync 4, %0;" ::"n"(PB_THREADS) : "memory");
 }
 
-// Forward pass: alpha of each chunk's last bin -> ckpt[chunk][n_tables][3]; the final alpha's sum -> expected[t][0]
-// (0 exactly when the table's total weight is 0: scaled rows never return from 0).
+// Forward pass: alpha of each chunk's last bin -> ckpt[chunk][n_tables][3]; 0 in expected[t][0] exactly when the
+// table's total weight is 0 (a positive value otherwise).
+template <bool LG>
 __global__ void __launch_bounds__(PB_THREADS, 3)
 posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
                      int is_log, double p01, double p02, double p12, double *__restrict__ ckpt, double *__restrict__ expected) {
@@ -182,7 +281,7 @@ posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                 if (c >= 2) sync_solved(b);  // the solver is done with chunk c - 2 in this buffer
                 ld.store(pre, em[b]);
                 if (c + 1 < nchunk) ld.fetch(c + 1, pre);  // in flight under this chunk's work
-                ld.emit(c, em[b], is_log);
+                ld.template emit<LG>(c, em[b], is_log);
                 arrive_ready(b);
             } else {
                 for (int k = max(0, nchunk - 2); k < nchunk; k++) sync_solved(k & 1);  // every arrival is consumed
@@ -192,7 +291,8 @@ posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
         const int lane = threadIdx.x;
         const int64_t n = s_len[lane];
         const int tb = tb0 + lane;
-        double a0 = 1, a1 = 1, a2 = 1;
+        const double one = LG ? 0.0 : 1.0;
+        double a0 = one, a1 = one, a2 = one;
         for (int c = 0; c < nchunk; c++) {
             const int b = c & 1;
             sync_ready(b);
@@ -200,7 +300,7 @@ posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
             const double *nr = &em[b][lane][0];
 #pragma unroll 4
             for (int q = 0; q < PB_BINS; q++)
-                fwd_step(a0, a1, a2, nr[q * 3], nr[q * 3 + 1], nr[q * 3 + 2], i0 + q == 0, i0 + q < n, p01, p02, p12);
+                fwd_step<LG>(a0, a1, a2, nr[q * 3], nr[q * 3 + 1], nr[q * 3 + 2], i0 + q == 0, i0 + q < n, p01, p02, p12);
             if (tb < n_tables) {
                 double *o = ckpt + ((size_t)c * n_tables + tb) * 3;
                 o[0] = a0; o[1] = a1; o[2] = a2;
@@ -208,11 +308,12 @@ posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
             __threadfence_block();
             arrive_solved(b);
         }
-        if (tb < n_tables) expected[(size_t)tb * 3] = a0 + a1 + a2;
+        if (tb < n_tables) expected[(size_t)tb * 3] = LG ? (fmax(a0, fmax(a1, a2)) > -INFINITY ? 1.0 : 0.0) : a0 + a1 + a2;
     }
 }
 
 // Backward pass: gamma -> posterior (the caller's layout), expected occupancy -> expected[t][3].
+template <bool LG>
 __global__ void __launch_bounds__(PB_THREADS, 3)
 posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
                      int is_log, double p01, double p02, double p12, const double *__restrict__ ckpt, double *__restrict__ posterior,
@@ -245,7 +346,7 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                 const int c = nchunk - 1 - r, b = r & 1;
                 ld.store(pre, em[b]);
                 if (c >= 1) ld.fetch(c - 1, pre);  // in flight under this chunk's work
-                ld.emit(c, em[b], is_log);
+                ld.template emit<LG>(c, em[b], is_log);
                 arrive_ready(b);
             }
             if (r >= 1) {  // gamma of the chunk the solver has just finished
@@ -257,10 +358,8 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                     const int idx = k * PB_WORKERS + w;
                     const int t = idx / PB_BINS, i = idx % PB_BINS;
                     if (i0 + i < s_len[t]) {
-                        const double *A = &al[pb][t][i * 3], *B = &em[pb][t][i * 3];
-                        const double g0 = A[0] * B[0], g1 = A[1] * B[1], g2 = A[2] * B[2];
-                        const double inv = s_dead[t] ? __longlong_as_double(0x7ff8000000000000LL) : recip(g0 + g1 + g2);
-                        const double y0 = g0 * inv, y1 = g1 * inv, y2 = g2 * inv;
+                        double y0, y1, y2;
+                        gamma<LG>(&al[pb][t][i * 3], &em[pb][t][i * 3], s_dead[t], y0, y1, y2);
                         double *o = posterior + (s_start[t] + i0 + i) * 3;
                         __stcs(o, y0);
                         __stcs(o + 1, y1);
@@ -277,10 +376,11 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
         const int lane = threadIdx.x;
         const int64_t n = s_len[lane];
         const int tb = tb0 + lane;
-        double b0 = 1, b1 = 1, b2 = 1;
+        const double one = LG ? 0.0 : 1.0;
+        double b0 = one, b1 = one, b2 = one;
         for (int r = 0; r < nchunk; r++) {
             const int c = nchunk - 1 - r, b = r & 1;
-            double a0 = 1, a1 = 1, a2 = 1;  // alpha entering the chunk: the previous chunk's checkpoint
+            double a0 = one, a1 = one, a2 = one;  // alpha entering the chunk: the previous chunk's checkpoint
             if (c >= 1 && tb < n_tables) {
                 const double *ck = ckpt + ((size_t)(c - 1) * n_tables + tb) * 3;
                 a0 = ck[0]; a1 = ck[1]; a2 = ck[2];
@@ -290,24 +390,15 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
             double *nr = &em[b][lane][0], *ao = &al[b][lane][0];
 #pragma unroll 4
             for (int q = 0; q < PB_BINS; q++) {
-                fwd_step(a0, a1, a2, nr[q * 3], nr[q * 3 + 1], nr[q * 3 + 2], i0 + q == 0, i0 + q < n, p01, p02, p12);
+                fwd_step<LG>(a0, a1, a2, nr[q * 3], nr[q * 3 + 1], nr[q * 3 + 2], i0 + q == 0, i0 + q < n, p01, p02, p12);
                 ao[q * 3] = a0; ao[q * 3 + 1] = a1; ao[q * 3 + 2] = a2;
             }
-            // beta down the chunk: the slot of bin i trades its emission for beta[i], then beta[i - 1] =
-            // sum_k pen(s, k) nrm[i][k] beta[i][k], rescaled
+            // beta down the chunk: the slot of bin i trades its emission for beta[i], then beta[i - 1]
 #pragma unroll 4
             for (int q = PB_BINS - 1; q >= 0; q--) {
                 const double e0 = nr[q * 3], e1 = nr[q * 3 + 1], e2 = nr[q * 3 + 2];
                 nr[q * 3] = b0; nr[q * 3 + 1] = b1; nr[q * 3 + 2] = b2;
-                const double v0 = e0 * b0, v1 = e1 * b1, v2 = e2 * b2;
-                const double t0 = fma(v2, p02, fma(v1, p01, v0));
-                const double t1 = fma(v2, p12, fma(v0, p01, v1));
-                const double t2 = fma(v1, p12, fma(v0, p02, v2));
-                const double sc = pow2_recip(t0 + t1 + t2);
-                const bool live = i0 + q < n;
-                b0 = live ? t0 * sc : b0;
-                b1 = live ? t1 * sc : b1;
-                b2 = live ? t2 * sc : b2;
+                bwd_step<LG>(b0, b1, b2, e0, e1, e2, i0 + q < n, p01, p02, p12);
             }
             __threadfence_block();
             arrive_solved(b);
@@ -350,6 +441,17 @@ bool bad_penalties(const char *fn, double p01, double p02, double p12) {
     return !ok;
 }
 
+// The linear-space kernels are exact to far below 1e-9 when every entry of the penalty matrix (1 on the diagonal) is
+// within a factor r = max(1, p) / min(1, p) <= 2^400 of every other.  Mixing keeps each alpha / beta entry above
+// 1/r of its row's share, so an entry flushed below 2^-1074 of its row, or an emission clipped below e^-700, moves
+// the next row by at most a relative 3 * 2^-1073 * r, or 3 * e^-700 * r^2 = 3 * 2^-210; such perturbations do not
+// grow along the table.  Rows stay within [2^-460, 2^403] before rescaling.  Zero penalties, and spreads above
+// 2^400, go to the same kernels in natural-log arithmetic, which has no range limit.
+bool linear_penalties(double p01, double p02, double p12) {
+    const double lo = std::min({1.0, p01, p02, p12}), hi = std::max({1.0, p01, p02, p12});
+    return lo > 0 && hi / lo <= 0x1p400;
+}
+
 // One batch of tables, everything in device memory (start / len per table); kernels only, no host synchronisation.
 int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
                         int is_log, double p01, double p02, double p12, double *d_post, double *d_expected) {
@@ -361,16 +463,33 @@ int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const i
     double *d_ckpt;
     if (scratch(e, SC_HG_CKPT, (size_t)nck * n_tables * 24, (void **)&d_ckpt)) return 1;
     const unsigned grid = (unsigned)((n_tables + PB_TABLES - 1) / PB_TABLES);
-    {
-        LaunchScope ls(e, K_POSTERIOR_FWD);
-        posterior_fwd_kernel<<<grid, PB_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt,
-                                                                           d_expected);
-    }
-    {
-        LaunchScope ls(e, K_POSTERIOR_BWD);
-        IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
-        posterior_bwd_kernel<<<grid, PB_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt,
-                                                                           d_post, d_expected);
+    if (linear_penalties(p01, p02, p12)) {
+        {
+            LaunchScope ls(e, K_POSTERIOR_FWD);
+            posterior_fwd_kernel<false><<<grid, PB_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
+                                                                                      d_ckpt, d_expected);
+        }
+        {
+            LaunchScope ls(e, K_POSTERIOR_BWD);
+            IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
+            posterior_bwd_kernel<false><<<grid, PB_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
+                                                                                      d_ckpt, d_post, d_expected);
+        }
+    } else {
+        const double l01 = log(p01), l02 = log(p02), l12 = log(p12);  // log(0) = -inf: a forbidden transition
+        {
+            LaunchScope ls(e, K_POSTERIOR_FWD);
+            e->k_launches[K_POSTERIOR_FWD_LOG]++;
+            posterior_fwd_kernel<true><<<grid, PB_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
+                                                                                     d_ckpt, d_expected);
+        }
+        {
+            LaunchScope ls(e, K_POSTERIOR_BWD);
+            e->k_launches[K_POSTERIOR_BWD_LOG]++;
+            IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
+            posterior_bwd_kernel<true><<<grid, PB_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
+                                                                                     d_ckpt, d_post, d_expected);
+        }
     }
     IBD_CUDA(cudaGetLastError());
     return 0;

@@ -250,7 +250,10 @@ int64_t hiddengem_last_flagged(ibdgem_engine *e);
  *     that is not finite) gets the uniform emission (1, 1, 1): it carries no information.  (The Viterbi entries
  *     propagate such a bin as the reference does.)
  *   - Penalties may be any finite value >= 0, above 1 included; anything else is an error.  A table whose total
- *     weight is 0 (possible only with zero penalties) gets NaN posteriors and NaN expected counts.
+ *     weight is 0 as a real number (possible only with zero penalties) gets NaN posteriors and NaN expected counts;
+ *     every other table gets the posteriors of the formula above, however far apart its states are.  Penalties with
+ *     max(1, p) / min(1, p) <= 2^400 (no zero among them) run in scaled fp64 linear space, all others in natural-log
+ *     arithmetic, which is slower but has no range limit.
  *   - An empty table has no posterior rows and expected counts 0; one bin has posterior = nrm.
  *   lik / bin_offsets   as for the Viterbi entry (host arrays)
  *   posterior           [sum(n_bins)][3], rows sum to 1

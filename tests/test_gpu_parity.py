@@ -278,7 +278,8 @@ def test_c3_full_size_spot_checks_against_oracle():
 
 @pytest.mark.parametrize("ragged", [False, True])
 def test_hiddengem_batched_pipeline_vs_oracle(ragged):
-    """>= 64 tables take the four-kernel batched path (bin-major intermediates); states must be
+    """>= 64 tables of similar lengths take the batched path (the fused kernel; the four-kernel pipeline only under
+    IBDGEM_VITERBI_FUSED=0, see test_hiddengem_edges_gpu.py); states must be
     bit-exact and scores within 1e-7 of the per-table oracle, for equal-length and ragged batches,
     with zero and all-zero (NaN) rows."""
     import ibdgem_b200 as ib

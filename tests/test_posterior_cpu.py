@@ -30,7 +30,7 @@ def log_emissions(lik, is_log):
         else:
             tot = (lik[:, 0] + lik[:, 1]) + lik[:, 2]
             bad = ~(tot > 0) | ~np.isfinite(tot)
-            out = np.log(lik / tot[:, None])
+            out = np.log(lik) - np.log(tot)[:, None]  # not log(lik / tot): that quotient can underflow to 0
     out[bad] = 0.0
     return out
 
@@ -42,9 +42,17 @@ def _lse3(x, axis):
         return (ms + np.log(np.exp(x - ms).sum(axis=axis, keepdims=True))).squeeze(axis)
 
 
+def _shift(x):
+    """Rows of log weights shifted so their maximum is 0 (a row of -inf stays -inf): magnitudes, and with them the
+    rounding of the sums, stay those of one row's spread however long the table."""
+    m = x.max(axis=-1, keepdims=True)
+    return x - np.where(np.isfinite(m), m, 0.0)
+
+
 def posterior_oracle(lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-3):
-    """Log-space forward-backward (np.logaddexp-style log-sum-exp), vectorised across tables, looped over bins.
-    Returns (posterior [n_bins, 3], expected [n_tables, 3])."""
+    """Log-space forward-backward (np.logaddexp-style log-sum-exp), vectorised across tables, looped over bins; each
+    row of log alpha / log beta shifted to maximum 0, each bin's posterior normalised on its own.  NaN for a table
+    whose final alpha is all -inf (total weight 0).  Returns (posterior [n_bins, 3], expected [n_tables, 3])."""
     off = np.asarray(bin_offsets, np.int64)
     T = len(off) - 1
     lens = np.diff(off)
@@ -60,15 +68,16 @@ def posterior_oracle(lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-
     if nmax:
         fa[:, 0] = E[:, 0]
     for i in range(1, nmax):
-        fa[:, i] = E[:, i] + _lse3(fa[:, i - 1][:, :, None] + lp[None], axis=1)
+        fa[:, i] = _shift(E[:, i] + _lse3(fa[:, i - 1][:, :, None] + lp[None], axis=1))
     for i in range(nmax - 2, -1, -1):
-        nxt = _lse3(lp[None] + (E[:, i + 1] + fb[:, i + 1])[:, None, :], axis=2)
+        nxt = _shift(_lse3(lp[None] + (E[:, i + 1] + fb[:, i + 1])[:, None, :], axis=2))
         fb[:, i] = np.where((i < lens - 1)[:, None], nxt, 0.0)
     last = fa[np.arange(T), np.maximum(lens - 1, 0)]
-    logz = _lse3(last, axis=1)
+    dead = np.isneginf(last).all(axis=1)
+    h = fa + fb
     with np.errstate(all="ignore"):
-        g = np.exp(fa + fb - logz[:, None, None])
-    g[np.isneginf(logz)] = np.nan
+        g = np.exp(h - _lse3(h, axis=2)[:, :, None])
+    g[dead] = np.nan
     post = g[idx]
     expected = np.where(idx[:, :, None], g, 0.0).sum(axis=1)
     return post, expected

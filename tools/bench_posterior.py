@@ -9,7 +9,9 @@ and seed), beside the Viterbi pass on the same tables.  Prints one JSON line (an
   - host-entry end-to-end time (page-locked host buffers through hiddengem_posterior_batch);
   - the card's name and power limit, read in the same run.
 
-`python tools/bench_posterior.py --out FILE` on a GPU box."""
+`python tools/bench_posterior.py [--p01 P --p02 P --p12 P] --out FILE` on a GPU box.  Penalties with a zero (for
+example --p02 0) or spread wider than 2^400 run the kernels in natural-log arithmetic (kernel_stats counts those launches
+again as posterior_fwd_log / posterior_bwd_log)."""
 import argparse
 import ctypes as C
 import json
@@ -38,6 +40,9 @@ def main():
     ap.add_argument("--bins", type=int, default=10_000)
     ap.add_argument("--reps", type=int, default=10)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--p01", type=float, default=1e-3)
+    ap.add_argument("--p02", type=float, default=1e-6)
+    ap.add_argument("--p12", type=float, default=1e-3)
     a = ap.parse_args()
     import torch
     import ibdgem_b200 as ib
@@ -60,13 +65,15 @@ def main():
     d_score = torch.empty((nb, 3), dtype=torch.float64, device=dev)
     d_counts = torch.empty((n_tables, 3), dtype=torch.int64, device=dev)
     out = {"workload": "hiddengem posterior, C4: %d tables x %d bins of natural-log window scores (tools/bench_aux.py leg_c4 "
-                       "tables), device-resident" % (n_tables, n_bins), "card": card(), "torch_device": torch.cuda.get_device_name(dev)}
+                       "tables), device-resident" % (n_tables, n_bins), "card": card(), "torch_device": torch.cuda.get_device_name(dev),
+           "penalties": {"p01": a.p01, "p02": a.p02, "p12": a.p12}}
+    pen = dict(p01=a.p01, p02=a.p02, p12=a.p12)
     with ib.Engine(ib.Params(device=0)) as e:
         def post():
-            e.posterior_batch_device(d_ll.data_ptr(), off, True, d_post.data_ptr(), d_exp.data_ptr())
+            e.posterior_batch_device(d_ll.data_ptr(), off, True, d_post.data_ptr(), d_exp.data_ptr(), **pen)
 
         def vit():
-            e.viterbi_batch_device(d_ll.data_ptr(), off, True, d_state.data_ptr(), d_score.data_ptr(), d_counts.data_ptr())
+            e.viterbi_batch_device(d_ll.data_ptr(), off, True, d_state.data_ptr(), d_score.data_ptr(), d_counts.data_ptr(), **pen)
 
         post()
         vit()
@@ -102,7 +109,7 @@ def main():
 
         def host():
             e._check(lib.hiddengem_posterior_batch(e._h, C.c_int32(n_tables), off.ctypes.data_as(C.c_void_p), C.c_void_p(h_ll.data_ptr()),
-                                                   C.c_int32(1), C.c_double(1e-3), C.c_double(1e-6), C.c_double(1e-3),
+                                                   C.c_int32(1), C.c_double(a.p01), C.c_double(a.p02), C.c_double(a.p12),
                                                    C.c_void_p(h_post.data_ptr()), h_exp.ctypes.data_as(C.c_void_p)))
 
         host()
