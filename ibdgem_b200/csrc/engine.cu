@@ -28,7 +28,7 @@ static const char *const kKernelNameList[] = {
     "site_table",     "scan_count",    "scan_offsets",  "scan_rank",    "window_nonld", "counters",
     "expand_sites",   "ld_general",    "ld_finalize",   "ld_compact",   "ld_c0",        "ld_transpose",
     "ld_stage",       "ld_expand_bg",  "ld_expand_tgt", "ld_windows",   "ld_ibd0",
-    "ld_mma",         "viterbi",       "viterbi_norm",  "viterbi_back", "viterbi_out", "fill",
+    "ld_mma",         "viterbi",       "viterbi_back",  "viterbi_out",  "fill",
     "v_slots",        "v_wmap",        "v_tw",          "v_sort",       "v_expand_a",  "v_expand_b",   "ld_vmma",
     "window_linear",  "posterior_fwd", "posterior_bwd", "posterior_fwd_log", "posterior_bwd_log",
 };

@@ -45,9 +45,8 @@ enum KernelId {
     K_LD_IBD0,          // tensor path: LIBD0 log-mean-exp over the background without the target
     K_LD_MMA,           // tensor path: tcgen05 window GEMM + fused log-sum-exp epilogue -> LIBD1
     K_VITERBI,          // H2 hiddengem forward pass (or the whole per-table kernel for small batches)
-    K_VITERBI_NORM,     // H1 ln of the normalised likelihoods, to bin-major
     K_VITERBI_BACK,     // H3 back-trace + state counts
-    K_VITERBI_OUT,      // scores / states back to table-major
+    K_VITERBI_OUT,      // states back to table-major
     K_FILL,             // NaN fill of device score buffers
     K_V_SLOTS,          // per-target-window tensor path: slots of the K axis (informative kept sites)
     K_V_WMAP,           // -v window map in rank space (one warp per target)
@@ -196,11 +195,14 @@ int pinned_stage(ibdgem_engine *e, size_t bytes, void **out);
 enum ScratchSlot {
     SC_TARGETS = 0, SC_BG, SC_TGT_COUNTS, SC_BLOCKCNT, SC_WFIRST, SC_WLAST, SC_NWIN, SC_KTOT, SC_WLL,
     SC_WN, SC_WS, SC_WE, SC_COUNTERS, SC_SITE_STATUS, SC_SITE_LIK, SC_LD_PART, SC_NREFPANEL,
-    SC_HG_LIK, SC_HG_OFF, SC_HG_STATE, SC_HG_SCORE, SC_HG_COUNTS, SC_HG_NRMT, SC_HG_SCORET, SC_HG_FROMT, SC_HG_LAST,
+    SC_HG_LIK, SC_HG_OFF, SC_HG_STATE, SC_HG_SCORE, SC_HG_COUNTS, SC_HG_FROMT, SC_HG_LAST,
     SC_MMA_TGT, SC_MMA_BG, SC_MMA_ROWLSE, SC_MMA_BGIDX, SC_MMA_MISC, SC_MMA_UNIT,
     SC_WLIN, SC_WLL_PACK, SC_V_KS, SC_V_KE, SC_V_TWBASE, SC_V_TWI, SC_V_TWD, SC_V_ORDER, SC_V_HIST, SC_V_TILES, SC_V_MISC, SC_HG_CKPT, SC_SLOTS
 };
 int scratch(ibdgem_engine *e, int slot, size_t bytes, void **out);
+// hiddengem: host start / length of every table of a call (hidden.cu; the Viterbi and posterior entries)
+int table_layout(const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, std::vector<int64_t> *sl, int64_t *maxbins,
+                 int64_t *total);
 
 // Makes the engine stream wait for the panel chunks that cover sites [0, s_end); ensure_table also
 // runs site_table on the part of [0, s_end) it has not covered yet.

@@ -16,16 +16,48 @@
 #include <vector>
 
 #include "engine.h"
+#include "hg_block.cuh"
 #include "tc_common.cuh"
 
 namespace ibdgem {
 
-__device__ __forceinline__ int argmax3(double c0, double c1, double c2) {
+constexpr uint8_t FROM_SELF = 0 | (1 << 2) | (2 << 4);  // back-pointers of bin 0: every state from itself
+
+__device__ __forceinline__ int argmax3(const double *c) {
     int b = 0;
-    double v = c0;
-    if (c1 > v) { b = 1; v = c1; }
-    if (c2 > v) { b = 2; }
+    double v = c[0];
+    if (c[1] > v) { b = 1; v = c[1]; }
+    if (c[2] > v) { b = 2; }
     return b;
+}
+__device__ __forceinline__ double pick3(const double *c, int k) { return k == 0 ? c[0] : (k == 1 ? c[1] : c[2]); }
+
+// c[s][k] = (prev_k + ln nrm_s) + ln pen(k, s), the candidates of state s; the diagonal has no penalty factor
+__device__ __forceinline__ void candidates(const double *p, const double *n, double lp01, double lp02, double lp12, double (&c)[3][3]) {
+    c[0][0] = p[0] + n[0], c[0][1] = (p[1] + n[0]) + lp01, c[0][2] = (p[2] + n[0]) + lp02;
+    c[1][0] = (p[0] + n[1]) + lp01, c[1][1] = p[1] + n[1], c[1][2] = (p[2] + n[1]) + lp12;
+    c[2][0] = (p[0] + n[2]) + lp02, c[2][1] = (p[1] + n[2]) + lp12, c[2][2] = p[2] + n[2];
+}
+
+// ln nrm = ln of the normalised likelihoods of one bin.  FAST_EXP: exp_nonpos (arguments are <= 0, degree-12
+// polynomial, error ~1 ulp, half the instructions of exp()) for the batched kernel; viterbi_kernel keeps libm exp.
+template <bool FAST_EXP>
+__device__ __forceinline__ void ln_nrm(const double *L, int is_log, double *n) {
+    if (is_log) {  // ln nrm = ll - logsumexp(ll)
+        const double m = fmax(L[0], fmax(L[1], L[2]));
+        if (m == -INFINITY) {
+            n[0] = n[1] = n[2] = __longlong_as_double(0x7ff8000000000000LL);  // 0/0 in the reference
+        } else {
+            const double z = FAST_EXP ? m + log(exp_nonpos(L[0] - m) + exp_nonpos(L[1] - m) + exp_nonpos(L[2] - m))
+                                      : m + log(exp(L[0] - m) + exp(L[1] - m) + exp(L[2] - m));
+            n[0] = L[0] - z; n[1] = L[1] - z; n[2] = L[2] - z;
+        }
+    } else {  // src/hiddengem.c:74-76: l_s / (l0 + l1 + l2) in fp64, then the log
+        const double tot = __dadd_rn(__dadd_rn(L[0], L[1]), L[2]);
+        n[0] = log(__ddiv_rn(L[0], tot));
+        n[1] = log(__ddiv_rn(L[1], tot));
+        n[2] = log(__ddiv_rn(L[2], tot));
+    }
 }
 
 // Near-tie guard.  The reference multiplies x87 long doubles (src/hiddengem.c:110-141); sums of fp64 logs carry a
@@ -35,19 +67,17 @@ __device__ __forceinline__ int argmax3(double c0, double c1, double c2) {
 // on the host in long double.  NaN / -inf candidates never flag: their comparisons are exact in both worlds.
 constexpr double LN_LDBL_MIN = -11355.137111933024;  // ln(3.3621e-4932)
 __device__ __forceinline__ double tie_scale(int64_t i) { return (double)(int)(i + 1) * 4.440892098500626e-16; }  // 4 (i + 1) 2^-53
-__device__ __forceinline__ bool near_tie(double c0, double c1, double c2, int best, double scale) {
-    const double w = best == 0 ? c0 : (best == 1 ? c1 : c2);
-    const double r = best == 0 ? fmax(c1, c2) : (best == 1 ? fmax(c0, c2) : fmax(c0, c1));
+__device__ __forceinline__ bool near_tie(const double *c, int best, double scale) {
+    const double w = pick3(c, best);
+    const double r = best == 0 ? fmax(c[1], c[2]) : (best == 1 ? fmax(c[0], c[2]) : fmax(c[0], c[1]));
     return (w - r) < fma(scale, fabs(w), 1e-12);  // false for NaN and for inf - inf
 }
-__device__ __forceinline__ bool near_tie(double c0, double c1, double c2, int best, int64_t i) {
-    return near_tie(c0, c1, c2, best, tie_scale(i));
-}
 // a finite score below the smallest normal long double: the reference's product is a denormal (or zero) there
-__device__ __forceinline__ bool below_ldbl(double s0, double s1, double s2) {
-    return (s0 < LN_LDBL_MIN && s0 > -INFINITY) || (s1 < LN_LDBL_MIN && s1 > -INFINITY) || (s2 < LN_LDBL_MIN && s2 > -INFINITY);
+__device__ __forceinline__ bool below_ldbl(const double *s) {
+    return (s[0] < LN_LDBL_MIN && s[0] > -INFINITY) || (s[1] < LN_LDBL_MIN && s[1] > -INFINITY) || (s[2] < LN_LDBL_MIN && s[2] > -INFINITY);
 }
 
+// One table per thread, for small or ragged batches.
 __global__ void __launch_bounds__(128)
 viterbi_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik, int is_log,
                double lp01, double lp02, double lp12, uint8_t *__restrict__ state,
@@ -61,49 +91,33 @@ viterbi_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *_
         flag[tb] = 0;
         return;
     }
-    double s0 = 0, s1 = 0, s2 = 0;
+    double s[3] = {0, 0, 0};
     bool tie = false;
     for (int64_t i = 0; i < n; i++) {
-        const double *L = lik + (b0 + i) * 3;
-        double n0, n1, n2;
-        if (is_log) {  // ln nrm = ll - logsumexp(ll)
-            const double m = fmax(L[0], fmax(L[1], L[2]));
-            if (m == -INFINITY) {
-                n0 = n1 = n2 = __longlong_as_double(0x7ff8000000000000LL);  // 0/0 in the reference
-            } else {
-                const double z = m + log(exp(L[0] - m) + exp(L[1] - m) + exp(L[2] - m));
-                n0 = L[0] - z; n1 = L[1] - z; n2 = L[2] - z;
-            }
-        } else {  // src/hiddengem.c:74-76: l_s / (l0 + l1 + l2) in fp64, then the log
-            const double tot = __dadd_rn(__dadd_rn(L[0], L[1]), L[2]);
-            n0 = log(__ddiv_rn(L[0], tot));
-            n1 = log(__ddiv_rn(L[1], tot));
-            n2 = log(__ddiv_rn(L[2], tot));
-        }
+        double nv[3];
+        ln_nrm<false>(lik + (b0 + i) * 3, is_log, nv);
         uint8_t from;
         if (i == 0) {  // src/hiddengem.c:112-118
-            s0 = n0; s1 = n1; s2 = n2;
-            from = 0 | (1 << 2) | (2 << 4);
+            s[0] = nv[0]; s[1] = nv[1]; s[2] = nv[2];
+            from = FROM_SELF;
         } else {
-            // candidates (prev_k + ln nrm_s) + ln pen(k, s), diagonal has no penalty factor
-            const double a0 = s0 + n0, a1 = (s1 + n0) + lp01, a2 = (s2 + n0) + lp02;
-            const double b0_ = (s0 + n1) + lp01, b1 = s1 + n1, b2 = (s2 + n1) + lp12;
-            const double c0 = (s0 + n2) + lp02, c1 = (s1 + n2) + lp12, c2 = s2 + n2;
-            const int k0 = argmax3(a0, a1, a2), k1 = argmax3(b0_, b1, b2), k2 = argmax3(c0, c1, c2);
+            double c[3][3];
+            candidates(s, nv, lp01, lp02, lp12, c);
+            const int k0 = argmax3(c[0]), k1 = argmax3(c[1]), k2 = argmax3(c[2]);
             const double ts = tie_scale(i);
-            tie |= near_tie(a0, a1, a2, k0, ts) | near_tie(b0_, b1, b2, k1, ts) | near_tie(c0, c1, c2, k2, ts);
-            s0 = k0 == 0 ? a0 : (k0 == 1 ? a1 : a2);
-            s1 = k1 == 0 ? b0_ : (k1 == 1 ? b1 : b2);
-            s2 = k2 == 0 ? c0 : (k2 == 1 ? c1 : c2);
+            tie |= near_tie(c[0], k0, ts) | near_tie(c[1], k1, ts) | near_tie(c[2], k2, ts);
+            s[0] = pick3(c[0], k0);
+            s[1] = pick3(c[1], k1);
+            s[2] = pick3(c[2], k2);
             from = (uint8_t)(k0 | (k1 << 2) | (k2 << 4));
         }
-        if (!is_log) tie |= below_ldbl(s0, s1, s2);
+        if (!is_log) tie |= below_ldbl(s);
         state[b0 + i] = from;
         double *o = score + (b0 + i) * 3;
-        o[0] = s0; o[1] = s1; o[2] = s2;
+        o[0] = s[0]; o[1] = s[1]; o[2] = s[2];
     }
-    int cur = argmax3(s0, s1, s2);  // src/hiddengem.c:246-249
-    tie |= near_tie(s0, s1, s2, cur, n);
+    int cur = argmax3(s);  // src/hiddengem.c:246-249
+    tie |= near_tie(s, cur, tie_scale(n));
     long long c[3] = {0, 0, 0};
     for (int64_t i = n - 1; i >= 0; i--) {  // src/hiddengem.c:252-257
         const uint8_t from = state[b0 + i];
@@ -118,127 +132,165 @@ viterbi_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *_
 }
 
 // ---------------------------------------------------------------------------------------------
-// Batched pipeline for many tables (C4: 10,000 tables x 10,000 bins).  The recursion is sequential
-// in bins and independent across tables, so the natural thread is a table — but the caller's
-// arrays are table-major and a thread-per-table walk over them is uncoalesced.  Four kernels, all
-// streaming: (1) ln nrm per bin, transposed to bin-major through shared memory; (2) forward pass,
-// thread = table, every load and store coalesced across tables, loads issued UNROLL bins ahead of
-// the recurrence; (3) back-trace, same layout; (4) scores and states transposed back to the
-// caller's table-major layout.  Arithmetic is operation-for-operation that of viterbi_kernel.
-__device__ __forceinline__ void ln_nrm(const double *L, int is_log, double &n0, double &n1, double &n2) {
-    if (is_log) {
-        const double m = fmax(L[0], fmax(L[1], L[2]));
-        if (m == -INFINITY) {
-            n0 = n1 = n2 = __longlong_as_double(0x7ff8000000000000LL);
-        } else {  // exp_nonpos: arguments are <= 0, degree-12 polynomial, error ~1 ulp (half the instructions of exp())
-            const double z = m + log(exp_nonpos(L[0] - m) + exp_nonpos(L[1] - m) + exp_nonpos(L[2] - m));
-            n0 = L[0] - z; n1 = L[1] - z; n2 = L[2] - z;
+// Batched pipeline for many tables (C4: 10,000 tables x 10,000 bins), three kernels: the fused forward pass, the
+// back-trace, and the states back to the caller's layout.
+//
+// Fused forward pass: one read of the likelihoods, one write of the scores, on the chunked block of hg_block.cuh.
+// The workers turn each chunk's likelihoods into ln nrm in shared memory — that is where the fp64 exp / log work is,
+// and it is parallel over bins; the solver walks the recursion.  The arithmetic is that of viterbi_kernel, operation
+// for operation.  Back-pointers leave bin-major (coalesced over tables) for viterbi_back_kernel; scores leave in the
+// caller's table-major layout.
+constexpr int VF_SMEM = 4 * HG_TABLES * HG_ROW * 8 + HG_HEAD_SMEM + 2 * HG_TABLES * 3 * 8 + HG_TABLES * 4 + 2 * HG_BINS * HG_TABLES;
+
+// The solver's walk over one chunk (lane = table, nq = bins of the table in the chunk, <= 0: none).  A single warp
+// walks the bins, so its time is (instructions per bin) x (issue latency): the step is branch-free.  FIRST: chunk 0,
+// whose bin 0 takes s = ln nrm and the identity back-pointers, as in viterbi_kernel.
+template <bool FIRST>
+__device__ __forceinline__ void solve_chunk(const double *nr, double *so, uint8_t (*frm)[HG_TABLES], int lane, int nq, double lp01,
+                                            double lp02, double lp12, double (&s)[3]) {
+    if (FIRST) {
+        s[0] = nr[0]; s[1] = nr[1]; s[2] = nr[2];
+        so[0] = s[0]; so[1] = s[1]; so[2] = s[2];
+        frm[0][lane] = FROM_SELF;
+    }
+#pragma unroll 4
+    for (int q = FIRST ? 1 : 0; q < HG_BINS; q++) {
+        double c[3][3];
+        candidates(s, nr + q * 3, lp01, lp02, lp12, c);
+        // strict '>' arg-max: lowest index wins, NaN never wins
+        const bool ga = c[0][1] > c[0][0], gb = c[1][1] > c[1][0], gc = c[2][1] > c[2][0];
+        const double ma = ga ? c[0][1] : c[0][0], mb = gb ? c[1][1] : c[1][0], mc = gc ? c[2][1] : c[2][0];
+        const bool ha = c[0][2] > ma, hb = c[1][2] > mb, hc = c[2][2] > mc;
+        const bool live = q < nq;
+        s[0] = live ? (ha ? c[0][2] : ma) : s[0];
+        s[1] = live ? (hb ? c[1][2] : mb) : s[1];
+        s[2] = live ? (hc ? c[2][2] : mc) : s[2];
+        so[q * 3] = s[0];
+        so[q * 3 + 1] = s[1];
+        so[q * 3 + 2] = s[2];
+        frm[q][lane] = (uint8_t)((ha ? 2 : (int)ga) | ((hb ? 2 : (int)gb) << 2) | ((hc ? 2 : (int)gc) << 4));
+    }
+}
+
+__global__ void __launch_bounds__(HG_THREADS, 3)
+viterbi_fused_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
+                     int is_log, double lp01, double lp02, double lp12, double *__restrict__ score,
+                     uint8_t *__restrict__ fromT /*[maxbins][n_tables]*/, double *__restrict__ last /*[n_tables][3]*/,
+                     uint8_t *__restrict__ flag) {
+    extern __shared__ double vf_smem[];
+    double (*nrm)[HG_TABLES][HG_ROW] = reinterpret_cast<double (*)[HG_TABLES][HG_ROW]>(vf_smem);
+    double (*sco)[HG_TABLES][HG_ROW] = reinterpret_cast<double (*)[HG_TABLES][HG_ROW]>(vf_smem + 2 * HG_TABLES * HG_ROW);
+    int64_t *s_start = reinterpret_cast<int64_t *>(vf_smem + 4 * HG_TABLES * HG_ROW), *s_len = s_start + HG_TABLES;
+    double (*prevlast)[HG_TABLES][3] = reinterpret_cast<double (*)[HG_TABLES][3]>(s_len + HG_TABLES);  // last bin's scores of a chunk
+    int *tieflag = reinterpret_cast<int *>(&prevlast[2][0][0]);
+    uint8_t (*frm)[HG_BINS][HG_TABLES] = reinterpret_cast<uint8_t (*)[HG_BINS][HG_TABLES]>(tieflag + HG_TABLES);
+    const int tb0 = blockIdx.x * HG_TABLES;
+    if (threadIdx.x < HG_TABLES) tieflag[threadIdx.x] = 0;
+    const int nchunk = block_tables(n_tables, start, len, s_start, s_len);
+    if (threadIdx.x >= 32) {
+        // ===== workers =====
+        const int w = threadIdx.x - 32;
+        const ChunkLoader ld{s_start, s_len, w};
+        // raw likelihoods of the NEXT chunk are fetched before this chunk's exp / log work starts, so DRAM latency
+        // hides under it
+        double pre[HG_NLD];
+        if (nchunk > 0) ld.fetch(lik, 0, pre);
+        for (int c = 0; c <= nchunk; c++) {
+            const int b = c & 1;
+            if (c < nchunk) {
+                const int64_t i0 = (int64_t)c * HG_BINS;
+                ld.store(pre, nrm[b]);
+                if (c + 1 < nchunk) ld.fetch(lik, c + 1, pre);
+                sync_workers();
+                // ln nrm in place: 512 bins, 2 per worker
+#pragma unroll
+                for (int k = 0; k < HG_NBIN; k++) {
+                    const int idx = k * HG_WORKERS + w;
+                    const int t = idx / HG_BINS, i = idx % HG_BINS;
+                    if (i0 + i < s_len[t]) {
+                        const double v[3] = {nrm[b][t][i * 3], nrm[b][t][i * 3 + 1], nrm[b][t][i * 3 + 2]};
+                        ln_nrm<true>(v, is_log, &nrm[b][t][i * 3]);
+                    }
+                }
+                __threadfence_block();
+                arrive_ready(b);
+            }
+            if (c >= 1) {  // drain the chunk the solver has just finished
+                const int pb = (c - 1) & 1;
+                sync_solved(pb);
+                const int64_t i0 = (int64_t)(c - 1) * HG_BINS;
+                // Near-tie and long-double-range tests, moved off the solver's critical path: with the scores of bin
+                // i - 1 and ln nrm of bin i both still in shared memory, every bin's nine candidates can be rebuilt
+                // independently (the same expressions, hence the same doubles) — 512 bins over 256 workers.
+#pragma unroll
+                for (int k = 0; k < HG_NBIN; k++) {
+                    const int idx = k * HG_WORKERS + w;
+                    const int t = idx / HG_BINS, i = idx % HG_BINS;
+                    const int64_t gi = i0 + i;
+                    if (gi < s_len[t]) {
+                        const double *cur = &sco[pb][t][i * 3];
+                        bool tie = !is_log && below_ldbl(cur);
+                        if (gi > 0) {
+                            const double *pv = i > 0 ? &sco[pb][t][(i - 1) * 3] : &prevlast[pb ^ 1][t][0];
+                            const double p[3] = {pv[0], pv[1], pv[2]};
+                            const double nv[3] = {nrm[pb][t][i * 3], nrm[pb][t][i * 3 + 1], nrm[pb][t][i * 3 + 2]};
+                            const double ts = tie_scale(gi);
+                            double cd[3][3];
+                            candidates(p, nv, lp01, lp02, lp12, cd);
+                            tie |= near_tie(cd[0], argmax3(cd[0]), ts) | near_tie(cd[1], argmax3(cd[1]), ts) |
+                                   near_tie(cd[2], argmax3(cd[2]), ts);
+                        }
+                        if (tie) tieflag[t] = 1;
+                        if (i == HG_BINS - 1) { prevlast[pb][t][0] = cur[0]; prevlast[pb][t][1] = cur[1]; prevlast[pb][t][2] = cur[2]; }
+                    }
+                }
+                ld.write(c - 1, sco[pb], score);
+#pragma unroll
+                for (int k = 0; k < HG_NBIN; k++) {
+                    const int idx = k * HG_WORKERS + w;
+                    const int i = idx / HG_TABLES, t = idx % HG_TABLES;
+                    if (tb0 + t < n_tables && i0 + i < s_len[t]) fromT[(size_t)(i0 + i) * n_tables + tb0 + t] = frm[pb][i][t];
+                }
+                sync_workers();  // buffer pb is free for chunk c + 1
+            }
         }
     } else {
-        const double tot = __dadd_rn(__dadd_rn(L[0], L[1]), L[2]);
-        n0 = log(__ddiv_rn(L[0], tot));
-        n1 = log(__ddiv_rn(L[1], tot));
-        n2 = log(__ddiv_rn(L[2], tot));
-    }
-}
-
-// (1) block = 32 tables x 32 bins.  Reads are contiguous runs of 32 bins of one table; writes are
-// runs of 32 tables of one (bin, state).
-__global__ void __launch_bounds__(1024)
-viterbi_norm_kernel(int n_tables, int64_t maxbins, const int64_t *__restrict__ start, const int64_t *__restrict__ len,
-                    const double *__restrict__ lik, int is_log, double *__restrict__ nrmT /*[maxbins][3][n_tables]*/) {
-    __shared__ double tile[3][32][33];
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-    const int t_in = blockIdx.x * 32 + ty;
-    const int64_t i_in = (int64_t)blockIdx.y * 32 + tx;
-    double n0 = 0, n1 = 0, n2 = 0;
-    if (t_in < n_tables) {
-        const int64_t b0 = start[t_in], n = len[t_in];
-        if (i_in < n) {
-            const double *L = lik + (b0 + i_in) * 3;
-            const double v[3] = {L[0], L[1], L[2]};
-            ln_nrm(v, is_log, n0, n1, n2);
+        // ===== solver: lane = table =====
+        const int lane = threadIdx.x;
+        const int64_t n = s_len[lane];
+        double s[3] = {0, 0, 0};
+        for (int c = 0; c < nchunk; c++) {
+            const int b = c & 1;
+            sync_ready(b);
+            const int nq = (int)min((int64_t)HG_BINS, n - (int64_t)c * HG_BINS);
+            if (c == 0) solve_chunk<true>(&nrm[b][lane][0], &sco[b][lane][0], frm[b], lane, nq, lp01, lp02, lp12, s);
+            else solve_chunk<false>(&nrm[b][lane][0], &sco[b][lane][0], frm[b], lane, nq, lp01, lp02, lp12, s);
+            __threadfence_block();
+            arrive_solved(b);
+        }
+        const int tb = tb0 + lane;
+        if (tb < n_tables) {
+            last[(size_t)tb * 3 + 0] = s[0];
+            last[(size_t)tb * 3 + 1] = s[1];
+            last[(size_t)tb * 3 + 2] = s[2];
         }
     }
-    tile[0][tx][ty] = n0;
-    tile[1][tx][ty] = n1;
-    tile[2][tx][ty] = n2;
-    __syncthreads();
-    const int t_out = blockIdx.x * 32 + tx;
-    const int64_t i_out = (int64_t)blockIdx.y * 32 + ty;
-    if (t_out < n_tables && i_out < maxbins) {
-#pragma unroll
-        for (int s = 0; s < 3; s++) nrmT[(i_out * 3 + s) * n_tables + t_out] = tile[s][ty][tx];
-    }
-}
-
-// (2) thread = table
-constexpr int VIT_UNROLL = 8;
-__global__ void __launch_bounds__(64)
-viterbi_forward_kernel(int n_tables, const int64_t *__restrict__ len, int is_log, const double *__restrict__ nrmT, double lp01,
-                       double lp02, double lp12, uint8_t *__restrict__ fromT /*[maxbins][n_tables]*/,
-                       double *__restrict__ scoreT /*[maxbins][3][n_tables]*/, double *__restrict__ last /*[n_tables][3]*/,
-                       uint8_t *__restrict__ flag) {
-    const int tb = blockIdx.x * blockDim.x + threadIdx.x;
-    if (tb >= n_tables) return;
-    const int64_t n = len[tb];
-    bool tie = false;
-    const size_t nT = (size_t)n_tables;
-    double s0 = 0, s1 = 0, s2 = 0;
-    // two register batches: the loads of batch k + 1 are in flight while batch k runs the recurrence
-    double nx[VIT_UNROLL][3];
-    auto fetch = [&](int64_t ib) {
-#pragma unroll
-        for (int u = 0; u < VIT_UNROLL; u++)
-            if (ib + u < n) {
-#pragma unroll
-                for (int s = 0; s < 3; s++) nx[u][s] = __ldcs(nrmT + ((size_t)(ib + u) * 3 + s) * nT + tb);
+    __syncthreads();  // the workers' last drain has set the tie flags
+    if (threadIdx.x < HG_TABLES) {
+        const int tb = tb0 + threadIdx.x;
+        if (tb < n_tables) {
+            const int64_t n = s_len[threadIdx.x];
+            bool tie = tieflag[threadIdx.x] != 0;
+            if (n > 0) {
+                const double l[3] = {last[(size_t)tb * 3], last[(size_t)tb * 3 + 1], last[(size_t)tb * 3 + 2]};
+                tie |= near_tie(l, argmax3(l), tie_scale(n));
             }
-    };
-    fetch(0);
-    for (int64_t ib = 0; ib < n; ib += VIT_UNROLL) {
-        double v[VIT_UNROLL][3];
-#pragma unroll
-        for (int u = 0; u < VIT_UNROLL; u++) {
-            v[u][0] = nx[u][0]; v[u][1] = nx[u][1]; v[u][2] = nx[u][2];
-        }
-        if (ib + VIT_UNROLL < n) fetch(ib + VIT_UNROLL);
-#pragma unroll
-        for (int u = 0; u < VIT_UNROLL; u++) {
-            const int64_t i = ib + u;
-            if (i >= n) break;
-            const double n0 = v[u][0], n1 = v[u][1], n2 = v[u][2];
-            uint8_t from;
-            if (i == 0) {
-                s0 = n0; s1 = n1; s2 = n2;
-                from = 0 | (1 << 2) | (2 << 4);
-            } else {
-                const double a0 = s0 + n0, a1 = (s1 + n0) + lp01, a2 = (s2 + n0) + lp02;
-                const double b0 = (s0 + n1) + lp01, b1 = s1 + n1, b2 = (s2 + n1) + lp12;
-                const double c0 = (s0 + n2) + lp02, c1 = (s1 + n2) + lp12, c2 = s2 + n2;
-                const int k0 = argmax3(a0, a1, a2), k1 = argmax3(b0, b1, b2), k2 = argmax3(c0, c1, c2);
-                const double ts = tie_scale(i);
-                tie |= near_tie(a0, a1, a2, k0, ts) | near_tie(b0, b1, b2, k1, ts) | near_tie(c0, c1, c2, k2, ts);
-                s0 = k0 == 0 ? a0 : (k0 == 1 ? a1 : a2);
-                s1 = k1 == 0 ? b0 : (k1 == 1 ? b1 : b2);
-                s2 = k2 == 0 ? c0 : (k2 == 1 ? c1 : c2);
-                from = (uint8_t)(k0 | (k1 << 2) | (k2 << 4));
-            }
-            if (!is_log) tie |= below_ldbl(s0, s1, s2);
-            fromT[(size_t)i * nT + tb] = from;
-            __stcs(scoreT + ((size_t)i * 3 + 0) * nT + tb, s0);
-            __stcs(scoreT + ((size_t)i * 3 + 1) * nT + tb, s1);
-            __stcs(scoreT + ((size_t)i * 3 + 2) * nT + tb, s2);
+            flag[tb] = tie ? 1 : 0;
         }
     }
-    last[(size_t)tb * 3 + 0] = s0;
-    last[(size_t)tb * 3 + 1] = s1;
-    last[(size_t)tb * 3 + 2] = s2;
-    if (n > 0) tie |= near_tie(s0, s1, s2, argmax3(s0, s1, s2), n);
-    flag[tb] = tie ? 1 : 0;
 }
 
-// (3) back-trace; the state overwrites the back-pointer byte in place
+// back-trace, thread = table; the state overwrites the back-pointer byte in place
 __global__ void __launch_bounds__(64)
 viterbi_back_kernel(int n_tables, const int64_t *__restrict__ len, uint8_t *__restrict__ fromT, const double *__restrict__ last,
                     long long *__restrict__ counts) {
@@ -248,7 +300,7 @@ viterbi_back_kernel(int n_tables, const int64_t *__restrict__ len, uint8_t *__re
     const size_t nT = (size_t)n_tables;
     long long c0 = 0, c1 = 0, c2 = 0;
     if (n > 0) {
-        int cur = argmax3(last[(size_t)tb * 3], last[(size_t)tb * 3 + 1], last[(size_t)tb * 3 + 2]);
+        int cur = argmax3(last + (size_t)tb * 3);
         constexpr int BU = 32;
         for (int64_t ib = n; ib > 0; ib -= BU) {
             uint8_t f[BU];
@@ -268,226 +320,6 @@ viterbi_back_kernel(int n_tables, const int64_t *__restrict__ len, uint8_t *__re
     counts[tb * 3 + 0] = c0;
     counts[tb * 3 + 1] = c1;
     counts[tb * 3 + 2] = c2;
-}
-
-// (4) bin-major -> the caller's table-major layout
-__global__ void __launch_bounds__(1024)
-viterbi_out_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const uint8_t *__restrict__ stateT,
-                   const double *__restrict__ scoreT, uint8_t *__restrict__ state, double *__restrict__ score) {
-    __shared__ double tile[3][32][33];
-    __shared__ uint8_t st[32][33];
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-    const int t_in = blockIdx.x * 32 + tx;
-    const int64_t i_in = (int64_t)blockIdx.y * 32 + ty;
-    const size_t nT = (size_t)n_tables;
-    if (t_in < n_tables && i_in < len[t_in]) {
-#pragma unroll
-        for (int s = 0; s < 3; s++) tile[s][ty][tx] = __ldcs(scoreT + ((size_t)i_in * 3 + s) * nT + t_in);
-        st[ty][tx] = stateT[(size_t)i_in * nT + t_in];
-    }
-    __syncthreads();
-    const int t_out = blockIdx.x * 32 + ty;
-    const int64_t i_out = (int64_t)blockIdx.y * 32 + tx;
-    if (t_out < n_tables) {
-        const int64_t b0 = start[t_out], n = len[t_out];
-        if (i_out < n) {
-            double *o = score + (b0 + i_out) * 3;
-            o[0] = tile[0][tx][ty];
-            o[1] = tile[1][tx][ty];
-            o[2] = tile[2][tx][ty];
-            state[b0 + i_out] = st[tx][ty];
-        }
-    }
-}
-
-
-// ---------------------------------------------------------------------------------------------
-// Fused forward pass for large batches (C4: 10,000 tables x 10,000 bins): one read of the likelihoods, one write of
-// the scores.  A block takes 32 tables.  Four worker warps move 16-bin chunks between global memory and shared
-// memory with coalesced accesses (a table's chunk is 384 contiguous bytes) and turn the likelihoods into ln nrm
-// there — that is where the fp64 exp / log work is, and it is parallel over bins; ONE solver warp (lane = table)
-// walks the chunk sequentially, which the recursion demands, touching shared memory only.  Chunks are double
-// buffered, so loads, normalisation, recursion and stores of neighbouring chunks overlap.  The arithmetic is that
-// of viterbi_kernel, operation for operation.  Back-pointers leave bin-major (coalesced over tables) for
-// viterbi_back_kernel; scores leave in the caller's table-major layout.
-constexpr int VF_TABLES = 32, VF_BINS = 16, VF_ROW = VF_BINS * 3 + 1;  // padded row: lanes hit distinct banks
-constexpr int VF_WORKERS = 256, VF_THREADS = VF_WORKERS + 32;
-constexpr int VF_SMEM = 4 * VF_TABLES * VF_ROW * 8 + 2 * VF_TABLES * 8 + 2 * VF_TABLES * 3 * 8 + VF_TABLES * 4 + 2 * VF_BINS * VF_TABLES;
-__global__ void __launch_bounds__(VF_THREADS, 3)
-viterbi_fused_kernel(int n_tables, int64_t maxbins, const int64_t *__restrict__ start, const int64_t *__restrict__ len,
-                     const double *__restrict__ lik, int is_log, double lp01, double lp02, double lp12, double *__restrict__ score,
-                     uint8_t *__restrict__ fromT /*[maxbins][n_tables]*/, double *__restrict__ last /*[n_tables][3]*/,
-                     uint8_t *__restrict__ flag) {
-    extern __shared__ double vf_smem[];
-    double (*nrm)[VF_TABLES][VF_ROW] = reinterpret_cast<double (*)[VF_TABLES][VF_ROW]>(vf_smem);
-    double (*sco)[VF_TABLES][VF_ROW] = reinterpret_cast<double (*)[VF_TABLES][VF_ROW]>(vf_smem + 2 * VF_TABLES * VF_ROW);
-    int64_t *s_start = reinterpret_cast<int64_t *>(vf_smem + 4 * VF_TABLES * VF_ROW), *s_len = s_start + VF_TABLES;
-    double (*prevlast)[VF_TABLES][3] = reinterpret_cast<double (*)[VF_TABLES][3]>(s_len + VF_TABLES);  // last bin's scores of a chunk
-    int *tieflag = reinterpret_cast<int *>(&prevlast[2][0][0]);
-    uint8_t (*frm)[VF_BINS][VF_TABLES] = reinterpret_cast<uint8_t (*)[VF_BINS][VF_TABLES]>(tieflag + VF_TABLES);
-    const int tb0 = blockIdx.x * VF_TABLES;
-    if (threadIdx.x < VF_TABLES) {
-        const int tb = tb0 + threadIdx.x;
-        s_start[threadIdx.x] = tb < n_tables ? start[tb] : 0;
-        s_len[threadIdx.x] = tb < n_tables ? len[tb] : 0;
-        tieflag[threadIdx.x] = 0;
-    }
-    __syncthreads();
-    int64_t blk_bins = 0;
-    for (int k = 0; k < VF_TABLES; k++) blk_bins = max(blk_bins, s_len[k]);
-    const int nchunk = (int)((blk_bins + VF_BINS - 1) / VF_BINS);
-    // named barriers: 1 + b = chunk in buffer b is normalised (workers arrive, solver syncs);
-    //                 3 + b = chunk in buffer b is solved (solver arrives, workers sync); 5 = workers only
-    if (threadIdx.x >= 32) {
-        // ===== workers =====
-        const int w = threadIdx.x - 32;
-        constexpr int NLD = VF_TABLES * VF_BINS * 3 / VF_WORKERS;
-        // raw likelihoods of the NEXT chunk are fetched (coalesced: 32 tables x 48 doubles) before this chunk's
-        // exp / log work starts, so DRAM latency hides under it
-        double pre[NLD];
-        auto fetch = [&](int c) {
-            const int64_t i0 = (int64_t)c * VF_BINS;
-#pragma unroll
-            for (int k = 0; k < NLD; k++) {
-                const int idx = k * VF_WORKERS + w;
-                const int t = idx / (VF_BINS * 3), d = idx % (VF_BINS * 3);
-                pre[k] = (i0 + d / 3 < s_len[t]) ? __ldcs(lik + (s_start[t] + i0) * 3 + d) : 0.0;
-            }
-        };
-        if (nchunk > 0) fetch(0);
-        for (int c = 0; c <= nchunk; c++) {
-            const int b = c & 1;
-            if (c < nchunk) {
-                const int64_t i0 = (int64_t)c * VF_BINS;
-#pragma unroll
-                for (int k = 0; k < NLD; k++) {
-                    const int idx = k * VF_WORKERS + w;
-                    nrm[b][idx / (VF_BINS * 3)][idx % (VF_BINS * 3)] = pre[k];
-                }
-                if (c + 1 < nchunk) fetch(c + 1);
-                asm volatile("bar.sync 5, %0;" ::"n"(VF_WORKERS) : "memory");
-                // ln nrm in place: 512 bins, 4 per worker
-#pragma unroll
-                for (int k = 0; k < VF_TABLES * VF_BINS / VF_WORKERS; k++) {
-                    const int idx = k * VF_WORKERS + w;
-                    const int t = idx / VF_BINS, i = idx % VF_BINS;
-                    if (i0 + i < s_len[t]) {
-                        const double v[3] = {nrm[b][t][i * 3], nrm[b][t][i * 3 + 1], nrm[b][t][i * 3 + 2]};
-                        double n0, n1, n2;
-                        ln_nrm(v, is_log, n0, n1, n2);
-                        nrm[b][t][i * 3] = n0;
-                        nrm[b][t][i * 3 + 1] = n1;
-                        nrm[b][t][i * 3 + 2] = n2;
-                    }
-                }
-                __threadfence_block();
-                if (b == 0) asm volatile("bar.arrive 1, %0;" ::"n"(VF_THREADS) : "memory");
-                else asm volatile("bar.arrive 2, %0;" ::"n"(VF_THREADS) : "memory");
-            }
-            if (c >= 1) {  // drain the chunk the solver has just finished
-                const int pb = (c - 1) & 1;
-                if (pb == 0) asm volatile("bar.sync 3, %0;" ::"n"(VF_THREADS) : "memory");
-                else asm volatile("bar.sync 4, %0;" ::"n"(VF_THREADS) : "memory");
-                const int64_t i0 = (int64_t)(c - 1) * VF_BINS;
-                // Near-tie and long-double-range tests, moved off the solver's critical path: with the scores of bin
-                // i - 1 and ln nrm of bin i both still in shared memory, every bin's nine candidates can be rebuilt
-                // independently (the same expressions, hence the same doubles) — 512 bins over 256 workers.
-#pragma unroll
-                for (int k = 0; k < VF_TABLES * VF_BINS / VF_WORKERS; k++) {
-                    const int idx = k * VF_WORKERS + w;
-                    const int t = idx / VF_BINS, i = idx % VF_BINS;
-                    const int64_t gi = i0 + i;
-                    if (gi < s_len[t]) {
-                        const double *cur = &sco[pb][t][i * 3];
-                        bool tie = !is_log && below_ldbl(cur[0], cur[1], cur[2]);
-                        if (gi > 0) {
-                            const double *pv = i > 0 ? &sco[pb][t][(i - 1) * 3] : &prevlast[pb ^ 1][t][0];
-                            const double p0 = pv[0], p1 = pv[1], p2 = pv[2];
-                            const double n0 = nrm[pb][t][i * 3], n1 = nrm[pb][t][i * 3 + 1], n2 = nrm[pb][t][i * 3 + 2];
-                            const double ts = tie_scale(gi);
-                            const double a0 = p0 + n0, a1 = (p1 + n0) + lp01, a2 = (p2 + n0) + lp02;
-                            const double b0 = (p0 + n1) + lp01, b1 = p1 + n1, b2 = (p2 + n1) + lp12;
-                            const double c0 = (p0 + n2) + lp02, c1 = (p1 + n2) + lp12, c2 = p2 + n2;
-                            tie |= near_tie(a0, a1, a2, argmax3(a0, a1, a2), ts) | near_tie(b0, b1, b2, argmax3(b0, b1, b2), ts) |
-                                   near_tie(c0, c1, c2, argmax3(c0, c1, c2), ts);
-                        }
-                        if (tie) tieflag[t] = 1;
-                        if (i == VF_BINS - 1) { prevlast[pb][t][0] = cur[0]; prevlast[pb][t][1] = cur[1]; prevlast[pb][t][2] = cur[2]; }
-                    }
-                }
-#pragma unroll
-                for (int k = 0; k < VF_TABLES * VF_BINS * 3 / VF_WORKERS; k++) {
-                    const int idx = k * VF_WORKERS + w;
-                    const int t = idx / (VF_BINS * 3), d = idx % (VF_BINS * 3);
-                    if (i0 + d / 3 < s_len[t]) __stcs(score + (s_start[t] + i0) * 3 + d, sco[pb][t][d]);
-                }
-#pragma unroll
-                for (int k = 0; k < VF_TABLES * VF_BINS / VF_WORKERS; k++) {
-                    const int idx = k * VF_WORKERS + w;
-                    const int i = idx / VF_TABLES, t = idx % VF_TABLES;
-                    if (tb0 + t < n_tables && i0 + i < s_len[t]) fromT[(size_t)(i0 + i) * n_tables + tb0 + t] = frm[pb][i][t];
-                }
-                asm volatile("bar.sync 5, %0;" ::"n"(VF_WORKERS) : "memory");  // buffer pb is free for chunk c + 1
-            }
-        }
-    } else {
-        // ===== solver: lane = table.  A single warp walks the bins, so its time is (instructions per bin) x (issue
-        // latency): the step is branch-free and starts from s = 0, which makes bin 0 an ordinary step (the diagonal
-        // candidate wins there, s_k = ln nrm_k exactly; its back-pointers are never followed). =====
-        const int lane = threadIdx.x;
-        const int64_t n = s_len[lane];
-        double s0 = 0, s1 = 0, s2 = 0;
-        for (int c = 0; c < nchunk; c++) {
-            const int b = c & 1;
-            if (b == 0) asm volatile("bar.sync 1, %0;" ::"n"(VF_THREADS) : "memory");
-            else asm volatile("bar.sync 2, %0;" ::"n"(VF_THREADS) : "memory");
-            const int64_t i0 = (int64_t)c * VF_BINS;
-            const double *nr = &nrm[b][lane][0];
-            double *so = &sco[b][lane][0];
-            const int nq = (int)min((int64_t)VF_BINS, n - i0);  // bins of this table in the chunk (<= 0: none)
-#pragma unroll 4
-            for (int q = 0; q < VF_BINS; q++) {
-                const double n0 = nr[q * 3], n1 = nr[q * 3 + 1], n2 = nr[q * 3 + 2];
-                // candidates (prev_k + ln nrm_s) + ln pen(k, s); strict '>' arg-max: lowest index wins, NaN never wins
-                const double a0 = s0 + n0, a1 = (s1 + n0) + lp01, a2 = (s2 + n0) + lp02;
-                const double b0 = (s0 + n1) + lp01, b1 = s1 + n1, b2 = (s2 + n1) + lp12;
-                const double c0 = (s0 + n2) + lp02, c1 = (s1 + n2) + lp12, c2 = s2 + n2;
-                const bool ga = a1 > a0, gb = b1 > b0, gc = c1 > c0;
-                const double ma = ga ? a1 : a0, mb = gb ? b1 : b0, mc = gc ? c1 : c0;
-                const bool ha = a2 > ma, hb = b2 > mb, hc = c2 > mc;
-                const bool live = q < nq;
-                s0 = live ? (ha ? a2 : ma) : s0;
-                s1 = live ? (hb ? b2 : mb) : s1;
-                s2 = live ? (hc ? c2 : mc) : s2;
-                so[q * 3] = s0;
-                so[q * 3 + 1] = s1;
-                so[q * 3 + 2] = s2;
-                frm[b][q][lane] = (uint8_t)((ha ? 2 : (int)ga) | ((hb ? 2 : (int)gb) << 2) | ((hc ? 2 : (int)gc) << 4));
-            }
-            __threadfence_block();
-            if (b == 0) asm volatile("bar.arrive 3, %0;" ::"n"(VF_THREADS) : "memory");
-            else asm volatile("bar.arrive 4, %0;" ::"n"(VF_THREADS) : "memory");
-        }
-        const int tb = tb0 + lane;
-        if (tb < n_tables) {
-            last[(size_t)tb * 3 + 0] = s0;
-            last[(size_t)tb * 3 + 1] = s1;
-            last[(size_t)tb * 3 + 2] = s2;
-        }
-    }
-    __syncthreads();  // the workers' last drain has set the tie flags
-    if (threadIdx.x < VF_TABLES) {
-        const int tb = tb0 + threadIdx.x;
-        if (tb < n_tables) {
-            const int64_t n = s_len[threadIdx.x];
-            bool tie = tieflag[threadIdx.x] != 0;
-            if (n > 0) {
-                const double l0 = last[(size_t)tb * 3], l1 = last[(size_t)tb * 3 + 1], l2 = last[(size_t)tb * 3 + 2];
-                tie |= near_tie(l0, l1, l2, argmax3(l0, l1, l2), n);
-            }
-            flag[tb] = tie ? 1 : 0;
-        }
-    }
 }
 
 // states of the back-trace (bin-major) -> the caller's table-major layout
@@ -591,48 +423,22 @@ int viterbi_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, int64_t t
     if (batched) {
         double *d_last;
         uint8_t *d_fromT;
-        const size_t cells = (size_t)maxbins * n_tables;
-        static const int fused_env = [] { const char *s = getenv("IBDGEM_VITERBI_FUSED"); return s ? atoi(s) : 1; }();
-        // the fused kernel starts from s = 0 and treats bin 0 as an ordinary step, which is the reference's bin 0 only
-        // while no switch is rewarded (penalties <= 1)
-        const bool fused = fused_env && p01 <= 1.0 && p02 <= 1.0 && p12 <= 1.0;
-        if (scratch(e, SC_HG_FROMT, cells, (void **)&d_fromT) || scratch(e, SC_HG_LAST, (size_t)n_tables * 24, (void **)&d_last)) return 1;
-        const dim3 tiles((unsigned)((n_tables + 31) / 32), (unsigned)((maxbins + 31) / 32));
-        if (fused) {
-            {
-                LaunchScope ls(e, K_VITERBI);
-                IBD_CUDA(cudaFuncSetAttribute(viterbi_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, VF_SMEM));
-                viterbi_fused_kernel<<<(n_tables + VF_TABLES - 1) / VF_TABLES, VF_THREADS, VF_SMEM, e->stream>>>(
-                    n_tables, maxbins, d_start, d_len, d_lik, is_log, log(p01), log(p02), log(p12), d_score, d_fromT, d_last, d_flag);
-            }
-            {
-                LaunchScope ls(e, K_VITERBI_BACK);
-                viterbi_back_kernel<<<(n_tables + 63) / 64, 64, 0, e->stream>>>(n_tables, d_len, d_fromT, d_last, d_counts);
-            }
-            {
-                LaunchScope ls(e, K_VITERBI_OUT);
-                viterbi_state_out_kernel<<<tiles, 1024, 0, e->stream>>>(n_tables, d_start, d_len, d_fromT, d_state);
-            }
-        } else {  // the four-kernel pipeline with bin-major intermediates (kept for A/B measurement)
-            double *d_nrmT, *d_scoreT;
-            if (scratch(e, SC_HG_NRMT, cells * 24, (void **)&d_nrmT) || scratch(e, SC_HG_SCORET, cells * 24, (void **)&d_scoreT)) return 1;
-            {
-                LaunchScope ls(e, K_VITERBI_NORM);
-                viterbi_norm_kernel<<<tiles, 1024, 0, e->stream>>>(n_tables, maxbins, d_start, d_len, d_lik, is_log, d_nrmT);
-            }
-            {
-                LaunchScope ls(e, K_VITERBI);
-                viterbi_forward_kernel<<<(n_tables + 63) / 64, 64, 0, e->stream>>>(n_tables, d_len, is_log, d_nrmT, log(p01), log(p02), log(p12),
-                                                                                 d_fromT, d_scoreT, d_last, d_flag);
-            }
-            {
-                LaunchScope ls(e, K_VITERBI_BACK);
-                viterbi_back_kernel<<<(n_tables + 63) / 64, 64, 0, e->stream>>>(n_tables, d_len, d_fromT, d_last, d_counts);
-            }
-            {
-                LaunchScope ls(e, K_VITERBI_OUT);
-                viterbi_out_kernel<<<tiles, 1024, 0, e->stream>>>(n_tables, d_start, d_len, d_fromT, d_scoreT, d_state, d_score);
-            }
+        if (scratch(e, SC_HG_FROMT, (size_t)maxbins * n_tables, (void **)&d_fromT) || scratch(e, SC_HG_LAST, (size_t)n_tables * 24, (void **)&d_last))
+            return 1;
+        {
+            LaunchScope ls(e, K_VITERBI);
+            IBD_CUDA(cudaFuncSetAttribute(viterbi_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, VF_SMEM));
+            viterbi_fused_kernel<<<(n_tables + HG_TABLES - 1) / HG_TABLES, HG_THREADS, VF_SMEM, e->stream>>>(
+                n_tables, d_start, d_len, d_lik, is_log, log(p01), log(p02), log(p12), d_score, d_fromT, d_last, d_flag);
+        }
+        {
+            LaunchScope ls(e, K_VITERBI_BACK);
+            viterbi_back_kernel<<<(n_tables + 63) / 64, 64, 0, e->stream>>>(n_tables, d_len, d_fromT, d_last, d_counts);
+        }
+        {
+            LaunchScope ls(e, K_VITERBI_OUT);
+            const dim3 tiles((unsigned)((n_tables + 31) / 32), (unsigned)((maxbins + 31) / 32));
+            viterbi_state_out_kernel<<<tiles, 1024, 0, e->stream>>>(n_tables, d_start, d_len, d_fromT, d_state);
         }
     } else {
         LaunchScope ls(e, K_VITERBI);
@@ -645,6 +451,26 @@ int viterbi_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, int64_t t
 
 }  // namespace
 
+// Host start / length of every table (stride > 0: table t starts at bin t * table_stride); 1 (error set) on a negative
+// length or one past the stride.
+int ibdgem::table_layout(const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, std::vector<int64_t> *sl,
+                         int64_t *maxbins, int64_t *total) {
+    sl->assign((size_t)n_tables * 2, 0);
+    *maxbins = *total = 0;
+    for (int t = 0; t < n_tables; t++) {
+        const int64_t n = bin_offsets[t + 1] - bin_offsets[t];
+        if (n < 0 || (table_stride > 0 && n > table_stride)) {
+            set_error("[::] ERROR in %s(): table %d has %lld bins (stride %lld).", fn, t, (long long)n, (long long)table_stride);
+            return 1;
+        }
+        (*sl)[(size_t)t] = table_stride > 0 ? (int64_t)t * table_stride : bin_offsets[t];
+        (*sl)[(size_t)n_tables + t] = n;
+        *maxbins = std::max(*maxbins, n);
+        *total += n;
+    }
+    return 0;
+}
+
 // Host buffers in, host buffers out.  The tables go through in batches: while batch b is scored, batch b + 1 is on its
 // way up and the results of batch b - 1 on their way down (three streams; page-locked buffers make the copies
 // asynchronous, pageable ones are simply staged by the driver).
@@ -656,6 +482,9 @@ extern "C" int hiddengem_viterbi_batch(ibdgem_engine *e, int32_t n_tables, const
         set_error("[::] ERROR in hiddengem_viterbi_batch(): bad arguments.");
         return 1;
     }
+    std::vector<int64_t> h_sl;
+    int64_t maxbins_all, total;
+    if (table_layout("hiddengem_viterbi_batch", n_tables, bin_offsets, 0, &h_sl, &maxbins_all, &total)) return 1;
     IBD_CUDA(cudaSetDevice(e->device));
     const int64_t nb = bin_offsets[n_tables];
     if (nb <= 0) {
@@ -672,11 +501,6 @@ extern "C" int hiddengem_viterbi_batch(ibdgem_engine *e, int32_t n_tables, const
         return 1;
     d_flag = d_state + nb;
     int64_t *d_len = d_start + n_tables;
-    std::vector<int64_t> h_sl((size_t)n_tables * 2);
-    for (int t = 0; t < n_tables; t++) {
-        h_sl[(size_t)t] = bin_offsets[t];
-        h_sl[(size_t)n_tables + t] = bin_offsets[t + 1] - bin_offsets[t];
-    }
     if (!e->copy_stream) {
         IBD_CUDA(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
         IBD_CUDA(cudaEventCreateWithFlags(&e->ev_order, cudaEventDisableTiming));
@@ -798,19 +622,9 @@ extern "C" int hiddengem_viterbi_batch_device(ibdgem_engine *e, int32_t n_tables
         return 1;
     }
     IBD_CUDA(cudaSetDevice(e->device));
-    std::vector<int64_t> h_sl((size_t)n_tables * 2);
-    int64_t maxbins = 0, total = 0;
-    for (int t = 0; t < n_tables; t++) {
-        const int64_t n = bin_offsets[t + 1] - bin_offsets[t];
-        if (n < 0 || (table_stride > 0 && n > table_stride)) {
-            set_error("[::] ERROR in hiddengem_viterbi_batch_device(): table %d has %lld bins (stride %lld).", t, (long long)n, (long long)table_stride);
-            return 1;
-        }
-        h_sl[(size_t)t] = table_stride > 0 ? (int64_t)t * table_stride : bin_offsets[t];
-        h_sl[(size_t)n_tables + t] = n;
-        maxbins = std::max(maxbins, n);
-        total += n;
-    }
+    std::vector<int64_t> h_sl;
+    int64_t maxbins, total;
+    if (table_layout("hiddengem_viterbi_batch_device", n_tables, bin_offsets, table_stride, &h_sl, &maxbins, &total)) return 1;
     if (total <= 0) {
         set_error("[::] ERROR parsing likelihood data; make sure input is valid.");
         return 1;

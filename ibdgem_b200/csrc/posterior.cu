@@ -14,9 +14,9 @@
 // entries.  Those calls run the same two kernels in natural-log arithmetic (LG = true: log-sum-exp mixing, rows
 // shifted to maximum 0), which has no range limit; they cost more fp64 work on the solver lane.
 //
-// Two kernels, each the structure of viterbi_fused_kernel: a block takes 32 tables, worker warps stage 16-bin chunks
-// with coalesced loads and compute the emissions in shared memory, ONE solver warp (lane = table) walks the chunk,
-// chunks are double buffered.
+// Two kernels on the chunked block of hg_block.cuh (shared with viterbi_fused_kernel): a block takes 32 tables, worker
+// warps stage 16-bin chunks with coalesced loads and compute the emissions in shared memory, ONE solver warp
+// (lane = table) walks the chunk, chunks are double buffered.
 //   forward   walks the chunks in order and stores only alpha of each chunk's last bin (a checkpoint, 24 B per table
 //             per 16 bins);
 //   backward  walks the chunks in reverse; per chunk the solver recomputes alpha from the previous chunk's checkpoint
@@ -41,17 +41,14 @@
 #include <vector>
 
 #include "engine.h"
+#include "hg_block.cuh"
 #include "tc_common.cuh"
 
 namespace ibdgem {
 
-constexpr int PB_TABLES = 32, PB_BINS = 16, PB_ROW = PB_BINS * 3 + 1;  // padded row: lanes hit distinct banks
-constexpr int PB_WORKERS = 256, PB_THREADS = PB_WORKERS + 32;
-constexpr int PB_NLD = PB_TABLES * PB_BINS * 3 / PB_WORKERS;  // doubles of a chunk each worker loads
-constexpr int PB_NBIN = PB_TABLES * PB_BINS / PB_WORKERS;     // bins of a chunk each worker normalises
-constexpr int PB_FWD_SMEM = 2 * PB_TABLES * PB_ROW * 8 + 2 * PB_TABLES * 8;
-constexpr int PB_BWD_SMEM = 4 * PB_TABLES * PB_ROW * 8 + 2 * PB_TABLES * 8 + PB_TABLES * 4;
-static_assert(PB_TABLES * PB_BINS * 3 <= PB_TABLES * PB_ROW, "expected-count partials fit in one staging buffer");
+constexpr int PB_FWD_SMEM = 2 * HG_TABLES * HG_ROW * 8 + HG_HEAD_SMEM;
+constexpr int PB_BWD_SMEM = 4 * HG_TABLES * HG_ROW * 8 + HG_HEAD_SMEM + HG_TABLES * 4;
+static_assert(HG_TABLES * HG_BINS * 3 <= HG_TABLES * HG_ROW, "expected-count partials fit in one staging buffer");
 
 // 2^-floor(log2 s) for s >= 0: multiplying by it is exact and brings s into [1, 2) (0 stays 0)
 __device__ __forceinline__ double pow2_recip(double s) {
@@ -196,92 +193,42 @@ __device__ __forceinline__ void gamma(const double *A, const double *B, bool dea
     y2 = g2 * inv;
 }
 
-// Workers: raw likelihoods of chunk c of the block's tables into registers (coalesced: a table's chunk is 384
-// contiguous bytes), rows past a table's end read as 0.
-struct ChunkLoader {
-    const double *lik;
-    const int64_t *s_start, *s_len;
-    int w;
-    __device__ __forceinline__ void fetch(int c, double (&pre)[PB_NLD]) const {
-        const int64_t i0 = (int64_t)c * PB_BINS;
-#pragma unroll
-        for (int k = 0; k < PB_NLD; k++) {
-            const int idx = k * PB_WORKERS + w;
-            const int t = idx / (PB_BINS * 3), d = idx % (PB_BINS * 3);
-            pre[k] = (i0 + d / 3 < s_len[t]) ? __ldcs(lik + (s_start[t] + i0) * 3 + d) : 0.0;
-        }
-    }
-    __device__ __forceinline__ void store(const double (&pre)[PB_NLD], double (*buf)[PB_ROW]) const {
-#pragma unroll
-        for (int k = 0; k < PB_NLD; k++) {
-            const int idx = k * PB_WORKERS + w;
-            buf[idx / (PB_BINS * 3)][idx % (PB_BINS * 3)] = pre[k];
-        }
-    }
-    // emissions of chunk c in place, once every worker has stored its part (workers' barrier)
-    template <bool LG>
-    __device__ __forceinline__ void emit(int c, double (*buf)[PB_ROW], int is_log) const {
-        asm volatile("bar.sync 5, %0;" ::"n"(PB_WORKERS) : "memory");
-        const int64_t i0 = (int64_t)c * PB_BINS;
+// Workers: emissions of chunk c in place, once every worker has stored its part
+template <bool LG>
+__device__ __forceinline__ void emit(const ChunkLoader &ld, int c, double (*buf)[HG_ROW], int is_log) {
+    sync_workers();
+    const int64_t i0 = (int64_t)c * HG_BINS;
 #pragma unroll 1  // unrolled, the two bins need more registers than three blocks per SM leave
-        for (int k = 0; k < PB_NBIN; k++) {
-            const int idx = k * PB_WORKERS + w;
-            const int t = idx / PB_BINS, i = idx % PB_BINS;
-            if (i0 + i < s_len[t]) emission<LG>(&buf[t][i * 3], is_log);
-        }
-        __threadfence_block();
+    for (int k = 0; k < HG_NBIN; k++) {
+        const int idx = k * HG_WORKERS + ld.w;
+        const int t = idx / HG_BINS, i = idx % HG_BINS;
+        if (i0 + i < ld.s_len[t]) emission<LG>(&buf[t][i * 3], is_log);
     }
-};
-
-// Named barriers: 1 + b = chunk in buffer b has its emissions (workers arrive, solver syncs);
-//                 3 + b = chunk in buffer b is solved (solver arrives, workers sync); 5 = workers only.
-__device__ __forceinline__ void arrive_ready(int b) {
-    if (b == 0) asm volatile("bar.arrive 1, %0;" ::"n"(PB_THREADS) : "memory");
-    else asm volatile("bar.arrive 2, %0;" ::"n"(PB_THREADS) : "memory");
-}
-__device__ __forceinline__ void sync_ready(int b) {
-    if (b == 0) asm volatile("bar.sync 1, %0;" ::"n"(PB_THREADS) : "memory");
-    else asm volatile("bar.sync 2, %0;" ::"n"(PB_THREADS) : "memory");
-}
-__device__ __forceinline__ void arrive_solved(int b) {
-    if (b == 0) asm volatile("bar.arrive 3, %0;" ::"n"(PB_THREADS) : "memory");
-    else asm volatile("bar.arrive 4, %0;" ::"n"(PB_THREADS) : "memory");
-}
-__device__ __forceinline__ void sync_solved(int b) {
-    if (b == 0) asm volatile("bar.sync 3, %0;" ::"n"(PB_THREADS) : "memory");
-    else asm volatile("bar.sync 4, %0;" ::"n"(PB_THREADS) : "memory");
+    __threadfence_block();
 }
 
 // Forward pass: alpha of each chunk's last bin -> ckpt[chunk][n_tables][3]; 0 in expected[t][0] exactly when the
 // table's total weight is 0 (a positive value otherwise).
 template <bool LG>
-__global__ void __launch_bounds__(PB_THREADS, 3)
+__global__ void __launch_bounds__(HG_THREADS, 3)
 posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
                      int is_log, double p01, double p02, double p12, double *__restrict__ ckpt, double *__restrict__ expected) {
     extern __shared__ double pb_smem[];
-    double (*em)[PB_TABLES][PB_ROW] = reinterpret_cast<double (*)[PB_TABLES][PB_ROW]>(pb_smem);
-    int64_t *s_start = reinterpret_cast<int64_t *>(pb_smem + 2 * PB_TABLES * PB_ROW), *s_len = s_start + PB_TABLES;
-    const int tb0 = blockIdx.x * PB_TABLES;
-    if (threadIdx.x < PB_TABLES) {
-        const int tb = tb0 + threadIdx.x;
-        s_start[threadIdx.x] = tb < n_tables ? start[tb] : 0;
-        s_len[threadIdx.x] = tb < n_tables ? len[tb] : 0;
-    }
-    __syncthreads();
-    int64_t blk_bins = 0;
-    for (int k = 0; k < PB_TABLES; k++) blk_bins = max(blk_bins, s_len[k]);
-    const int nchunk = (int)((blk_bins + PB_BINS - 1) / PB_BINS);
+    double (*em)[HG_TABLES][HG_ROW] = reinterpret_cast<double (*)[HG_TABLES][HG_ROW]>(pb_smem);
+    int64_t *s_start = reinterpret_cast<int64_t *>(pb_smem + 2 * HG_TABLES * HG_ROW), *s_len = s_start + HG_TABLES;
+    const int tb0 = blockIdx.x * HG_TABLES;
+    const int nchunk = block_tables(n_tables, start, len, s_start, s_len);
     if (threadIdx.x >= 32) {
-        const ChunkLoader ld{lik, s_start, s_len, (int)threadIdx.x - 32};
-        double pre[PB_NLD];
-        if (nchunk > 0) ld.fetch(0, pre);
+        const ChunkLoader ld{s_start, s_len, (int)threadIdx.x - 32};
+        double pre[HG_NLD];
+        if (nchunk > 0) ld.fetch(lik, 0, pre);
         for (int c = 0; c <= nchunk; c++) {
             if (c < nchunk) {
                 const int b = c & 1;
                 if (c >= 2) sync_solved(b);  // the solver is done with chunk c - 2 in this buffer
                 ld.store(pre, em[b]);
-                if (c + 1 < nchunk) ld.fetch(c + 1, pre);  // in flight under this chunk's work
-                ld.template emit<LG>(c, em[b], is_log);
+                if (c + 1 < nchunk) ld.fetch(lik, c + 1, pre);  // in flight under this chunk's work
+                emit<LG>(ld, c, em[b], is_log);
                 arrive_ready(b);
             } else {
                 for (int k = max(0, nchunk - 2); k < nchunk; k++) sync_solved(k & 1);  // every arrival is consumed
@@ -296,10 +243,10 @@ posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
         for (int c = 0; c < nchunk; c++) {
             const int b = c & 1;
             sync_ready(b);
-            const int64_t i0 = (int64_t)c * PB_BINS;
+            const int64_t i0 = (int64_t)c * HG_BINS;
             const double *nr = &em[b][lane][0];
 #pragma unroll 4
-            for (int q = 0; q < PB_BINS; q++)
+            for (int q = 0; q < HG_BINS; q++)
                 fwd_step<LG>(a0, a1, a2, nr[q * 3], nr[q * 3 + 1], nr[q * 3 + 2], i0 + q == 0, i0 + q < n, p01, p02, p12);
             if (tb < n_tables) {
                 double *o = ckpt + ((size_t)c * n_tables + tb) * 3;
@@ -314,49 +261,43 @@ posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
 
 // Backward pass: gamma -> posterior (the caller's layout), expected occupancy -> expected[t][3].
 template <bool LG>
-__global__ void __launch_bounds__(PB_THREADS, 3)
+__global__ void __launch_bounds__(HG_THREADS, 3)
 posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
                      int is_log, double p01, double p02, double p12, const double *__restrict__ ckpt, double *__restrict__ posterior,
                      double *__restrict__ expected) {
     extern __shared__ double pb_smem[];
-    double (*em)[PB_TABLES][PB_ROW] = reinterpret_cast<double (*)[PB_TABLES][PB_ROW]>(pb_smem);  // emissions, then beta
-    double (*al)[PB_TABLES][PB_ROW] = reinterpret_cast<double (*)[PB_TABLES][PB_ROW]>(pb_smem + 2 * PB_TABLES * PB_ROW);
-    int64_t *s_start = reinterpret_cast<int64_t *>(pb_smem + 4 * PB_TABLES * PB_ROW), *s_len = s_start + PB_TABLES;
-    int *s_dead = reinterpret_cast<int *>(s_len + PB_TABLES);
-    const int tb0 = blockIdx.x * PB_TABLES;
-    if (threadIdx.x < PB_TABLES) {
+    double (*em)[HG_TABLES][HG_ROW] = reinterpret_cast<double (*)[HG_TABLES][HG_ROW]>(pb_smem);  // emissions, then beta
+    double (*al)[HG_TABLES][HG_ROW] = reinterpret_cast<double (*)[HG_TABLES][HG_ROW]>(pb_smem + 2 * HG_TABLES * HG_ROW);
+    int64_t *s_start = reinterpret_cast<int64_t *>(pb_smem + 4 * HG_TABLES * HG_ROW), *s_len = s_start + HG_TABLES;
+    int *s_dead = reinterpret_cast<int *>(s_len + HG_TABLES);
+    const int tb0 = blockIdx.x * HG_TABLES;
+    if (threadIdx.x < HG_TABLES) {
         const int tb = tb0 + threadIdx.x;
-        const int64_t n = tb < n_tables ? len[tb] : 0;
-        s_start[threadIdx.x] = tb < n_tables ? start[tb] : 0;
-        s_len[threadIdx.x] = n;
-        s_dead[threadIdx.x] = n > 0 && !(expected[(size_t)tb * 3] > 0);  // total weight 0
+        s_dead[threadIdx.x] = tb < n_tables && len[tb] > 0 && !(expected[(size_t)tb * 3] > 0);  // total weight 0
     }
-    __syncthreads();
-    int64_t blk_bins = 0;
-    for (int k = 0; k < PB_TABLES; k++) blk_bins = max(blk_bins, s_len[k]);
-    const int nchunk = (int)((blk_bins + PB_BINS - 1) / PB_BINS);
+    const int nchunk = block_tables(n_tables, start, len, s_start, s_len);
     const int w = (int)threadIdx.x - 32;
-    double E[PB_NBIN][3] = {};  // a worker's share of the expected counts: the same (table, bin slot) every chunk
+    double E[HG_NBIN][3] = {};  // a worker's share of the expected counts: the same (table, bin slot) every chunk
     if (threadIdx.x >= 32) {
-        const ChunkLoader ld{lik, s_start, s_len, w};
-        double pre[PB_NLD];
-        if (nchunk > 0) ld.fetch(nchunk - 1, pre);
+        const ChunkLoader ld{s_start, s_len, w};
+        double pre[HG_NLD];
+        if (nchunk > 0) ld.fetch(lik, nchunk - 1, pre);
         for (int r = 0; r <= nchunk; r++) {  // r-th chunk from the end
             if (r < nchunk) {
                 const int c = nchunk - 1 - r, b = r & 1;
                 ld.store(pre, em[b]);
-                if (c >= 1) ld.fetch(c - 1, pre);  // in flight under this chunk's work
-                ld.template emit<LG>(c, em[b], is_log);
+                if (c >= 1) ld.fetch(lik, c - 1, pre);  // in flight under this chunk's work
+                emit<LG>(ld, c, em[b], is_log);
                 arrive_ready(b);
             }
             if (r >= 1) {  // gamma of the chunk the solver has just finished
                 const int c = nchunk - r, pb = (r - 1) & 1;
                 sync_solved(pb);
-                const int64_t i0 = (int64_t)c * PB_BINS;
+                const int64_t i0 = (int64_t)c * HG_BINS;
 #pragma unroll
-                for (int k = 0; k < PB_NBIN; k++) {
-                    const int idx = k * PB_WORKERS + w;
-                    const int t = idx / PB_BINS, i = idx % PB_BINS;
+                for (int k = 0; k < HG_NBIN; k++) {
+                    const int idx = k * HG_WORKERS + w;
+                    const int t = idx / HG_BINS, i = idx % HG_BINS;
                     if (i0 + i < s_len[t]) {
                         double y0, y1, y2;
                         gamma<LG>(&al[pb][t][i * 3], &em[pb][t][i * 3], s_dead[t], y0, y1, y2);
@@ -369,7 +310,7 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                         E[k][2] += y2;
                     }
                 }
-                asm volatile("bar.sync 5, %0;" ::"n"(PB_WORKERS) : "memory");  // buffer pb is free for the next chunk
+                sync_workers();  // buffer pb is free for the next chunk
             }
         }
     } else {
@@ -386,16 +327,16 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                 a0 = ck[0]; a1 = ck[1]; a2 = ck[2];
             }
             sync_ready(b);
-            const int64_t i0 = (int64_t)c * PB_BINS;
+            const int64_t i0 = (int64_t)c * HG_BINS;
             double *nr = &em[b][lane][0], *ao = &al[b][lane][0];
 #pragma unroll 4
-            for (int q = 0; q < PB_BINS; q++) {
+            for (int q = 0; q < HG_BINS; q++) {
                 fwd_step<LG>(a0, a1, a2, nr[q * 3], nr[q * 3 + 1], nr[q * 3 + 2], i0 + q == 0, i0 + q < n, p01, p02, p12);
                 ao[q * 3] = a0; ao[q * 3 + 1] = a1; ao[q * 3 + 2] = a2;
             }
             // beta down the chunk: the slot of bin i trades its emission for beta[i], then beta[i - 1]
 #pragma unroll 4
-            for (int q = PB_BINS - 1; q >= 0; q--) {
+            for (int q = HG_BINS - 1; q >= 0; q--) {
                 const double e0 = nr[q * 3], e1 = nr[q * 3 + 1], e2 = nr[q * 3 + 2];
                 nr[q * 3] = b0; nr[q * 3 + 1] = b1; nr[q * 3 + 2] = b2;
                 bwd_step<LG>(b0, b1, b2, e0, e1, e2, i0 + q < n, p01, p02, p12);
@@ -406,23 +347,23 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
     }
     __syncthreads();
     // expected[t] = the 16 bin slots' partial sums of table t, added in a fixed order (reproducible)
-    double *part = &em[0][0][0];  // [PB_TABLES][PB_BINS][3]
+    double *part = &em[0][0][0];  // [HG_TABLES][HG_BINS][3]
     if (threadIdx.x >= 32) {
 #pragma unroll
-        for (int k = 0; k < PB_NBIN; k++) {
-            const int idx = k * PB_WORKERS + w;
-            const int t = idx / PB_BINS, i = idx % PB_BINS;
+        for (int k = 0; k < HG_NBIN; k++) {
+            const int idx = k * HG_WORKERS + w;
+            const int t = idx / HG_BINS, i = idx % HG_BINS;
 #pragma unroll
-            for (int s = 0; s < 3; s++) part[(t * PB_BINS + i) * 3 + s] = E[k][s];
+            for (int s = 0; s < 3; s++) part[(t * HG_BINS + i) * 3 + s] = E[k][s];
         }
     }
     __syncthreads();
-    if (threadIdx.x < PB_TABLES) {
+    if (threadIdx.x < HG_TABLES) {
         const int tb = tb0 + threadIdx.x;
         if (tb < n_tables) {
             double x[3] = {0, 0, 0};
-            for (int i = 0; i < PB_BINS; i++)
-                for (int s = 0; s < 3; s++) x[s] += part[(threadIdx.x * PB_BINS + i) * 3 + s];
+            for (int i = 0; i < HG_BINS; i++)
+                for (int s = 0; s < 3; s++) x[s] += part[(threadIdx.x * HG_BINS + i) * 3 + s];
             const double nan = __longlong_as_double(0x7ff8000000000000LL);
             for (int s = 0; s < 3; s++) expected[(size_t)tb * 3 + s] = s_dead[threadIdx.x] ? nan : x[s];
         }
@@ -455,24 +396,24 @@ bool linear_penalties(double p01, double p02, double p12) {
 // One batch of tables, everything in device memory (start / len per table); kernels only, no host synchronisation.
 int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
                         int is_log, double p01, double p02, double p12, double *d_post, double *d_expected) {
-    const int64_t nck = (maxbins + PB_BINS - 1) / PB_BINS;
+    const int64_t nck = (maxbins + HG_BINS - 1) / HG_BINS;
     if (nck == 0) {  // only empty tables: no bins, expected occupancy 0
         IBD_CUDA(cudaMemsetAsync(d_expected, 0, (size_t)n_tables * 24, e->stream));
         return 0;
     }
     double *d_ckpt;
     if (scratch(e, SC_HG_CKPT, (size_t)nck * n_tables * 24, (void **)&d_ckpt)) return 1;
-    const unsigned grid = (unsigned)((n_tables + PB_TABLES - 1) / PB_TABLES);
+    const unsigned grid = (unsigned)((n_tables + HG_TABLES - 1) / HG_TABLES);
     if (linear_penalties(p01, p02, p12)) {
         {
             LaunchScope ls(e, K_POSTERIOR_FWD);
-            posterior_fwd_kernel<false><<<grid, PB_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
+            posterior_fwd_kernel<false><<<grid, HG_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
                                                                                       d_ckpt, d_expected);
         }
         {
             LaunchScope ls(e, K_POSTERIOR_BWD);
             IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
-            posterior_bwd_kernel<false><<<grid, PB_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
+            posterior_bwd_kernel<false><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
                                                                                       d_ckpt, d_post, d_expected);
         }
     } else {
@@ -480,37 +421,18 @@ int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const i
         {
             LaunchScope ls(e, K_POSTERIOR_FWD);
             e->k_launches[K_POSTERIOR_FWD_LOG]++;
-            posterior_fwd_kernel<true><<<grid, PB_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
+            posterior_fwd_kernel<true><<<grid, HG_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
                                                                                      d_ckpt, d_expected);
         }
         {
             LaunchScope ls(e, K_POSTERIOR_BWD);
             e->k_launches[K_POSTERIOR_BWD_LOG]++;
             IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
-            posterior_bwd_kernel<true><<<grid, PB_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
+            posterior_bwd_kernel<true><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
                                                                                      d_ckpt, d_post, d_expected);
         }
     }
     IBD_CUDA(cudaGetLastError());
-    return 0;
-}
-
-// host start / length of every table; 1 (error set) on a negative length or one past the stride
-int table_layout(const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, std::vector<int64_t> *sl, int64_t *maxbins,
-                 int64_t *total) {
-    sl->assign((size_t)n_tables * 2, 0);
-    *maxbins = *total = 0;
-    for (int t = 0; t < n_tables; t++) {
-        const int64_t n = bin_offsets[t + 1] - bin_offsets[t];
-        if (n < 0 || (table_stride > 0 && n > table_stride)) {
-            set_error("[::] ERROR in %s(): table %d has %lld bins (stride %lld).", fn, t, (long long)n, (long long)table_stride);
-            return 1;
-        }
-        (*sl)[(size_t)t] = table_stride > 0 ? (int64_t)t * table_stride : bin_offsets[t];
-        (*sl)[(size_t)n_tables + t] = n;
-        *maxbins = std::max(*maxbins, n);
-        *total += n;
-    }
     return 0;
 }
 

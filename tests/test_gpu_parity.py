@@ -195,7 +195,7 @@ def test_hiddengem_vs_oracle_and_reference(golden_dir):
         tables.append(l)
         offs.append(offs[-1] + n)
     lik = np.concatenate(tables)
-    for pen in ((1e-3, 1e-6, 1e-3), (0.2, 0.05, 0.3)):
+    for pen in ((1e-3, 1e-6, 1e-3), (0.2, 0.05, 0.3), (2.0, 0.5, 4.0)):
         with ib.Engine(ib.Params()) as e:
             state, score, counts = e.viterbi_batch(lik, offs, False, *pen)
         for i, l in enumerate(tables):
@@ -278,10 +278,9 @@ def test_c3_full_size_spot_checks_against_oracle():
 
 @pytest.mark.parametrize("ragged", [False, True])
 def test_hiddengem_batched_pipeline_vs_oracle(ragged):
-    """>= 64 tables of similar lengths take the batched path (the fused kernel; the four-kernel pipeline only under
-    IBDGEM_VITERBI_FUSED=0, see test_hiddengem_edges_gpu.py); states must be
-    bit-exact and scores within 1e-7 of the per-table oracle, for equal-length and ragged batches,
-    with zero and all-zero (NaN) rows."""
+    """>= 64 tables of similar lengths take the batched path (viterbi_fused_kernel, back-trace, state transpose);
+    states must be bit-exact and scores within 1e-7 of the per-table oracle, for equal-length and ragged batches,
+    with zero and all-zero (NaN) rows, at penalties below 1 and at penalties above 1 that reward a switch."""
     import ibdgem_b200 as ib
     import oracle
     rng = np.random.default_rng(12)
@@ -299,7 +298,7 @@ def test_hiddengem_batched_pipeline_vs_oracle(ragged):
         tables.append(l)
         offs.append(offs[-1] + int(n))
     lik = np.concatenate(tables)
-    for pen in ((1e-3, 1e-6, 1e-3), (0.2, 0.05, 0.3)):
+    for pen in ((1e-3, 1e-6, 1e-3), (0.2, 0.05, 0.3), (2.0, 0.5, 4.0)):
         with ib.Engine(ib.Params()) as e:
             state, score, counts = e.viterbi_batch(lik, offs, False, *pen)
             stats = e.kernel_stats()
