@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -60,6 +61,8 @@ enum KernelId {
     K_POSTERIOR_BWD,    // hiddengem posterior: backward pass, posteriors + expected occupancy
     K_POSTERIOR_FWD_LOG,  // of the posterior_fwd / _bwd launches, those in natural-log arithmetic (zero or widely
     K_POSTERIOR_BWD_LOG,  // spread penalties); counted only, their time is in posterior_fwd / _bwd
+    K_TRACT_COUNT,      // hiddengem tracts: runs of equal state per table, state bytes checked
+    K_TRACT_EMIT,       // hiddengem tracts: one 64-byte record per run (likelihood sums, posterior mean / minimum)
     K_COUNT
 };
 
@@ -170,6 +173,7 @@ struct ibdgem_engine {
     bool t0_set = false;
 
     int64_t hg_flagged = 0;  // tables of the last hiddengem call re-evaluated on the host (near-tie guard)
+    int64_t hg_tracts = -1;  // records in SC_HG_TRACTS from the last tract call; -1: none, or that call failed
     int last_ld_path = -1;
     int force_general = 0;
 };
@@ -197,12 +201,29 @@ enum ScratchSlot {
     SC_WN, SC_WS, SC_WE, SC_COUNTERS, SC_SITE_STATUS, SC_SITE_LIK, SC_LD_PART, SC_NREFPANEL,
     SC_HG_LIK, SC_HG_OFF, SC_HG_STATE, SC_HG_SCORE, SC_HG_COUNTS, SC_HG_FROMT, SC_HG_LAST,
     SC_MMA_TGT, SC_MMA_BG, SC_MMA_ROWLSE, SC_MMA_BGIDX, SC_MMA_MISC, SC_MMA_UNIT,
-    SC_WLIN, SC_WLL_PACK, SC_V_KS, SC_V_KE, SC_V_TWBASE, SC_V_TWI, SC_V_TWD, SC_V_ORDER, SC_V_HIST, SC_V_TILES, SC_V_MISC, SC_HG_CKPT, SC_SLOTS
+    SC_WLIN, SC_WLL_PACK, SC_V_KS, SC_V_KE, SC_V_TWBASE, SC_V_TWI, SC_V_TWD, SC_V_ORDER, SC_V_HIST, SC_V_TILES, SC_V_MISC, SC_HG_CKPT,
+    SC_HG_TRACTS,  // the tract records of the last tract call (hiddengem_last_tracts); nothing else writes it
+    SC_HG_TOFF, SC_SLOTS
 };
 int scratch(ibdgem_engine *e, int slot, size_t bytes, void **out);
 // hiddengem: host start / length of every table of a call (hidden.cu; the Viterbi and posterior entries)
 int table_layout(const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, std::vector<int64_t> *sl, int64_t *maxbins,
                  int64_t *total);
+// Viterbi kernels for one batch of tables in device memory (hidden.cu); no host synchronisation.  d_flag[t] = 1 marks
+// a table the near-tie guard hands to the host.
+int viterbi_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, int64_t total_bins, const int64_t *d_start, const int64_t *d_len,
+                      const double *d_lik, int is_log, double p01, double p02, double p12, uint8_t *d_state, double *d_score,
+                      long long *d_counts, uint8_t *d_flag);
+// The flagged tables, table t = flagged[k] at host lik + bin_offsets[t] * 3, re-evaluated in long double on a few host
+// threads; sink(k, t, state, score_log, counts) receives each result (concurrently, one call per k).
+void viterbi_redo_flagged(const std::vector<int> &flagged, const int64_t *bin_offsets, const double *lik, int is_log, double p01,
+                          double p02, double p12,
+                          const std::function<void(size_t, int, const uint8_t *, const double *, const int64_t *)> &sink);
+// posterior.cu: penalty check of the posterior entries (1 and the error set when rejected), and its kernels for one
+// batch of tables in device memory (no host synchronisation)
+bool bad_penalties(const char *fn, double p01, double p02, double p12);
+int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
+                        int is_log, double p01, double p02, double p12, double *d_post, double *d_expected);
 
 // Makes the engine stream wait for the panel chunks that cover sites [0, s_end); ensure_table also
 // runs site_table on the part of [0, s_end) it has not covered yet.

@@ -414,9 +414,11 @@ void viterbi_long_double(const double *lik, int64_t n, int is_log, double p01, d
     }
 }
 
+}  // namespace
+
 // One batch of tables, everything in device memory.  start / len describe where each table's bins sit in lik /
 // state / score; counts and flag are per table.  Kernels only (no host synchronisation).
-int viterbi_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, int64_t total_bins, const int64_t *d_start, const int64_t *d_len,
+int ibdgem::viterbi_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, int64_t total_bins, const int64_t *d_start, const int64_t *d_len,
                       const double *d_lik, int is_log, double p01, double p02, double p12, uint8_t *d_state, double *d_score,
                       long long *d_counts, uint8_t *d_flag) {
     const bool batched = n_tables >= 64 && (double)maxbins * n_tables <= 2.0 * (double)total_bins;
@@ -449,7 +451,32 @@ int viterbi_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, int64_t t
     return 0;
 }
 
-}  // namespace
+// Flagged tables: the reference's long double recurrence decides (tables are independent: a few host threads).
+void ibdgem::viterbi_redo_flagged(const std::vector<int> &flagged, const int64_t *bin_offsets, const double *lik, int is_log, double p01,
+                                  double p02, double p12,
+                                  const std::function<void(size_t, int, const uint8_t *, const double *, const int64_t *)> &sink) {
+    auto redo = [&](size_t k0, size_t step) {
+        std::vector<uint8_t> st_tmp;
+        std::vector<double> sc_tmp;
+        for (size_t k = k0; k < flagged.size(); k += step) {
+            const int t = flagged[k];
+            const int64_t b0 = bin_offsets[t], n = bin_offsets[t + 1] - b0;
+            int64_t c[3];
+            st_tmp.resize((size_t)n);
+            sc_tmp.resize((size_t)n * 3);
+            viterbi_long_double(lik + b0 * 3, n, is_log, p01, p02, p12, st_tmp.data(), sc_tmp.data(), c);
+            sink(k, t, st_tmp.data(), sc_tmp.data(), c);
+        }
+    };
+    const size_t nthr = std::max<size_t>(1, std::min<size_t>({flagged.size(), (size_t)16, (size_t)std::thread::hardware_concurrency()}));
+    if (nthr <= 1) {
+        redo(0, 1);
+    } else {
+        std::vector<std::thread> pool;
+        for (size_t k = 0; k < nthr; k++) pool.emplace_back(redo, k, nthr);
+        for (auto &th : pool) th.join();
+    }
+}
 
 // Host start / length of every table (stride > 0: table t starts at bin t * table_stride); 1 (error set) on a negative
 // length or one past the stride.
@@ -567,7 +594,6 @@ extern "C" int hiddengem_viterbi_batch(ibdgem_engine *e, int32_t n_tables, const
     if (rc) return 1;
     IBD_CUDA(cudaGetLastError());
     settle_timers(e);
-    // flagged tables: the reference's long double recurrence decides (tables are independent: a few host threads)
     std::vector<int> flagged;
     for (int t = 0; t < n_tables; t++) {
         if (state_counts) {
@@ -578,33 +604,17 @@ extern "C" int hiddengem_viterbi_batch(ibdgem_engine *e, int32_t n_tables, const
         if (h_flag[(size_t)t]) flagged.push_back(t);
     }
     e->hg_flagged = (int64_t)flagged.size();
-    auto redo = [&](size_t k0, size_t step) {
-        std::vector<uint8_t> st_tmp;
-        std::vector<double> sc_tmp;
-        for (size_t k = k0; k < flagged.size(); k += step) {
-            const int t = flagged[k];
-            const int64_t b0 = bin_offsets[t], n = bin_offsets[t + 1] - b0;
-            int64_t c[3];
-            st_tmp.resize((size_t)n);
-            sc_tmp.resize((size_t)n * 3);
-            viterbi_long_double(lik + b0 * 3, n, is_log, p01, p02, p12, st_tmp.data(), sc_tmp.data(), c);
-            if (state) memcpy(state + b0, st_tmp.data(), (size_t)n);
-            if (score_log) memcpy(score_log + b0 * 3, sc_tmp.data(), (size_t)n * 24);
-            if (state_counts) {
-                state_counts[(size_t)t * 3] = c[0];
-                state_counts[(size_t)t * 3 + 1] = c[1];
-                state_counts[(size_t)t * 3 + 2] = c[2];
-            }
-        }
-    };
-    const size_t nthr = std::max<size_t>(1, std::min<size_t>({flagged.size(), (size_t)16, (size_t)std::thread::hardware_concurrency()}));
-    if (nthr <= 1) {
-        redo(0, 1);
-    } else {
-        std::vector<std::thread> pool;
-        for (size_t k = 0; k < nthr; k++) pool.emplace_back(redo, k, nthr);
-        for (auto &th : pool) th.join();
-    }
+    viterbi_redo_flagged(flagged, bin_offsets, lik, is_log, p01, p02, p12,
+                         [&](size_t, int t, const uint8_t *st, const double *sc, const int64_t *c) {
+                             const int64_t b0 = bin_offsets[t], n = bin_offsets[t + 1] - b0;
+                             if (state) memcpy(state + b0, st, (size_t)n);
+                             if (score_log) memcpy(score_log + b0 * 3, sc, (size_t)n * 24);
+                             if (state_counts) {
+                                 state_counts[(size_t)t * 3] = c[0];
+                                 state_counts[(size_t)t * 3 + 1] = c[1];
+                                 state_counts[(size_t)t * 3 + 2] = c[2];
+                             }
+                         });
     return 0;
 }
 

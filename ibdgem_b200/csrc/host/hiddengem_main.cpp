@@ -4,7 +4,8 @@
 // long-double running products are re-synthesised for printing from their logarithms.
 // Additive: -s may be given several times; the tables are read in parallel, scored in one batch and
 // printed in order (formatted in parallel).  --posterior (additive) also prints each bin's posterior state
-// probabilities (hiddengem_posterior_batch) and the expected state fractions.
+// probabilities (hiddengem_posterior_batch) and the expected state fractions.  --tracts FILE (additive) writes the IBD
+// tracts, maximal runs of one state, to FILE (hiddengem_tracts_batch); stdout is unchanged.
 #include <getopt.h>
 
 #include <cmath>
@@ -33,6 +34,10 @@ void print_help(int code) {
           "--p12  FLOAT             Penalty for switching between states IBD1 and IBD2 (default: 1e-3)\n"
           "--posterior              Also print each segment's posterior probability of every state (columns\n"
           "                            P_IBD0, P_IBD1, P_IBD2) and the expected share of segments per state\n"
+          "--tracts  FILE           Also write the IBD tracts (maximal runs of segments in one state) to FILE: per\n"
+          "                            tract its summary file, state, first and last segment, START, END, number\n"
+          "                            of segments and sites, LOD10 of its state against the next best (and with\n"
+          "                            --posterior the mean and minimum posterior of its state)\n"
           "--help                   Show this help message and exit\n\n"
           "Format of output table is tab-delimited with columns:\n"
           "Segment, IBD0_Score, IBD1_Score, IBD2_Score, Inferred_State\n",
@@ -81,7 +86,13 @@ void parallel_for(size_t n, F fn) {
 }
 
 // init_summary, src/hiddengem.c:51-84: skip leading '#' lines, then every line that parses
-int read_summary(const std::string &fn, std::vector<double> *lik) {
+// (START, END and NUM_SITES of each bin are kept for --tracts)
+struct Summary {
+    std::vector<double> lik;
+    std::vector<uint64_t> start, end;
+    std::vector<int64_t> n_sites;
+};
+int read_summary(const std::string &fn, Summary *sm) {
     LineReader lr;
     if (!lr.open(fn)) return 1;
     const char *line;
@@ -96,9 +107,12 @@ int read_summary(const std::string &fn, std::vector<double> *lik) {
         double l0, l1, l2;
         int n;
         if (sscanf(z.c_str(), "%*s\t%zu\t%zu\t%lf\t%lf\t%lf\t%d", &a, &b, &l0, &l1, &l2, &n) == 6) {
-            lik->push_back(l0);
-            lik->push_back(l1);
-            lik->push_back(l2);
+            sm->lik.push_back(l0);
+            sm->lik.push_back(l1);
+            sm->lik.push_back(l2);
+            sm->start.push_back(a);
+            sm->end.push_back(b);
+            sm->n_sites.push_back(n);
         }
     }
     return 0;
@@ -110,9 +124,11 @@ int main(int argc, char *argv[]) {
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
     std::vector<std::string> files;
     bool posterior = false;
+    const char *tracts_fn = nullptr;
     static struct option longopts[] = {{"summary", required_argument, 0, 's'}, {"p01", required_argument, 0, 1},
                                        {"p02", required_argument, 0, 2},       {"p12", required_argument, 0, 3},
                                        {"posterior", no_argument, 0, 4},       // additive
+                                       {"tracts", required_argument, 0, 5},    // additive
                                        {"help", no_argument, 0, 'h'},          {0, 0, 0, 0}};
     if (argc == 1) print_help(0);
     int option;
@@ -123,6 +139,7 @@ int main(int argc, char *argv[]) {
             case 2: p02 = atof(optarg); break;
             case 3: p12 = atof(optarg); break;
             case 4: posterior = true; break;
+            case 5: tracts_fn = optarg; break;
             case 'h': print_help(0); break;
             case ':':
                 fprintf(stderr, "Option -%c missing required argument.\n", optopt);
@@ -139,15 +156,15 @@ int main(int argc, char *argv[]) {
     for (int i = optind; i < argc; i++) fprintf(stderr, "Given extra argument %s.\n", argv[i]);
 
     // the tables are independent files: read by a few threads, concatenated in command-line order
-    std::vector<std::vector<double>> per_file(files.size());
+    std::vector<Summary> per_file(files.size());
     std::vector<int> read_rc(files.size(), 0);
     parallel_for(files.size(), [&](size_t i) { read_rc[i] = read_summary(files[i], &per_file[i]); });
     std::vector<double> lik;
     std::vector<int64_t> off{0};
     for (size_t i = 0; i < files.size(); i++) {
         if (read_rc[i]) exit(1);
-        lik.insert(lik.end(), per_file[i].begin(), per_file[i].end());
-        std::vector<double>().swap(per_file[i]);
+        lik.insert(lik.end(), per_file[i].lik.begin(), per_file[i].lik.end());
+        std::vector<double>().swap(per_file[i].lik);
         off.push_back((int64_t)(lik.size() / 3));
     }
     if (files.empty() || lik.empty()) {
@@ -169,6 +186,41 @@ int main(int argc, char *argv[]) {
                                                 expected.data()))) {
         fprintf(stderr, "%s\n", ibdgem_last_error());
         exit(1);
+    }
+    if (tracts_fn) {  // the same tables once more, through the tract entry: only the records come back
+        std::vector<int64_t> toff(off.size());
+        std::vector<hiddengem_tract> tr;
+        int rc = hiddengem_tracts_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, posterior ? 1 : 0, toff.data());
+        if (!rc) {
+            tr.resize((size_t)toff.back());
+            rc = hiddengem_last_tracts(e, tr.data(), 0);
+        }
+        if (rc) {
+            fprintf(stderr, "%s\n", ibdgem_last_error());
+            exit(1);
+        }
+        FILE *f = fopen(tracts_fn, "w");
+        if (!f) {
+            fprintf(stderr, "[::] ERROR: Cannot open '%s' for writing.\n", tracts_fn);
+            exit(1);
+        }
+        const std::string head = tract_header(true, posterior);
+        fwrite(head.data(), 1, head.size(), f);
+        for (size_t t = 0; t + 1 < off.size(); t++) {
+            const Summary &sm = per_file[t];
+            for (int64_t k = toff[t]; k < toff[t + 1]; k++) {
+                const hiddengem_tract &r = tr[(size_t)k];
+                const size_t a = (size_t)r.first_bin, b = (size_t)(r.first_bin + r.n_bins);
+                int64_t sites = 0;
+                for (size_t i = a; i < b; i++) sites += sm.n_sites[i];
+                const std::string row = files[t] + "\t" + tract_row(r, k - toff[t], sm.start[a], sm.end[b - 1], sites, posterior);
+                fwrite(row.data(), 1, row.size(), f);
+            }
+        }
+        if (fclose(f)) {
+            fprintf(stderr, "[::] ERROR: Cannot write '%s'.\n", tracts_fn);
+            exit(1);
+        }
     }
     ibdgem_engine_destroy(e);
     // one table's text does not depend on another's: formatted by a few threads, a wave of tables at a

@@ -4,7 +4,8 @@
 // (include/ibdgem_b200.h) and there is no CPU fallback.  Additive options: --gpus N (shard the
 // targets over N devices), --batch N (targets per engine call), --no-tab (skip *.tab.txt),
 // --panel-cache FILE (binary cache of the parsed IMPUTE or VCF panel), --hiddengem [--p01/--p02/--p12] (chain the
-// batched Viterbi pass over each target's window scores: <pileup>.<target>.hiddengem.txt).
+// batched Viterbi pass over each target's window scores: <pileup>.<target>.hiddengem.txt; with --tracts also the IBD
+// tracts, maximal runs of one state, in <pileup>.<target>.tracts.txt).
 #include <getopt.h>
 #include <limits.h>
 #include <unistd.h>
@@ -25,6 +26,7 @@
 #include "../../../include/ibdgem_b200.h"
 #include "panel.h"
 #include "pileup_store.h"
+#include "textio.h"
 
 using namespace ibdhost;
 
@@ -42,6 +44,7 @@ struct Options {
     int gpus = 1, batch = 0, no_tab = 0;
     int hiddengem = 0;  // --hiddengem: also write <pileup>.<target>.hiddengem.txt from the window scores
     int posterior = 0;  // --posterior (with --hiddengem): posterior state probabilities in those files
+    int tracts = 0;     // --tracts (with --hiddengem): also write <pileup>.<target>.tracts.txt
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
 };
 
@@ -92,6 +95,10 @@ void print_help(int code) {
         "                                   <pileup-name>.<target>.hiddengem.txt (penalties --p01, --p02, --p12)\n"
         "--posterior                     With --hiddengem: add each segment's posterior state probabilities\n"
         "                                   (P_IBD0, P_IBD1, P_IBD2) and the expected share of segments per state\n"
+        "--tracts                        With --hiddengem: also write the IBD tracts (maximal runs of segments in\n"
+        "                                   one state) to <pileup-name>.<target>.tracts.txt: state, first and last\n"
+        "                                   segment, START, END, number of segments and sites, LOD10 of the state\n"
+        "                                   against the next best (and with --posterior its mean and minimum posterior)\n"
         "-h, --help                      Show this help message and exit\n\n"
         "Format of likelihood table is tab-delimited with columns:\n"
         "CHR, rsID, POS, REF, ALT, AF, DP, SQ_NREF, SQ_NALT, GT_A0, GT_A1, LIBD0, LIBD1, LIBD2\n\n"
@@ -349,6 +356,8 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
         std::vector<double> hg_score;
         std::vector<int64_t> hg_counts, hg_off;
         std::vector<double> hg_post, hg_expected;
+        std::vector<int64_t> tr_off;
+        std::vector<hiddengem_tract> tracts;
         if (o.hiddengem) {
             std::vector<double> packed;
             hg_off.assign(1, 0);
@@ -369,6 +378,13 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
                 if (nbins && hiddengem_posterior_batch(e, (int32_t)T, hg_off.data(), packed.data(), 1, o.p01, o.p02, o.p12, hg_post.data(),
                                                        hg_expected.data()))
                     return fail_engine();
+            }
+            if (o.tracts && nbins) {  // the same packed scores through the tract entry: only the records come back
+                tr_off.resize(T + 1);
+                if (hiddengem_tracts_batch(e, (int32_t)T, hg_off.data(), packed.data(), 1, o.p01, o.p02, o.p12, o.posterior, tr_off.data()))
+                    return fail_engine();
+                tracts.resize((size_t)tr_off[T]);
+                if (hiddengem_last_tracts(e, tracts.data(), 0)) return fail_engine();
             }
         }
 
@@ -480,6 +496,26 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
                         fprintf(hg, "#%% posterior IBD%d (n = %.2f): %.2f\n", c, hg_expected[k * 3 + (size_t)c], (hg_expected[k * 3 + (size_t)c] / n) * 100);
                 fclose(hg);
             }
+            if (o.tracts && nw[k] > 0) {  // START / END / NUM_SITES from the run's own window bookkeeping
+                const std::string tr_fn = o.out_dir + "/" + o.sq_id + "." + smp.name + ".tracts.txt";
+                FILE *tf = fopen(tr_fn.c_str(), "w");
+                if (!tf) {
+                    fprintf(stderr, "[::] ERROR: Cannot open '%s' for writing.\n", tr_fn.c_str());
+                    return 1;
+                }
+                const std::string head = tract_header(false, o.posterior);
+                fwrite(head.data(), 1, head.size(), tf);
+                const size_t w0 = k * (size_t)maxW;
+                for (int64_t j = tr_off[k]; j < tr_off[k + 1]; j++) {
+                    const hiddengem_tract &r = tracts[(size_t)j];
+                    int64_t sites = 0;
+                    for (int64_t w = r.first_bin; w < r.first_bin + r.n_bins; w++) sites += wn[w0 + (size_t)w];
+                    const std::string row = tract_row(r, j - tr_off[k], ws[w0 + (size_t)r.first_bin], we[w0 + (size_t)(r.first_bin + r.n_bins - 1)],
+                                                      sites, o.posterior);
+                    fwrite(row.data(), 1, row.size(), tf);
+                }
+                fclose(tf);
+            }
             return 0;
         };
         const size_t n_writers = std::max<size_t>(1, std::min<size_t>({T, (size_t)WRITER_THREADS, (size_t)std::thread::hardware_concurrency()}));
@@ -510,7 +546,7 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
 int main(int argc, char *argv[]) {
     const clock_t start = clock();
     Options o;
-    static int ld_flag = 0, no_tab_flag = 0, hg_flag = 0, post_flag = 0;
+    static int ld_flag = 0, no_tab_flag = 0, hg_flag = 0, post_flag = 0, tracts_flag = 0;
     static struct option longopts[] = {{"LD", no_argument, &ld_flag, 1},
                                        {"vcf", required_argument, 0, 'V'},
                                        {"hap", required_argument, 0, 'H'},
@@ -540,6 +576,7 @@ int main(int argc, char *argv[]) {
                                        {"no-tab", no_argument, &no_tab_flag, 1},  // additive
                                        {"hiddengem", no_argument, &hg_flag, 1},   // additive: chain the Viterbi pass
                                        {"posterior", no_argument, &post_flag, 1},  // additive: posteriors in the hiddengem files
+                                       {"tracts", no_argument, &tracts_flag, 1},   // additive: IBD tracts beside the hiddengem files
                                        {"p01", required_argument, 0, 1004},
                                        {"p02", required_argument, 0, 1005},
                                        {"p12", required_argument, 0, 1006},
@@ -595,6 +632,7 @@ int main(int argc, char *argv[]) {
     o.no_tab = no_tab_flag;
     o.hiddengem = hg_flag;
     o.posterior = post_flag;
+    o.tracts = tracts_flag;
     for (int i = optind; i < argc; i++) fprintf(stderr, "Given extra argument %s.\n", argv[i]);
     // validation: the reference exits with status 0 on invalid values (src/ibdgem.c:966-989)
     if (o.opt_d && o.target_dp <= 0) {
@@ -623,6 +661,10 @@ int main(int argc, char *argv[]) {
     }
     if (o.posterior && !o.hiddengem) {
         fprintf(stderr, "[::] ERROR: --posterior needs --hiddengem (the posteriors are written to the hiddengem files).\n");
+        exit(0);
+    }
+    if (o.tracts && !o.hiddengem) {
+        fprintf(stderr, "[::] ERROR: --tracts needs --hiddengem (the tracts are runs of the hiddengem states).\n");
         exit(0);
     }
     if (o.max_cov > IBDGEM_MAX_COV_LIMIT) o.max_cov = IBDGEM_MAX_COV_LIMIT;  // pileup lines with cov >= 128 never load

@@ -1,11 +1,33 @@
 #include "textio.h"
 
+#include <cinttypes>
+#include <cmath>
 #include <cstring>
 
 namespace ibdhost {
 
 bool ends_with_gz(const std::string &fn) {
     return fn.size() >= 3 && fn.compare(fn.size() - 3, 3, ".gz") == 0;
+}
+
+std::string tract_header(bool summary, bool posterior) {
+    std::string h = summary ? "Summary\t" : "";
+    h += "Tract\tInferred_State\tFirst_Segment\tLast_Segment\tSTART\tEND\tN_Segments\tNUM_SITES\tLOD10";
+    h += posterior ? "\tP_Mean\tP_Min\n" : "\n";
+    return h;
+}
+
+// LOD10: log10 of the likelihood ratio of the called state against the better of the other two over the tract; it
+// is negative where the penalties, not the likelihoods, decided the call
+std::string tract_row(const hiddengem_tract &r, int64_t k, uint64_t start, uint64_t end, int64_t n_sites, bool posterior) {
+    const int s = r.state;
+    const double lod = (r.loglik[s] - std::fmax(r.loglik[(s + 1) % 3], r.loglik[(s + 2) % 3])) / std::log(10.0);
+    char row[320];
+    int n = snprintf(row, sizeof row, "%" PRId64 "\t%d\t%" PRId64 "\t%" PRId64 "\t%" PRIu64 "\t%" PRIu64 "\t%" PRId64 "\t%" PRId64 "\t%.4f", k + 1, s,
+                     r.first_bin + 1, r.first_bin + r.n_bins, start, end, r.n_bins, n_sites, lod);
+    if (posterior) n += snprintf(row + n, sizeof row - (size_t)n, "\t%.6f\t%.6f", r.post_mean, r.post_min);
+    row[n++] = '\n';
+    return std::string(row, (size_t)n);
 }
 
 bool LineReader::open(const std::string &path) {

@@ -9,6 +9,8 @@
 #include <string>
 #include <vector>
 
+#include "../../../include/ibdgem_b200.h"
+
 namespace ibdhost {
 
 class LineReader {
@@ -38,5 +40,11 @@ private:
 
 // true iff the name ends in ".gz" (src/file-io.c:10-18)
 bool ends_with_gz(const std::string &fn);
+
+// --tracts tables (hiddengem --tracts, ibdgem --hiddengem --tracts): the header line (with the leading Summary column
+// or without it), and one tract's columns from Tract on (k = 0-based index within its table; start / end: START of its
+// first bin and END of its last; n_sites: NUM_SITES summed over its bins), each ending in '\n'.
+std::string tract_header(bool summary, bool posterior);
+std::string tract_row(const hiddengem_tract &r, int64_t k, uint64_t start, uint64_t end, int64_t n_sites, bool posterior);
 
 }  // namespace ibdhost

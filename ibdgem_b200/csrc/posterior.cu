@@ -374,13 +374,13 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
 
 using namespace ibdgem;
 
-namespace {
-
-bool bad_penalties(const char *fn, double p01, double p02, double p12) {
+bool ibdgem::bad_penalties(const char *fn, double p01, double p02, double p12) {
     const bool ok = std::isfinite(p01) && std::isfinite(p02) && std::isfinite(p12) && p01 >= 0 && p02 >= 0 && p12 >= 0;
     if (!ok) set_error("[::] ERROR in %s(): penalties must be finite and >= 0 (p01 = %g, p02 = %g, p12 = %g).", fn, p01, p02, p12);
     return !ok;
 }
+
+namespace {
 
 // The linear-space kernels are exact to far below 1e-9 when every entry of the penalty matrix (1 on the diagonal) is
 // within a factor r = max(1, p) / min(1, p) <= 2^400 of every other.  Mixing keeps each alpha / beta entry above
@@ -393,8 +393,10 @@ bool linear_penalties(double p01, double p02, double p12) {
     return lo > 0 && hi / lo <= 0x1p400;
 }
 
+}  // namespace
+
 // One batch of tables, everything in device memory (start / len per table); kernels only, no host synchronisation.
-int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
+int ibdgem::posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
                         int is_log, double p01, double p02, double p12, double *d_post, double *d_expected) {
     const int64_t nck = (maxbins + HG_BINS - 1) / HG_BINS;
     if (nck == 0) {  // only empty tables: no bins, expected occupancy 0
@@ -435,8 +437,6 @@ int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const i
     IBD_CUDA(cudaGetLastError());
     return 0;
 }
-
-}  // namespace
 
 // Host buffers in, host buffers out: the likelihoods go up, both passes run, posteriors and expected counts come down.
 extern "C" int hiddengem_posterior_batch(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, const double *lik, int32_t is_log,

@@ -58,6 +58,12 @@ class Scores:
     extra: dict = field(default_factory=dict)
 
 
+# hiddengem_tract (include/ibdgem_b200.h): one IBD tract, a maximal run of one Viterbi state within a table
+TRACT_DTYPE = np.dtype([("first_bin", "<i8"), ("n_bins", "<i8"), ("state", "<i4"), ("reserved", "<i4"),
+                        ("loglik", "<f8", (3,)), ("post_mean", "<f8"), ("post_min", "<f8")])
+assert TRACT_DTYPE.itemsize == 64
+
+
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
@@ -273,6 +279,37 @@ class Engine:
             self._h, C.c_int32(len(off) - 1), _ptr(off), C.c_int64(table_stride), C.c_void_p(d_lik_ptr),
             C.c_int32(1 if is_log else 0), C.c_double(p01), C.c_double(p02), C.c_double(p12),
             C.c_void_p(d_posterior_ptr), C.c_void_p(d_expected_ptr)))
+
+    def tracts_batch(self, lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-3, posterior=True):
+        """IBD tracts (runs of one Viterbi state) with likelihood sums and, with posterior, the mean and minimum
+        posterior of their state (hiddengem_tracts_batch + hiddengem_last_tracts): (tract_offsets [n_tables + 1],
+        tracts, a TRACT_DTYPE array)."""
+        lik = np.ascontiguousarray(lik, np.float64)
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        nt = len(off) - 1
+        toff = np.zeros(nt + 1, np.int64)
+        self._check(self._lib.hiddengem_tracts_batch(self._h, C.c_int32(nt), _ptr(off), _ptr(lik), C.c_int32(1 if is_log else 0),
+                                                     C.c_double(p01), C.c_double(p02), C.c_double(p12),
+                                                     C.c_int32(1 if posterior else 0), _ptr(toff)))
+        return toff, self.last_tracts(toff[-1])
+
+    def tracts_device(self, d_lik_ptr: int, bin_offsets, is_log: bool, d_state_ptr: int, d_posterior_ptr: int = 0,
+                      table_stride: int = 0):
+        """Tracts of device states (and posteriors, 0: none) (hiddengem_tracts_device); bin_offsets stays on the host.
+        Returns (tract_offsets, tracts) copied to the host."""
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        nt = len(off) - 1
+        toff = np.zeros(nt + 1, np.int64)
+        self._check(self._lib.hiddengem_tracts_device(self._h, C.c_int32(nt), _ptr(off), C.c_int64(table_stride),
+                                                      C.c_void_p(d_lik_ptr), C.c_int32(1 if is_log else 0),
+                                                      C.c_void_p(d_state_ptr), C.c_void_p(d_posterior_ptr or None), _ptr(toff)))
+        return toff, self.last_tracts(toff[-1])
+
+    def last_tracts(self, n: int):
+        """The n records of the last successful tract call (hiddengem_last_tracts), as a TRACT_DTYPE array."""
+        tracts = np.zeros(max(int(n), 1), TRACT_DTYPE)
+        self._check(self._lib.hiddengem_last_tracts(self._h, _ptr(tracts), C.c_int32(0)))
+        return tracts[: int(n)]
 
     def viterbi_last_flagged(self) -> int:
         """Tables of the last hiddengem call re-evaluated on the host in long double (near-tie guard)."""

@@ -269,6 +269,43 @@ int hiddengem_posterior_batch_device(ibdgem_engine *e, int32_t n_tables, const i
                                      const double *d_lik, int32_t is_log, double p01, double p02, double p12,
                                      double *d_posterior, double *d_expected);
 
+/* IBD tracts.  A tract is a maximal run [first_bin, first_bin + n_bins) of bins of one table with the same Viterbi
+ * state (in IBDGem a "segment" is one window, i.e. one bin).  Tracts never cross tables; an empty table has none.
+ * Records are ordered table by table, then by first_bin; table t's are records [tract_offsets[t], tract_offsets[t+1]).
+ *   loglik[s]    sum over the tract's bins of the natural log of the RAW likelihood of state s: the input as is for
+ *                is_log = 1, ln l_s for is_log = 0 (a zero likelihood gives -inf, a NaN row NaN sums).  Differences
+ *                between states are the tract's log likelihood ratios; the called state need not have the largest,
+ *                since penalties can outweigh it.
+ *   post_mean    mean over the tract's bins of the posterior of `state`, and post_min its minimum; both NaN without
+ *   post_min     posteriors, or when any of them is NaN (a table of zero total weight).
+ * Sums are reduced in a fixed order: the same inputs give the same bits. */
+typedef struct {            /* 64 bytes, layout fixed */
+    int64_t first_bin;      /* 0-based within its table */
+    int64_t n_bins;
+    int32_t state;          /* 0, 1, 2 = IBD0/1/2 */
+    int32_t reserved;       /* 0 */
+    double  loglik[3];      /* sum of ln likelihood of each state over the tract */
+    double  post_mean;      /* mean posterior of `state` over the tract; NaN without posteriors */
+    double  post_min;
+} hiddengem_tract;
+
+/* Viterbi (with its near-tie guard: the states are exactly those of hiddengem_viterbi_batch, and
+ * hiddengem_last_flagged reports the call's flagged tables) + optional posterior (with_posterior != 0; penalties
+ * checked as by hiddengem_posterior_batch) + tracts on the GPU; per-bin arrays never leave the device.  lik /
+ * bin_offsets / is_log as for hiddengem_viterbi_batch (host arrays).  tract_offsets: host [n_tables + 1]; the records
+ * stay in the engine for hiddengem_last_tracts. */
+int hiddengem_tracts_batch(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, const double *lik, int32_t is_log,
+                           double p01, double p02, double p12, int32_t with_posterior, int64_t *tract_offsets);
+/* Tracts of states (and posteriors; d_posterior may be NULL) already on the device, e.g. from the two *_device
+ * entries, with their layouts (table_stride = 0 packed, > 0 table t at bin t * table_stride).  d_lik is the input those
+ * entries took.  A state byte above 2 fails the call. */
+int hiddengem_tracts_device(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, int64_t table_stride,
+                            const double *d_lik, int32_t is_log, const uint8_t *d_state, const double *d_posterior,
+                            int64_t *tract_offsets);
+/* Copy the records of the last successful tract call (tract_offsets[n_tables] of them) to dst, host memory or
+ * (dst_on_device != 0) device memory of the engine's GPU.  Fails if no tract call has succeeded on this engine. */
+int hiddengem_last_tracts(ibdgem_engine *e, hiddengem_tract *dst, int32_t dst_on_device);
+
 /* ---- instrumentation --------------------------------------------------------------------- */
 
 /* When enabled every kernel launch is bracketed by CUDA events on the engine stream. */
