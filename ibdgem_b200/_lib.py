@@ -21,6 +21,7 @@ ABI_SYMBOLS = [
     "ibdgem_engine_set_window_shard", "ibdgem_engine_window_shard", "ibdgem_peer_alloc", "ibdgem_peer_open",
     "ibdgem_peer_close", "hiddengem_viterbi_batch_device", "hiddengem_last_flagged", "ibdgem_engine_clone_panel", "ibdgem_engine_set_shard_compact_output",
     "hiddengem_posterior_batch", "hiddengem_posterior_batch_device",
+    "hiddengem_posterior_moments_batch", "hiddengem_posterior_moments_device",
     "hiddengem_tracts_batch", "hiddengem_tracts_device", "hiddengem_last_tracts",
 ]
 

@@ -31,7 +31,7 @@ static const char *const kKernelNameList[] = {
     "ld_mma",         "viterbi",       "viterbi_back",  "viterbi_out",  "fill",
     "v_slots",        "v_wmap",        "v_tw",          "v_sort",       "v_expand_a",  "v_expand_b",   "ld_vmma",
     "window_linear",  "posterior_fwd", "posterior_bwd", "posterior_fwd_log", "posterior_bwd_log",
-    "tract_count",    "tract_emit",
+    "tract_count",    "tract_emit",    "posterior_bwd_moments",
 };
 static_assert(sizeof(kKernelNameList) / sizeof(kKernelNameList[0]) == K_COUNT, "one name per KernelId, in enum order");
 const char *const *const kKernelNames = kKernelNameList;

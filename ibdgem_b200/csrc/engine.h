@@ -63,6 +63,8 @@ enum KernelId {
     K_POSTERIOR_BWD_LOG,  // spread penalties); counted only, their time is in posterior_fwd / _bwd
     K_TRACT_COUNT,      // hiddengem tracts: runs of equal state per table, state bytes checked
     K_TRACT_EMIT,       // hiddengem tracts: one 64-byte record per run (likelihood sums, posterior mean / minimum)
+    K_POSTERIOR_BWD_MOMENTS,  // hiddengem posterior moments: the backward pass with the covariance recursion (its
+                              // forward pass is posterior_fwd; in log arithmetic both are counted under _log too)
     K_COUNT
 };
 
@@ -220,10 +222,11 @@ void viterbi_redo_flagged(const std::vector<int> &flagged, const int64_t *bin_of
                           double p02, double p12,
                           const std::function<void(size_t, int, const uint8_t *, const double *, const int64_t *)> &sink);
 // posterior.cu: penalty check of the posterior entries (1 and the error set when rejected), and its kernels for one
-// batch of tables in device memory (no host synchronisation)
+// batch of tables in device memory (no host synchronisation).  d_cov != null runs the moment variant of the backward
+// pass: covariances into d_cov [n_tables][3][3], and d_post may then be null.
 bool bad_penalties(const char *fn, double p01, double p02, double p12);
 int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
-                        int is_log, double p01, double p02, double p12, double *d_post, double *d_expected);
+                        int is_log, double p01, double p02, double p12, double *d_post, double *d_expected, double *d_cov = nullptr);
 
 // Makes the engine stream wait for the panel chunks that cover sites [0, s_end); ensure_table also
 // runs site_table on the part of [0, s_end) it has not covered yet.

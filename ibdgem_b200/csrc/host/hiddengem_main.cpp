@@ -5,7 +5,9 @@
 // Additive: -s may be given several times; the tables are read in parallel, scored in one batch and
 // printed in order (formatted in parallel).  --posterior (additive) also prints each bin's posterior state
 // probabilities (hiddengem_posterior_batch) and the expected state fractions.  --tracts FILE (additive) writes the IBD
-// tracts, maximal runs of one state, to FILE (hiddengem_tracts_batch); stdout is unchanged.
+// tracts, maximal runs of one state, to FILE (hiddengem_tracts_batch); stdout is unchanged.  --share-sd (additive,
+// with --posterior) runs hiddengem_posterior_moments_batch in place of hiddengem_posterior_batch and adds the
+// standard deviations of the posterior state shares and of the kinship, per table and over all tables.
 #include <getopt.h>
 
 #include <cmath>
@@ -34,6 +36,10 @@ void print_help(int code) {
           "--p12  FLOAT             Penalty for switching between states IBD1 and IBD2 (default: 1e-3)\n"
           "--posterior              Also print each segment's posterior probability of every state (columns\n"
           "                            P_IBD0, P_IBD1, P_IBD2) and the expected share of segments per state\n"
+          "--share-sd               With --posterior: also print the standard deviation of each state's share\n"
+          "                            of segments and the window-share kinship (N_IBD1/4 + N_IBD2/2)/n with its\n"
+          "                            standard deviation, from the posterior covariance; with several -s, also\n"
+          "                            these figures over all tables together\n"
           "--tracts  FILE           Also write the IBD tracts (maximal runs of segments in one state) to FILE: per\n"
           "                            tract its summary file, state, first and last segment, START, END, number\n"
           "                            of segments and sites, LOD10 of its state against the next best (and with\n"
@@ -123,12 +129,13 @@ int read_summary(const std::string &fn, Summary *sm) {
 int main(int argc, char *argv[]) {
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
     std::vector<std::string> files;
-    bool posterior = false;
+    bool posterior = false, share_sd = false;
     const char *tracts_fn = nullptr;
     static struct option longopts[] = {{"summary", required_argument, 0, 's'}, {"p01", required_argument, 0, 1},
                                        {"p02", required_argument, 0, 2},       {"p12", required_argument, 0, 3},
                                        {"posterior", no_argument, 0, 4},       // additive
                                        {"tracts", required_argument, 0, 5},    // additive
+                                       {"share-sd", no_argument, 0, 6},        // additive
                                        {"help", no_argument, 0, 'h'},          {0, 0, 0, 0}};
     if (argc == 1) print_help(0);
     int option;
@@ -140,6 +147,7 @@ int main(int argc, char *argv[]) {
             case 3: p12 = atof(optarg); break;
             case 4: posterior = true; break;
             case 5: tracts_fn = optarg; break;
+            case 6: share_sd = true; break;
             case 'h': print_help(0); break;
             case ':':
                 fprintf(stderr, "Option -%c missing required argument.\n", optopt);
@@ -154,6 +162,10 @@ int main(int argc, char *argv[]) {
         }
     }
     for (int i = optind; i < argc; i++) fprintf(stderr, "Given extra argument %s.\n", argv[i]);
+    if (share_sd && !posterior) {
+        fprintf(stderr, "[::] ERROR: --share-sd needs --posterior (the standard deviations are those of the posterior counts).\n");
+        exit(0);
+    }
 
     // the tables are independent files: read by a few threads, concatenated in command-line order
     std::vector<Summary> per_file(files.size());
@@ -179,11 +191,14 @@ int main(int argc, char *argv[]) {
     std::vector<double> score(nb * 3);
     std::vector<int64_t> counts((off.size() - 1) * 3);
     std::vector<double> post(posterior ? nb * 3 : 0), expected(posterior ? (off.size() - 1) * 3 : 0);
+    std::vector<double> cov(share_sd ? (off.size() - 1) * 9 : 0);
     if (ibdgem_engine_create(&prm, &e) ||
         hiddengem_viterbi_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, state.data(), score.data(),
                                 counts.data()) ||
-        (posterior && hiddengem_posterior_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, post.data(),
-                                                expected.data()))) {
+        (posterior && !share_sd &&
+         hiddengem_posterior_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, post.data(), expected.data())) ||
+        (share_sd && hiddengem_posterior_moments_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, post.data(),
+                                                       expected.data(), cov.data()))) {
         fprintf(stderr, "%s\n", ibdgem_last_error());
         exit(1);
     }
@@ -258,8 +273,24 @@ int main(int argc, char *argv[]) {
                     const double x = expected[t * 3 + (size_t)k];
                     out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d (n = %.2f): %.2f\n", k, x, (x / n) * 100));
                 }
+            if (share_sd) out += share_sd_lines(&expected[t * 3], &cov[t * 9], n);
         });
         for (size_t k = 0; k < nt; k++) fwrite(text[k].data(), 1, text[k].size(), stdout);
+    }
+    if (share_sd && n_tables > 1) {  // the tables are independent: their means and covariances add
+        double x[3] = {0, 0, 0}, c[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+        for (size_t t = 0; t < n_tables; t++) {
+            for (int k = 0; k < 3; k++) x[k] += expected[t * 3 + (size_t)k];
+            for (int k = 0; k < 9; k++) c[k] += cov[t * 9 + (size_t)k];
+        }
+        const double n = (double)off.back();
+        std::string out;
+        char row[160];
+        out.append(row, (size_t)snprintf(row, sizeof row, "#%% all %zu tables (n = %.0f)\n", n_tables, n));
+        for (int k = 0; k < 3; k++)
+            out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d (n = %.2f): %.2f\n", k, x[k], (x[k] / n) * 100));
+        out += share_sd_lines(x, c, n);
+        fwrite(out.data(), 1, out.size(), stdout);
     }
     return 0;
 }

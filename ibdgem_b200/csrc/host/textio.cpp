@@ -98,4 +98,20 @@ bool LineReader::next(const char **line, size_t *len) {
     }
 }
 
+// sqrt of a variance; one a rounding below 0 is 0, NaN stays NaN
+static double sd_of(double v) { return v > 0 ? std::sqrt(v) : (v == v ? 0.0 : v); }
+
+std::string share_sd_lines(const double *expected, const double *cov, double n) {
+    std::string out;
+    char row[160];
+    for (int k = 0; k < 3; k++) {
+        const double sd = sd_of(cov[k * 4]);
+        out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d sd (n = %.2f): %.2f\n", k, sd, (sd / n) * 100));
+    }
+    const double phi = (expected[1] / 4 + expected[2] / 2) / n;
+    const double var = (cov[4] / 16 + cov[8] / 4 + cov[5] / 4) / (n * n);
+    out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior kinship (sd = %.4f): %.4f\n", sd_of(var), phi));
+    return out;
+}
+
 }  // namespace ibdhost

@@ -47,4 +47,9 @@ bool ends_with_gz(const std::string &fn);
 std::string tract_header(bool summary, bool posterior);
 std::string tract_row(const hiddengem_tract &r, int64_t k, uint64_t start, uint64_t end, int64_t n_sites, bool posterior);
 
+// --share-sd lines (hiddengem, ibdgem --hiddengem): from the posterior mean (expected[3]) and covariance (cov[3][3]) of
+// the bins per state of n bins, "#% posterior IBDk sd (n = <sd of N_k>): <sd of the share in %>" for k = 0, 1, 2 and
+// "#% posterior kinship (sd = <sd>): <phi>" with phi = (N_1 / 4 + N_2 / 2) / n, each ending in '\n'.
+std::string share_sd_lines(const double *expected, const double *cov, double n);
+
 }  // namespace ibdhost

@@ -24,6 +24,11 @@
 //             gamma = alpha * beta / sum, write it and accumulate the expected occupancy.
 // Bytes per bin: 24 read by each pass, 24 written once, plus the checkpoints (3 B): ~75 B, against ~120 B for a
 // design that stores alpha of every bin and reads it back.
+//   moments   (hiddengem_posterior_moments_*) the backward kernel with MOM = true: the solver lane also carries the
+//             moment recursion down the table (moment_step) and sums each table's covariance terms in bin order
+//             (moment_acc).  The sums stay on the solver lane: staging its per-bin state in shared memory for the
+//             workers would add 32-74 KB per block and drop residency from three blocks per SM to two or one, and at
+//             C4 the 313 blocks then need two waves.  The posteriors are optional there.
 //
 // Emissions (nrm; any positive per-bin factor cancels in gamma, so only the direction is needed):
 //   is_log = 0  l_s / ((l0 + l1) + l2) as hiddengem normalises summary-file likelihoods, with the division replaced
@@ -193,6 +198,80 @@ __device__ __forceinline__ void gamma(const double *A, const double *B, bool dea
     y2 = g2 * inv;
 }
 
+// Moments (the MOM variant of the backward pass).  Conditioned on x_{i-1} = k the rest of the path is Markov with
+// P(x_i = l | k) = pen(k, l) nrm[i][l] beta[i][l] / t_k, t_k = sum_l pen(k, l) nrm[i][l] beta[i][l] (the sum bwd_step
+// forms).  With h_i^t[k] = E[#{j > i : x_j = t} | x_i = k],
+//     h_{i-1}^t[k] = sum_l P(l | k) (delta_lt + h_i^t[l]),   h_{n-1} = 0,
+//     Cov(N_s, N_t) = sum_i gamma_i(s) (delta_st - gamma_i(t)) + gamma_i(s) (h_i^t[s] - H_i^t) + gamma_i(t) (h_i^s[t] - H_i^s),
+// H_i^t = sum_k gamma_i(k) h_i^t[k].  Every term is invariant to adding one constant per t to h_i^t[0..2], so the
+// solver carries u^t[k] = h^t[k] minus h^t of the state with the largest t_k (a live state): bounded by the
+// correlation length, where h grows with n and its differences would lose a digit per factor 10 of table length.
+// u^2 is -u^0 - u^1 up to such a constant (sum_t h^t[k] = n - 1 - i for every k), so only t = 0, 1 are carried.
+// A state with t_k = 0 (or below the normal range) has gamma 0 there and no weight in the next step: its m is set to 0.
+template <bool LG>
+__device__ __forceinline__ void moment_step(double (&u)[2][3], double e0, double e1, double e2, double b0, double b1, double b2,
+                                            double p01, double p02, double p12) {
+    double m[2][3], t0, t1, t2;
+    if (LG) {  // P(l | k) = exp(lp(k, l) + v_l - t_k), 0 where t_k = -inf
+        const double v0 = e0 + b0, v1 = e1 + b1, v2 = e2 + b2;
+        t0 = lse3(v0, v1 + p01, v2 + p02);
+        t1 = lse3(v0 + p01, v1, v2 + p12);
+        t2 = lse3(v0 + p02, v1 + p12, v2);
+        const double x[3][3] = {{v0, v1 + p01, v2 + p02}, {v0 + p01, v1, v2 + p12}, {v0 + p02, v1 + p12, v2}};
+        const double tk[3] = {t0, t1, t2};
+#pragma unroll
+        for (int k = 0; k < 3; k++) {
+            const bool ok = tk[k] > -INFINITY;
+            const double q0 = ok ? exp_nonpos(x[k][0] - tk[k]) : 0.0, q1 = ok ? exp_nonpos(x[k][1] - tk[k]) : 0.0,
+                         q2 = ok ? exp_nonpos(x[k][2] - tk[k]) : 0.0;
+#pragma unroll
+            for (int t = 0; t < 2; t++) m[t][k] = fma(q0, u[t][0], fma(q1, u[t][1], fma(q2, u[t][2], t == 0 ? q0 : q1)));
+        }
+    } else {  // m^t[k] = (sum_l pen(k, l) v_l (delta_lt + u^t[l])) / t_k
+        const double v0 = e0 * b0, v1 = e1 * b1, v2 = e2 * b2;
+        t0 = fma(v2, p02, fma(v1, p01, v0));
+        t1 = fma(v2, p12, fma(v0, p01, v1));
+        t2 = fma(v1, p12, fma(v0, p02, v2));
+        const double r0 = t0 >= 0x1p-1022 ? recip(t0) : 0.0, r1 = t1 >= 0x1p-1022 ? recip(t1) : 0.0,
+                     r2 = t2 >= 0x1p-1022 ? recip(t2) : 0.0;
+#pragma unroll
+        for (int t = 0; t < 2; t++) {
+            const double w0 = v0 * (u[t][0] + (t == 0)), w1 = v1 * (u[t][1] + (t == 1)), w2 = v2 * u[t][2];
+            m[t][0] = r0 * fma(w2, p02, fma(w1, p01, w0));
+            m[t][1] = r1 * fma(w2, p12, fma(w0, p01, w1));
+            m[t][2] = r2 * fma(w1, p12, fma(w0, p02, w2));
+        }
+    }
+    const int r = (t1 > t0) ? (t2 > t1 ? 2 : 1) : (t2 > t0 ? 2 : 0);  // a live state (largest t_k)
+#pragma unroll
+    for (int t = 0; t < 2; t++) {
+        const double ref = r == 0 ? m[t][0] : r == 1 ? m[t][1] : m[t][2];
+        u[t][0] = m[t][0] - ref;
+        u[t][1] = m[t][1] - ref;
+        u[t][2] = m[t][2] - ref;
+    }
+}
+
+// one bin's cross terms (gamma y of the bin, u of the bin) into the upper triangle C = {00, 01, 02, 11, 12, 22}
+__device__ __forceinline__ void moment_acc(double (&C)[6], const double (&u)[2][3], double y0, double y1, double y2) {
+    const double y[3] = {y0, y1, y2};
+    double d[3][3];  // d[t][s] = gamma(s) (u^t[s] - U^t)
+#pragma unroll
+    for (int t = 0; t < 3; t++) {
+        const double a0 = t < 2 ? u[t][0] : -u[0][0] - u[1][0], a1 = t < 2 ? u[t][1] : -u[0][1] - u[1][1],
+                     a2 = t < 2 ? u[t][2] : -u[0][2] - u[1][2];
+        const double U = fma(y2, a2, fma(y1, a1, y0 * a0));
+        d[t][0] = y0 * (a0 - U);
+        d[t][1] = y1 * (a1 - U);
+        d[t][2] = y2 * (a2 - U);
+    }
+    int k = 0;
+#pragma unroll
+    for (int s = 0; s < 3; s++)
+#pragma unroll
+        for (int t = s; t < 3; t++, k++) C[k] += fma(y[s], (s == t ? 1.0 : 0.0) - y[t], d[t][s] + d[s][t]);
+}
+
 // Workers: emissions of chunk c in place, once every worker has stored its part
 template <bool LG>
 __device__ __forceinline__ void emit(const ChunkLoader &ld, int c, double (*buf)[HG_ROW], int is_log) {
@@ -259,12 +338,15 @@ posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
     }
 }
 
-// Backward pass: gamma -> posterior (the caller's layout), expected occupancy -> expected[t][3].
-template <bool LG>
+// Backward pass: gamma -> posterior (the caller's layout), expected occupancy -> expected[t][3].  MOM: the solver
+// also carries the moment recursion (moment_step) and sums each table's cross terms in bin order, from the last bin
+// down, into cov[t][3][3]; posterior may then be null (nothing per bin is written).  The workers' gamma, posterior and
+// expected are those of the plain pass, bit for bit.
+template <bool LG, bool MOM = false>
 __global__ void __launch_bounds__(HG_THREADS, 3)
 posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
                      int is_log, double p01, double p02, double p12, const double *__restrict__ ckpt, double *__restrict__ posterior,
-                     double *__restrict__ expected) {
+                     double *__restrict__ expected, double *__restrict__ cov = nullptr) {
     extern __shared__ double pb_smem[];
     double (*em)[HG_TABLES][HG_ROW] = reinterpret_cast<double (*)[HG_TABLES][HG_ROW]>(pb_smem);  // emissions, then beta
     double (*al)[HG_TABLES][HG_ROW] = reinterpret_cast<double (*)[HG_TABLES][HG_ROW]>(pb_smem + 2 * HG_TABLES * HG_ROW);
@@ -278,6 +360,7 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
     const int nchunk = block_tables(n_tables, start, len, s_start, s_len);
     const int w = (int)threadIdx.x - 32;
     double E[HG_NBIN][3] = {};  // a worker's share of the expected counts: the same (table, bin slot) every chunk
+    double mu[2][3] = {}, mc[6] = {};  // MOM, solver lane: u of the bin below, the table's cross-term sums
     if (threadIdx.x >= 32) {
         const ChunkLoader ld{s_start, s_len, w};
         double pre[HG_NLD];
@@ -301,10 +384,12 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                     if (i0 + i < s_len[t]) {
                         double y0, y1, y2;
                         gamma<LG>(&al[pb][t][i * 3], &em[pb][t][i * 3], s_dead[t], y0, y1, y2);
-                        double *o = posterior + (s_start[t] + i0 + i) * 3;
-                        __stcs(o, y0);
-                        __stcs(o + 1, y1);
-                        __stcs(o + 2, y2);
+                        if (!MOM || posterior) {
+                            double *o = posterior + (s_start[t] + i0 + i) * 3;
+                            __stcs(o, y0);
+                            __stcs(o + 1, y1);
+                            __stcs(o + 2, y2);
+                        }
                         E[k][0] += y0;
                         E[k][1] += y1;
                         E[k][2] += y2;
@@ -335,11 +420,27 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                 ao[q * 3] = a0; ao[q * 3 + 1] = a1; ao[q * 3 + 2] = a2;
             }
             // beta down the chunk: the slot of bin i trades its emission for beta[i], then beta[i - 1]
+            if (!MOM) {
 #pragma unroll 4
-            for (int q = HG_BINS - 1; q >= 0; q--) {
-                const double e0 = nr[q * 3], e1 = nr[q * 3 + 1], e2 = nr[q * 3 + 2];
-                nr[q * 3] = b0; nr[q * 3 + 1] = b1; nr[q * 3 + 2] = b2;
-                bwd_step<LG>(b0, b1, b2, e0, e1, e2, i0 + q < n, p01, p02, p12);
+                for (int q = HG_BINS - 1; q >= 0; q--) {
+                    const double e0 = nr[q * 3], e1 = nr[q * 3 + 1], e2 = nr[q * 3 + 2];
+                    nr[q * 3] = b0; nr[q * 3 + 1] = b1; nr[q * 3 + 2] = b2;
+                    bwd_step<LG>(b0, b1, b2, e0, e1, e2, i0 + q < n, p01, p02, p12);
+                }
+            } else {
+                const bool dead = s_dead[lane];
+#pragma unroll 1
+                for (int q = HG_BINS - 1; q >= 0; q--) {
+                    const double e0 = nr[q * 3], e1 = nr[q * 3 + 1], e2 = nr[q * 3 + 2];
+                    nr[q * 3] = b0; nr[q * 3 + 1] = b1; nr[q * 3 + 2] = b2;
+                    if (i0 + q < n) {  // the bin's cross terms with u of bin i, then u of bin i - 1
+                        double y0, y1, y2;
+                        gamma<LG>(&ao[q * 3], &nr[q * 3], dead, y0, y1, y2);
+                        moment_acc(mc, mu, y0, y1, y2);
+                        moment_step<LG>(mu, e0, e1, e2, b0, b1, b2, p01, p02, p12);
+                    }
+                    bwd_step<LG>(b0, b1, b2, e0, e1, e2, i0 + q < n, p01, p02, p12);
+                }
             }
             __threadfence_block();
             arrive_solved(b);
@@ -366,6 +467,12 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                 for (int s = 0; s < 3; s++) x[s] += part[(threadIdx.x * HG_BINS + i) * 3 + s];
             const double nan = __longlong_as_double(0x7ff8000000000000LL);
             for (int s = 0; s < 3; s++) expected[(size_t)tb * 3 + s] = s_dead[threadIdx.x] ? nan : x[s];
+            if (MOM) {  // this thread is the table's solver lane: its own sums
+                double *o = cov + (size_t)tb * 9;
+                const int ix[9] = {0, 1, 2, 1, 3, 4, 2, 4, 5};
+#pragma unroll
+                for (int k = 0; k < 9; k++) o[k] = s_dead[threadIdx.x] ? nan : mc[ix[k]];
+            }
         }
     }
 }
@@ -397,10 +504,11 @@ bool linear_penalties(double p01, double p02, double p12) {
 
 // One batch of tables, everything in device memory (start / len per table); kernels only, no host synchronisation.
 int ibdgem::posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
-                        int is_log, double p01, double p02, double p12, double *d_post, double *d_expected) {
+                        int is_log, double p01, double p02, double p12, double *d_post, double *d_expected, double *d_cov) {
     const int64_t nck = (maxbins + HG_BINS - 1) / HG_BINS;
-    if (nck == 0) {  // only empty tables: no bins, expected occupancy 0
+    if (nck == 0) {  // only empty tables: no bins, expected occupancy 0 (and covariance 0)
         IBD_CUDA(cudaMemsetAsync(d_expected, 0, (size_t)n_tables * 24, e->stream));
+        if (d_cov) IBD_CUDA(cudaMemsetAsync(d_cov, 0, (size_t)n_tables * 72, e->stream));
         return 0;
     }
     double *d_ckpt;
@@ -412,7 +520,12 @@ int ibdgem::posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins,
             posterior_fwd_kernel<false><<<grid, HG_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
                                                                                       d_ckpt, d_expected);
         }
-        {
+        if (d_cov) {
+            LaunchScope ls(e, K_POSTERIOR_BWD_MOMENTS);
+            IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
+            posterior_bwd_kernel<false, true><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02,
+                                                                                            p12, d_ckpt, d_post, d_expected, d_cov);
+        } else {
             LaunchScope ls(e, K_POSTERIOR_BWD);
             IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
             posterior_bwd_kernel<false><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
@@ -426,7 +539,13 @@ int ibdgem::posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins,
             posterior_fwd_kernel<true><<<grid, HG_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
                                                                                      d_ckpt, d_expected);
         }
-        {
+        if (d_cov) {
+            LaunchScope ls(e, K_POSTERIOR_BWD_MOMENTS);
+            e->k_launches[K_POSTERIOR_BWD_LOG]++;
+            IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
+            posterior_bwd_kernel<true, true><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02,
+                                                                                           l12, d_ckpt, d_post, d_expected, d_cov);
+        } else {
             LaunchScope ls(e, K_POSTERIOR_BWD);
             e->k_launches[K_POSTERIOR_BWD_LOG]++;
             IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
@@ -490,6 +609,67 @@ extern "C" int hiddengem_posterior_batch_device(ibdgem_engine *e, int32_t n_tabl
     if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start)) return 1;
     IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
     if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_posterior, d_expected)) return 1;
+    IBD_CUDA(cudaStreamSynchronize(e->stream));  // h_sl is read by the copy above
+    settle_timers(e);
+    return 0;
+}
+
+// Posterior moments: the posterior pass with the moment variant of the backward kernel.  Host buffers in, host
+// buffers out; without posterior (null) only the 96 B of expected + cov per table come back.
+extern "C" int hiddengem_posterior_moments_batch(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, const double *lik,
+                                                 int32_t is_log, double p01, double p02, double p12, double *posterior, double *expected,
+                                                 double *cov) {
+    if (!e || n_tables <= 0 || !bin_offsets || !expected || !cov) {
+        set_error("[::] ERROR in hiddengem_posterior_moments_batch(): bad arguments.");
+        return 1;
+    }
+    if (bad_penalties("hiddengem_posterior_moments_batch", p01, p02, p12)) return 1;
+    std::vector<int64_t> h_sl;
+    int64_t maxbins, total;
+    if (table_layout("hiddengem_posterior_moments_batch", n_tables, bin_offsets, 0, &h_sl, &maxbins, &total)) return 1;
+    const int64_t nb = total > 0 ? bin_offsets[n_tables] : 0;  // bins of lik / posterior
+    if (nb > 0 && !lik) {
+        set_error("[::] ERROR in hiddengem_posterior_moments_batch(): bad arguments.");
+        return 1;
+    }
+    IBD_CUDA(cudaSetDevice(e->device));
+    double *d_lik = nullptr, *d_post = nullptr, *d_out;
+    int64_t *d_start;
+    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start) || scratch(e, SC_HG_COUNTS, (size_t)n_tables * 96, (void **)&d_out))
+        return 1;
+    if (nb > 0 && scratch(e, SC_HG_LIK, (size_t)nb * 24, (void **)&d_lik)) return 1;
+    if (nb > 0 && posterior && scratch(e, SC_HG_SCORE, (size_t)nb * 24, (void **)&d_post)) return 1;
+    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
+    if (nb > 0) IBD_CUDA(cudaMemcpyAsync(d_lik, lik, (size_t)nb * 24, cudaMemcpyHostToDevice, e->stream));
+    double *d_cov = d_out + (size_t)n_tables * 3;
+    if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_post, d_out, d_cov)) return 1;
+    if (d_post) IBD_CUDA(cudaMemcpyAsync(posterior, d_post, (size_t)nb * 24, cudaMemcpyDeviceToHost, e->stream));
+    IBD_CUDA(cudaMemcpyAsync(expected, d_out, (size_t)n_tables * 24, cudaMemcpyDeviceToHost, e->stream));
+    IBD_CUDA(cudaMemcpyAsync(cov, d_cov, (size_t)n_tables * 72, cudaMemcpyDeviceToHost, e->stream));
+    IBD_CUDA(cudaStreamSynchronize(e->stream));
+    settle_timers(e);
+    return 0;
+}
+
+// Device buffers in, device buffers out (d_posterior may be null); bin_offsets is a HOST array, table_stride as for
+// hiddengem_posterior_batch_device.
+extern "C" int hiddengem_posterior_moments_device(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, int64_t table_stride,
+                                                  const double *d_lik, int32_t is_log, double p01, double p02, double p12, double *d_posterior,
+                                                  double *d_expected, double *d_cov) {
+    if (!e || n_tables <= 0 || !bin_offsets || !d_lik || !d_expected || !d_cov || table_stride < 0) {
+        set_error("[::] ERROR in hiddengem_posterior_moments_device(): bad arguments.");
+        return 1;
+    }
+    if (bad_penalties("hiddengem_posterior_moments_device", p01, p02, p12)) return 1;
+    std::vector<int64_t> h_sl;
+    int64_t maxbins, total;
+    if (table_layout("hiddengem_posterior_moments_device", n_tables, bin_offsets, table_stride, &h_sl, &maxbins, &total)) return 1;
+    IBD_CUDA(cudaSetDevice(e->device));
+    int64_t *d_start;
+    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start)) return 1;
+    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
+    if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_posterior, d_expected, d_cov))
+        return 1;
     IBD_CUDA(cudaStreamSynchronize(e->stream));  // h_sl is read by the copy above
     settle_timers(e);
     return 0;

@@ -280,6 +280,32 @@ class Engine:
             C.c_int32(1 if is_log else 0), C.c_double(p01), C.c_double(p02), C.c_double(p12),
             C.c_void_p(d_posterior_ptr), C.c_void_p(d_expected_ptr)))
 
+    def posterior_moments_batch(self, lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-3, posterior=False):
+        """Posterior mean and covariance of the bins per IBD state (hiddengem_posterior_moments_batch): (expected
+        [n_tables, 3], cov [n_tables, 3, 3]), and with posterior=True also the per-bin posteriors [n_bins, 3]."""
+        lik = np.ascontiguousarray(lik, np.float64)
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        nt = len(off) - 1
+        post = np.zeros((int(off[-1]), 3)) if posterior else None
+        expected = np.zeros((nt, 3))
+        cov = np.zeros((nt, 3, 3))
+        self._check(self._lib.hiddengem_posterior_moments_batch(self._h, C.c_int32(nt), _ptr(off), _ptr(lik),
+                                                                C.c_int32(1 if is_log else 0), C.c_double(p01),
+                                                                C.c_double(p02), C.c_double(p12), _ptr(post), _ptr(expected),
+                                                                _ptr(cov)))
+        return (expected, cov, post) if posterior else (expected, cov)
+
+    def posterior_moments_device(self, d_lik_ptr: int, bin_offsets: np.ndarray, is_log: bool, d_expected_ptr: int,
+                                 d_cov_ptr: int, d_posterior_ptr: int = 0, table_stride: int = 0, p01=1e-3, p02=1e-6,
+                                 p12=1e-3):
+        """Device buffers in, device buffers out (hiddengem_posterior_moments_device; d_posterior_ptr 0: none);
+        bin_offsets stays on the host."""
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        self._check(self._lib.hiddengem_posterior_moments_device(
+            self._h, C.c_int32(len(off) - 1), _ptr(off), C.c_int64(table_stride), C.c_void_p(d_lik_ptr),
+            C.c_int32(1 if is_log else 0), C.c_double(p01), C.c_double(p02), C.c_double(p12),
+            C.c_void_p(d_posterior_ptr or None), C.c_void_p(d_expected_ptr), C.c_void_p(d_cov_ptr)))
+
     def tracts_batch(self, lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-3, posterior=True):
         """IBD tracts (runs of one Viterbi state) with likelihood sums and, with posterior, the mean and minimum
         posterior of their state (hiddengem_tracts_batch + hiddengem_last_tracts): (tract_offsets [n_tables + 1],

@@ -269,6 +269,32 @@ int hiddengem_posterior_batch_device(ibdgem_engine *e, int32_t n_tables, const i
                                      const double *d_lik, int32_t is_log, double p01, double p02, double p12,
                                      double *d_posterior, double *d_expected);
 
+/* Posterior moments: the posterior entries' model, emissions, uniform rule and penalties, plus the 3 x 3 posterior
+ * covariance of N_s = #{i : x_i = s}, the bins a path puts in state s.  expected[t][s] = E[N_s] (the posterior
+ * entries' expected, bit for bit, as are the posteriors) and cov[t][s][u] = Cov(N_s, N_u), exact in the model: one
+ * extra recursion in the backward pass, h_i^u[k] = E[#{j > i : x_j = u} | x_i = k], and
+ *     Cov(N_s, N_u) = sum_i gamma_i(s) (delta_su - gamma_i(u)) + gamma_i(s) (h_i^u[s] - H_i^u) + gamma_i(u) (h_i^s[u] - H_i^s)
+ * with gamma the posteriors and H_i^u = sum_k gamma_i(k) h_i^u[k] (the centred form: no E[N_s N_u] - E[N_s] E[N_u]).
+ * Each table's sums run over its bins in a fixed order: the same inputs give the same bits in any batch or layout.
+ * Rows of cov sum to 0 (sum_s N_s = n) and cov is positive semi-definite, both up to rounding.
+ *   - An empty table has expected 0 and cov 0; one bin has cov = diag(gamma) - gamma gamma^T; a table of total
+ *     weight 0 has NaN expected and NaN cov.
+ *   - Independent tables (e.g. the chromosomes of one pair) add: the means and covariances of the genome are the sums
+ *     of the tables'.  The sd of the IBD1 share is sqrt(cov[1][1]) / n; the kinship phi = (N_1 / 4 + N_2 / 2) / n has
+ *     variance (cov[1][1] / 16 + cov[2][2] / 4 + cov[1][2] / 4) / n^2.
+ *   posterior   [sum(n_bins)][3] or NULL: with NULL no per-bin array is written, and only 96 B per table come back
+ *   expected    [n_tables][3]
+ *   cov         [n_tables][3][3], symmetric
+ * Arguments, penalties and bin_offsets are checked as by hiddengem_posterior_batch. */
+int hiddengem_posterior_moments_batch(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, const double *lik,
+                                      int32_t is_log, double p01, double p02, double p12,
+                                      double *posterior, double *expected, double *cov);
+/* The same on DEVICE buffers (bin_offsets a HOST array), with the layouts of hiddengem_posterior_batch_device
+ * (table_stride = max_windows takes ibdgem_scores.w_loglik_device as is); d_posterior may be NULL. */
+int hiddengem_posterior_moments_device(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, int64_t table_stride,
+                                       const double *d_lik, int32_t is_log, double p01, double p02, double p12,
+                                       double *d_posterior, double *d_expected, double *d_cov);
+
 /* IBD tracts.  A tract is a maximal run [first_bin, first_bin + n_bins) of bins of one table with the same Viterbi
  * state (in IBDGem a "segment" is one window, i.e. one bin).  Tracts never cross tables; an empty table has none.
  * Records are ordered table by table, then by first_bin; table t's are records [tract_offsets[t], tract_offsets[t+1]).
