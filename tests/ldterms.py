@@ -24,14 +24,16 @@ import refio
 
 
 def ld_case(seed, S, N, window, targets, *, src=0, share=(), twins=None, bg=None, pu_idx=-1, opt_v=0, depth=2.0,
-            eps=0.02, max_cov=20, cull_p=1.0, keep_frac=0.97):
+            eps=0.02, max_cov=20, cull_p=1.0, keep_frac=0.97, af=None):
     """Synthetic --LD case.  Reads are drawn from individual `src` (its genotype, error rate `eps`, Poisson(`depth`)
     bases per site).  Haplotype 0 of every individual in `share` is a copy of haplotype 1 of `src` (a relative sharing
     one haplotype).  `twins` maps an individual to another whose two haplotypes it copies; copies are made after the
     shared haplotypes are planted, and the reads are drawn last.  `bg` is the background list as given on the command
-    line (order and repeats kept)."""
+    line (order and repeats kept).  `af` gives the panel's alternate-allele frequency per site (a scalar or S values);
+    by default they are drawn from Beta(0.5, 2)."""
     rng = np.random.default_rng(seed)
-    af = np.clip(rng.beta(0.5, 2.0, S), 0.01, 0.99)
+    drawn = np.clip(rng.beta(0.5, 2.0, S), 0.01, 0.99)
+    af = drawn if af is None else np.broadcast_to(np.asarray(af, np.float64), (S,))
     hap = (rng.random((S, 2 * N)) < af[:, None]).astype(np.uint8)
     for t in share:
         hap[:, 2 * t] = hap[:, 2 * src + 1]
@@ -146,6 +148,39 @@ def column_terms(case, window_sites, target):
 
 def kappa(eps):
     return float(np.log(4 * eps * (1 - eps)))
+
+
+def depth_coefficients(eps, max_cov):
+    """(alpha, beta, kappa) of the depth-linear class table, read off the oracle's ln P(D|G): one REF base adds alpha
+    to l1 - l0, one ALT base adds beta, and every base adds kappa to l2 - 2 l1 + l0."""
+    L = ln_pdg(eps, max_cov)
+    return L[1, 0, 1] - L[1, 0, 0], L[0, 1, 1] - L[0, 1, 0], L[1, 0, 2] - 2 * L[1, 0, 1] + L[1, 0, 0]
+
+
+def mma_mode(eps, ncols):
+    """(table, delta, dpos) of the ld_mma epilogue for `ncols` background haplotype columns: the screen's reach in key
+    units, the head-room a row's maximum may climb above its reference key before the reference moves, and whether
+    the exp table (delta + dpos + 1 entries of at most 512) is used.  Mirrors screen_nats and ld_mma.cu:1377-1387."""
+    k = -kappa(eps)
+    screen = min(32.0, np.log(max(ncols, 2)) + 16.2)
+    delta = int(np.ceil(screen / k)) + 2
+    dpos = int(min(256.0, np.floor(600.0 / k)))
+    return dpos >= 8 and delta + dpos + 1 <= 512, delta, dpos
+
+
+def screen_operands(case, sites, target):
+    """Y[k] + kappa M[a_i, k] in float64 for each target haplotype row i and background column k (column_terms'
+    order): the part of a term that the window's C0 + R[a_i] does not carry, and what ld_vmma screens in fp32."""
+    pk = case.pk
+    alpha, beta, kap = depth_coefficients(case.params.epsilon, case.params.max_cov)
+    s = np.asarray(sites)
+    nr, na = pk.n_ref[s].astype(np.float64), pk.n_alt[s].astype(np.float64)
+    bgU = column_terms(case, sites, target).bgU
+    cols = pk.hap[s][:, np.stack([2 * bgU, 2 * bgU + 1], axis=1).ravel()].astype(np.float64)  # [W, 2 nU]
+    rows = pk.hap[s][:, [2 * target, 2 * target + 1]].astype(np.float64)                      # [W, 2]
+    Y = (alpha * nr + beta * na) @ cols
+    M = (rows * (nr + na)[:, None]).T @ cols
+    return Y[None, :] + kap * M
 
 
 def first_tile_climb(terms, tile_cols):

@@ -90,3 +90,40 @@ def test_thinned_view_reproduces_the_oracle_under_downsampling(opt_v):
         for w, sites in enumerate(wins):
             got = np.array(lt.column_terms(view, sites, t).libd())
             assert np.all(np.abs(got - ora["w_log"][w, :2]) <= 1e-9), (k, w, got, ora["w_log"][w, :2])
+
+
+@pytest.mark.parametrize("eps,nats", [(0.001, 596), (0.02, 598), (0.1, 262), (0.3, 45)])
+def test_mma_mode_table_at_the_usual_error_rates(eps, nats):
+    """Table mode, with the head-room dpos |kappa| a row's maximum may climb before its reference key moves."""
+    table, delta, dpos = lt.mma_mode(eps, 600)
+    assert table and delta + dpos + 1 <= 512
+    assert round(dpos * -lt.kappa(eps)) == nats
+
+
+def test_mma_mode_switches_to_the_exp_path():
+    """At 600 columns the table holds the screen's reach up to eps = 0.353; from 0.354 on the exp path runs, and at
+    0.45 the reach is thousands of keys."""
+    assert lt.mma_mode(0.353, 600) == (True, 252, 256)
+    assert lt.mma_mode(0.354, 600) == (False, 256, 256)
+    assert not lt.mma_mode(0.45, 600)[0] and lt.mma_mode(0.45, 600)[1] > 2000
+    # the screen's reach grows with ln(ncols) up to 32 nats
+    assert lt.mma_mode(0.02, 2)[1] == 9 and lt.mma_mode(0.02, 40962)[1] == 13
+
+
+@pytest.mark.parametrize("opt_v", [0, 1])
+def test_screen_operands_complete_the_column_terms(opt_v):
+    """C0 + R[a_i] + (Y + kappa M) is the LIBD1 term of every row and column, with alpha, beta, kappa read off the
+    oracle's P(D|G); frequencies given to the builder reach the panel."""
+    case = lt.ld_case(8, 1500, 30, 200, [4], src=17, share=[4], depth=9.0, max_cov=40, eps=0.01, opt_v=opt_v, af=0.9)
+    assert abs(case.pk.hap.mean() - 0.9) < 0.01
+    alpha, beta, kap = lt.depth_coefficients(0.01, 40)
+    assert np.isclose(alpha, np.log(0.5 / 0.99)) and np.isclose(beta, np.log(50)) and np.isclose(kap, lt.kappa(0.01))
+    L = lt.ln_pdg(0.01, 40)
+    pk = case.pk
+    for sites in lt.windows(case, 4):
+        C0 = L[pk.n_ref[sites], pk.n_alt[sites], 0].sum()
+        a = pk.hap[sites][:, [8, 9]].astype(np.float64)
+        R = (alpha * pk.n_ref[sites] + beta * pk.n_alt[sites]) @ a
+        got = C0 + R[:, None] + lt.screen_operands(case, sites, 4)
+        want = lt.column_terms(case, sites, 4).l1
+        assert np.abs(got - want).max() <= 1e-9 * np.abs(want).max()
