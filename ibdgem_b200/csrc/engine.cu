@@ -462,7 +462,9 @@ window_nonld_kernel(SiteView v, WindowMapView m, const int32_t *__restrict__ tar
 // shared load per site and target), and LIBD0 — the same for every target — is summed once per CTA
 // from the values the threads stage.
 constexpr int NONLD_TILE = 256;  // sites staged per pass
-template <int NONLD_BATCH>  // genotype loads in flight per thread
+// genotype loads in flight per thread (measured 0.154 / 0.181 / 0.242 ms at C2 for 8 / 16 / 32: more loads in flight
+// cost more in resident CTAs than they save)
+constexpr int NONLD_BATCH = 8;
 __global__ void __launch_bounds__(128)
 window_nonld_shared_kernel(SiteView v, WindowMapView m, const int32_t *__restrict__ targets, int T,
                            const uint64_t *__restrict__ pos, const uint8_t *__restrict__ status,
@@ -1620,11 +1622,8 @@ static int score_common(ibdgem_engine *e, int32_t T, const int32_t *targets, int
         {
             LaunchScope ls(e, K_WINDOW_NONLD);
             if (shared) {
-                // IBDGEM_NONLD_BATCH: 8 / 16 / 32 genotype loads in flight per thread (A/B: measured 0.154 / 0.181 / 0.242 ms at C2 — more loads in flight cost more in resident CTAs than they save)
-                static const int batch = [] { const char *sb = getenv("IBDGEM_NONLD_BATCH"); return sb ? atoi(sb) : 8; }();
                 const dim3 grid((unsigned)std::max(e->nW_shared, 1), (unsigned)((T + 127) / 128));
-                auto kern = batch >= 32 ? window_nonld_shared_kernel<32> : (batch >= 16 ? window_nonld_shared_kernel<16> : window_nonld_shared_kernel<8>);
-                kern<<<grid, 128, 0, e->stream>>>(v, m, d_targets, T, e->d_pos, e->d_status, e->d_lnlik7, outW, d_wll, d_wn, d_ws, d_we, d_nwout);
+                window_nonld_shared_kernel<<<grid, 128, 0, e->stream>>>(v, m, d_targets, T, e->d_pos, e->d_status, e->d_lnlik7, outW, d_wll, d_wn, d_ws, d_we, d_nwout);
             } else {
                 const int64_t warps = (int64_t)nWT;
                 window_nonld_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, e->stream>>>(

@@ -249,6 +249,21 @@ constexpr size_t PANEL_CHUNK_MIN_BYTES = (size_t)16 << 20;  // ~0.3 ms of PCIe; 
 void ld_tensor_invalidate(ibdgem_engine *e);
 // site-major bits -> [block][haplotype][WP32 words] for `nwin` blocks of Wpad slots listed in `infsite` (ld_mma.cu)
 int ld_transpose_launch(ibdgem_engine *e, int w_begin, int w_end, const int32_t *infsite, int Wpad, int WP32, int H, uint32_t *tbits);
+// The call's background as both tensor paths see it (ld_mma.cu): the unique individuals in ascending order with
+// ln(multiplicity) — the pileup's own individual never contributes (src/ibdgem.c:714) — and per target its own index in
+// that list (-1: none) and nb, the background size without it, with ln nb (NaN when nb = 0: 0/0 in the reference).
+struct LdBackground {
+    std::vector<int32_t> bgU;
+    std::vector<double> lnc;
+    std::vector<int32_t> own;
+    std::vector<int64_t> nb;
+    std::vector<double> lognb;
+};
+void ld_background(int32_t N, int32_t T, const int32_t *h_targets, int32_t n_bg, const int32_t *h_bg, int32_t pu_idx, LdBackground *out);
+// device alias of the caller's host table e->h_wll_out when it is page-locked and mapped, else nullptr (ld_mma.cu)
+double *host_table_alias(ibdgem_engine *e);
+// *ev = e->range_ev[k], creating the events up to k as needed (ld_mma.cu)
+int range_event(ibdgem_engine *e, size_t k, cudaEvent_t *ev);
 // per-target-window tensor path (ld_vmma.cu): -v / -D
 bool ld_vtensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t n_bg);
 int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const int32_t *d_targets, int32_t n_bg, const int32_t *h_bg,

@@ -24,8 +24,6 @@
 // ld_expand_bg, ld_expand_tgt, ld_windows, ld_mma, ld_ibd0 (per call).
 #include <cuda.h>
 #include <math.h>
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
@@ -56,7 +54,6 @@ struct LdCache {
 
 constexpr int KEY_PAD = -(1 << 30);   // key of padding / excluded columns
 constexpr int KEY_INIT = -(1 << 29);  // initial running maximum
-constexpr double SCREEN_NATS = 32.0;
 constexpr int MAX_GRID_Y = 65535;  // windows ride on gridDim.y of the transposition and expansion kernels
 constexpr size_t LD_OPERAND_BUDGET = (size_t)12 << 30;  // bytes of expanded int8 operands per window batch
 
@@ -154,18 +151,11 @@ ld_transpose_kernel(int w_off, const uint32_t *__restrict__ bits, int64_t Wh, in
 // ---------------------------------------------------------------------------------------------
 // per-call kernels
 
-__device__ __forceinline__ uint32_t spread4(uint32_t nib) { return (nib * 0x00204081u) & 0x01010101u; }
 // One 32-site word of a haplotype as 0/1 bytes (eight 32-bit lanes of four sites).
 __device__ __forceinline__ void spread32(uint32_t x, uint32_t (&e)[8]) {
 #pragma unroll
     for (int k = 0; k < 8; k++) e[k] = spread4((x >> (4 * k)) & 15u);
 }
-__device__ __forceinline__ unsigned warp_sum(unsigned v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
 // K_LD_STAGE: words from pinned (mapped) host memory to the device
 __global__ void __launch_bounds__(256) ld_stage_kernel(uint32_t *__restrict__ dst, const uint32_t *__restrict__ src, int n) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -438,32 +428,30 @@ constexpr int ETAB_N = 512;           // entries of the exp(|kappa| d) table in 
 // unit ahead of the MMA issuer (operand rings), which is at most two tiles ahead of the epilogue
 // (accumulator slots), which is at most one unit ahead of the merge warps (bar 2) — 3 < URING.
 
-// CG = CTAs per MMA (tcgen05 cta_group).  CG = 2 pairs two SMs on one 256 x 256 tile: each CTA keeps
-// its own 128 target rows resident and streams HALF of every background tile, which halves the
-// shared-memory traffic per MMA — the resource ncu showed saturated with CG = 1.
-template <int CG_, int NSTAGE_>
-struct Cfg {
-    static constexpr int CG = CG_, NSTAGE = NSTAGE_;
-    static constexpr int TILE_N = BN * CG;          // accumulator tile columns
-    static constexpr int NACC = 512 / TILE_N;       // TMEM accumulator slots
-    static constexpr int SETCOLS = TILE_N / NSETS;  // accumulator columns per epilogue set
-    static constexpr int THREADS = 128 + NSETS * 128;
-    static constexpr int OFF_A = 0;
-    static constexpr int OFF_B = OFF_A + MAXKB * A_SLAB;
-    static constexpr int OFF_KEYS = OFF_B + NSTAGE * B_SLAB;             // per epilogue warp: 128 int32
-    static constexpr int OFF_MERGE = OFF_KEYS + NSETS * 4 * SETCOLS * 4;  // NSETS x 128 x double2: the sets' (max, sum) per row
-    static constexpr int OFF_KMAX = OFF_MERGE + NSETS * BM * 16;          // 2 x 128 int32, shared by the sets
-    static constexpr int OFF_BAR = OFF_KMAX + 2 * BM * 4;
-    static constexpr int NBAR = 2 * MAXKB + 2 * NSTAGE + 2 * NACC + URING;
-    static constexpr int OFF_TMEM = OFF_BAR + NBAR * 8;
-    static constexpr int OFF_URING = OFF_TMEM + 16;                      // URING unit numbers handed out by the scheduler
-    static constexpr int OFF_ETAB = OFF_URING + URING * 4;               // ETAB_N doubles: exp(|kappa| d) over the screen's reach
-    static constexpr int SMEM_BYTES = OFF_ETAB + ETAB_N * 8 + 1024;      // + alignment slack
-    static constexpr uint32_t IDESC = (2u << 4) /* D = s32 */ | (0u << 7) /* A = u8 */ | (0u << 10) /* B = u8 */ |
-                                      ((uint32_t)(TILE_N >> 3) << 17) | ((uint32_t)((BM * CG) >> 4) << 24);
-    static_assert(SMEM_BYTES <= 232448, "over the 227 KB shared memory limit");
-    static_assert(SETCOLS % 32 == 0 && SETCOLS <= BN, "epilogue sets split the tile into 32-column chunks");
-};
+// CTA pairs (tcgen05 cta_group::2) on 256 x 256 tiles: each CTA keeps its own 128 target rows resident and streams
+// HALF of every background tile, which halves the shared-memory traffic per MMA — the resource ncu showed saturated
+// with single-CTA 128 x 128 tiles.
+constexpr int CG = 2;                           // CTAs per MMA
+constexpr int NSTAGE = 5;                       // background stages
+constexpr int TILE_N = BN * CG;                 // accumulator tile columns
+constexpr int NACC = 512 / TILE_N;              // TMEM accumulator slots
+constexpr int SETCOLS = TILE_N / NSETS;         // accumulator columns per epilogue set
+constexpr int THREADS = 128 + NSETS * 128;
+constexpr int OFF_A = 0;
+constexpr int OFF_B = OFF_A + MAXKB * A_SLAB;
+constexpr int OFF_KEYS = OFF_B + NSTAGE * B_SLAB;             // per epilogue warp: 128 int32
+constexpr int OFF_MERGE = OFF_KEYS + NSETS * 4 * SETCOLS * 4;  // NSETS x 128 x double2: the sets' (max, sum) per row
+constexpr int OFF_KMAX = OFF_MERGE + NSETS * BM * 16;          // 2 x 128 int32, shared by the sets
+constexpr int OFF_BAR = OFF_KMAX + 2 * BM * 4;
+constexpr int NBAR = 2 * MAXKB + 2 * NSTAGE + 2 * NACC + URING;
+constexpr int OFF_TMEM = OFF_BAR + NBAR * 8;
+constexpr int OFF_URING = OFF_TMEM + 16;                      // URING unit numbers handed out by the scheduler
+constexpr int OFF_ETAB = OFF_URING + URING * 4;               // ETAB_N doubles: exp(|kappa| d) over the screen's reach
+constexpr int SMEM_BYTES = OFF_ETAB + ETAB_N * 8 + 1024;      // + alignment slack
+constexpr uint32_t IDESC = (2u << 4) /* D = s32 */ | (0u << 7) /* A = u8 */ | (0u << 10) /* B = u8 */ |
+                           ((uint32_t)(TILE_N >> 3) << 17) | ((uint32_t)((BM * CG) >> 4) << 24);
+static_assert(SMEM_BYTES <= 232448, "over the 227 KB shared memory limit");
+static_assert(SETCOLS % 32 == 0 && SETCOLS <= BN, "epilogue sets split the tile into 32-column chunks");
 
 struct Params {
     int w0;                  // first window of this batch (operands hold windows w0 .. w0 + nW - 1)
@@ -484,25 +472,11 @@ struct Params {
     const double *lognb4;    // [T] ln(4 n_refpanel) or NaN
     double *wll;             // [T][outW][3]
     double *wll_host;        // the same table in the caller's page-locked host memory (device alias), or nullptr
-    int debug;               // IBDGEM_MMA_DEBUG experiments (0 = product behaviour)
-    int warm_tiles;          // leading tiles of a unit whose maximum is taken before they are screened
     int *unit_counter;       // next unit to hand out (zeroed before the launch)
-    int pf_tiles;            // L2 prefetch distance of the background stream, in tiles
-    unsigned long long *trace;  // IBDGEM_MMA_TRACE: [4][1024] event log of CTA 0 (nullptr = off)
 };
-// event log entry: clock64 << 16 | event << 12 | tile; one lane per traced warp writes
-#define IBD_TRACE(role, ev, tile)                                                                          \
-    do {                                                                                                   \
-        if (p.trace && blockIdx.x == 0 && lane == 0 && tr_n < 1024 && (p.debug != 9 || (ev) == 5))        \
-            p.trace[(role) * 1024 + tr_n++] = ((unsigned long long)clock64() << 16) | ((ev) << 12) | ((tile) & 0xfff); \
-    } while (0)
 
-template <class CF>
-__global__ void __launch_bounds__(CF::THREADS, 1)
+__global__ void __launch_bounds__(THREADS, 1)
 ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__ CUtensorMap tmapB, const Params p) {
-    constexpr int CG = CF::CG, NSTAGE = CF::NSTAGE, NACC = CF::NACC, TILE_N = CF::TILE_N;
-    constexpr int OFF_A = CF::OFF_A, OFF_B = CF::OFF_B, OFF_KEYS = CF::OFF_KEYS, OFF_MERGE = CF::OFF_MERGE;
-    constexpr int OFF_BAR = CF::OFF_BAR, OFF_TMEM = CF::OFF_TMEM, OFF_KMAX = CF::OFF_KMAX;
     extern __shared__ unsigned char smem_raw[];
     unsigned char *smem = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem + OFF_BAR);
@@ -512,21 +486,13 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
     uint64_t *b_full = bars + 2 * MAXKB, *b_empty = b_full + NSTAGE;
     uint64_t *acc_full = b_empty + NSTAGE, *acc_empty = acc_full + NACC;
     uint64_t *ufull = acc_empty + NACC;
-    int *uring = reinterpret_cast<int *>(smem + CF::OFF_URING);
+    int *uring = reinterpret_cast<int *>(smem + OFF_URING);
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(smem + OFF_TMEM);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint32_t rank = 0;  // CTA rank in the pair; rank 0 issues the MMAs
-    if constexpr (CG == 2) asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+    uint32_t rank;  // CTA rank in the pair; rank 0 issues the MMAs
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
 
-    if (p.trace && warp == 1 && lane == 0 && blockIdx.x < 256) {  // per-CTA start stamp (global timer, ns)
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        p.trace[3 * 1024 + blockIdx.x * 4] = t;
-        unsigned smid;
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        p.trace[3 * 1024 + blockIdx.x * 4 + 2] = smid;
-    }
     if (warp == 0 && lane == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmapA) : "memory");
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmapB) : "memory");
@@ -540,20 +506,15 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
     }
     if (warp == 3)
         for (int i = lane; i < 2 * BM; i += 32) reinterpret_cast<int *>(smem + OFF_KMAX)[i] = KEY_INIT;
-    for (int i = threadIdx.x; i < p.tab_n; i += CF::THREADS)
-        reinterpret_cast<double *>(smem + CF::OFF_ETAB)[i] = exp(-p.kappa * (double)(i - p.delta));
+    for (int i = threadIdx.x; i < p.tab_n; i += THREADS)
+        reinterpret_cast<double *>(smem + OFF_ETAB)[i] = exp(-p.kappa * (double)(i - p.delta));
     if (warp == 2) {
-        if constexpr (CG == 1) {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
     }
     tc_fence_before();
     __syncthreads();
-    if constexpr (CG == 2) cluster_sync_all();  // peer barriers are initialised before anyone signals them
+    cluster_sync_all();  // peer barriers are initialised before anyone signals them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
 
@@ -575,7 +536,7 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
             int pending = -1;
             if (rank == 0) {
                 u_next = fetch_unit();
-                unit_publish<CG>(uring, ufull, 0, u_next);
+                unit_publish(uring, ufull, 0, u_next);
                 pending = atomicAdd(p.unit_counter, 1);
             }
             for (int it = 0;; it++) {
@@ -591,24 +552,24 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
                 auto load_a = [&](int kb) {
                     mbar_wait(a_empty + kb, (uint32_t)((it & 1) ^ 1));
                     if (rank == 0) mbar_expect_tx(a_full + kb, (uint32_t)(CG * A_SLAB));
-                    tma_load_3d_cg<CG>(smem + OFF_A + kb * A_SLAB, &tmapA, a_full + kb, kb * KBYTES, (mb * CG + (int)rank) * BM, w);
+                    tma_load_3d_cg(smem + OFF_A + kb * A_SLAB, &tmapA, a_full + kb, kb * KBYTES, (mb * CG + (int)rank) * BM, w);
                 };
                 for (int n = 0; n < p.NT; n++)
                     for (int kb = 0; kb < p.KB; kb++) {
                         // the unit's target k-blocks are interleaved with its first background tile, in
                         // the order the MMA issuer needs them
                         if (n == 0) load_a(kb);
-                        if (n + p.pf_tiles < p.NT)  // pull the same k-block of a later tile into L2
-                            tma_prefetch_3d(&tmapB, kb * KBYTES, ((n + p.pf_tiles) * CG + (int)rank) * BN, w);
+                        if (n + PF_TILES < p.NT)  // pull the same k-block of a later tile into L2
+                            tma_prefetch_3d(&tmapB, kb * KBYTES, ((n + PF_TILES) * CG + (int)rank) * BN, w);
                         mbar_wait(b_empty + st, ph ^ 1u);
                         if (rank == 0) mbar_expect_tx(b_full + st, (uint32_t)(CG * B_SLAB));
-                        tma_load_3d_cg<CG>(smem + OFF_B + st * B_SLAB, &tmapB, b_full + st, kb * KBYTES,
+                        tma_load_3d_cg(smem + OFF_B + st * B_SLAB, &tmapB, b_full + st, kb * KBYTES,
                                            (n * CG + (int)rank) * BN, w);
                         if (++st == NSTAGE) { st = 0; ph ^= 1u; }
                     }
                 if (rank == 0) {
                     u_next = pending < p.n_units ? pending : -1;
-                    unit_publish<CG>(uring, ufull, it + 1, u_next);
+                    unit_publish(uring, ufull, it + 1, u_next);
                     if (u_next >= 0) pending = atomicAdd(p.unit_counter, 1);
                 }
             }
@@ -621,7 +582,6 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
             uint32_t ph = 0;
             int it = 0;
             uint32_t g = 0;  // accumulator tile counter
-            int tr_n = 0;
             const uint64_t adesc0 = umma_desc_sw128(smem_u32(smem + OFF_A));
             const uint64_t bdesc0 = umma_desc_sw128(smem_u32(smem + OFF_B));
             for (;; it++) {
@@ -630,9 +590,7 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
                 for (int n = 0; n < p.NT; n++, g++) {
                     const bool first = n == 0, last = n == p.NT - 1;
                     const uint32_t acc = g % NACC, use = g / NACC;
-                    IBD_TRACE(0, 1, g);
                     mbar_wait(acc_empty + acc, (use & 1u) ^ 1u);
-                    IBD_TRACE(0, 2, g);
                     const uint32_t d_tmem = tmem_base + acc * TILE_N;
                     // two k-blocks per trip: both barrier probes are in flight together
                     for (int kb = 0; kb < p.KB; kb += 2) {
@@ -642,15 +600,11 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
                         if (st2 == NSTAGE) { st2 = 0; ph2 ^= 1u; }
                         const bool r1 = mbar_test(b_full + st, ph);
                         const bool r2 = two ? mbar_test(b_full + st2, ph2) : true;
-                        if (!r1 || !r2) IBD_TRACE(0, 3, g);
                         if (!r1) mbar_wait(b_full + st, ph);
                         if (!r2) mbar_wait(b_full + st2, ph2);
-                        if (!r1 || !r2) IBD_TRACE(0, 4, g);
                         if (first) {  // the unit's target k-blocks arrive one by one
-                            IBD_TRACE(0, 6, kb);
                             mbar_wait(a_full + kb, (uint32_t)(it & 1));
                             if (two) mbar_wait(a_full + kb + 1, (uint32_t)(it & 1));
-                            IBD_TRACE(0, 7, kb);
                         }
                         tc_fence_after();
                         if (elect_one()) {
@@ -658,29 +612,27 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
                             const uint64_t bd = bdesc0 + (uint64_t)((st * B_SLAB) >> 4);
 #pragma unroll
                             for (int k = 0; k < KBYTES / UK; k++)
-                                umma_i8_cg<CG>(d_tmem, ad + (uint64_t)(k * (UK >> 4)), bd + (uint64_t)(k * (UK >> 4)), CF::IDESC,
-                                               (uint32_t)((kb | k) != 0));
-                            tc_commit_cg<CG>(b_empty + st);
-                            if (last) tc_commit_cg<CG>(a_empty + kb);
+                                umma_i8_cg(d_tmem, ad + (uint64_t)(k * (UK >> 4)), bd + (uint64_t)(k * (UK >> 4)), IDESC,
+                                           (uint32_t)((kb | k) != 0));
+                            tc_commit_cg(b_empty + st);
+                            if (last) tc_commit_cg(a_empty + kb);
                             if (two) {
                                 const uint64_t ad2 = ad + (uint64_t)(A_SLAB >> 4);
                                 const uint64_t bd2 = bdesc0 + (uint64_t)((st2 * B_SLAB) >> 4);
 #pragma unroll
                                 for (int k = 0; k < KBYTES / UK; k++)
-                                    umma_i8_cg<CG>(d_tmem, ad2 + (uint64_t)(k * (UK >> 4)), bd2 + (uint64_t)(k * (UK >> 4)), CF::IDESC, 1u);
-                                tc_commit_cg<CG>(b_empty + st2);
-                                if (last) tc_commit_cg<CG>(a_empty + kb + 1);
+                                    umma_i8_cg(d_tmem, ad2 + (uint64_t)(k * (UK >> 4)), bd2 + (uint64_t)(k * (UK >> 4)), IDESC, 1u);
+                                tc_commit_cg(b_empty + st2);
+                                if (last) tc_commit_cg(a_empty + kb + 1);
                             }
-                            if (kb + 2 >= p.KB) tc_commit_cg<CG>(acc_full + acc);
+                            if (kb + 2 >= p.KB) tc_commit_cg(acc_full + acc);
                         }
                         __syncwarp();
                         if (two) { st = st2; ph = ph2; }
                         if (++st == NSTAGE) { st = 0; ph ^= 1u; }
                     }
                 }
-                IBD_TRACE(0, 5, (u_cur % p.MB) | (((u_cur / p.MB) & 0x1ff) << 3));
             }
-            if (p.trace && lane == 0 && blockIdx.x < 256) p.trace[3 * 1024 + blockIdx.x * 4 + 3] = (unsigned long long)it;
         }
     } else {
         // ===== merge warps (2, 3): at the end of every unit the four epilogue sets leave their partial
@@ -747,7 +699,6 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
         // every set works on every tile: set q owns columns [q * SETCOLS, (q + 1) * SETCOLS) of the
         // accumulator, so all four epilogue warps of a scheduler drain the slot together and the
         // slot is handed back to the MMA issuer in half the time; each thread owns one target row
-        constexpr int SETCOLS = CF::SETCOLS;
         const int ew = warp - EPI_WARP0, set = ew >> 2, quarter = warp & 3;
         const int rloc = quarter * 32 + lane;
         int *skeys = reinterpret_cast<int *>(smem + OFF_KEYS) + ew * SETCOLS;
@@ -755,8 +706,6 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
         int *skmax_all = reinterpret_cast<int *>(smem + OFF_KMAX);
         uint32_t g0 = 0;  // tile counter at the start of the unit
         int it = 0;
-        int tr_n = 0;
-        const int tr_role = ew == 0 ? 1 : (ew == 15 ? 2 : 3);
         for (;; it++, g0 += (uint32_t)p.NT) {
             const int u = unit_of(uring, ufull, it);
             if (u < 0) break;
@@ -770,7 +719,7 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
             // candidate path, which is what rows with many near-maximal columns (a pileup whose source is not in the
             // background) spend their time on.  The row's partial is (|kappa| vref, s).
             const bool tab = p.tab_n > 0;
-            const double *etab = reinterpret_cast<const double *>(smem + CF::OFF_ETAB);
+            const double *etab = reinterpret_cast<const double *>(smem + OFF_ETAB);
             const double *rpw = (tab ? p.Fp : p.Rp) + (size_t)w * p.ncolpad;
             int vref = KEY_INIT;
             int kmax = row_ok ? KEY_INIT : (1 << 30);  // padding rows never reach the fp64 path
@@ -806,9 +755,7 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
                 const bool own_here = own0 >= col0 && own0 < col0 + SETCOLS;
                 const bool any_own = __any_sync(0xffffffffu, own_here);
                 kmax = max(kmax, *skmax);
-                if (tr_role < 3) IBD_TRACE(tr_role, 1, g);
                 mbar_wait_relaxed(acc_full + slot, use & 1u);
-                if (tr_role < 3) IBD_TRACE(tr_role, 2, g);
                 tc_fence_after();
                 const uint32_t taddr = tmem_base + slot * TILE_N + set * SETCOLS + ((uint32_t)(quarter * 32) << 16);
                 // chunk c of this warp's columns: v[j] = key[j] - M[row, j], returns the chunk maximum
@@ -840,7 +787,7 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
                     c0 = __vimax3_s32(c0, v[7], c1); c2 = __vimax3_s32(c2, v[15], c3);
                     return __vimax3_s32(c0, c2, max(v[23], v[31]));
                 };
-                if (n < p.warm_tiles && p.debug != 1) {
+                if (n == 0) {
                     // The screen is relative to the RUNNING row maximum, which starts at -inf: without
                     // help the first tile of a unit sends nearly every element down the fp64 path
                     // (measured: ~40k cycles per unit, 1/3 of the kernel).  So the first tile is read
@@ -861,7 +808,6 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
                 }
 #pragma unroll
                 for (int c = 0; c < NCH; c++) {
-                    if (p.debug == 1) break;  // roofline experiment: MMA + operand feed only
                     int v[32];
                     const int cm = load_chunk(c, v);
                     if (cm > kmax) {
@@ -904,123 +850,33 @@ ld_mma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__
                 }
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) mbar_arrive_leader<CG>(acc_empty + slot);
-                if (tr_role < 3) IBD_TRACE(tr_role, 3, g);
+                if (lane == 0) mbar_arrive_leader(acc_empty + slot);
             }
             // hand the partial (max, sum) of this set's columns to the merge warps and move on
             if (set == 0) skmax_all[((it + 1) & 1) * BM + rloc] = KEY_INIT;  // next unit's slot (idle since unit it - 1)
-            if (tr_role < 3) IBD_TRACE(tr_role, 4, g0);
             asm volatile("bar.sync 2, %0;" ::"n"(NSETS * 128 + 64) : "memory");  // previous unit's partials consumed
             merge[set * BM + rloc] = tab ? make_double2(-p.kappa * (double)vref, s) : make_double2(m, s);
             asm volatile("bar.arrive 1, %0;" ::"n"(NSETS * 128 + 64) : "memory");
-            if (tr_role < 3) IBD_TRACE(tr_role, 7, g0);
         }
     }
 
     tc_fence_before();
     __syncthreads();
-    if (p.trace && warp == 1 && lane == 0 && blockIdx.x < 256) {  // per-CTA end stamp
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        p.trace[3 * 1024 + blockIdx.x * 4 + 1] = t;
-    }
-    if constexpr (CG == 2) cluster_sync_all();  // the peer's shared memory and barriers stay alive until both are done
+    cluster_sync_all();  // the peer's shared memory and barriers stay alive until both are done
     if (warp == 2) {
         tc_fence_after();
-        if constexpr (CG == 1)
-            asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-        else
-            asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
     }
 }
 }  // namespace mma
 
 // ---------------------------------------------------------------------------------------------
 // host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-static EncodeTiledFn get_encode_fn() {
-    static const EncodeTiledFn fn = [] {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || !p)
-            return (EncodeTiledFn) nullptr;
-        return reinterpret_cast<EncodeTiledFn>(p);
-    }();
-    return fn;
-}
-
-// [windows][rows][Wpad] bytes, box = 128 bytes x 128 rows, 128-byte swizzle, zero fill outside
+// [windows][rows][Wpad] bytes, box = 128 bytes x 128 rows
 static int make_operand_map(CUtensorMap *m, void *base, int Wpad, int rows, int nW) {
-    EncodeTiledFn fn = get_encode_fn();
-    if (!fn) {
-        set_error("[::] ERROR: cuTensorMapEncodeTiled is not available from the CUDA driver.");
-        return 1;
-    }
-    const cuuint64_t dims[3] = {(cuuint64_t)Wpad, (cuuint64_t)rows, (cuuint64_t)nW};
-    const cuuint64_t strides[2] = {(cuuint64_t)Wpad, (cuuint64_t)Wpad * (cuuint64_t)rows};
-    const cuuint32_t box[3] = {(cuuint32_t)mma::KBYTES, (cuuint32_t)mma::BM, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    const CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_error("[::] ERROR: cuTensorMapEncodeTiled failed (%d) for a %d x %d x %d operand.", (int)r, Wpad, rows, nW);
-        return 1;
-    }
-    return 0;
-}
-
-template <class CF>
-static int launch_mma_cfg(int n_units, int sm_count, cudaStream_t st, const CUtensorMap &a, const CUtensorMap &b,
-                          const mma::Params &p) {
-    // function attributes are per device (the command-line front-end drives one engine per GPU from
-    // threads of one process); setting it is cheap enough to do on every launch
-    IBD_CUDA(cudaFuncSetAttribute(mma::ld_mma_kernel<CF>, cudaFuncAttributeMaxDynamicSharedMemorySize, CF::SMEM_BYTES));
-    const int groups = std::max(1, std::min(n_units, sm_count / CF::CG));  // persistent: one CTA (pair) per SM (pair)
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(groups * CF::CG));
-    cfg.blockDim = dim3((unsigned)CF::THREADS);
-    cfg.dynamicSmemBytes = CF::SMEM_BYTES;
-    cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = CF::CG;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    IBD_CUDA(cudaLaunchKernelEx(&cfg, mma::ld_mma_kernel<CF>, a, b, p));
-    return 0;
-}
-// IBDGEM_MMA_VARIANT: 2 = CTA pairs (cta_group::2, 256 x 256 tiles; default), 1 = single CTA
-// (128 x 128 tiles; shared-memory bound, kept for A/B measurement)
-static int mma_variant() {
-    static const int v = [] {
-        const char *s = getenv("IBDGEM_MMA_VARIANT");
-        return s ? atoi(s) : 2;
-    }();
-    return v;
-}
-static int mma_cg(int variant) { return variant == 1 ? 1 : 2; }
-static int launch_mma(int variant, int n_units, int sm_count, cudaStream_t st, const CUtensorMap &a, const CUtensorMap &b,
-                      const mma::Params &p) {
-    if (variant == 1) return launch_mma_cfg<mma::Cfg<1, 5>>(n_units, sm_count, st, a, b, p);
-    return launch_mma_cfg<mma::Cfg<2, 5>>(n_units, sm_count, st, a, b, p);
-}
-// Screening distance in nats.  An element more than D below its row maximum contributes at most
-// e^-D of the row's sum, so dropping every such element of a row with `ncols` columns changes the
-// row's log-sum-exp by less than ncols * e^-D.  D = ln(ncols) + ln(1e7) keeps that below 1e-7 (the
-// window tolerance is 1e-6); IBDGEM_SCREEN_NATS overrides it.
-static double screen_nats(int ncols) {
-    static const double forced = [] {  // validated before it is published
-        const char *s = getenv("IBDGEM_SCREEN_NATS");
-        const double f = s ? atof(s) : 0.0;
-        return (f >= 8.0 && f <= 700.0) ? f : 0.0;
-    }();
-    if (forced > 0.0) return forced;
-    return std::min(SCREEN_NATS, log((double)std::max(ncols, 2)) + 16.2);
+    return encode_u8_3d(m, base, {(cuuint64_t)Wpad, (cuuint64_t)rows, (cuuint64_t)nW}, {(cuuint64_t)Wpad, (cuuint64_t)Wpad * rows},
+                        {(cuuint32_t)mma::KBYTES, (cuuint32_t)mma::BM, 1});
 }
 
 bool ld_tensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t n_bg, const uint8_t *tgt_counts) {
@@ -1108,6 +964,51 @@ int ld_transpose_launch(ibdgem_engine *e, int w_begin, int w_end, const int32_t 
     return 0;
 }
 
+void ld_background(int32_t N, int32_t T, const int32_t *h_targets, int32_t n_bg, const int32_t *h_bg, int32_t pu_idx, LdBackground *out) {
+    // (ordinals were range-checked by the caller; plain arrays — this runs on the host between two stretches of device work)
+    std::vector<int32_t> mult((size_t)N, 0), where((size_t)N, -1);
+    int64_t total_bg = 0;
+    for (int n = 0; n < n_bg; n++)
+        if (h_bg[n] != pu_idx) { mult[h_bg[n]]++; total_bg++; }
+    out->bgU.clear();
+    out->lnc.clear();
+    for (int32_t b = 0; b < N; b++)
+        if (mult[b]) {
+            where[b] = (int32_t)out->bgU.size();
+            out->bgU.push_back(b);
+            out->lnc.push_back(mult[b] == 1 ? 0.0 : log((double)mult[b]));
+        }
+    out->own.resize((size_t)T);
+    out->nb.resize((size_t)T);
+    out->lognb.resize((size_t)T);
+    for (int t = 0; t < T; t++) {
+        const int own = where[h_targets[t]];
+        const int64_t nb = total_bg - (own >= 0 ? mult[h_targets[t]] : 0);
+        out->own[t] = own;
+        out->nb[t] = nb;
+        out->lognb[t] = nb > 0 ? log((double)nb) : (double)NAN;
+    }
+}
+
+double *host_table_alias(ibdgem_engine *e) {
+    if (!e->h_wll_out) return nullptr;
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, e->h_wll_out) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
+        return static_cast<double *>(attr.devicePointer);
+    cudaGetLastError();
+    return nullptr;
+}
+
+int range_event(ibdgem_engine *e, size_t k, cudaEvent_t *ev) {
+    while (e->range_ev.size() <= k) {
+        cudaEvent_t x;
+        IBD_CUDA(cudaEventCreateWithFlags(&x, cudaEventDisableTiming));
+        e->range_ev.push_back(x);
+    }
+    *ev = e->range_ev[k];
+    return 0;
+}
+
 // Transposed bits of windows [tw_upto, w_hi).  The caller has made the engine stream
 // wait for the panel rows of those windows (wait_panel_upto / ensure_table).
 static int cache_windows(ibdgem_engine *e, int w_hi) {
@@ -1134,35 +1035,15 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
                     uint64_t *d_we, int32_t *d_nwout) {
     if (build_cache(e)) return 1;
     LdCache *c = e->ld;
-    // unique background individuals with multiplicities; the pileup's own individual never
-    // contributes (src/ibdgem.c:714), duplicates become a ln(multiplicity) weight
-    // (ordinals were range-checked by the caller; plain arrays — this runs on the host between two
-    // stretches of device work)
-    std::vector<int32_t> mult((size_t)c->N, 0), where((size_t)c->N, -1);
-    int64_t total_bg = 0;
-    for (int n = 0; n < n_bg; n++)
-        if (h_bg[n] != pu_idx) { mult[h_bg[n]]++; total_bg++; }
-    std::vector<int32_t> bgU;
-    std::vector<double> lnc;
-    bgU.reserve((size_t)c->N);
-    lnc.reserve((size_t)c->N);
-    for (int32_t b = 0; b < c->N; b++)
-        if (mult[b]) {
-            where[b] = (int32_t)bgU.size();
-            bgU.push_back(b);
-            lnc.push_back(mult[b] == 1 ? 0.0 : log((double)mult[b]));
-        }
-    const int nU = (int)bgU.size();
-    const double nan = (double)NAN;
-    std::vector<int32_t> ownU(T), row_own(2 * (size_t)T);
-    std::vector<double> lognb(T), lognb4(T);
+    // duplicate background entries become a ln(multiplicity) weight on one individual
+    LdBackground bg;
+    ld_background(c->N, T, h_targets, n_bg, h_bg, pu_idx, &bg);
+    const int nU = (int)bg.bgU.size();
+    std::vector<int32_t> row_own(2 * (size_t)T);
+    std::vector<double> lognb4(T);
     for (int t = 0; t < T; t++) {
-        const int own = where[h_targets[t]];
-        const int64_t nb = total_bg - (own >= 0 ? mult[h_targets[t]] : 0);
-        ownU[t] = own;
-        lognb[t] = nb > 0 ? log((double)nb) : nan;
-        lognb4[t] = nb > 0 ? log(4.0 * (double)nb) : nan;
-        row_own[2 * t] = row_own[2 * t + 1] = own >= 0 ? 2 * own : -1;
+        lognb4[t] = bg.nb[t] > 0 ? log(4.0 * (double)bg.nb[t]) : (double)NAN;
+        row_own[2 * t] = row_own[2 * t + 1] = bg.own[t] >= 0 ? 2 * bg.own[t] : -1;
     }
     const int nW = c->nW;
     // Window ranges: one per panel chunk still in flight (a range is the windows whose last site has
@@ -1178,12 +1059,9 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
             range_end.push_back(k + 1 == e->chunk_end.size() ? nW : w);
         }
     } else {
-        // Panel resident: one range.  IBDGEM_LD_TAIL_DIV=d splits off the last 1/d of the windows so that the
-        // first range's columns of the score table travel to the host while the second is scored; measured
-        // at C3 it buys nothing (8.70 ms one range, 8.68 ms d = 8, 8.78 ms d = 5: a second round of launches
-        // costs what the hidden 0.4 ms copy saves), so it is off by default.
-        static const int tail_div = [] { const char *st = getenv("IBDGEM_LD_TAIL_DIV"); return st ? atoi(st) : 0; }();
-        if (e->h_wll_out && tail_div > 1 && nW >= 8 * tail_div) range_end.push_back(nW - nW / tail_div);
+        // Panel resident: one range.  (Splitting off a tail range, so that the first range's columns travel to the host
+        // while the tail is scored, was measured at C3 to buy nothing: a second round of launches costs what the
+        // hidden 0.4 ms copy saves.)
         range_end.push_back(nW);
     }
     bool by_chunk = in_flight && c->tw_upto == 0;
@@ -1197,7 +1075,7 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
         // three sub-ranges when results go to the host and the shard is large: the copy of a sub-range's columns runs
         // under the next sub-range's GEMM, so only the last one's is left at the end
         const int span = shard_we - shard_wb;
-        static const int parts_env = [] { const char *sp = getenv("IBDGEM_SHARD_PARTS"); return sp ? atoi(sp) : 3; }();
+        static const int parts_env = env_int("IBDGEM_SHARD_PARTS", 3);
         // ... as long as every sub-range still keeps the persistent GEMM busy for >= 8 rounds of units (IBDGEM_SHARD_PARTS < 0
         // forces |value| parts, for tests)
         const int64_t units = (int64_t)span * ((2 * T + 255) / 256);
@@ -1239,18 +1117,14 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
         return 0;
     }
     const int ncols = 2 * nU;
-    const int variant = mma_variant();
-    const int CG = mma_cg(variant);
-    const int NT = (ncols + mma::BN * CG - 1) / (mma::BN * CG);
-    const int ncolpad = NT * mma::BN * CG;
-    const int MB = (nrows + mma::BM * CG - 1) / (mma::BM * CG);
+    const int NT = (ncols + mma::TILE_N - 1) / mma::TILE_N;
+    const int ncolpad = NT * mma::TILE_N;
+    const int MB = (nrows + mma::BM * mma::CG - 1) / (mma::BM * mma::CG);
 
     const size_t per_window = (size_t)(ncols + nrows) * c->Wpad;
     // IBDGEM_LD_BUDGET_MB: operand budget override (tests exercise the window batching with it)
-    static const size_t budget = [] {
-        const char *sb = getenv("IBDGEM_LD_BUDGET_MB");
-        return sb && atol(sb) > 0 ? (size_t)atol(sb) << 20 : LD_OPERAND_BUDGET;
-    }();
+    static const int budget_mb = env_int("IBDGEM_LD_BUDGET_MB", 0);
+    const size_t budget = budget_mb > 0 ? (size_t)budget_mb << 20 : LD_OPERAND_BUDGET;
     const int nWb = (int)std::max<size_t>(1, std::min<size_t>({(size_t)nW, budget / per_window, (size_t)MAX_GRID_Y}));
     int32_t *d_bgU, *d_ownU, *d_rowown, *d_akey;
     double *d_lnc, *d_lognb, *d_lognb4, *d_Rp, *d_Qp, *d_Rt, *d_Fp;
@@ -1276,12 +1150,12 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
         void *h_misc;
         if (pinned_stage(e, misc_d * 8 + misc_i * 4, &h_misc)) return 1;
         double *hd = static_cast<double *>(h_misc);
-        memcpy(hd, lnc.data(), (size_t)nU * 8);
-        memcpy(hd + nU, lognb.data(), (size_t)T * 8);
+        memcpy(hd, bg.lnc.data(), (size_t)nU * 8);
+        memcpy(hd + nU, bg.lognb.data(), (size_t)T * 8);
         memcpy(hd + nU + T, lognb4.data(), (size_t)T * 8);
         int32_t *hi = reinterpret_cast<int32_t *>(hd + misc_d);
-        memcpy(hi, bgU.data(), (size_t)nU * 4);
-        memcpy(hi + nU, ownU.data(), (size_t)T * 4);
+        memcpy(hi, bg.bgU.data(), (size_t)nU * 4);
+        memcpy(hi + nU, bg.own.data(), (size_t)T * 4);
         memcpy(hi + nU + T, row_own.data(), (size_t)T * 8);
         // Not a cudaMemcpyAsync: a DMA copy would queue on the host-to-device copy engine behind the panel
         // chunks still in flight and hold the scoring of the first windows back until the whole panel is up.
@@ -1296,21 +1170,13 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
     // filled range by range too
     const bool stream_dev = e->d_wll_out_device != nullptr;
     // page-locked host destination: its device alias, for stores from a kernel
-    double *h_wll_mapped = nullptr;
-    if (e->h_wll_out) {
-        cudaPointerAttributes attr;
-        if (cudaPointerGetAttributes(&attr, e->h_wll_out) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
-            h_wll_mapped = static_cast<double *>(attr.devicePointer);
-        else
-            cudaGetLastError();
-    }
+    double *h_wll_mapped = host_table_alias(e);
     // direct mode: the GEMM's merge warps store finished score triples into the page-locked host table themselves
-    static const int direct_env = [] { const char *sd = getenv("IBDGEM_LD_DIRECT_STORE"); return sd ? atoi(sd) : 1; }();
     // (not while panel chunks are still arriving: measured at C3 end to end, the 24-byte posted writes of every range
     // compete with the upload on the link — 13.3 ms against 12.6 with the per-range store kernel)
     // (nor for window shards: eight ranks scattering 24-byte writes over a 10,000-row host table — one 4 KB page per
     // write — slowed the GEMM by 15 % at C5 over 8 GPUs; there the shard's columns leave by one store kernel at the end)
-    const bool direct = direct_env && h_wll_mapped != nullptr && !by_chunk && !sharded;
+    const bool direct = h_wll_mapped != nullptr && !by_chunk && !sharded;
     if (stream_out || stream_dev || direct) {
         if (!e->d2h_stream) IBD_CUDA(cudaStreamCreateWithFlags(&e->d2h_stream, cudaStreamNonBlocking));
         e->wll_streamed = stream_out || direct;
@@ -1323,6 +1189,28 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
         const size_t q_smem = (size_t)nU * 8 <= 160 * 1024 ? (size_t)nU * 8 : 0;
         IBD_CUDA(cudaFuncSetAttribute(ld_ibd0_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
         ld_ibd0_kernel<<<wb_ - wa, 256, q_smem, e->stream>>>(wa, T, nU, outW, d_Qp, d_ownU, d_lognb, d_wll, q_smem ? 1 : 0);
+        return 0;
+    };
+    // columns [w, w + n) of d_wll to the same columns of dst [T][outW][3] on d2h_stream; many short rows go by coalesced
+    // stores from a kernel (ld_store_cols_kernel) where dst has a device address dst_dev (local, peer or mapped host
+    // memory), not by T DMA descriptors
+    auto export_cols = [&](double *dst, double *dst_dev, int w, int n) -> int {
+        if (dst_dev && T >= 256) {
+            const int64_t cnt = (int64_t)T * n * 3;
+            ld_store_cols_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, e->d2h_stream>>>(d_wll, dst_dev, T, outW, w, n);
+            e->k_launches[K_LD_WINDOWS]++;
+        } else {
+            IBD_CUDA(cudaMemcpy2DAsync(dst + (size_t)w * 3, (size_t)outW * 24, d_wll + (size_t)w * 3, (size_t)outW * 24, (size_t)n * 24,
+                                       (size_t)T, cudaMemcpyDefault, e->d2h_stream));
+        }
+        return 0;
+    };
+    // d2h_stream waits for the engine stream's work so far (range event k)
+    auto d2h_after = [&](size_t k) -> int {
+        cudaEvent_t ev;
+        if (range_event(e, k, &ev)) return 1;
+        IBD_CUDA(cudaEventRecord(ev, e->stream));
+        IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, ev, 0));
         return 0;
     };
     int w_lo = shard_wb;
@@ -1380,11 +1268,10 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
         p.Fp = d_Fp;
         {
             // table mode when the screen's reach plus the head-room above a row's reference key fits the shared-memory
-            // table and exp(|kappa| dpos) stays far from overflow; IBDGEM_MMA_TABLE=0 keeps the exp path (A/B)
-            static const int tab_env = [] { const char *st = getenv("IBDGEM_MMA_TABLE"); return st ? atoi(st) : 1; }();
+            // table and exp(|kappa| dpos) stays far from overflow
             const int dpos = (int)std::min(256.0, floor(600.0 / -e->kappa));
             const int tab_n = p.delta + dpos + 1;
-            const bool tab = tab_env && dpos >= 8 && tab_n <= mma::ETAB_N;
+            const bool tab = dpos >= 8 && tab_n <= mma::ETAB_N;
             p.tab_n = tab ? tab_n : 0;
             p.dpos = dpos;
         }
@@ -1393,65 +1280,22 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
         p.wll_host = direct ? h_wll_mapped : nullptr;
         if (direct && launch_ibd0(w0, w0 + nw)) return 1;  // LIBD0 must be in the table before the GEMM's merge warps read it
         {
-            static const int dbg = [] { const char *sdbg = getenv("IBDGEM_MMA_DEBUG"); return sdbg ? atoi(sdbg) : 0; }();
-            p.debug = dbg;
-        }
-        {
-            static const int wt = [] { const char *sw = getenv("IBDGEM_MMA_WARM_TILES"); return sw ? atoi(sw) : 1; }();
-            p.warm_tiles = wt;
-        }
-        {
             int *d_unit;
             if (scratch(e, SC_MMA_UNIT, 64, (void **)&d_unit)) return 1;
             IBD_CUDA(cudaMemsetAsync(d_unit, 0, 4, e->stream));
             p.unit_counter = d_unit;
-            static const int pf = [] { const char *spf = getenv("IBDGEM_MMA_PF"); return spf ? atoi(spf) : mma::PF_TILES; }();
-            p.pf_tiles = pf;
-        }
-        p.trace = nullptr;
-        const char *trace_path = getenv("IBDGEM_MMA_TRACE");
-        unsigned long long *d_trace = nullptr;
-        if (trace_path) {
-            IBD_CUDA(cudaMalloc(&d_trace, 4 * 1024 * 8));
-            IBD_CUDA(cudaMemsetAsync(d_trace, 0, 4 * 1024 * 8, e->stream));
-            p.trace = d_trace;
         }
         {
             LaunchScope ls(e, K_LD_MMA);
-            if (launch_mma(variant, p.n_units, e->sm_count, e->stream, mapA, mapB, p)) return 1;
+            if (launch_pairs(mma::ld_mma_kernel, mma::THREADS, mma::SMEM_BYTES, p.n_units, e->sm_count, e->stream, mapA, mapB, p)) return 1;
         }
         IBD_CUDA(cudaGetLastError());
-        if (d_trace) {
-            std::vector<unsigned long long> h(4 * 1024);
-            IBD_CUDA(cudaMemcpyAsync(h.data(), d_trace, h.size() * 8, cudaMemcpyDeviceToHost, e->stream));
-            IBD_CUDA(cudaStreamSynchronize(e->stream));
-            if (FILE *fh = fopen(trace_path, "wb")) {
-                fwrite(h.data(), 8, h.size(), fh);
-                fclose(fh);
-            }
-            cudaFree(d_trace);
-        }
     }
     if (!direct && launch_ibd0(w_lo, w_hi)) return 1;
     if (stream_out || stream_dev) {
-        // the range's columns of d_wll [T][outW][3] are final: strided copies on their own stream
-        while (e->range_ev.size() <= rk) {
-            cudaEvent_t ev;
-            IBD_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            e->range_ev.push_back(ev);
-        }
-        IBD_CUDA(cudaEventRecord(e->range_ev[rk], e->stream));
-        IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, e->range_ev[rk], 0));
-        if (stream_dev) {
-            if (T >= 256) {  // many short rows: coalesced stores from a kernel (to local or peer memory alike), not T DMA descriptors
-                const int64_t n = (int64_t)T * (w_hi - w_lo) * 3;
-                ld_store_cols_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->d2h_stream>>>(d_wll, e->d_wll_out_device, T, outW, w_lo, w_hi - w_lo);
-                e->k_launches[K_LD_WINDOWS]++;
-            } else {
-                IBD_CUDA(cudaMemcpy2DAsync(e->d_wll_out_device + (size_t)w_lo * 3, (size_t)outW * 24, d_wll + (size_t)w_lo * 3,
-                                           (size_t)outW * 24, (size_t)(w_hi - w_lo) * 24, (size_t)T, cudaMemcpyDefault, e->d2h_stream));
-            }
-        }
+        // the range's columns of d_wll [T][outW][3] are final: they leave on their own stream
+        if (d2h_after(rk)) return 1;
+        if (stream_dev && export_cols(e->d_wll_out_device, e->d_wll_out_device, w_lo, w_hi - w_lo)) return 1;
         if (stream_out && sharded && e->shard_compact) {
             // compact host table of a window shard: pack on the device, one contiguous copy
             double *d_pack;
@@ -1461,35 +1305,13 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
             e->k_launches[K_LD_WINDOWS]++;
             IBD_CUDA(cudaMemcpyAsync(e->h_wll_out + off, d_pack + off, (size_t)n * 8, cudaMemcpyDeviceToHost, e->d2h_stream));
         } else if (stream_out && !direct) {
-            if (h_wll_mapped && T >= 256) {  // many short rows: store them from a kernel (see ld_store_cols_kernel)
-                const int64_t n = (int64_t)T * (w_hi - w_lo) * 3;
-                ld_store_cols_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->d2h_stream>>>(d_wll, h_wll_mapped, T, outW, w_lo, w_hi - w_lo);
-                e->k_launches[K_LD_WINDOWS]++;
-            } else {
-                IBD_CUDA(cudaMemcpy2DAsync(e->h_wll_out + (size_t)w_lo * 3, (size_t)outW * 24, d_wll + (size_t)w_lo * 3, (size_t)outW * 24,
-                                           (size_t)(w_hi - w_lo) * 24, (size_t)T, cudaMemcpyDeviceToHost, e->d2h_stream));
-            }
+            if (export_cols(e->h_wll_out, h_wll_mapped, w_lo, w_hi - w_lo)) return 1;
         }
     }
     w_lo = w_hi;
     }  // window ranges
     if ((stream_out || direct) && outW > nW && !sharded) {  // the unused columns nW .. outW-1 (NaN since the fill at the start of the call)
-        const size_t rk = range_end.size();
-        while (e->range_ev.size() <= rk) {
-            cudaEvent_t ev;
-            IBD_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            e->range_ev.push_back(ev);
-        }
-        IBD_CUDA(cudaEventRecord(e->range_ev[rk], e->stream));
-        IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, e->range_ev[rk], 0));
-        if (h_wll_mapped && T >= 256) {
-            const int64_t n = (int64_t)T * (outW - nW) * 3;
-            ld_store_cols_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->d2h_stream>>>(d_wll, h_wll_mapped, T, outW, nW, outW - nW);
-            e->k_launches[K_LD_WINDOWS]++;
-        } else {
-            IBD_CUDA(cudaMemcpy2DAsync(e->h_wll_out + (size_t)nW * 3, (size_t)outW * 24, d_wll + (size_t)nW * 3, (size_t)outW * 24,
-                                       (size_t)(outW - nW) * 24, (size_t)T, cudaMemcpyDeviceToHost, e->d2h_stream));
-        }
+        if (d2h_after(range_end.size()) || export_cols(e->h_wll_out, h_wll_mapped, nW, outW - nW)) return 1;
     }
     IBD_CUDA(cudaGetLastError());
     return 0;

@@ -30,8 +30,6 @@
 // v_expand_b, ld_vmma (per call).
 #include <cuda.h>
 #include <math.h>
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
@@ -61,8 +59,6 @@ struct VCache {
     cudaStream_t side = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
 };
-
-__device__ __forceinline__ uint32_t vspread4(uint32_t nib) { return (nib * 0x00204081u) & 0x01010101u; }
 
 namespace vmma {
 using namespace tcx;
@@ -117,7 +113,6 @@ struct Params {
     double *wll;                 // [T][outW][3]
     double *wll_host;            // the caller's page-locked table (device alias) or nullptr: finished scores go there too
     int *unit_counter;
-    int debug;
 };
 
 // order-preserving float <-> int map, so that atomicMax on ints is a max on floats
@@ -182,7 +177,7 @@ ld_vmma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant_
             if (rank == 0) {
                 const int v = atomicAdd(p.unit_counter, 1);
                 u_next = v < p.n_units ? v : -1;
-                unit_publish<CG>(uring, ufull, 0, u_next);
+                unit_publish(uring, ufull, 0, u_next);
                 pending = atomicAdd(p.unit_counter, 1);
             }
             for (int it = 0;; it++) {
@@ -200,18 +195,15 @@ ld_vmma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant_
                     const int slabB = (n * 2 + (int)rank) * p.nKB + kb0;
                     for (int kr = 0; kr < nkb; kr++) {
                         mbar_wait(s_empty + st, ph ^ 1u);
-                        // p.debug (IBDGEM_VMMA_DEBUG, timing experiments only — results are wrong): 1 = the row operand
-                        // is loaded for the first k-block of a column tile only, 2 = the same for the column operand
-                        const bool ldA = !(p.debug == 1 && kr > 0), ldB = !(p.debug == 2 && kr > 0);
-                        if (rank == 0) mbar_expect_tx(s_full + st, (uint32_t)(CG * ((ldA ? A_SLAB : 0) + (ldB ? B_SLAB : 0))));
-                        if (ldA) tma_load_3d_cg<CG>(smem + OFF_A + st * A_SLAB, &tmapA, s_full + st, 0, 0, slabA + kr);
-                        if (ldB) tma_load_3d_cg<CG>(smem + OFF_B + st * B_SLAB, &tmapB, s_full + st, 0, 0, slabB + kr);
+                        if (rank == 0) mbar_expect_tx(s_full + st, (uint32_t)(CG * (A_SLAB + B_SLAB)));
+                        tma_load_3d_cg(smem + OFF_A + st * A_SLAB, &tmapA, s_full + st, 0, 0, slabA + kr);
+                        tma_load_3d_cg(smem + OFF_B + st * B_SLAB, &tmapB, s_full + st, 0, 0, slabB + kr);
                         if (++st == NSTAGE) { st = 0; ph ^= 1u; }
                     }
                 }
                 if (rank == 0) {
                     u_next = pending < p.n_units ? pending : -1;
-                    unit_publish<CG>(uring, ufull, it + 1, u_next);
+                    unit_publish(uring, ufull, it + 1, u_next);
                     if (u_next >= 0) pending = atomicAdd(p.unit_counter, 1);
                 }
             }
@@ -240,10 +232,10 @@ ld_vmma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant_
                             const uint64_t bd = bdesc0 + (uint64_t)((st * B_SLAB) >> 4);
 #pragma unroll
                             for (int k = 0; k < KBYTES / UK; k++)
-                                umma_i8_cg<CG>(d_tmem, ad + (uint64_t)(k * (UK >> 4)), bd + (uint64_t)(k * (UK >> 4)), IDESC,
-                                               (uint32_t)((kr | k) != 0));
-                            tc_commit_cg<CG>(s_empty + st);
-                            if (kr + 1 == nkb) tc_commit_cg<CG>(acc_full + acc);
+                                umma_i8_cg(d_tmem, ad + (uint64_t)(k * (UK >> 4)), bd + (uint64_t)(k * (UK >> 4)), IDESC,
+                                           (uint32_t)((kr | k) != 0));
+                            tc_commit_cg(s_empty + st);
+                            if (kr + 1 == nkb) tc_commit_cg(acc_full + acc);
                         }
                         __syncwarp();
                         if (++st == NSTAGE) { st = 0; ph ^= 1u; }
@@ -332,7 +324,7 @@ ld_vmma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant_
                 fmx = fmaxf(fmx, ord2f(*reinterpret_cast<volatile int *>(smax)));
                 // the screen is relative to the running row maximum, which starts at -inf: the first tile of a unit is
                 // read twice, once for its maximum alone (shared by the sets)
-                for (int pass = (n == 0 ? 0 : 1); pass < 2 && p.debug != 3; pass++) {
+                for (int pass = (n == 0 ? 0 : 1); pass < 2; pass++) {
                     if (pass == 1 && n == 0) {
                         atomicMax(smax, f2ord(fmx));
                         asm volatile("bar.sync 3, %0;" ::"n"(NSETS * 128) : "memory");
@@ -380,7 +372,7 @@ ld_vmma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant_
                         }
                         fmx = fmaxf(fmx, cmx);
                         if (pass == 0) continue;
-                        const float thr = p.debug == 4 ? INFINITY : fmx - p.screen_f;  // (debug 4: nothing passes)
+                        const float thr = fmx - p.screen_f;
                         uint32_t mask = 0;
 #pragma unroll
                         for (int i = 0; i < 4; i++) mask |= (t0[i] > thr ? 1u << (2 * i) : 0u) | (t1[i] > thr ? 2u << (2 * i) : 0u);
@@ -407,7 +399,7 @@ ld_vmma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant_
                 atomicMax(smax, f2ord(fmx));
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) mbar_arrive_leader<CG>(acc_empty + slot);
+                if (lane == 0) mbar_arrive_leader(acc_empty + slot);
             }
             if (set == 0) reinterpret_cast<int *>(smem + OFF_SMAX)[((it + 1) & 1) * BM + rloc] = ORD_NEG_INF;  // next unit's slot (idle since unit it - 1)
             asm volatile("bar.sync 2, %0;" ::"n"(NSETS * 128 + 32) : "memory");  // previous unit's partials consumed
@@ -440,17 +432,6 @@ v_slots_kernel(int64_t S, const uint8_t *__restrict__ status, const uint32_t *__
     nk[j] = (uint8_t)(a + b);
     nr[j] = (uint8_t)a;
     l0[j] = lnP[(size_t)(a * C + b) * 3];
-}
-
-__device__ __forceinline__ unsigned vwarp_sum(unsigned v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ double vwarp_sum_d(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
 }
 
 // -v window map in rank space: one warp per target walks the words v = x0 | x1 of the target's two haplotype
@@ -585,7 +566,7 @@ v_tw_kernel(int T, int mapW, int outW, const int32_t *__restrict__ targets, cons
         const uint32_t nn[8] = {n0.x, n0.y, n0.z, n0.w, n1.x, n1.y, n1.z, n1.w};
 #pragma unroll
         for (int k = 0; k < 8; k++) {
-            const uint32_t e0 = vspread4((x0 >> (4 * k)) & 15u), e1 = vspread4((x1 >> (4 * k)) & 15u);
+            const uint32_t e0 = spread4((x0 >> (4 * k)) & 15u), e1 = spread4((x1 >> (4 * k)) & 15u);
             A0 = __dp4a(e0, rr[k], A0);
             N0 = __dp4a(e0, nn[k], N0);
             A1 = __dp4a(e1, rr[k], A1);
@@ -613,8 +594,8 @@ v_tw_kernel(int T, int mapW, int outW, const int32_t *__restrict__ targets, cons
             c0 += (q0 + q1) + (q2 + q3);
         }
     }
-    A0 = vwarp_sum(A0); N0 = vwarp_sum(N0); A1 = vwarp_sum(A1); N1 = vwarp_sum(N1); M = vwarp_sum(M); cnt = vwarp_sum(cnt);
-    c0 = vwarp_sum_d(c0);
+    A0 = warp_sum(A0); N0 = warp_sum(N0); A1 = warp_sum(A1); N1 = warp_sum(N1); M = warp_sum(M); cnt = warp_sum(cnt);
+    c0 = warp_sum(c0);
     if (lane == 0) {
         const int tw = twbase[t] + w;
         const double R0 = fma(alpha, (double)A0, beta * (double)(N0 - A0));
@@ -659,8 +640,8 @@ v_tw_site_kernel(SiteView v, int T, int mapW, int outW, const int32_t *__restric
         A0 += a0 * r; B0 += a0 * a; A1 += a1 * r; B1 += a1 * a; M += (a0 & a1) * (r + a);
         c0 += __ldg(lnP + (size_t)(r * C + a) * 3);
     }
-    A0 = vwarp_sum(A0); B0 = vwarp_sum(B0); A1 = vwarp_sum(A1); B1 = vwarp_sum(B1); M = vwarp_sum(M); cnt = vwarp_sum(cnt);
-    c0 = vwarp_sum_d(c0);
+    A0 = warp_sum(A0); B0 = warp_sum(B0); A1 = warp_sum(A1); B1 = warp_sum(B1); M = warp_sum(M); cnt = warp_sum(cnt);
+    c0 = warp_sum(c0);
     if (lane == 0) {
         const int tw = twbase[t] + w;
         const double R0 = fma(alpha, (double)A0, beta * (double)B0), R1 = fma(alpha, (double)A1, beta * (double)B1);
@@ -799,8 +780,8 @@ v_expand_a_kernel(int unit0, const int32_t *__restrict__ tile_kb0, const int32_t
             }
 #pragma unroll
             for (int k = 0; k < 8; k++) {
-                const uint32_t m0 = vspread4((x0 >> (4 * k)) & 15u) * 0xFFu, m1 = vspread4((x1 >> (4 * k)) & 15u) * 0xFFu;
-                const uint32_t mv = vspread4((vm >> (4 * k)) & 15u) * 0xFFu;
+                const uint32_t m0 = spread4((x0 >> (4 * k)) & 15u) * 0xFFu, m1 = spread4((x1 >> (4 * k)) & 15u) * 0xFFu;
+                const uint32_t mv = spread4((vm >> (4 * k)) & 15u) * 0xFFu;
                 e[0][k] = m0 & nn[k];
                 e[1][k] = m1 & nn[k];
                 e[2][k] = mv & rr[k];
@@ -848,7 +829,7 @@ v_expand_b_kernel(int nKB, int nU, const int32_t *__restrict__ bgU, const uint32
         for (int c = 0; c < 3; c++) {
             uint32_t e[8];
 #pragma unroll
-            for (int k = 0; k < 8; k++) e[k] = vspread4((xs[c] >> (4 * k)) & 15u);
+            for (int k = 0; k < 8; k++) e[k] = spread4((xs[c] >> (4 * k)) & 15u);
             uint4 *o = reinterpret_cast<uint4 *>(slab + (size_t)(c * vmma::IND_HALF + i) * 128 + part * 32);
             __stcs(o, make_uint4(e[0], e[1], e[2], e[3]));
             __stcs(o + 1, make_uint4(e[4], e[5], e[6], e[7]));
@@ -858,31 +839,9 @@ v_expand_b_kernel(int nKB, int nU, const int32_t *__restrict__ bgU, const uint32
 
 // ---------------------------------------------------------------------------------------------
 // host side
+// `nslabs` slabs of `rows` rows of 128 bytes, box = one slab
 static int make_slab_map(CUtensorMap *m, void *base, int rows, int64_t nslabs) {
-    typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                      const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static const EncodeTiledFn fn = [] {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || !p) return (EncodeTiledFn) nullptr;
-        return reinterpret_cast<EncodeTiledFn>(p);
-    }();
-    if (!fn) {
-        set_error("[::] ERROR: cuTensorMapEncodeTiled is not available from the CUDA driver.");
-        return 1;
-    }
-    const cuuint64_t dims[3] = {128, (cuuint64_t)rows, (cuuint64_t)nslabs};
-    const cuuint64_t strides[2] = {128, (cuuint64_t)rows * 128};
-    const cuuint32_t box[3] = {128, (cuuint32_t)rows, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    const CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_error("[::] ERROR: cuTensorMapEncodeTiled failed (%d) for %lld slabs of %d rows.", (int)r, (long long)nslabs, rows);
-        return 1;
-    }
-    return 0;
+    return encode_u8_3d(m, base, {128, (cuuint64_t)rows, (cuuint64_t)nslabs}, {128, (cuuint64_t)rows * 128}, {128, (cuuint32_t)rows, 1});
 }
 
 constexpr size_t V_A_BUDGET = (size_t)8 << 30;    // bytes of A slabs per batch of row tiles
@@ -905,8 +864,6 @@ void ld_vtensor_release(ibdgem_engine *e) {
 void ld_vtensor_invalidate(ibdgem_engine *e) {
     if (e->vc) e->vc->valid = false;
 }
-
-static double v_screen_nats(int ncols) { return std::min(32.0, log((double)std::max(ncols, 2)) + 16.2); }
 
 bool ld_vtensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t n_bg) {
     if (!e->depth_linear || !(e->kappa < -1e-3)) return false;
@@ -970,29 +927,14 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
     const int W = e->prm.window_size;
     const int mapW = (int)(e->S / W + 2);
 
-    // unique background individuals with multiplicities (src/ibdgem.c:714: the pileup's own individual never contributes)
-    std::vector<int32_t> mult((size_t)c->N, 0), where((size_t)c->N, -1);
-    int64_t total_bg = 0;
-    for (int n = 0; n < n_bg; n++)
-        if (h_bg[n] != pu_idx) { mult[h_bg[n]]++; total_bg++; }
-    std::vector<int32_t> bgU;
-    for (int32_t b = 0; b < c->N; b++)
-        if (mult[b]) { where[b] = (int32_t)bgU.size(); bgU.push_back(b); }
-    const int nU = (int)bgU.size();
+    LdBackground bg;
+    ld_background(c->N, T, h_targets, n_bg, h_bg, pu_idx, &bg);
+    const int nU = (int)bg.bgU.size();
     if (nU == 0) return 2;
     const int NT = (nU + TILE_IND - 1) / TILE_IND;
-    std::vector<double> lnc((size_t)NT * TILE_IND, -INFINITY), lognb(T);
-    for (int u = 0; u < nU; u++) lnc[(size_t)u] = mult[bgU[u]] == 1 ? 0.0 : log((double)mult[bgU[u]]);
-    std::vector<int32_t> ownT(T);
-    for (int t = 0; t < T; t++) {
-        const int own = where[h_targets[t]];
-        const int64_t nb = total_bg - (own >= 0 ? mult[h_targets[t]] : 0);
-        ownT[t] = own;
-        lognb[t] = nb > 0 ? log((double)nb) : (double)NAN;
-    }
+    bg.lnc.resize((size_t)NT * TILE_IND, -INFINITY);  // padding columns of the last tile
 
     // ---- background operand over the whole K axis, on the side stream ----------------------------
-    static const int vdebug = [] { const char *sb = getenv("IBDGEM_VMMA_DEBUG"); return sb ? atoi(sb) : 0; }();
     const int nKB = c->nKB;
     double *d_lnc, *d_lognb;
     int32_t *d_bgU, *d_ownT;
@@ -1000,10 +942,10 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
     d_lognb = d_lnc + (size_t)NT * TILE_IND;
     d_bgU = reinterpret_cast<int32_t *>(d_lognb + T);
     d_ownT = d_bgU + nU;
-    IBD_CUDA(cudaMemcpyAsync(d_lnc, lnc.data(), lnc.size() * 8, cudaMemcpyHostToDevice, e->stream));
-    IBD_CUDA(cudaMemcpyAsync(d_lognb, lognb.data(), (size_t)T * 8, cudaMemcpyHostToDevice, e->stream));
-    IBD_CUDA(cudaMemcpyAsync(d_bgU, bgU.data(), (size_t)nU * 4, cudaMemcpyHostToDevice, e->stream));
-    IBD_CUDA(cudaMemcpyAsync(d_ownT, ownT.data(), (size_t)T * 4, cudaMemcpyHostToDevice, e->stream));
+    IBD_CUDA(cudaMemcpyAsync(d_lnc, bg.lnc.data(), bg.lnc.size() * 8, cudaMemcpyHostToDevice, e->stream));
+    IBD_CUDA(cudaMemcpyAsync(d_lognb, bg.lognb.data(), (size_t)T * 8, cudaMemcpyHostToDevice, e->stream));
+    IBD_CUDA(cudaMemcpyAsync(d_bgU, bg.bgU.data(), (size_t)nU * 4, cudaMemcpyHostToDevice, e->stream));
+    IBD_CUDA(cudaMemcpyAsync(d_ownT, bg.own.data(), (size_t)T * 4, cudaMemcpyHostToDevice, e->stream));
     unsigned char *d_B;
     const size_t b_bytes = (size_t)NT * 2 * nKB * B_SLAB;
     if (scratch(e, SC_MMA_BG, b_bytes, (void **)&d_B)) return 1;
@@ -1012,15 +954,13 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
         IBD_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
         IBD_CUDA(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
     }
-    static const int use_side = [] { const char *sv = getenv("IBDGEM_V_SIDE"); return sv ? atoi(sv) : 1; }();  // 0: A/B, all on the engine stream
-    cudaStream_t bstream = use_side ? c->side : e->stream;
     IBD_CUDA(cudaEventRecord(c->ev_fork, e->stream));
-    IBD_CUDA(cudaStreamWaitEvent(bstream, c->ev_fork, 0));
+    IBD_CUDA(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
     {
-        LaunchScope ls(e, K_V_EXPAND_B, bstream);
-        v_expand_b_kernel<<<dim3((unsigned)((nKB + 7) / 8), (unsigned)(NT * 2)), 160, 0, bstream>>>(nKB, nU, d_bgU, c->d_tbits, c->H, d_B);
+        LaunchScope ls(e, K_V_EXPAND_B, c->side);
+        v_expand_b_kernel<<<dim3((unsigned)((nKB + 7) / 8), (unsigned)(NT * 2)), 160, 0, c->side>>>(nKB, nU, d_bgU, c->d_tbits, c->H, d_B);
     }
-    IBD_CUDA(cudaEventRecord(c->ev_join, bstream));
+    IBD_CUDA(cudaEventRecord(c->ev_join, c->side));
     // every way out of this function rejoins the side stream: the scratch it writes belongs to the engine stream's next call
     struct Join {
         ibdgem_engine *e;
@@ -1101,26 +1041,16 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
         IBD_CUDA(cudaEventRecord(e->ev_book, e->stream));
         e->book_ready = true;
     }
-    double *h_wll_mapped = nullptr;
-    static const int direct_env = [] { const char *sd = getenv("IBDGEM_LD_DIRECT_STORE"); return sd ? atoi(sd) : 1; }();
-    if (e->h_wll_out && direct_env) {
-        cudaPointerAttributes attr;
-        if (cudaPointerGetAttributes(&attr, e->h_wll_out) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
-            h_wll_mapped = static_cast<double *>(attr.devicePointer);
-        else
-            cudaGetLastError();
-    }
+    double *h_wll_mapped = host_table_alias(e);
+    cudaEvent_t ev_table = nullptr;  // the copy of the whole table is done
     if (h_wll_mapped) {
         if (!e->d2h_stream) IBD_CUDA(cudaStreamCreateWithFlags(&e->d2h_stream, cudaStreamNonBlocking));
-        while (e->range_ev.size() < 2) {
-            cudaEvent_t ev;
-            IBD_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-            e->range_ev.push_back(ev);
-        }
-        IBD_CUDA(cudaEventRecord(e->range_ev[0], e->stream));
-        IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, e->range_ev[0], 0));
+        cudaEvent_t ev_ready;
+        if (range_event(e, 0, &ev_ready) || range_event(e, 1, &ev_table)) return 1;
+        IBD_CUDA(cudaEventRecord(ev_ready, e->stream));
+        IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, ev_ready, 0));
         IBD_CUDA(cudaMemcpyAsync(e->h_wll_out, d_wll, (size_t)T * outW * 24, cudaMemcpyDeviceToHost, e->d2h_stream));
-        IBD_CUDA(cudaEventRecord(e->range_ev[1], e->d2h_stream));
+        IBD_CUDA(cudaEventRecord(ev_table, e->d2h_stream));
         e->wll_streamed = true;
     }
     {
@@ -1138,14 +1068,11 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
     IBD_CUDA(cudaStreamSynchronize(e->stream));
 
     // ---- row tiles in batches under the A budget ---------------------------------------------------
-    static const size_t a_budget = [] {
-        const char *sb = getenv("IBDGEM_V_BUDGET_MB");
-        return sb && atol(sb) > 0 ? (size_t)atol(sb) << 20 : V_A_BUDGET;
-    }();
+    static const int budget_mb = env_int("IBDGEM_V_BUDGET_MB", 0);  // (tests exercise the row-tile batching with it)
+    const size_t a_budget = budget_mb > 0 ? (size_t)budget_mb << 20 : V_A_BUDGET;
     std::vector<int64_t> h_slab((size_t)n_tiles);
     int *d_unit;
     if (scratch(e, SC_MMA_UNIT, 64, (void **)&d_unit)) return 1;
-    IBD_CUDA(cudaFuncSetAttribute(ld_vmma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     int u0 = 0;
     // slab offsets restart at every batch; all batches' offsets go up in one copy
     std::vector<std::pair<int, int>> batches;
@@ -1189,34 +1116,20 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
         p.NT = NT; p.nKB = nKB; p.n_tw = n_tw; p.outW = outW;
         p.alpha = e->alpha; p.beta = e->beta; p.kappa = e->kappa;
         p.alpha_f = (float)e->alpha; p.beta_f = (float)e->beta; p.kappa_f = (float)e->kappa;
-        p.screen_f = (float)(v_screen_nats(2 * nU) + 2.0);
+        p.screen_f = (float)(screen_nats(2 * nU) + 2.0);
         p.tile_kb0 = d_tile_kb0; p.tile_nkb = d_tile_nkb; p.tile_slab = d_tile_slab; p.order = d_order;
         p.tw_t = d_tw_t; p.tw_w = d_tw_w; p.tw_own = d_tw_own; p.tw_C0 = d_tw_C0; p.tw_R0 = d_tw_R0; p.tw_R1 = d_tw_R1;
         p.lnc = d_lnc; p.lognb = d_lognb; p.wll = d_wll;
         p.wll_host = h_wll_mapped;
-        p.debug = vdebug;
         IBD_CUDA(cudaMemsetAsync(d_unit, 0, 8, e->stream));
         p.unit_counter = d_unit;
         if (bi == 0) {
             IBD_CUDA(cudaStreamWaitEvent(e->stream, c->ev_join, 0));
-            if (h_wll_mapped) IBD_CUDA(cudaStreamWaitEvent(e->stream, e->range_ev[1], 0));
+            if (h_wll_mapped) IBD_CUDA(cudaStreamWaitEvent(e->stream, ev_table, 0));
         }
         {
             LaunchScope ls(e, K_LD_VMMA);
-            const int groups = std::max(1, std::min(p.n_units, e->sm_count / 2));
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3((unsigned)(groups * 2));
-            cfg.blockDim = dim3((unsigned)THREADS);
-            cfg.dynamicSmemBytes = SMEM_BYTES;
-            cfg.stream = e->stream;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeClusterDimension;
-            at[0].val.clusterDim.x = 2;
-            at[0].val.clusterDim.y = 1;
-            at[0].val.clusterDim.z = 1;
-            cfg.attrs = at;
-            cfg.numAttrs = 1;
-            IBD_CUDA(cudaLaunchKernelEx(&cfg, ld_vmma_kernel, mapA, mapB, p));
+            if (launch_pairs(ld_vmma_kernel, THREADS, SMEM_BYTES, p.n_units, e->sm_count, e->stream, mapA, mapB, p)) return 1;
         }
         IBD_CUDA(cudaGetLastError());
     }

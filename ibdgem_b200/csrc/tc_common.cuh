@@ -1,11 +1,18 @@
-// tc_common.cuh — sm_100a PTX wrappers (mbarrier, TMA, tcgen05) and the fp64 exp / log-sum-exp helpers
-// shared by the tensor-core --LD kernels (ld_mma.cu: shared windows; ld_vmma.cu: per-target windows).
+// tc_common.cuh — sm_100a PTX wrappers (mbarrier, TMA, tcgen05), the fp64 exp / log-sum-exp helpers and the
+// tensor-map / CTA-pair launch plumbing shared by the tensor-core --LD kernels (ld_mma.cu: shared windows;
+// ld_vmma.cu: per-target windows).
 #pragma once
 
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
+#include <stdlib.h>
+
+#include <algorithm>
+#include <utility>
+
+#include "engine.h"
 
 namespace ibdgem {
 
@@ -15,9 +22,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)_
 
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
@@ -64,12 +68,6 @@ __device__ __forceinline__ void mbar_wait_relaxed(uint64_t *bar, uint32_t parity
         __nanosleep(64);
     }
 }
-__device__ __forceinline__ void tma_load_3d(void *dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, int c2) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(smem_u32(dst)),
-        "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;
     asm volatile(
@@ -83,19 +81,6 @@ __device__ __forceinline__ bool elect_one() {
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint64_t *bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// D[tmem] (+)= A[smem] . B[smem]^T, int8 x int8 -> int32
-__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
 // 32 consecutive accumulator columns of this thread's TMEM lane
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, int (&v)[32]) {
     asm volatile(
@@ -206,6 +191,18 @@ __device__ __forceinline__ int pick_tree(const int *v, int j) {
 }
 __device__ __forceinline__ int pick32(const int (&v)[32], int j) { return pick_tree<32>(v, j); }
 
+// 4 bits -> 4 bytes of 0 / 1 (bit i to byte i)
+__device__ __forceinline__ uint32_t spread4(uint32_t nib) { return (nib * 0x00204081u) & 0x01010101u; }
+__device__ __forceinline__ unsigned warp_sum(unsigned v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+__device__ __forceinline__ double warp_sum(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
 
 // ---------------------------------------------------------------------------------------------
 // CTA-pair (tcgen05 cta_group::2) helpers and the dynamic unit ring shared by the persistent kernels
@@ -216,56 +213,39 @@ namespace tcx {
 constexpr int URING = 8;
 constexpr uint32_t PEER_MASK = 0xFEFFFFFFu;  // clears the CTA-rank bit of a shared::cluster address -> CTA 0 of the pair
 
-template <int CG>
+// executed by both CTAs of the pair; the bytes are counted on CTA 0's barrier
 __device__ __forceinline__ void tma_load_3d_cg(void *dst, const CUtensorMap *map, uint64_t *bar, int c0, int c1, int c2) {
-    if constexpr (CG == 1) {
-        tma_load_3d(dst, map, bar, c0, c1, c2);
-    } else {  // executed by both CTAs of the pair; the bytes are counted on CTA 0's barrier
-        asm volatile(
-            "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
-                smem_u32(dst)),
-            "l"(map), "r"(smem_u32(bar) & PEER_MASK), "r"(c0), "r"(c1), "r"(c2)
-            : "memory");
-    }
+    asm volatile(
+        "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
+            smem_u32(dst)),
+        "l"(map), "r"(smem_u32(bar) & PEER_MASK), "r"(c0), "r"(c1), "r"(c2)
+        : "memory");
 }
 __device__ __forceinline__ void tma_prefetch_3d(const CUtensorMap *map, int c0, int c1, int c2) {
     asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global [%0, {%1, %2, %3}];" ::"l"(map), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 constexpr int PF_TILES = 2;
-template <int CG>
+// arrives on the barrier at this offset in BOTH CTAs once the pair's MMAs retire
 __device__ __forceinline__ void tc_commit_cg(uint64_t *bar) {
-    if constexpr (CG == 1) {
-        tc_commit(bar);
-    } else {  // arrives on the barrier at this offset in BOTH CTAs once the pair's MMAs retire
-        asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                         smem_u32(bar)),
-                     "h"((uint16_t)3)
-                     : "memory");
-    }
+    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+                     smem_u32(bar)),
+                 "h"((uint16_t)3)
+                 : "memory");
 }
-template <int CG>
+// D[tmem] (+)= A[smem] . B[smem]^T, int8 x int8 -> int32, over the pair's 256 rows
 __device__ __forceinline__ void umma_i8_cg(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    if constexpr (CG == 1) {
-        umma_i8(tmem_d, adesc, bdesc, idesc, accumulate);
-    } else {
-        asm volatile(
-            "{\n\t"
-            ".reg .pred p;\n\t"
-            "setp.ne.b32 p, %4, 0;\n\t"
-            "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t"
-            "}" ::"r"(tmem_d),
-            "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-            : "memory");
-    }
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t"
+        "}" ::"r"(tmem_d),
+        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+        : "memory");
 }
 // arrive on CTA 0's copy of a barrier (CTA 0 itself: a plain local arrive)
-template <int CG>
 __device__ __forceinline__ void mbar_arrive_leader(uint64_t *bar) {
-    if constexpr (CG == 1) {
-        mbar_arrive(bar);
-    } else {
-        asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & PEER_MASK) : "memory");
-    }
+    asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & PEER_MASK) : "memory");
 }
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
@@ -294,20 +274,83 @@ __device__ __forceinline__ int unit_of(const int *uring, uint64_t *ufull, int it
     return *reinterpret_cast<const volatile int *>(uring + (it % URING));
 }
 // scheduler (producer lane of CTA 0): publish unit u for iteration `it` in both CTAs of the pair
-template <int CG>
 __device__ __forceinline__ void unit_publish(int *uring, uint64_t *ufull, int it, int u) {
     const int i = it % URING;
     *reinterpret_cast<volatile int *>(uring + i) = u;
     asm volatile("mbarrier.arrive.release.cluster.shared::cta.b64 _, [%0];" ::"r"(smem_u32(ufull + i)) : "memory");
-    if constexpr (CG == 2) {
-        uint32_t rdata, rbar;
-        asm volatile("mapa.shared::cluster.u32 %0, %1, 1;" : "=r"(rdata) : "r"(smem_u32(uring + i)));
-        asm volatile("mapa.shared::cluster.u32 %0, %1, 1;" : "=r"(rbar) : "r"(smem_u32(ufull + i)));
-        asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(rdata), "r"(u) : "memory");
-        asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(rbar) : "memory");
-    }
+    uint32_t rdata, rbar;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, 1;" : "=r"(rdata) : "r"(smem_u32(uring + i)));
+    asm volatile("mapa.shared::cluster.u32 %0, %1, 1;" : "=r"(rbar) : "r"(smem_u32(ufull + i)));
+    asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(rdata), "r"(u) : "memory");
+    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(rbar) : "memory");
 }
 
 }  // namespace tcx
+
+// ---------------------------------------------------------------------------------------------
+// host side of the persistent CTA-pair GEMMs
+
+// Screening distance in nats.  An element more than D below its row maximum contributes at most e^-D of the row's
+// sum, so dropping every such element of a row with `ncols` columns changes the row's log-sum-exp by less than
+// ncols * e^-D.  D = ln(ncols) + ln(1e7) keeps that below 1e-7 (the window tolerance is 1e-6).
+constexpr double SCREEN_NATS = 32.0;
+inline double screen_nats(int ncols) { return std::min(SCREEN_NATS, log((double)std::max(ncols, 2)) + 16.2); }
+
+// integer value of the environment variable `name` (read by the caller once per process), or dflt when it is unset
+inline int env_int(const char *name, int dflt) {
+    const char *s = getenv(name);
+    return s ? atoi(s) : dflt;
+}
+
+// TMA map of a 3-D uint8 array (dims[0] bytes contiguous; strides of dims 1 and 2 in bytes): 128-byte swizzle,
+// zero fill outside
+inline int encode_u8_3d(CUtensorMap *m, void *base, const cuuint64_t (&dims)[3], const cuuint64_t (&strides)[2],
+                        const cuuint32_t (&box)[3]) {
+    typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
+                                      const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+    static const EncodeTiledFn fn = [] {
+        void *p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || !p) return (EncodeTiledFn) nullptr;
+        return reinterpret_cast<EncodeTiledFn>(p);
+    }();
+    if (!fn) {
+        set_error("[::] ERROR: cuTensorMapEncodeTiled is not available from the CUDA driver.");
+        return 1;
+    }
+    const cuuint32_t estr[3] = {1, 1, 1};
+    const CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        set_error("[::] ERROR: cuTensorMapEncodeTiled failed (%d) for a %llu x %llu x %llu operand.", (int)r, (unsigned long long)dims[0],
+                  (unsigned long long)dims[1], (unsigned long long)dims[2]);
+        return 1;
+    }
+    return 0;
+}
+
+// Persistent launch of a CTA-pair kernel: clusters of 2 x 1 x 1, one pair per two SMs and at most one per unit.
+template <class... Exp, class... Act>
+inline int launch_pairs(void (*kernel)(Exp...), int threads, int smem_bytes, int n_units, int sm_count, cudaStream_t st, Act &&...args) {
+    // function attributes are per device (the command-line front-end drives one engine per GPU from threads of one
+    // process); setting it is cheap enough to do on every launch
+    IBD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+    const int groups = std::max(1, std::min(n_units, sm_count / 2));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(groups * 2));
+    cfg.blockDim = dim3((unsigned)threads);
+    cfg.dynamicSmemBytes = smem_bytes;
+    cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = 2;
+    at[0].val.clusterDim.y = 1;
+    at[0].val.clusterDim.z = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = 1;
+    IBD_CUDA(cudaLaunchKernelEx(&cfg, kernel, std::forward<Act>(args)...));
+    return 0;
+}
 
 }  // namespace ibdgem

@@ -160,7 +160,8 @@ def depth_coefficients(eps, max_cov):
 def mma_mode(eps, ncols):
     """(table, delta, dpos) of the ld_mma epilogue for `ncols` background haplotype columns: the screen's reach in key
     units, the head-room a row's maximum may climb above its reference key before the reference moves, and whether
-    the exp table (delta + dpos + 1 entries of at most 512) is used.  Mirrors screen_nats and ld_mma.cu:1377-1387."""
+    the exp table (delta + dpos + 1 entries of at most 512) is used.  Mirrors screen_nats (tc_common.cuh) and
+    ld_mma.cu:1265-1276."""
     k = -kappa(eps)
     screen = min(32.0, np.log(max(ncols, 2)) + 16.2)
     delta = int(np.ceil(screen / k)) + 2

@@ -7,10 +7,6 @@ a later maximum in fp32, and ld_ibd0's own entry always sits at chunk 0, positio
 test here builds a case that reaches one of those branches (ldterms.ld_case), asserts in float64 that it does before
 the engine runs, checks which path ran (ld_path 1 = ld_mma + ld_ibd0, 2 = ld_vmma, 0 = the general path) and compares
 every target with the oracle at the parity bar: integers exact, window sums to 1e-6 absolute."""
-import os
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 
@@ -19,8 +15,7 @@ import refcases
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-MMA_TILE = 256        # background columns per ld_mma tile (CTA pairs); 128 with IBDGEM_MMA_VARIANT=1
+MMA_TILE = 256        # background columns per ld_mma tile (CTA pairs)
 VMMA_TILE = 2 * 80    # background columns per ld_vmma tile (80 individuals)
 
 
@@ -37,16 +32,6 @@ def check(case, path):
         worst = np.fmax(worst, np.nanmax(d, axis=0, initial=0.0))
     print(f"ld_path={path} max|dLIBD0|={worst[0]:.3g} max|dLIBD1|={worst[1]:.3g}")
     return res
-
-
-def in_subprocess(env, body):
-    """Runs `body` in a fresh interpreter with the environment knobs `env` (the engine reads each knob once per
-    process) and this module imported as `g`."""
-    code = "import sys; sys.path[:0] = ['tests', '.']\nimport test_ld_epilogue_gpu as g\n" + body + "\nprint('ok')\n"
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=dict(os.environ, **env),
-                       cwd=ROOT, timeout=600)
-    print(r.stdout[-2000:])
-    assert r.returncode == 0 and r.stdout.rstrip().endswith("ok"), r.stdout[-2000:] + r.stderr[-3000:]
 
 
 def climbs(case, targets, tile_cols, view=None):
@@ -128,34 +113,12 @@ def test_mma_deep_coverage_repeated_moves():
 
 
 def test_mma_late_maximum_on_the_exp_path():
-    in_subprocess({"IBDGEM_MMA_TABLE": "0"},
-                  "case = g.late_case(0.02, 300)\n"
-                  "g.assert_late(case, g.MMA_TILE, 600.0)\n"
-                  "g.check(case, 1)")
-
-
-def test_mma_late_maximum_single_cta_tiles():
-    """128-column tiles: the maximum at column 600 is four tiles in."""
-    in_subprocess({"IBDGEM_MMA_VARIANT": "1"},
-                  "case = g.late_case(0.02, 300)\n"
-                  "_, _, dpos = g.lt.mma_mode(0.02, 1400)\n"
-                  "g.assert_late(case, 128, dpos * -g.lt.kappa(0.02))\n"
-                  "g.check(case, 1)")
-
-
-def test_mma_late_maximum_without_the_max_only_pass():
-    """No warm tile: the first tile is screened against the running maximum as it comes, so with the source in the
-    second 32-column chunk of set 0 the reference moves inside tile 0, over the sum of the first chunk."""
-    in_subprocess({"IBDGEM_MMA_WARM_TILES": "0"},
-                  "_, _, dpos = g.lt.mma_mode(0.02, 1400)\n"
-                  "reach = dpos * -g.lt.kappa(0.02)\n"
-                  "case = g.late_case(0.02, 300)\n"
-                  "g.assert_late(case, g.MMA_TILE, reach)\n"
-                  "g.check(case, 1)\n"
-                  "case = g.late_case(0.02, 20, seed=14)\n"
-                  "assert 32 <= 2 * 20 < 64\n"
-                  "g.assert_late(case, 32, reach)\n"
-                  "g.check(case, 1)")
+    """eps = 0.354: delta + dpos + 1 passes the 512 table entries, so the candidates take the exp path; deep reads
+    (max_cov = 127) make the row maximum climb hundreds of nats after the first tile."""
+    assert not lt.mma_mode(0.354, 1400)[0]
+    case = late_case(0.354, 300, depth=100.0, max_cov=127)
+    assert_late(case, MMA_TILE, 600.0)
+    check(case, 1)
 
 
 @pytest.mark.parametrize("eps,table", [(0.353, True), (0.354, False)])
@@ -258,7 +221,7 @@ def v_case(src, opt_v=1, cull_p=1.0, seed=31, targets=None, S=1500, window=300):
 
 
 def v_reach(nU=250):
-    return min(32.0, np.log(2 * nU) + 16.2) + 2.0  # ld_vmma's screen in nats (v_screen_nats + 2)
+    return min(32.0, np.log(2 * nU) + 16.2) + 2.0  # ld_vmma's screen in nats (screen_nats + 2)
 
 
 @pytest.mark.parametrize("opt_v,cull_p", [(1, 1.0), (1, 0.5), (0, 0.5)])
