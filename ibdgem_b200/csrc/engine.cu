@@ -129,6 +129,13 @@ int scratch(ibdgem_engine *e, int slot, size_t bytes, void **out) {
     return 0;
 }
 
+int side_streams(ibdgem_engine *e) {
+    if (!e->copy_stream) IBD_CUDA(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
+    if (!e->ev_order) IBD_CUDA(cudaEventCreateWithFlags(&e->ev_order, cudaEventDisableTiming));
+    if (!e->d2h_stream) IBD_CUDA(cudaStreamCreateWithFlags(&e->d2h_stream, cudaStreamNonBlocking));
+    return 0;
+}
+
 // ---------------------------------------------------------------------------------------------
 // device helpers
 __device__ __forceinline__ int warp_sum_i(int v) {
@@ -1149,10 +1156,7 @@ int ibdgem_engine_upload_panel(ibdgem_engine *e, int64_t n_sites, int32_t n_indi
     }
     e->N = n_indiv;
     // chunked copy on the copy stream, ordered after whatever the engine stream still reads from d_bits
-    if (!e->copy_stream) {
-        IBD_CUDA(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
-        IBD_CUDA(cudaEventCreateWithFlags(&e->ev_order, cudaEventDisableTiming));
-    }
+    if (side_streams(e)) return 1;
     // Equal chunks.  Scoring a chunk's windows takes less time than copying it (C3: 9.0 ms of scoring
     // against 11.6 ms of PCIe for the whole panel), so the GPU keeps up with the copy and the end-to-end
     // step is ~ copy + one chunk's scoring + its result copy.  Measured at C3 (bench.py e2e, ms):
@@ -1262,10 +1266,7 @@ int ibdgem_engine_clone_panel(ibdgem_engine *e, ibdgem_engine *src) {
         if (dev_alloc(e, (void **)&e->d_bits, (size_t)e->S * e->Wh * 4)) return 1;
     }
     e->N = src->N;
-    if (!e->copy_stream) {
-        IBD_CUDA(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
-        IBD_CUDA(cudaEventCreateWithFlags(&e->ev_order, cudaEventDisableTiming));
-    }
+    if (side_streams(e)) return 1;
     if (e->device != src->device) {
         int can = 0;
         cudaDeviceCanAccessPeer(&can, e->device, src->device);
@@ -1574,10 +1575,7 @@ static int score_common(ibdgem_engine *e, int32_t T, const int32_t *targets, int
     IBD_CUDA(cudaMemsetAsync(d_we, 0, nWT * 8, e->stream));
     const bool tensor = ld && !e->force_general && shared && ld_tensor_eligible(e, T, n_bg, tgt_counts);
     e->book_ready = false;
-    if ((tensor || vtensor) && !e->copy_stream) {  // (a panel set in device memory never went through upload_panel)
-        IBD_CUDA(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
-        IBD_CUDA(cudaEventCreateWithFlags(&e->ev_order, cudaEventDisableTiming));
-    }
+    if ((tensor || vtensor) && side_streams(e)) return 1;  // (a panel set in device memory never went through upload_panel)
     if ((tensor || vtensor) && !e->ev_book) IBD_CUDA(cudaEventCreateWithFlags(&e->ev_book, cudaEventDisableTiming));
     // everything but the tensor path reads the per-site table and the whole panel up front; the
     // tensor path asks for them window range by window range (upload / scoring overlap)

@@ -5,7 +5,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <functional>
 #include <string>
 #include <vector>
 
@@ -208,19 +207,44 @@ enum ScratchSlot {
     SC_HG_TOFF, SC_SLOTS
 };
 int scratch(ibdgem_engine *e, int slot, size_t bytes, void **out);
-// hiddengem: host start / length of every table of a call (hidden.cu; the Viterbi and posterior entries)
-int table_layout(const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, std::vector<int64_t> *sl, int64_t *maxbins,
-                 int64_t *total);
-// Viterbi kernels for one batch of tables in device memory (hidden.cu); no host synchronisation.  d_flag[t] = 1 marks
-// a table the near-tie guard hands to the host.
+// copy_stream with ev_order, and d2h_stream, created on first use (engine.cu)
+int side_streams(ibdgem_engine *e);
+
+// hiddengem (hidden.cu): the tables of one call.  Table t holds len(t) bins from bin start(t) of every per-bin array:
+// start(t) = bin_offsets[t] (packed, table_stride = 0) or t * table_stride.
+struct HgCall {
+    int n = 0;
+    std::vector<int64_t> sl;  // [n] starts, then [n] lengths
+    int64_t maxbins = 0, total = 0;
+    int64_t *d_start = nullptr, *d_len = nullptr;  // the same in device memory (SC_HG_OFF)
+    int64_t start(int t) const { return sl[(size_t)t]; }
+    int64_t len(int t) const { return sl[(size_t)n + t]; }
+};
+// The prologue of every hiddengem entry: the layout (1 and the error set on a negative length or one past the
+// stride; with need_bins, also when the call has no bins), the engine's device, and start / length uploaded on the
+// engine stream.
+int hg_begin(ibdgem_engine *e, const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, bool need_bins,
+             HgCall *c);
+// Scratch of a Viterbi pass over nb host bins: likelihoods, scores (nb x 24 B), states and, behind them, the per-table
+// near-tie flags (d_flag = d_state + nb), and counts.  The posterior pass may reuse SC_HG_SCORE and SC_HG_COUNTS (the
+// tract entry runs it after the Viterbi pass); nothing but the Viterbi pass writes SC_HG_STATE.
+struct HgViterbiScratch {
+    double *lik, *score;
+    uint8_t *state, *flag;
+    long long *counts;
+};
+int viterbi_scratch(ibdgem_engine *e, int n_tables, int64_t nb, HgViterbiScratch *s);
+// Viterbi kernels for one batch of tables in device memory; no host synchronisation.  d_flag[t] = 1 marks a table the
+// near-tie guard hands to the host.
 int viterbi_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, int64_t total_bins, const int64_t *d_start, const int64_t *d_len,
                       const double *d_lik, int is_log, double p01, double p02, double p12, uint8_t *d_state, double *d_score,
                       long long *d_counts, uint8_t *d_flag);
-// The flagged tables, table t = flagged[k] at host lik + bin_offsets[t] * 3, re-evaluated in long double on a few host
-// threads; sink(k, t, state, score_log, counts) receives each result (concurrently, one call per k).
-void viterbi_redo_flagged(const std::vector<int> &flagged, const int64_t *bin_offsets, const double *lik, int is_log, double p01,
-                          double p02, double p12,
-                          const std::function<void(size_t, int, const uint8_t *, const double *, const int64_t *)> &sink);
+// The near-tie guard's verdict: the tables with h_flag[t] != 0 re-evaluated in long double on a few host threads, and
+// e->hg_flagged set to their number.  Table t is read at bin c.start(t) of lik (device memory when lik_on_device) and
+// its states, scores and counts are written to the same places of state, score and counts (each may be null; device
+// memory when out_on_device, written on the engine stream, which is then synchronised).
+int viterbi_resolve(ibdgem_engine *e, const HgCall &c, const std::vector<uint8_t> &h_flag, const double *lik, bool lik_on_device,
+                    int is_log, double p01, double p02, double p12, uint8_t *state, double *score, int64_t *counts, bool out_on_device);
 // posterior.cu: penalty check of the posterior entries (1 and the error set when rejected), and its kernels for one
 // batch of tables in device memory (no host synchronisation).  d_cov != null runs the moment variant of the backward
 // pass: covariances into d_cov [n_tables][3][3], and d_post may then be null.

@@ -451,24 +451,84 @@ int ibdgem::viterbi_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, i
     return 0;
 }
 
-// Flagged tables: the reference's long double recurrence decides (tables are independent: a few host threads).
-void ibdgem::viterbi_redo_flagged(const std::vector<int> &flagged, const int64_t *bin_offsets, const double *lik, int is_log, double p01,
-                                  double p02, double p12,
-                                  const std::function<void(size_t, int, const uint8_t *, const double *, const int64_t *)> &sink) {
+// The layout of the call's tables: start / length per table on the host and uploaded to SC_HG_OFF on the engine stream.
+int ibdgem::hg_begin(ibdgem_engine *e, const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, bool need_bins,
+                     HgCall *c) {
+    c->n = n_tables;
+    c->sl.assign((size_t)n_tables * 2, 0);
+    c->maxbins = c->total = 0;
+    for (int t = 0; t < n_tables; t++) {
+        const int64_t n = bin_offsets[t + 1] - bin_offsets[t];
+        if (n < 0 || (table_stride > 0 && n > table_stride)) {
+            set_error("[::] ERROR in %s(): table %d has %lld bins (stride %lld).", fn, t, (long long)n, (long long)table_stride);
+            return 1;
+        }
+        c->sl[(size_t)t] = table_stride > 0 ? (int64_t)t * table_stride : bin_offsets[t];
+        c->sl[(size_t)n_tables + t] = n;
+        c->maxbins = std::max(c->maxbins, n);
+        c->total += n;
+    }
+    if (need_bins && c->total <= 0) {
+        set_error("[::] ERROR parsing likelihood data; make sure input is valid.");
+        return 1;
+    }
+    IBD_CUDA(cudaSetDevice(e->device));
+    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&c->d_start)) return 1;
+    c->d_len = c->d_start + n_tables;
+    IBD_CUDA(cudaMemcpyAsync(c->d_start, c->sl.data(), c->sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
+    return 0;
+}
+
+int ibdgem::viterbi_scratch(ibdgem_engine *e, int n_tables, int64_t nb, HgViterbiScratch *s) {
+    if (scratch(e, SC_HG_LIK, (size_t)nb * 24, (void **)&s->lik) || scratch(e, SC_HG_STATE, (size_t)nb + (size_t)n_tables, (void **)&s->state) ||
+        scratch(e, SC_HG_SCORE, (size_t)nb * 24, (void **)&s->score) || scratch(e, SC_HG_COUNTS, (size_t)n_tables * 24, (void **)&s->counts))
+        return 1;
+    s->flag = s->state + nb;
+    return 0;
+}
+
+// The reference's long double recurrence decides the flagged tables (tables are independent: a few host threads).
+int ibdgem::viterbi_resolve(ibdgem_engine *e, const HgCall &c, const std::vector<uint8_t> &h_flag, const double *lik, bool lik_on_device,
+                            int is_log, double p01, double p02, double p12, uint8_t *state, double *score, int64_t *counts,
+                            bool out_on_device) {
+    std::vector<int> flagged;
+    std::vector<int64_t> at{0};  // at[k]: bins of the flagged tables before flagged[k] (their place in the host copies below)
+    for (int t = 0; t < c.n; t++)
+        if (h_flag[(size_t)t]) {
+            flagged.push_back(t);
+            at.push_back(at.back() + c.len(t));
+        }
+    const size_t nf = flagged.size();
+    e->hg_flagged = (int64_t)nf;
+    if (nf == 0) return 0;
+    std::vector<double> h_lik;  // the flagged tables' likelihoods, when they are on the device
+    if (lik_on_device) {
+        h_lik.resize((size_t)at[nf] * 3);
+        for (size_t k = 0; k < nf; k++)
+            IBD_CUDA(cudaMemcpyAsync(h_lik.data() + at[k] * 3, lik + c.start(flagged[k]) * 3, (size_t)c.len(flagged[k]) * 24,
+                                     cudaMemcpyDeviceToHost, e->stream));
+        IBD_CUDA(cudaStreamSynchronize(e->stream));
+    }
+    // results bound for device memory wait here for their copies
+    std::vector<uint8_t> up_state(out_on_device && state ? (size_t)at[nf] : 0);
+    std::vector<double> up_score(out_on_device && score ? (size_t)at[nf] * 3 : 0);
+    std::vector<int64_t> up_counts(out_on_device && counts ? nf * 3 : 0);
     auto redo = [&](size_t k0, size_t step) {
-        std::vector<uint8_t> st_tmp;
-        std::vector<double> sc_tmp;
-        for (size_t k = k0; k < flagged.size(); k += step) {
+        std::vector<uint8_t> st;
+        std::vector<double> sc;
+        for (size_t k = k0; k < nf; k += step) {
             const int t = flagged[k];
-            const int64_t b0 = bin_offsets[t], n = bin_offsets[t + 1] - b0;
-            int64_t c[3];
-            st_tmp.resize((size_t)n);
-            sc_tmp.resize((size_t)n * 3);
-            viterbi_long_double(lik + b0 * 3, n, is_log, p01, p02, p12, st_tmp.data(), sc_tmp.data(), c);
-            sink(k, t, st_tmp.data(), sc_tmp.data(), c);
+            const int64_t b0 = c.start(t), n = c.len(t);
+            int64_t cnt[3];
+            st.resize((size_t)n);
+            sc.resize((size_t)n * 3);
+            viterbi_long_double(lik_on_device ? h_lik.data() + at[k] * 3 : lik + b0 * 3, n, is_log, p01, p02, p12, st.data(), sc.data(), cnt);
+            if (state) memcpy(out_on_device ? up_state.data() + at[k] : state + b0, st.data(), (size_t)n);
+            if (score) memcpy(out_on_device ? up_score.data() + at[k] * 3 : score + b0 * 3, sc.data(), (size_t)n * 24);
+            if (counts) memcpy(out_on_device ? up_counts.data() + k * 3 : counts + (size_t)t * 3, cnt, 24);
         }
     };
-    const size_t nthr = std::max<size_t>(1, std::min<size_t>({flagged.size(), (size_t)16, (size_t)std::thread::hardware_concurrency()}));
+    const size_t nthr = std::max<size_t>(1, std::min<size_t>({nf, (size_t)16, (size_t)std::thread::hardware_concurrency()}));
     if (nthr <= 1) {
         redo(0, 1);
     } else {
@@ -476,25 +536,15 @@ void ibdgem::viterbi_redo_flagged(const std::vector<int> &flagged, const int64_t
         for (size_t k = 0; k < nthr; k++) pool.emplace_back(redo, k, nthr);
         for (auto &th : pool) th.join();
     }
-}
-
-// Host start / length of every table (stride > 0: table t starts at bin t * table_stride); 1 (error set) on a negative
-// length or one past the stride.
-int ibdgem::table_layout(const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, std::vector<int64_t> *sl,
-                         int64_t *maxbins, int64_t *total) {
-    sl->assign((size_t)n_tables * 2, 0);
-    *maxbins = *total = 0;
-    for (int t = 0; t < n_tables; t++) {
-        const int64_t n = bin_offsets[t + 1] - bin_offsets[t];
-        if (n < 0 || (table_stride > 0 && n > table_stride)) {
-            set_error("[::] ERROR in %s(): table %d has %lld bins (stride %lld).", fn, t, (long long)n, (long long)table_stride);
-            return 1;
-        }
-        (*sl)[(size_t)t] = table_stride > 0 ? (int64_t)t * table_stride : bin_offsets[t];
-        (*sl)[(size_t)n_tables + t] = n;
-        *maxbins = std::max(*maxbins, n);
-        *total += n;
+    if (!out_on_device) return 0;
+    for (size_t k = 0; k < nf; k++) {
+        const int t = flagged[k];
+        const int64_t b0 = c.start(t), n = c.len(t);
+        if (state) IBD_CUDA(cudaMemcpyAsync(state + b0, up_state.data() + at[k], (size_t)n, cudaMemcpyHostToDevice, e->stream));
+        if (score) IBD_CUDA(cudaMemcpyAsync(score + b0 * 3, up_score.data() + at[k] * 3, (size_t)n * 24, cudaMemcpyHostToDevice, e->stream));
+        if (counts) IBD_CUDA(cudaMemcpyAsync(counts + (size_t)t * 3, up_counts.data() + k * 3, 24, cudaMemcpyHostToDevice, e->stream));
     }
+    IBD_CUDA(cudaStreamSynchronize(e->stream));
     return 0;
 }
 
@@ -509,35 +559,11 @@ extern "C" int hiddengem_viterbi_batch(ibdgem_engine *e, int32_t n_tables, const
         set_error("[::] ERROR in hiddengem_viterbi_batch(): bad arguments.");
         return 1;
     }
-    std::vector<int64_t> h_sl;
-    int64_t maxbins_all, total;
-    if (table_layout("hiddengem_viterbi_batch", n_tables, bin_offsets, 0, &h_sl, &maxbins_all, &total)) return 1;
-    IBD_CUDA(cudaSetDevice(e->device));
+    HgCall c;
+    HgViterbiScratch d;
     const int64_t nb = bin_offsets[n_tables];
-    if (nb <= 0) {
-        set_error("[::] ERROR parsing likelihood data; make sure input is valid.");
+    if (hg_begin(e, "hiddengem_viterbi_batch", n_tables, bin_offsets, 0, true, &c) || viterbi_scratch(e, n_tables, nb, &d) || side_streams(e))
         return 1;
-    }
-    double *d_lik, *d_score;
-    int64_t *d_start;
-    uint8_t *d_state, *d_flag;
-    long long *d_counts;
-    if (scratch(e, SC_HG_LIK, (size_t)nb * 24, (void **)&d_lik) || scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start) ||
-        scratch(e, SC_HG_STATE, (size_t)nb + (size_t)n_tables, (void **)&d_state) || scratch(e, SC_HG_SCORE, (size_t)nb * 24, (void **)&d_score) ||
-        scratch(e, SC_HG_COUNTS, (size_t)n_tables * 24, (void **)&d_counts))
-        return 1;
-    d_flag = d_state + nb;
-    int64_t *d_len = d_start + n_tables;
-    if (!e->copy_stream) {
-        IBD_CUDA(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
-        IBD_CUDA(cudaEventCreateWithFlags(&e->ev_order, cudaEventDisableTiming));
-    }
-    if (!e->d2h_stream) IBD_CUDA(cudaStreamCreateWithFlags(&e->d2h_stream, cudaStreamNonBlocking));
-    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
-    // earlier work on the engine stream may still use the scratch buffers: the side streams start after it
-    IBD_CUDA(cudaEventRecord(e->ev_order, e->stream));
-    IBD_CUDA(cudaStreamWaitEvent(e->copy_stream, e->ev_order, 0));
-    IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, e->ev_order, 0));
     // Batches of whole tables, at least 64 so the batched kernels apply.  A batch's kernels take the time of one block
     // (the recursion is sequential in bins) however few tables it holds, so batches are few: about six per call —
     // copy-bound with ~1/6 of the upload exposed at the front and ~1/6 of the download at the back — and never below
@@ -552,70 +578,53 @@ extern "C" int hiddengem_viterbi_batch(ibdgem_engine *e, int32_t n_tables, const
         t = t1;
     }
     const size_t nbatch = cuts.size() - 1;
-    std::vector<cudaEvent_t> ev_up(nbatch), ev_done(nbatch);
-    for (size_t b = 0; b < nbatch; b++) {
-        IBD_CUDA(cudaEventCreateWithFlags(&ev_up[b], cudaEventDisableTiming));
-        IBD_CUDA(cudaEventCreateWithFlags(&ev_done[b], cudaEventDisableTiming));
-    }
-    int rc = 0;
-    for (size_t b = 0; b < nbatch && !rc; b++) {
-        const int t0 = cuts[b], t1 = cuts[b + 1];
-        const int64_t b0 = bin_offsets[t0], b1 = bin_offsets[t1];
-        IBD_CUDA(cudaMemcpyAsync(d_lik + b0 * 3, lik + b0 * 3, (size_t)(b1 - b0) * 24, cudaMemcpyHostToDevice, e->copy_stream));
-        IBD_CUDA(cudaEventRecord(ev_up[b], e->copy_stream));
-    }
-    for (size_t b = 0; b < nbatch && !rc; b++) {
-        const int t0 = cuts[b], t1 = cuts[b + 1];
-        const int64_t b0 = bin_offsets[t0], b1 = bin_offsets[t1];
-        int64_t maxbins = 0;
-        for (int t = t0; t < t1; t++) maxbins = std::max<int64_t>(maxbins, bin_offsets[t + 1] - bin_offsets[t]);
-        IBD_CUDA(cudaStreamWaitEvent(e->stream, ev_up[b], 0));
-        rc = viterbi_on_device(e, t1 - t0, maxbins, b1 - b0, d_start + t0, d_len + t0, d_lik, is_log, p01, p02, p12, d_state, d_score,
-                               d_counts + (size_t)t0 * 3, d_flag + t0);
-        if (rc) break;
-        IBD_CUDA(cudaEventRecord(ev_done[b], e->stream));
-        IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, ev_done[b], 0));
-        if (state) IBD_CUDA(cudaMemcpyAsync(state + b0, d_state + b0, (size_t)(b1 - b0), cudaMemcpyDeviceToHost, e->d2h_stream));
-        if (score_log) IBD_CUDA(cudaMemcpyAsync(score_log + b0 * 3, d_score + b0 * 3, (size_t)(b1 - b0) * 24, cudaMemcpyDeviceToHost, e->d2h_stream));
-    }
-    std::vector<uint8_t> h_flag((size_t)n_tables, 0);
+    std::vector<uint8_t> h_flag((size_t)n_tables);
     std::vector<long long> h_counts((size_t)n_tables * 3);
-    if (!rc) {
-        IBD_CUDA(cudaMemcpyAsync(h_counts.data(), d_counts, (size_t)n_tables * 24, cudaMemcpyDeviceToHost, e->stream));
-        IBD_CUDA(cudaMemcpyAsync(h_flag.data(), d_flag, (size_t)n_tables, cudaMemcpyDeviceToHost, e->stream));
-    }
+    // Batch b's upload is done at range event 2b, its kernels at 2b + 1 (every ABI call ends synchronised, so the
+    // engine's events are free here).
+    auto enqueue = [&]() -> int {
+        // earlier work on the engine stream may still use the scratch buffers: the side streams start after it
+        IBD_CUDA(cudaEventRecord(e->ev_order, e->stream));
+        IBD_CUDA(cudaStreamWaitEvent(e->copy_stream, e->ev_order, 0));
+        IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, e->ev_order, 0));
+        for (size_t b = 0; b < nbatch; b++) {
+            const int64_t b0 = bin_offsets[cuts[b]], b1 = bin_offsets[cuts[b + 1]];
+            cudaEvent_t up;
+            if (range_event(e, 2 * b, &up)) return 1;
+            IBD_CUDA(cudaMemcpyAsync(d.lik + b0 * 3, lik + b0 * 3, (size_t)(b1 - b0) * 24, cudaMemcpyHostToDevice, e->copy_stream));
+            IBD_CUDA(cudaEventRecord(up, e->copy_stream));
+        }
+        for (size_t b = 0; b < nbatch; b++) {
+            const int t0 = cuts[b], t1 = cuts[b + 1];
+            const int64_t b0 = bin_offsets[t0], b1 = bin_offsets[t1];
+            int64_t maxbins = 0;
+            for (int t = t0; t < t1; t++) maxbins = std::max<int64_t>(maxbins, bin_offsets[t + 1] - bin_offsets[t]);
+            cudaEvent_t up, done;
+            if (range_event(e, 2 * b, &up) || range_event(e, 2 * b + 1, &done)) return 1;
+            IBD_CUDA(cudaStreamWaitEvent(e->stream, up, 0));
+            if (viterbi_on_device(e, t1 - t0, maxbins, b1 - b0, c.d_start + t0, c.d_len + t0, d.lik, is_log, p01, p02, p12, d.state, d.score,
+                                  d.counts + (size_t)t0 * 3, d.flag + t0))
+                return 1;
+            IBD_CUDA(cudaEventRecord(done, e->stream));
+            IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, done, 0));
+            if (state) IBD_CUDA(cudaMemcpyAsync(state + b0, d.state + b0, (size_t)(b1 - b0), cudaMemcpyDeviceToHost, e->d2h_stream));
+            if (score_log)
+                IBD_CUDA(cudaMemcpyAsync(score_log + b0 * 3, d.score + b0 * 3, (size_t)(b1 - b0) * 24, cudaMemcpyDeviceToHost, e->d2h_stream));
+        }
+        IBD_CUDA(cudaMemcpyAsync(h_counts.data(), d.counts, (size_t)n_tables * 24, cudaMemcpyDeviceToHost, e->stream));
+        IBD_CUDA(cudaMemcpyAsync(h_flag.data(), d.flag, (size_t)n_tables, cudaMemcpyDeviceToHost, e->stream));
+        return 0;
+    };
+    // one way out: whatever was queued has finished with the caller's buffers before the call returns, failed or not
+    const int rc = enqueue();
     cudaStreamSynchronize(e->copy_stream);
     cudaStreamSynchronize(e->stream);
     cudaStreamSynchronize(e->d2h_stream);
-    for (size_t b = 0; b < nbatch; b++) {
-        cudaEventDestroy(ev_up[b]);
-        cudaEventDestroy(ev_done[b]);
-    }
     if (rc) return 1;
     IBD_CUDA(cudaGetLastError());
     settle_timers(e);
-    std::vector<int> flagged;
-    for (int t = 0; t < n_tables; t++) {
-        if (state_counts) {
-            state_counts[(size_t)t * 3] = h_counts[(size_t)t * 3];
-            state_counts[(size_t)t * 3 + 1] = h_counts[(size_t)t * 3 + 1];
-            state_counts[(size_t)t * 3 + 2] = h_counts[(size_t)t * 3 + 2];
-        }
-        if (h_flag[(size_t)t]) flagged.push_back(t);
-    }
-    e->hg_flagged = (int64_t)flagged.size();
-    viterbi_redo_flagged(flagged, bin_offsets, lik, is_log, p01, p02, p12,
-                         [&](size_t, int t, const uint8_t *st, const double *sc, const int64_t *c) {
-                             const int64_t b0 = bin_offsets[t], n = bin_offsets[t + 1] - b0;
-                             if (state) memcpy(state + b0, st, (size_t)n);
-                             if (score_log) memcpy(score_log + b0 * 3, sc, (size_t)n * 24);
-                             if (state_counts) {
-                                 state_counts[(size_t)t * 3] = c[0];
-                                 state_counts[(size_t)t * 3 + 1] = c[1];
-                                 state_counts[(size_t)t * 3 + 2] = c[2];
-                             }
-                         });
-    return 0;
+    if (state_counts) std::copy(h_counts.begin(), h_counts.end(), state_counts);
+    return viterbi_resolve(e, c, h_flag, lik, false, is_log, p01, p02, p12, state, score_log, state_counts, false);
 }
 
 // Device buffers in, device buffers out: the hiddengem front-end for scores that never left the GPU (SURVEY.md 8f-3).
@@ -631,41 +640,20 @@ extern "C" int hiddengem_viterbi_batch_device(ibdgem_engine *e, int32_t n_tables
         set_error("[::] ERROR in hiddengem_viterbi_batch_device(): bad arguments.");
         return 1;
     }
-    IBD_CUDA(cudaSetDevice(e->device));
-    std::vector<int64_t> h_sl;
-    int64_t maxbins, total;
-    if (table_layout("hiddengem_viterbi_batch_device", n_tables, bin_offsets, table_stride, &h_sl, &maxbins, &total)) return 1;
-    if (total <= 0) {
-        set_error("[::] ERROR parsing likelihood data; make sure input is valid.");
-        return 1;
-    }
-    int64_t *d_start;
+    HgCall c;
     uint8_t *d_flag;
-    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start) || scratch(e, SC_HG_STATE, (size_t)n_tables, (void **)&d_flag)) return 1;
-    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
+    if (hg_begin(e, "hiddengem_viterbi_batch_device", n_tables, bin_offsets, table_stride, true, &c) ||
+        scratch(e, SC_HG_STATE, (size_t)n_tables, (void **)&d_flag))
+        return 1;
     static_assert(sizeof(long long) == sizeof(int64_t), "state counts are 64-bit");
-    if (viterbi_on_device(e, n_tables, maxbins, total, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_state, d_score_log,
+    if (viterbi_on_device(e, n_tables, c.maxbins, c.total, c.d_start, c.d_len, d_lik, is_log, p01, p02, p12, d_state, d_score_log,
                           reinterpret_cast<long long *>(d_state_counts), d_flag))
         return 1;
     std::vector<uint8_t> h_flag((size_t)n_tables);
     IBD_CUDA(cudaMemcpyAsync(h_flag.data(), d_flag, (size_t)n_tables, cudaMemcpyDeviceToHost, e->stream));
     IBD_CUDA(cudaStreamSynchronize(e->stream));
     settle_timers(e);
-    e->hg_flagged = 0;
-    for (int t = 0; t < n_tables; t++) {
-        if (!h_flag[(size_t)t]) continue;
-        const int64_t b0 = h_sl[(size_t)t], n = h_sl[(size_t)n_tables + t];
-        std::vector<double> l((size_t)n * 3), sc((size_t)n * 3);
-        std::vector<uint8_t> st((size_t)n);
-        int64_t c[3];
-        IBD_CUDA(cudaMemcpy(l.data(), d_lik + b0 * 3, (size_t)n * 24, cudaMemcpyDeviceToHost));
-        viterbi_long_double(l.data(), n, is_log, p01, p02, p12, st.data(), sc.data(), c);
-        IBD_CUDA(cudaMemcpy(d_state + b0, st.data(), (size_t)n, cudaMemcpyHostToDevice));
-        IBD_CUDA(cudaMemcpy(d_score_log + b0 * 3, sc.data(), (size_t)n * 24, cudaMemcpyHostToDevice));
-        IBD_CUDA(cudaMemcpy(d_state_counts + (size_t)t * 3, c, 24, cudaMemcpyHostToDevice));
-        e->hg_flagged++;
-    }
-    return 0;
+    return viterbi_resolve(e, c, h_flag, d_lik, true, is_log, p01, p02, p12, d_state, d_score_log, d_state_counts, true);
 }
 
 // Tables of the last hiddengem call that were re-evaluated on the host in long double (near-tie guard).

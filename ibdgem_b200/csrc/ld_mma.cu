@@ -1178,7 +1178,7 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
     // write — slowed the GEMM by 15 % at C5 over 8 GPUs; there the shard's columns leave by one store kernel at the end)
     const bool direct = h_wll_mapped != nullptr && !by_chunk && !sharded;
     if (stream_out || stream_dev || direct) {
-        if (!e->d2h_stream) IBD_CUDA(cudaStreamCreateWithFlags(&e->d2h_stream, cudaStreamNonBlocking));
+        if (side_streams(e)) return 1;
         e->wll_streamed = stream_out || direct;
         e->wll_dev_streamed = stream_dev;
     }

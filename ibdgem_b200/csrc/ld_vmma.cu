@@ -1044,7 +1044,7 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
     double *h_wll_mapped = host_table_alias(e);
     cudaEvent_t ev_table = nullptr;  // the copy of the whole table is done
     if (h_wll_mapped) {
-        if (!e->d2h_stream) IBD_CUDA(cudaStreamCreateWithFlags(&e->d2h_stream, cudaStreamNonBlocking));
+        if (side_streams(e)) return 1;
         cudaEvent_t ev_ready;
         if (range_event(e, 0, &ev_ready) || range_event(e, 1, &ev_table)) return 1;
         IBD_CUDA(cudaEventRecord(ev_ready, e->stream));

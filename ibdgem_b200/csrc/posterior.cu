@@ -500,6 +500,62 @@ bool linear_penalties(double p01, double p02, double p12) {
     return lo > 0 && hi / lo <= 0x1p400;
 }
 
+// Both passes in arithmetic LG; p01 / p02 / p12 as the kernels take them (LG: their logs).  d_cov selects the moment
+// variant of the backward pass.
+template <bool LG>
+int posterior_launch(ibdgem_engine *e, int n_tables, const int64_t *d_start, const int64_t *d_len, const double *d_lik, int is_log,
+                     double p01, double p02, double p12, double *d_ckpt, double *d_post, double *d_expected, double *d_cov) {
+    const unsigned grid = (unsigned)((n_tables + HG_TABLES - 1) / HG_TABLES);
+    {
+        LaunchScope ls(e, K_POSTERIOR_FWD);
+        if (LG) e->k_launches[K_POSTERIOR_FWD_LOG]++;
+        posterior_fwd_kernel<LG><<<grid, HG_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt,
+                                                                               d_expected);
+    }
+    LaunchScope ls(e, d_cov ? K_POSTERIOR_BWD_MOMENTS : K_POSTERIOR_BWD);
+    if (LG) e->k_launches[K_POSTERIOR_BWD_LOG]++;
+    const auto bwd = d_cov ? posterior_bwd_kernel<LG, true> : posterior_bwd_kernel<LG, false>;
+    IBD_CUDA(cudaFuncSetAttribute(bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
+    bwd<<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt, d_post, d_expected,
+                                                      d_cov);
+    return 0;
+}
+
+// The body of the four posterior entries.  lik, post, expected and cov are host buffers (packed, table_stride 0) or,
+// with on_device, device buffers in the layout of table_stride; post and cov may be null, not both.
+int posterior_call(ibdgem_engine *e, const char *fn, int n_tables, const int64_t *bin_offsets, int64_t table_stride, const double *lik,
+                   bool on_device, int is_log, double p01, double p02, double p12, double *post, double *expected, double *cov) {
+    if (bad_penalties(fn, p01, p02, p12)) return 1;
+    HgCall c;
+    if (hg_begin(e, fn, n_tables, bin_offsets, table_stride, false, &c)) return 1;
+    const int64_t nb = c.total > 0 && !on_device ? bin_offsets[n_tables] : 0;  // host bins of lik / post
+    if (c.total > 0 && (!lik || (!cov && !post))) {
+        set_error("[::] ERROR in %s(): bad arguments.", fn);
+        return 1;
+    }
+    const double *d_lik = lik;
+    double *d_post = post, *d_expected = expected, *d_cov = cov;
+    if (!on_device) {  // expected (and cov) come back in one copy each from SC_HG_COUNTS
+        double *d_lik_up = nullptr;
+        d_post = nullptr;
+        if (scratch(e, SC_HG_COUNTS, (size_t)n_tables * (cov ? 96 : 24), (void **)&d_expected)) return 1;
+        if (nb > 0 && scratch(e, SC_HG_LIK, (size_t)nb * 24, (void **)&d_lik_up)) return 1;
+        if (nb > 0 && post && scratch(e, SC_HG_SCORE, (size_t)nb * 24, (void **)&d_post)) return 1;
+        if (nb > 0) IBD_CUDA(cudaMemcpyAsync(d_lik_up, lik, (size_t)nb * 24, cudaMemcpyHostToDevice, e->stream));
+        d_lik = d_lik_up;
+        d_cov = cov ? d_expected + (size_t)n_tables * 3 : nullptr;
+    }
+    if (posterior_on_device(e, n_tables, c.maxbins, c.d_start, c.d_len, d_lik, is_log, p01, p02, p12, d_post, d_expected, d_cov)) return 1;
+    if (!on_device) {
+        if (d_post) IBD_CUDA(cudaMemcpyAsync(post, d_post, (size_t)nb * 24, cudaMemcpyDeviceToHost, e->stream));
+        IBD_CUDA(cudaMemcpyAsync(expected, d_expected, (size_t)n_tables * 24, cudaMemcpyDeviceToHost, e->stream));
+        if (cov) IBD_CUDA(cudaMemcpyAsync(cov, d_cov, (size_t)n_tables * 72, cudaMemcpyDeviceToHost, e->stream));
+    }
+    IBD_CUDA(cudaStreamSynchronize(e->stream));
+    settle_timers(e);
+    return 0;
+}
+
 }  // namespace
 
 // One batch of tables, everything in device memory (start / len per table); kernels only, no host synchronisation.
@@ -513,46 +569,12 @@ int ibdgem::posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins,
     }
     double *d_ckpt;
     if (scratch(e, SC_HG_CKPT, (size_t)nck * n_tables * 24, (void **)&d_ckpt)) return 1;
-    const unsigned grid = (unsigned)((n_tables + HG_TABLES - 1) / HG_TABLES);
-    if (linear_penalties(p01, p02, p12)) {
-        {
-            LaunchScope ls(e, K_POSTERIOR_FWD);
-            posterior_fwd_kernel<false><<<grid, HG_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
-                                                                                      d_ckpt, d_expected);
-        }
-        if (d_cov) {
-            LaunchScope ls(e, K_POSTERIOR_BWD_MOMENTS);
-            IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
-            posterior_bwd_kernel<false, true><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02,
-                                                                                            p12, d_ckpt, d_post, d_expected, d_cov);
-        } else {
-            LaunchScope ls(e, K_POSTERIOR_BWD);
-            IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
-            posterior_bwd_kernel<false><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12,
-                                                                                      d_ckpt, d_post, d_expected);
-        }
-    } else {
-        const double l01 = log(p01), l02 = log(p02), l12 = log(p12);  // log(0) = -inf: a forbidden transition
-        {
-            LaunchScope ls(e, K_POSTERIOR_FWD);
-            e->k_launches[K_POSTERIOR_FWD_LOG]++;
-            posterior_fwd_kernel<true><<<grid, HG_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
-                                                                                     d_ckpt, d_expected);
-        }
-        if (d_cov) {
-            LaunchScope ls(e, K_POSTERIOR_BWD_MOMENTS);
-            e->k_launches[K_POSTERIOR_BWD_LOG]++;
-            IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
-            posterior_bwd_kernel<true, true><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02,
-                                                                                           l12, d_ckpt, d_post, d_expected, d_cov);
-        } else {
-            LaunchScope ls(e, K_POSTERIOR_BWD);
-            e->k_launches[K_POSTERIOR_BWD_LOG]++;
-            IBD_CUDA(cudaFuncSetAttribute(posterior_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PB_BWD_SMEM));
-            posterior_bwd_kernel<true><<<grid, HG_THREADS, PB_BWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, l01, l02, l12,
-                                                                                     d_ckpt, d_post, d_expected);
-        }
-    }
+    // log(0) = -inf: a forbidden transition
+    if (linear_penalties(p01, p02, p12) ? posterior_launch<false>(e, n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt, d_post,
+                                                                  d_expected, d_cov)
+                                        : posterior_launch<true>(e, n_tables, d_start, d_len, d_lik, is_log, log(p01), log(p02), log(p12),
+                                                                 d_ckpt, d_post, d_expected, d_cov))
+        return 1;
     IBD_CUDA(cudaGetLastError());
     return 0;
 }
@@ -564,30 +586,8 @@ extern "C" int hiddengem_posterior_batch(ibdgem_engine *e, int32_t n_tables, con
         set_error("[::] ERROR in hiddengem_posterior_batch(): bad arguments.");
         return 1;
     }
-    if (bad_penalties("hiddengem_posterior_batch", p01, p02, p12)) return 1;
-    std::vector<int64_t> h_sl;
-    int64_t maxbins, total;
-    if (table_layout("hiddengem_posterior_batch", n_tables, bin_offsets, 0, &h_sl, &maxbins, &total)) return 1;
-    const int64_t nb = total > 0 ? bin_offsets[n_tables] : 0;  // bins of lik / posterior
-    if (nb > 0 && (!lik || !posterior)) {
-        set_error("[::] ERROR in hiddengem_posterior_batch(): bad arguments.");
-        return 1;
-    }
-    IBD_CUDA(cudaSetDevice(e->device));
-    double *d_lik = nullptr, *d_post = nullptr, *d_expected;
-    int64_t *d_start;
-    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start) || scratch(e, SC_HG_COUNTS, (size_t)n_tables * 24, (void **)&d_expected))
-        return 1;
-    if (nb > 0 && (scratch(e, SC_HG_LIK, (size_t)nb * 24, (void **)&d_lik) || scratch(e, SC_HG_SCORE, (size_t)nb * 24, (void **)&d_post)))
-        return 1;
-    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
-    if (nb > 0) IBD_CUDA(cudaMemcpyAsync(d_lik, lik, (size_t)nb * 24, cudaMemcpyHostToDevice, e->stream));
-    if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_post, d_expected)) return 1;
-    if (nb > 0) IBD_CUDA(cudaMemcpyAsync(posterior, d_post, (size_t)nb * 24, cudaMemcpyDeviceToHost, e->stream));
-    IBD_CUDA(cudaMemcpyAsync(expected, d_expected, (size_t)n_tables * 24, cudaMemcpyDeviceToHost, e->stream));
-    IBD_CUDA(cudaStreamSynchronize(e->stream));
-    settle_timers(e);
-    return 0;
+    return posterior_call(e, "hiddengem_posterior_batch", n_tables, bin_offsets, 0, lik, false, is_log, p01, p02, p12, posterior, expected,
+                          nullptr);
 }
 
 // Device buffers in, device buffers out; bin_offsets is a HOST array.  table_stride > 0: table t starts at bin
@@ -600,18 +600,8 @@ extern "C" int hiddengem_posterior_batch_device(ibdgem_engine *e, int32_t n_tabl
         set_error("[::] ERROR in hiddengem_posterior_batch_device(): bad arguments.");
         return 1;
     }
-    if (bad_penalties("hiddengem_posterior_batch_device", p01, p02, p12)) return 1;
-    std::vector<int64_t> h_sl;
-    int64_t maxbins, total;
-    if (table_layout("hiddengem_posterior_batch_device", n_tables, bin_offsets, table_stride, &h_sl, &maxbins, &total)) return 1;
-    IBD_CUDA(cudaSetDevice(e->device));
-    int64_t *d_start;
-    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start)) return 1;
-    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
-    if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_posterior, d_expected)) return 1;
-    IBD_CUDA(cudaStreamSynchronize(e->stream));  // h_sl is read by the copy above
-    settle_timers(e);
-    return 0;
+    return posterior_call(e, "hiddengem_posterior_batch_device", n_tables, bin_offsets, table_stride, d_lik, true, is_log, p01, p02, p12,
+                          d_posterior, d_expected, nullptr);
 }
 
 // Posterior moments: the posterior pass with the moment variant of the backward kernel.  Host buffers in, host
@@ -623,32 +613,8 @@ extern "C" int hiddengem_posterior_moments_batch(ibdgem_engine *e, int32_t n_tab
         set_error("[::] ERROR in hiddengem_posterior_moments_batch(): bad arguments.");
         return 1;
     }
-    if (bad_penalties("hiddengem_posterior_moments_batch", p01, p02, p12)) return 1;
-    std::vector<int64_t> h_sl;
-    int64_t maxbins, total;
-    if (table_layout("hiddengem_posterior_moments_batch", n_tables, bin_offsets, 0, &h_sl, &maxbins, &total)) return 1;
-    const int64_t nb = total > 0 ? bin_offsets[n_tables] : 0;  // bins of lik / posterior
-    if (nb > 0 && !lik) {
-        set_error("[::] ERROR in hiddengem_posterior_moments_batch(): bad arguments.");
-        return 1;
-    }
-    IBD_CUDA(cudaSetDevice(e->device));
-    double *d_lik = nullptr, *d_post = nullptr, *d_out;
-    int64_t *d_start;
-    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start) || scratch(e, SC_HG_COUNTS, (size_t)n_tables * 96, (void **)&d_out))
-        return 1;
-    if (nb > 0 && scratch(e, SC_HG_LIK, (size_t)nb * 24, (void **)&d_lik)) return 1;
-    if (nb > 0 && posterior && scratch(e, SC_HG_SCORE, (size_t)nb * 24, (void **)&d_post)) return 1;
-    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
-    if (nb > 0) IBD_CUDA(cudaMemcpyAsync(d_lik, lik, (size_t)nb * 24, cudaMemcpyHostToDevice, e->stream));
-    double *d_cov = d_out + (size_t)n_tables * 3;
-    if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_post, d_out, d_cov)) return 1;
-    if (d_post) IBD_CUDA(cudaMemcpyAsync(posterior, d_post, (size_t)nb * 24, cudaMemcpyDeviceToHost, e->stream));
-    IBD_CUDA(cudaMemcpyAsync(expected, d_out, (size_t)n_tables * 24, cudaMemcpyDeviceToHost, e->stream));
-    IBD_CUDA(cudaMemcpyAsync(cov, d_cov, (size_t)n_tables * 72, cudaMemcpyDeviceToHost, e->stream));
-    IBD_CUDA(cudaStreamSynchronize(e->stream));
-    settle_timers(e);
-    return 0;
+    return posterior_call(e, "hiddengem_posterior_moments_batch", n_tables, bin_offsets, 0, lik, false, is_log, p01, p02, p12, posterior,
+                          expected, cov);
 }
 
 // Device buffers in, device buffers out (d_posterior may be null); bin_offsets is a HOST array, table_stride as for
@@ -660,17 +626,6 @@ extern "C" int hiddengem_posterior_moments_device(ibdgem_engine *e, int32_t n_ta
         set_error("[::] ERROR in hiddengem_posterior_moments_device(): bad arguments.");
         return 1;
     }
-    if (bad_penalties("hiddengem_posterior_moments_device", p01, p02, p12)) return 1;
-    std::vector<int64_t> h_sl;
-    int64_t maxbins, total;
-    if (table_layout("hiddengem_posterior_moments_device", n_tables, bin_offsets, table_stride, &h_sl, &maxbins, &total)) return 1;
-    IBD_CUDA(cudaSetDevice(e->device));
-    int64_t *d_start;
-    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start)) return 1;
-    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
-    if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_posterior, d_expected, d_cov))
-        return 1;
-    IBD_CUDA(cudaStreamSynchronize(e->stream));  // h_sl is read by the copy above
-    settle_timers(e);
-    return 0;
+    return posterior_call(e, "hiddengem_posterior_moments_device", n_tables, bin_offsets, table_stride, d_lik, true, is_log, p01, p02, p12,
+                          d_posterior, d_expected, d_cov);
 }

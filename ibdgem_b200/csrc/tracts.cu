@@ -211,50 +211,23 @@ extern "C" int hiddengem_tracts_batch(ibdgem_engine *e, int32_t n_tables, const 
         return 1;
     }
     if (with_posterior && bad_penalties("hiddengem_tracts_batch", p01, p02, p12)) return 1;
-    std::vector<int64_t> h_sl;
-    int64_t maxbins, total;
-    if (table_layout("hiddengem_tracts_batch", n_tables, bin_offsets, 0, &h_sl, &maxbins, &total)) return 1;
+    HgCall c;
+    HgViterbiScratch d;
     const int64_t nb = bin_offsets[n_tables];
-    if (nb <= 0) {
-        set_error("[::] ERROR parsing likelihood data; make sure input is valid.");
-        return 1;
-    }
-    IBD_CUDA(cudaSetDevice(e->device));
-    double *d_lik, *d_score;
-    int64_t *d_start;
-    uint8_t *d_state;
-    long long *d_counts;
-    if (scratch(e, SC_HG_LIK, (size_t)nb * 24, (void **)&d_lik) || scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start) ||
-        scratch(e, SC_HG_STATE, (size_t)nb + (size_t)n_tables, (void **)&d_state) || scratch(e, SC_HG_SCORE, (size_t)nb * 24, (void **)&d_score) ||
-        scratch(e, SC_HG_COUNTS, (size_t)n_tables * 24, (void **)&d_counts))
-        return 1;
-    uint8_t *d_flag = d_state + nb;
-    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
-    IBD_CUDA(cudaMemcpyAsync(d_lik, lik, (size_t)nb * 24, cudaMemcpyHostToDevice, e->stream));
-    if (viterbi_on_device(e, n_tables, maxbins, total, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_state, d_score, d_counts,
-                          d_flag))
+    if (hg_begin(e, "hiddengem_tracts_batch", n_tables, bin_offsets, 0, true, &c) || viterbi_scratch(e, n_tables, nb, &d)) return 1;
+    IBD_CUDA(cudaMemcpyAsync(d.lik, lik, (size_t)nb * 24, cudaMemcpyHostToDevice, e->stream));
+    if (viterbi_on_device(e, n_tables, c.maxbins, c.total, c.d_start, c.d_len, d.lik, is_log, p01, p02, p12, d.state, d.score, d.counts,
+                          d.flag))
         return 1;
     std::vector<uint8_t> h_flag((size_t)n_tables);
-    IBD_CUDA(cudaMemcpyAsync(h_flag.data(), d_flag, (size_t)n_tables, cudaMemcpyDeviceToHost, e->stream));
-    double *d_post = nullptr;
-    if (with_posterior) {
-        d_post = d_score;
-        if (posterior_on_device(e, n_tables, maxbins, d_start, d_start + n_tables, d_lik, is_log, p01, p02, p12, d_post,
-                                reinterpret_cast<double *>(d_counts)))
-            return 1;
-    }
+    IBD_CUDA(cudaMemcpyAsync(h_flag.data(), d.flag, (size_t)n_tables, cudaMemcpyDeviceToHost, e->stream));
+    double *d_post = with_posterior ? d.score : nullptr;
+    if (d_post && posterior_on_device(e, n_tables, c.maxbins, c.d_start, c.d_len, d.lik, is_log, p01, p02, p12, d_post,
+                                      reinterpret_cast<double *>(d.counts)))
+        return 1;
     IBD_CUDA(cudaStreamSynchronize(e->stream));
-    std::vector<int> flagged;
-    for (int t = 0; t < n_tables; t++)
-        if (h_flag[(size_t)t]) flagged.push_back(t);
-    e->hg_flagged = (int64_t)flagged.size();
-    std::vector<std::vector<uint8_t>> patch(flagged.size());
-    viterbi_redo_flagged(flagged, bin_offsets, lik, is_log, p01, p02, p12, [&](size_t k, int t, const uint8_t *st, const double *, const int64_t *) {
-        patch[k].assign(st, st + (bin_offsets[t + 1] - bin_offsets[t]));
-    });
-    for (size_t k = 0; k < flagged.size(); k++)
-        IBD_CUDA(cudaMemcpyAsync(d_state + bin_offsets[flagged[k]], patch[k].data(), patch[k].size(), cudaMemcpyHostToDevice, e->stream));
-    return tracts_on_device(e, "hiddengem_tracts_batch", n_tables, d_start, d_lik, is_log, d_state, d_post, tract_offsets);
+    if (viterbi_resolve(e, c, h_flag, lik, false, is_log, p01, p02, p12, d.state, nullptr, nullptr, true)) return 1;
+    return tracts_on_device(e, "hiddengem_tracts_batch", n_tables, c.d_start, d.lik, is_log, d.state, d_post, tract_offsets);
 }
 
 // Device states (and posteriors) in, tract records kept on the device; bin_offsets is a HOST array.
@@ -265,14 +238,9 @@ extern "C" int hiddengem_tracts_device(ibdgem_engine *e, int32_t n_tables, const
         set_error("[::] ERROR in hiddengem_tracts_device(): bad arguments.");
         return 1;
     }
-    std::vector<int64_t> h_sl;
-    int64_t maxbins, total;
-    if (table_layout("hiddengem_tracts_device", n_tables, bin_offsets, table_stride, &h_sl, &maxbins, &total)) return 1;
-    IBD_CUDA(cudaSetDevice(e->device));
-    int64_t *d_start;
-    if (scratch(e, SC_HG_OFF, (size_t)n_tables * 16, (void **)&d_start)) return 1;
-    IBD_CUDA(cudaMemcpyAsync(d_start, h_sl.data(), h_sl.size() * 8, cudaMemcpyHostToDevice, e->stream));
-    return tracts_on_device(e, "hiddengem_tracts_device", n_tables, d_start, d_lik, is_log, d_state, d_posterior, tract_offsets);
+    HgCall c;
+    if (hg_begin(e, "hiddengem_tracts_device", n_tables, bin_offsets, table_stride, false, &c)) return 1;
+    return tracts_on_device(e, "hiddengem_tracts_device", n_tables, c.d_start, d_lik, is_log, d_state, d_posterior, tract_offsets);
 }
 
 extern "C" int hiddengem_last_tracts(ibdgem_engine *e, hiddengem_tract *dst, int32_t dst_on_device) {

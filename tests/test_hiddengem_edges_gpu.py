@@ -8,9 +8,11 @@ numbers sit at the kernels' 16-bin chunks, 32-table blocks and the 64-table thre
 import numpy as np
 import pytest
 
+from test_cli_gpu import TIE_PENALTIES, _long_table, _tie_tables
 from test_hiddengem_edges_cpu import GAPS, LOG_CASES, PENALTY_SETS, gap_rows, to_text
 from test_posterior_cpu import posterior_oracle
 from test_posterior_gpu import _check
+from test_tracts_gpu import _as_text
 
 pytestmark = pytest.mark.gpu
 
@@ -361,6 +363,59 @@ def test_viterbi_special_layouts(pen):
     ll = [np.log(t) for t in _text_tables(rng, [int(n) for n in rng.integers(100, 140, 70)])]
     with np.errstate(divide="ignore"):
         _viterbi_check(ll, p, True, is_log=True)
+
+
+@pytest.mark.parametrize("layout", ["packed", "strided"])
+@pytest.mark.parametrize("tag", list(TIE_PENALTIES))
+def test_viterbi_device_entry_near_ties(tag, layout):
+    """The tie tables (and, at the default penalties, the long table) of test_tracts_gpu.test_near_tie_guard_states
+    through hiddengem_viterbi_batch_device: the tables the near-tie guard flags are re-evaluated in long double and
+    written back to the device buffers.  States, counts and the number of flagged tables equal the host entry's,
+    scores of the flagged tables bit for bit (both from the long double recurrence), and nothing outside a table's bins
+    is written."""
+    import torch
+    import ibdgem_b200 as ib
+    opt = dict(zip(TIE_PENALTIES[tag][0::2], map(float, TIE_PENALTIES[tag][1::2])))
+    pen = (opt.get("--p01", 1e-3), opt.get("--p02", 1e-6), opt.get("--p12", 1e-3))
+    tables = [_as_text(l) for l in _tie_tables()]
+    if tag == "default":
+        tables.append(_as_text(_long_table()))
+    off = _offsets(tables)
+    lens = np.diff(off)
+    lik = np.concatenate(tables)
+    stride = int(lens.max()) + 37 if layout == "strided" else 0
+    starts = np.arange(len(tables)) * stride if stride else off[:-1]
+    rows = len(tables) * stride if stride else int(off[-1]) + 64
+    inside = np.zeros(rows, bool)
+    lay = np.full((rows, 3), np.nan)
+    for t, l in enumerate(tables):
+        inside[starts[t]: starts[t] + lens[t]] = True
+        lay[starts[t]: starts[t] + lens[t]] = l
+    with ib.Engine(ib.Params()) as e:
+        flagged = []
+        for l in tables:  # which tables the guard hands to the host: fewer than 64 tables run the per-table kernel
+            e.viterbi_batch(l, [0, len(l)], False, *pen)
+            flagged.append(e.viterbi_last_flagged() == 1)
+        state, score, counts = e.viterbi_batch(lik, off, False, *pen)
+        n_flagged = e.viterbi_last_flagged()
+        d_lik = torch.from_numpy(lay).cuda()
+        d_state = torch.full((rows,), 9, dtype=torch.uint8, device="cuda")
+        d_score = torch.full((rows, 3), 7.0, dtype=torch.float64, device="cuda")
+        d_cnt = torch.full((len(tables), 3), -1, dtype=torch.int64, device="cuda")
+        e.viterbi_batch_device(d_lik.data_ptr(), off, False, d_state.data_ptr(), d_score.data_ptr(), d_cnt.data_ptr(),
+                               table_stride=stride, p01=pen[0], p02=pen[1], p12=pen[2])
+        assert e.viterbi_last_flagged() == n_flagged
+        s2, sc2 = d_state.cpu().numpy(), d_score.cpu().numpy()
+        np.testing.assert_array_equal(d_cnt.cpu().numpy(), counts)
+    assert n_flagged > 0 and n_flagged == sum(flagged)
+    for t in range(len(tables)):
+        a, b, s = off[t], off[t + 1], starts[t]
+        np.testing.assert_array_equal(s2[s: s + lens[t]], state[a:b])
+        if flagged[t]:
+            np.testing.assert_array_equal(sc2[s: s + lens[t]], score[a:b])
+        else:
+            np.testing.assert_allclose(sc2[s: s + lens[t]], score[a:b], rtol=0, atol=1e-9)
+    assert (s2[~inside] == 9).all() and (sc2[~inside] == 7.0).all()
 
 
 def test_non_monotone_offsets_rejected():
