@@ -87,6 +87,22 @@ int resolve_timers(ibdgem_engine *e) {
     return 0;
 }
 
+// IBDGEM_TIMELINE: the end of a scoring step in the timeline file, after its launches (resolve_timers) — when each panel
+// chunk arrived and when the window scores and the bookkeeping were on the host
+static void timeline_step(ibdgem_engine *e) {
+    if (!e->t0_set) return;
+    FILE *tl = fopen(e->timeline_path, "a");
+    if (!tl) return;
+    float ms = 0;
+    for (size_t k = 0; k < e->chunk_end.size(); k++)
+        if (cudaEventElapsedTime(&ms, e->ev_t0, e->chunk_ev[k]) == cudaSuccess) fprintf(tl, "chunk%d_arrived %.4f %.4f\n", (int)k, ms, ms);
+    if (cudaEventElapsedTime(&ms, e->ev_t0, e->ev_wll) == cudaSuccess) fprintf(tl, "wll_on_host %.4f %.4f\n", ms, ms);
+    if (cudaEventElapsedTime(&ms, e->ev_t0, e->ev_bookdone) == cudaSuccess) fprintf(tl, "bookkeeping_on_host %.4f %.4f\n", ms, ms);
+    fprintf(tl, "---\n");
+    fclose(tl);
+    cudaGetLastError();  // an event made before the timeline was switched on has no timestamp: not an engine error
+}
+
 int dev_alloc(ibdgem_engine *e, void **p, size_t bytes) {
     *p = nullptr;
     if (bytes == 0) bytes = 16;
@@ -1024,7 +1040,8 @@ static void free_panel(ibdgem_engine *e, int64_t S) {
     e->owns_bits = true;
     e->have_panel = false;
 }
-static void free_prepared(ibdgem_engine *e, int64_t S) {
+static void free_prepared(ibdgem_engine *e) {
+    const int64_t S = e->S;
     if (e->d_f) {
         dev_free(e, e->d_f, (size_t)S * 8);
         dev_free(e, e->d_keep, (size_t)S);
@@ -1034,7 +1051,7 @@ static void free_prepared(ibdgem_engine *e, int64_t S) {
         dev_free(e, e->d_rank, (size_t)S * 4);
     }
     if (e->d_wfirst) {
-        const size_t cap = (size_t)(S / std::max(e->prm.window_size, 1) + 2) * 8;
+        const size_t cap = (size_t)map_windows(e) * 8;
         dev_free(e, e->d_wfirst, cap);
         dev_free(e, e->d_wlast, cap);
         dev_free(e, e->d_nwin_shared, 4);
@@ -1050,15 +1067,32 @@ static void free_prepared(ibdgem_engine *e, int64_t S) {
     ld_tensor_release(e);
     ld_vtensor_release(e);
 }
+// New panel rows, a new shard or an explicit invalidation: the prepared state, the per-site table and the tensor caches
+// are stale (their buffers are kept)
+static void drop_prepared(ibdgem_engine *e) {
+    e->prepared = false;
+    e->table_from = e->table_upto = 0;
+    ld_tensor_invalidate(e);
+    ld_vtensor_invalidate(e);
+}
+// *ev = e->chunk_ev[k], creating the events up to k as needed
+static int chunk_event(ibdgem_engine *e, size_t k, cudaEvent_t *ev) {
+    while (e->chunk_ev.size() <= k) {
+        cudaEvent_t x;
+        IBD_CUDA(cudaEventCreateWithFlags(&x, e->t0_set ? cudaEventDefault : cudaEventDisableTiming));
+        e->chunk_ev.push_back(x);
+    }
+    *ev = e->chunk_ev[k];
+    return 0;
+}
 
 int ibdgem_engine_destroy(ibdgem_engine *e) {
     if (!e) return 0;
     cudaSetDevice(e->device);
     cudaStreamSynchronize(e->stream);
     resolve_timers(e);
-    const int64_t S = e->S;
-    free_prepared(e, S);
-    free_panel(e, S);
+    free_prepared(e);
+    free_panel(e, e->S);
     if (e->have_sites) free_sites(e);
     dev_free(e, e->d_P, e->h_P.size() * 8);
     dev_free(e, e->d_lnP, e->h_lnP.size() * 8);
@@ -1110,8 +1144,7 @@ int ibdgem_engine_upload_sites(ibdgem_engine *e, int64_t n_sites, const uint64_t
         return 1;
     }
     if (e->have_sites && (e->S != n_sites || (af_user != nullptr) != (e->d_afuser != nullptr))) {
-        const int64_t S_old = e->S;
-        free_prepared(e, S_old);
+        free_prepared(e);
         free_sites(e);
     }
     if (!e->have_sites) {
@@ -1145,7 +1178,7 @@ int ibdgem_engine_upload_panel(ibdgem_engine *e, int64_t n_sites, int32_t n_indi
         return 1;
     }
     if (e->have_panel && (e->S != n_sites || e->Wh != words_per_site)) {
-        free_prepared(e, e->S);
+        free_prepared(e);
         free_panel(e, e->S);
     }
     if (e->have_panel && !e->owns_bits) free_panel(e, e->S);  // never copy into the caller's device buffer
@@ -1162,49 +1195,30 @@ int ibdgem_engine_upload_panel(ibdgem_engine *e, int64_t n_sites, int32_t n_indi
     // step is ~ copy + one chunk's scoring + its result copy.  Measured at C3 (bench.py e2e, ms):
     // 1 chunk 22.5, 5: 13.6, 8: 13.1, 12: 12.8, 16: 12.65, 20: 12.6, 24: 13.3, 32: 14.9, 64: 20.2 — past ~20 the
     // per-range launches (a dozen per range) cost more than the shorter tail saves.  Tapered sizes
-    // (IBDGEM_PANEL_TAPER < 1) measured no better: the scoring rate is too close to the copy rate for
+    // (each smaller than the one before) measured no better: the scoring rate is too close to the copy rate for
     // shrinking chunks to stay ahead.
     // read once (C++11 static initialisers are thread-safe: `ibdgem --gpus N` calls this from one host
     // thread per device)
-    static const int want_chunks = [] {
-        const char *sc = getenv("IBDGEM_PANEL_CHUNKS");
-        return sc ? std::max(1, atoi(sc)) : PANEL_CHUNKS;
-    }();
-    static const double taper = [] {  // each chunk is `taper` times the size of the one before it
-        const char *st = getenv("IBDGEM_PANEL_TAPER");
-        const double t = st ? atof(st) : PANEL_TAPER;
-        return (t > 0.1 && t <= 1.0) ? t : 1.0;
-    }();
+    static const int want_chunks = std::max(1, env_int("IBDGEM_PANEL_CHUNKS", PANEL_CHUNKS));
     const size_t panel_bytes = (size_t)n_sites * (size_t)words_per_site * 4;
     const int nchunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)want_chunks, panel_bytes / PANEL_CHUNK_MIN_BYTES));
-    while ((int)e->chunk_ev.size() < nchunk) {
-        cudaEvent_t ev;
-        IBD_CUDA(cudaEventCreateWithFlags(&ev, e->t0_set ? cudaEventDefault : cudaEventDisableTiming));
-        e->chunk_ev.push_back(ev);
-    }
     IBD_CUDA(cudaEventRecord(e->ev_order, e->stream));
     IBD_CUDA(cudaStreamWaitEvent(e->copy_stream, e->ev_order, 0));
     e->chunk_end.assign((size_t)nchunk, 0);
-    double wsum = 0, wk = 1;
-    for (int k = 0; k < nchunk; k++, wk *= taper) wsum += wk;
     int64_t s0 = 0;
-    double acc = 0;
-    wk = 1;
-    for (int k = 0; k < nchunk; k++, wk *= taper) {
-        acc += wk / wsum;
-        const int64_t s1 = k + 1 == nchunk ? n_sites : std::min<int64_t>(n_sites, std::max<int64_t>(s0 + 1, (int64_t)(acc * (double)n_sites)));
+    for (int k = 0; k < nchunk; k++) {
+        const int64_t s1 = std::min<int64_t>(n_sites, std::max<int64_t>(s0 + 1, n_sites * (k + 1) / nchunk));
+        cudaEvent_t ev;
+        if (chunk_event(e, (size_t)k, &ev)) return 1;
         IBD_CUDA(cudaMemcpyAsync(e->d_bits + (size_t)s0 * words_per_site, bits + (size_t)s0 * words_per_site,
                                  (size_t)(s1 - s0) * words_per_site * 4, cudaMemcpyHostToDevice, e->copy_stream));
-        IBD_CUDA(cudaEventRecord(e->chunk_ev[(size_t)k], e->copy_stream));
+        IBD_CUDA(cudaEventRecord(ev, e->copy_stream));
         e->chunk_end[(size_t)k] = s1;
         s0 = s1;
     }
     e->chunks_waited = 0;
     e->have_panel = true;
-    e->prepared = false;
-    e->table_from = e->table_upto = 0;
-    ld_tensor_invalidate(e);
-    ld_vtensor_invalidate(e);
+    drop_prepared(e);
     return 0;
 }
 
@@ -1227,7 +1241,7 @@ int ibdgem_engine_set_panel_device(ibdgem_engine *e, int64_t n_sites, int32_t n_
     }
     // kernels of an earlier call may still read the old buffer
     IBD_CUDA(cudaStreamSynchronize(e->stream));
-    if (e->have_panel && (e->S != n_sites || e->Wh != words_per_site)) free_prepared(e, e->S);
+    if (e->have_panel && (e->S != n_sites || e->Wh != words_per_site)) free_prepared(e);
     if (e->have_panel) free_panel(e, e->S);
     e->S = n_sites;
     e->Wh = words_per_site;
@@ -1237,10 +1251,7 @@ int ibdgem_engine_set_panel_device(ibdgem_engine *e, int64_t n_sites, int32_t n_
     e->chunk_end.clear();
     e->chunks_waited = 0;
     e->have_panel = true;
-    e->prepared = false;
-    e->table_from = e->table_upto = 0;
-    ld_tensor_invalidate(e);
-    ld_vtensor_invalidate(e);
+    drop_prepared(e);
     return 0;
 }
 
@@ -1257,7 +1268,7 @@ int ibdgem_engine_clone_panel(ibdgem_engine *e, ibdgem_engine *src) {
     }
     IBD_CUDA(cudaSetDevice(e->device));
     if (e->have_panel && (e->S != src->S || e->Wh != src->Wh || !e->owns_bits)) {
-        free_prepared(e, e->S);
+        free_prepared(e);
         free_panel(e, e->S);
     }
     if (!e->have_panel) {
@@ -1276,29 +1287,23 @@ int ibdgem_engine_clone_panel(ibdgem_engine *e, ibdgem_engine *src) {
     IBD_CUDA(cudaStreamWaitEvent(e->copy_stream, e->ev_order, 0));
     // src's chunk layout: a caller-owned source panel (no chunks of its own) is taken as one piece, already complete
     const size_t nchunk = std::max<size_t>(1, src->chunk_end.size());
-    while (e->chunk_ev.size() < nchunk) {
-        cudaEvent_t ev;
-        IBD_CUDA(cudaEventCreateWithFlags(&ev, e->t0_set ? cudaEventDefault : cudaEventDisableTiming));
-        e->chunk_ev.push_back(ev);
-    }
     e->chunk_end.assign(nchunk, 0);
     int64_t s0 = 0;
     for (size_t k = 0; k < nchunk; k++) {
         const int64_t s1 = src->chunk_end.empty() ? src->S : src->chunk_end[k];
+        cudaEvent_t ev;
+        if (chunk_event(e, k, &ev)) return 1;
         if (!src->chunk_end.empty()) IBD_CUDA(cudaStreamWaitEvent(e->copy_stream, src->chunk_ev[k], 0));
         IBD_CUDA(cudaMemcpyPeerAsync(e->d_bits + (size_t)s0 * e->Wh, e->device, src->d_bits + (size_t)s0 * e->Wh, src->device,
                                      (size_t)(s1 - s0) * e->Wh * 4, e->copy_stream));
-        IBD_CUDA(cudaEventRecord(e->chunk_ev[k], e->copy_stream));
+        IBD_CUDA(cudaEventRecord(ev, e->copy_stream));
         e->chunk_end[k] = s1;
         s0 = s1;
     }
     e->chunks_waited = 0;
     e->have_panel = true;
     e->owns_bits = true;
-    e->prepared = false;
-    e->table_from = e->table_upto = 0;
-    ld_tensor_invalidate(e);
-    ld_vtensor_invalidate(e);
+    drop_prepared(e);
     return 0;
 }
 
@@ -1312,13 +1317,9 @@ int ibdgem_engine_panel_rows_ready(ibdgem_engine *e, int64_t row_end, void *stre
         return 1;
     }
     IBD_CUDA(cudaSetDevice(e->device));
-    const size_t k = e->chunk_end.size();
-    while (e->chunk_ev.size() <= k) {
-        cudaEvent_t ev;
-        IBD_CUDA(cudaEventCreateWithFlags(&ev, e->t0_set ? cudaEventDefault : cudaEventDisableTiming));
-        e->chunk_ev.push_back(ev);
-    }
-    IBD_CUDA(cudaEventRecord(e->chunk_ev[k], stream ? static_cast<cudaStream_t>(stream) : e->stream));
+    cudaEvent_t ev;
+    if (chunk_event(e, e->chunk_end.size(), &ev)) return 1;
+    IBD_CUDA(cudaEventRecord(ev, stream ? static_cast<cudaStream_t>(stream) : e->stream));
     e->chunk_end.push_back(row_end);
     return 0;
 }
@@ -1390,7 +1391,7 @@ int ibdgem_engine_prepare(ibdgem_engine *e) {
     }
     IBD_CUDA(cudaSetDevice(e->device));
     const int64_t S = e->S;
-    const int maxW = (int)(S / e->prm.window_size + 2);
+    const int maxW = map_windows(e);
     if (!e->d_f) {
         if (dev_alloc(e, (void **)&e->d_f, (size_t)S * 8) || dev_alloc(e, (void **)&e->d_keep, (size_t)S) ||
             dev_alloc(e, (void **)&e->d_status, (size_t)S) || dev_alloc(e, (void **)&e->d_lik7, (size_t)S * 56) ||
@@ -1450,10 +1451,7 @@ int ibdgem_engine_prepare(ibdgem_engine *e) {
 
 int ibdgem_engine_invalidate(ibdgem_engine *e) {
     if (!e) return 1;
-    e->prepared = false;
-    e->table_from = e->table_upto = 0;
-    ld_tensor_invalidate(e);
-    ld_vtensor_invalidate(e);
+    drop_prepared(e);
     return 0;
 }
 
@@ -1461,7 +1459,6 @@ int ibdgem_engine_get_site_table(ibdgem_engine *e, double *f, uint8_t *status, d
     if (!e) return 1;
     if (ibdgem_engine_prepare(e)) return 1;
     if (e->table_from > 0) {  // a window shard skipped the rows before its own: the whole table is wanted now
-        e->table_from = 0;
         e->table_from = e->table_upto = 0;
     }
     if (ensure_table(e, e->S)) return 1;
@@ -1470,6 +1467,22 @@ int ibdgem_engine_get_site_table(ibdgem_engine *e, double *f, uint8_t *status, d
     if (status) IBD_CUDA(cudaMemcpyAsync(status, e->d_status, (size_t)e->S, cudaMemcpyDeviceToHost, e->stream));
     if (lik7) IBD_CUDA(cudaMemcpyAsync(lik7, e->d_lik7, (size_t)e->S * 56, cudaMemcpyDeviceToHost, e->stream));
     IBD_CUDA(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+// The per-target window map of a call (the shared map serves the rest; the per-target-window tensor path builds its
+// own, in rank space for -v).  -v ranks sites by the target's genotype, i.e. reads panel rows: the engine stream must
+// depend on every panel chunk (and the per-site table) BEFORE the map is built, not only before the scoring kernels — a
+// lazily prepared engine has so far only looked at the site arrays.
+static int target_window_map(ibdgem_engine *e, const ScoreCall &c, WindowMapView *m) {
+    const int mapW = map_windows(e);
+    int64_t *d_wf, *d_wl, *d_ktot;
+    int32_t *d_nwin;
+    if (scratch(e, SC_WFIRST, (size_t)c.T * mapW * 8, (void **)&d_wf) || scratch(e, SC_WLAST, (size_t)c.T * mapW * 8, (void **)&d_wl) ||
+        scratch(e, SC_NWIN, (size_t)c.T * 4, (void **)&d_nwin) || scratch(e, SC_KTOT, (size_t)c.T * 8, (void **)&d_ktot))
+        return 1;
+    if (ensure_table(e, e->S) || build_window_map(e, c.v, c.d_targets, c.T, mapW, d_wf, d_wl, d_nwin, d_ktot, nullptr)) return 1;
+    *m = WindowMapView{d_wf, d_wl, d_nwin, c.T, mapW};
     return 0;
 }
 
@@ -1496,10 +1509,9 @@ static int score_common(ibdgem_engine *e, int32_t T, const int32_t *targets, int
     const int C = e->C;
     const int vflag = e->prm.variable_sites_only ? 1 : 0;
     const bool shared = !vflag && !tgt_counts;
-    const int mapW = shared ? std::max(e->nW_shared, 1) : (int)(S / e->prm.window_size + 2);
     const bool want_windows = out->n_windows || out->w_start || out->w_end || out->w_nsites || out->w_loglik ||
                               out->w_loglik_device || out->w_lik_linear;
-    const int outW = want_windows ? out->max_windows : mapW;
+    const int outW = want_windows ? out->max_windows : shared ? std::max(e->nW_shared, 1) : map_windows(e);
     if (want_windows && outW <= 0) {
         set_error("[::] ERROR: ibdgem_scores.max_windows must be positive.");
         return 1;
@@ -1509,137 +1521,91 @@ static int score_common(ibdgem_engine *e, int32_t T, const int32_t *targets, int
         return 1;
     }
 
-    int32_t *d_targets;
-    if (scratch(e, SC_TARGETS, (size_t)T * 4, (void **)&d_targets)) return 1;
-    IBD_CUDA(cudaMemcpyAsync(d_targets, targets, (size_t)T * 4, cudaMemcpyHostToDevice, e->stream));
-    uint8_t *d_tc = nullptr;
-    if (tgt_counts) {
-        if (scratch(e, SC_TGT_COUNTS, (size_t)T * S * 2, (void **)&d_tc)) return 1;
-        IBD_CUDA(cudaMemcpyAsync(d_tc, tgt_counts, (size_t)T * S * 2, cudaMemcpyHostToDevice, e->stream));
-    }
-    SiteView v = make_view(e, d_tc, vflag);
-
-    // window map
-    bool vtensor = false;
-    WindowMapView m;
-    int32_t *d_nwin;
-    int64_t *d_ktot;
-    if (shared) {
-        d_nwin = e->d_nwin_shared;
-        m.wfirst = e->d_wfirst;
-        m.wlast = e->d_wlast;
-        m.nwin = d_nwin;
-        m.rows = 1;
-        m.maxW = (int)(S / e->prm.window_size + 2);
-    } else if (ld && !e->force_general && ld_vtensor_eligible(e, T, n_bg)) {
-        vtensor = true;  // the per-target-window tensor path builds its own window map (in rank space for -v)
-        d_nwin = nullptr;
-        m.wfirst = m.wlast = nullptr;
-        m.nwin = nullptr;
-        m.rows = T;
-        m.maxW = mapW;
-    } else {
-        int64_t *d_wf, *d_wl;
-        if (scratch(e, SC_WFIRST, (size_t)T * mapW * 8, (void **)&d_wf) ||
-            scratch(e, SC_WLAST, (size_t)T * mapW * 8, (void **)&d_wl) ||
-            scratch(e, SC_NWIN, (size_t)std::max(T, 1) * 4, (void **)&d_nwin) ||
-            scratch(e, SC_KTOT, (size_t)std::max(T, 1) * 8, (void **)&d_ktot))
-            return 1;
-        // -v ranks sites by the target's genotype, i.e. reads panel rows: the engine stream must depend on
-        // every panel chunk (and the per-site table) BEFORE the map is built, not only before the scoring
-        // kernels — a lazily prepared engine has so far only looked at the site arrays
-        if (ensure_table(e, S)) return 1;
-        if (build_window_map(e, v, d_targets, T, mapW, d_wf, d_wl, d_nwin, d_ktot, nullptr)) return 1;
-        m.wfirst = d_wf;
-        m.wlast = d_wl;
-        m.nwin = d_nwin;
-        m.rows = T;
-        m.maxW = mapW;
-    }
-
-    // non-LD window sums (LIBD2 of --LD runs is the non-LD product too, src/ibdgem.c:752)
-    double *d_wll;
-    int32_t *d_wn, *d_nwout;
-    uint64_t *d_ws, *d_we;
-    const size_t nWT = (size_t)T * outW;
-    if (scratch(e, SC_WLL, nWT * 24, (void **)&d_wll) || scratch(e, SC_WN, nWT * 4 + (size_t)T * 4, (void **)&d_wn) ||
-        scratch(e, SC_WS, nWT * 8, (void **)&d_ws) || scratch(e, SC_WE, nWT * 8, (void **)&d_we))
+    ScoreCall c;
+    c.T = T;
+    c.outW = outW;
+    c.w_loglik = out->w_loglik;
+    c.w_loglik_device = static_cast<double *>(out->w_loglik_device);
+    if (ld) ld_background(e->N, T, targets, n_bg, bg, pu_idx, &c.bg);
+    // the path, chosen once: with every background member excluded (nU = 0) per-target windows take the general path,
+    // while the shared-window tensor path handles that case itself
+    int path = NONLD;
+    if (ld && !e->force_general && shared && ld_tensor_eligible(e, T, n_bg, tgt_counts))
+        path = LD_TENSOR;
+    else if (ld && !e->force_general && !shared && ld_vtensor_eligible(e, T, (int32_t)c.bg.bgU.size()))
+        path = LD_VTENSOR;
+    else if (ld)
+        path = LD_GENERAL;
+    if (path != LD_TENSOR && e->shard_count > 1) {
+        set_error("[::] ERROR: a window shard (ibdgem_engine_set_window_shard) needs the shared-window tensor --LD path; "
+                  "shard the target list instead for non-LD, -v and -D runs.");
         return 1;
-    d_nwout = d_wn + nWT;
-    {
-        LaunchScope ls(e, K_FILL);
-        fill_nan_kernel<<<(unsigned)std::min<int64_t>((int64_t)(nWT * 3 + 255) / 256, 4096), 256, 0, e->stream>>>(d_wll, (int64_t)nWT * 3);
     }
-    IBD_CUDA(cudaMemsetAsync(d_wn, 0, nWT * 4 + (size_t)T * 4, e->stream));
-    IBD_CUDA(cudaMemsetAsync(d_ws, 0, nWT * 8, e->stream));
-    IBD_CUDA(cudaMemsetAsync(d_we, 0, nWT * 8, e->stream));
-    const bool tensor = ld && !e->force_general && shared && ld_tensor_eligible(e, T, n_bg, tgt_counts);
-    e->book_ready = false;
-    if ((tensor || vtensor) && side_streams(e)) return 1;  // (a panel set in device memory never went through upload_panel)
-    if ((tensor || vtensor) && !e->ev_book) IBD_CUDA(cudaEventCreateWithFlags(&e->ev_book, cudaEventDisableTiming));
-    // everything but the tensor path reads the per-site table and the whole panel up front; the
-    // tensor path asks for them window range by window range (upload / scoring overlap)
-    if (!tensor) {
-        if (e->shard_count > 1) {
-            set_error("[::] ERROR: a window shard (ibdgem_engine_set_window_shard) needs the shared-window tensor --LD path; "
-                      "shard the target list instead for non-LD, -v and -D runs.");
-            return 1;
-        }
-        if (ensure_table(e, S)) return 1;
-    }
-    e->wll_streamed = false;
-    e->wll_dev_streamed = false;
-    e->h_wll_out = out->w_loglik;
-    e->d_wll_out_device = static_cast<double *>(out->w_loglik_device);
-    if (vtensor) {
-        const int rc = ld_vtensor_score(e, T, targets, d_targets, n_bg, bg, pu_idx, d_tc, outW, d_wll, d_wn, d_ws, d_we, d_nwout);
-        if (rc == 1) return 1;
-        if (rc == 2) {  // not taken after all (e.g. every background member excluded): the general path, with its own map
-            vtensor = false;
-            int64_t *d_wf, *d_wl;
-            if (scratch(e, SC_WFIRST, (size_t)T * mapW * 8, (void **)&d_wf) ||
-                scratch(e, SC_WLAST, (size_t)T * mapW * 8, (void **)&d_wl) ||
-                scratch(e, SC_NWIN, (size_t)std::max(T, 1) * 4, (void **)&d_nwin) ||
-                scratch(e, SC_KTOT, (size_t)std::max(T, 1) * 8, (void **)&d_ktot))
-                return 1;
-            if (build_window_map(e, v, d_targets, T, mapW, d_wf, d_wl, d_nwin, d_ktot, nullptr)) return 1;
-            m.wfirst = d_wf;
-            m.wlast = d_wl;
-            m.nwin = d_nwin;
-        } else {
-            e->last_ld_path = 2;
-        }
-    }
-    if (vtensor) {
-        // done: window bookkeeping, LIBD0, LIBD1 and LIBD2 of every target are in place
-    } else if (tensor) {
-        // tensor path: fills window bookkeeping, LIBD0, LIBD1 and LIBD2 of every target
-        if (ld_tensor_score(e, T, targets, d_targets, n_bg, bg, pu_idx, outW, d_wll, d_wn, d_ws, d_we, d_nwout)) return 1;
-        e->last_ld_path = 1;
-    } else {
-        {
-            LaunchScope ls(e, K_WINDOW_NONLD);
-            if (shared) {
-                const dim3 grid((unsigned)std::max(e->nW_shared, 1), (unsigned)((T + 127) / 128));
-                window_nonld_shared_kernel<<<grid, 128, 0, e->stream>>>(v, m, d_targets, T, e->d_pos, e->d_status, e->d_lnlik7, outW, d_wll, d_wn, d_ws, d_we, d_nwout);
-            } else {
-                const int64_t warps = (int64_t)nWT;
-                window_nonld_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, e->stream>>>(
-                    v, m, d_targets, T, e->d_pos, e->d_f, e->d_lnlik7, e->d_P, C, outW, d_wll, d_wn, d_ws, d_we, d_nwout);
-            }
-        }
-        IBD_CUDA(cudaGetLastError());
-    }
+    const bool want_counters = out->processed || out->skipped || out->final_total_cov || out->final_dist;
+    const int crow = C + 3;
+    const int crows = shared ? 1 : T;
+    std::vector<int32_t> h_nw(T);
+    std::vector<unsigned long long> h_cnt(want_counters ? (size_t)crows * crow : 0);
 
-    if (ld && !tensor && !vtensor) {
-        std::vector<int32_t> h_nref(T);
-        for (int t = 0; t < T; t++) {
-            int c = 0;
-            for (int n = 0; n < n_bg; n++)
-                if (bg[n] != targets[t] && bg[n] != pu_idx) c++;
-            h_nref[t] = c;
+    auto enqueue = [&]() -> int {
+        int32_t *d_targets;
+        if (scratch(e, SC_TARGETS, (size_t)T * 4, (void **)&d_targets)) return 1;
+        IBD_CUDA(cudaMemcpyAsync(d_targets, targets, (size_t)T * 4, cudaMemcpyHostToDevice, e->stream));
+        c.d_targets = d_targets;
+        uint8_t *d_tc = nullptr;
+        if (tgt_counts) {
+            if (scratch(e, SC_TGT_COUNTS, (size_t)T * S * 2, (void **)&d_tc)) return 1;
+            IBD_CUDA(cudaMemcpyAsync(d_tc, tgt_counts, (size_t)T * S * 2, cudaMemcpyHostToDevice, e->stream));
         }
+        c.v = make_view(e, d_tc, vflag);
+        const SiteView &v = c.v;
+        WindowMapView m{};
+        if (shared)
+            m = WindowMapView{e->d_wfirst, e->d_wlast, e->d_nwin_shared, 1, map_windows(e)};
+        else if (path != LD_VTENSOR && target_window_map(e, c, &m))
+            return 1;
+
+        // window outputs (LIBD2 of --LD runs is the non-LD product too, src/ibdgem.c:752)
+        const size_t nWT = (size_t)T * outW;
+        if (scratch(e, SC_WLL, nWT * 24, (void **)&c.d_wll) || scratch(e, SC_WN, nWT * 4 + (size_t)T * 4, (void **)&c.d_wn) ||
+            scratch(e, SC_WS, nWT * 8, (void **)&c.d_ws) || scratch(e, SC_WE, nWT * 8, (void **)&c.d_we))
+            return 1;
+        c.d_nwout = c.d_wn + nWT;
         {
+            LaunchScope ls(e, K_FILL);
+            fill_nan_kernel<<<(unsigned)std::min<int64_t>((int64_t)(nWT * 3 + 255) / 256, 4096), 256, 0, e->stream>>>(c.d_wll, (int64_t)nWT * 3);
+        }
+        IBD_CUDA(cudaMemsetAsync(c.d_wn, 0, nWT * 4 + (size_t)T * 4, e->stream));
+        IBD_CUDA(cudaMemsetAsync(c.d_ws, 0, nWT * 8, e->stream));
+        IBD_CUDA(cudaMemsetAsync(c.d_we, 0, nWT * 8, e->stream));
+        if (path == LD_TENSOR || path == LD_VTENSOR) {
+            if (side_streams(e)) return 1;  // (a panel set in device memory never went through upload_panel)
+            if (!e->ev_book) IBD_CUDA(cudaEventCreateWithFlags(&e->ev_book, cudaEventDisableTiming));
+        }
+        // everything but the shared-window tensor path reads the per-site table and the whole panel up front; that
+        // path asks for them window range by window range (upload / scoring overlap)
+        if (path != LD_TENSOR && ensure_table(e, S)) return 1;
+        if (path == LD_TENSOR) {
+            // window bookkeeping, LIBD0, LIBD1 and LIBD2 of every target
+            if (ld_tensor_score(e, c)) return 1;
+        } else if (path == LD_VTENSOR) {
+            if (ld_vtensor_score(e, c)) return 1;
+        } else {
+            {
+                LaunchScope ls(e, K_WINDOW_NONLD);
+                if (shared) {
+                    const dim3 grid((unsigned)std::max(e->nW_shared, 1), (unsigned)((T + 127) / 128));
+                    window_nonld_shared_kernel<<<grid, 128, 0, e->stream>>>(v, m, d_targets, T, e->d_pos, e->d_status, e->d_lnlik7, outW, c.d_wll, c.d_wn,
+                                                                            c.d_ws, c.d_we, c.d_nwout);
+                } else {
+                    const int64_t warps = (int64_t)nWT;
+                    window_nonld_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, e->stream>>>(
+                        v, m, d_targets, T, e->d_pos, e->d_f, e->d_lnlik7, e->d_P, C, outW, c.d_wll, c.d_wn, c.d_ws, c.d_we, c.d_nwout);
+                }
+            }
+            IBD_CUDA(cudaGetLastError());
+        }
+        if (path == LD_GENERAL) {
             int32_t *d_bg, *d_nrp;
             LdPartial *d_part;
             const int nz = std::max(1, (n_bg + LD_THREADS * LD_PER - 1) / (LD_THREADS * LD_PER));
@@ -1648,7 +1614,7 @@ static int score_common(ibdgem_engine *e, int32_t T, const int32_t *targets, int
                 scratch(e, SC_LD_PART, nWT * nz * sizeof(LdPartial), (void **)&d_part))
                 return 1;
             if (n_bg > 0) IBD_CUDA(cudaMemcpyAsync(d_bg, bg, (size_t)n_bg * 4, cudaMemcpyHostToDevice, e->stream));
-            IBD_CUDA(cudaMemcpyAsync(d_nrp, h_nref.data(), (size_t)T * 4, cudaMemcpyHostToDevice, e->stream));
+            IBD_CUDA(cudaMemcpyAsync(d_nrp, c.bg.nb.data(), (size_t)T * 4, cudaMemcpyHostToDevice, e->stream));
             // grid.y/z are limited to 65535: chunk the targets
             for (int t0 = 0; t0 < T; t0 += 32768) {
                 const int tc = std::min(32768, T - t0);
@@ -1666,104 +1632,87 @@ static int score_common(ibdgem_engine *e, int32_t T, const int32_t *targets, int
             }
             {
                 LaunchScope ls(e, K_LD_FINALIZE);
-                ld_finalize_kernel<<<(unsigned)((nWT + 255) / 256), 256, 0, e->stream>>>(d_part, nz, m, T, outW, d_nrp, d_wll);
+                ld_finalize_kernel<<<(unsigned)((nWT + 255) / 256), 256, 0, e->stream>>>(d_part, nz, m, T, outW, d_nrp, c.d_wll);
             }
             IBD_CUDA(cudaGetLastError());
-            e->last_ld_path = 0;
         }
-    }
 
-    if (e->shard_count == 1 && ensure_table(e, S)) return 1;  // no-op unless the tensor path left a tail
-    // the reference's own linear window products, on request (not for --LD with per-target windows: that path keeps its
-    // window map in rank space)
-    double *d_wlin = nullptr;
-    if (out->w_lik_linear && e->shard_count == 1) {
-        if (scratch(e, SC_WLIN, nWT * 24, (void **)&d_wlin)) return 1;
-        {
-            LaunchScope ls(e, K_FILL);
-            fill_nan_kernel<<<(unsigned)std::min<int64_t>((int64_t)(nWT * 3 + 255) / 256, 4096), 256, 0, e->stream>>>(d_wlin, (int64_t)nWT * 3);
+        if (e->shard_count == 1 && ensure_table(e, S)) return 1;  // no-op unless the tensor path left a tail
+        // the reference's own linear window products, on request (not for --LD with per-target windows: that path keeps its
+        // window map in rank space)
+        double *d_wlin = nullptr;
+        if (out->w_lik_linear && e->shard_count == 1) {
+            if (scratch(e, SC_WLIN, nWT * 24, (void **)&d_wlin)) return 1;
+            {
+                LaunchScope ls(e, K_FILL);
+                fill_nan_kernel<<<(unsigned)std::min<int64_t>((int64_t)(nWT * 3 + 255) / 256, 4096), 256, 0, e->stream>>>(d_wlin, (int64_t)nWT * 3);
+            }
+            if (path != LD_VTENSOR) {
+                LaunchScope ls(e, K_WINDOW_LINEAR);
+                window_linear_kernel<<<(unsigned)((nWT + 127) / 128), 128, 0, e->stream>>>(v, m, d_targets, T, e->d_f, e->d_lik7, e->d_P, C, outW, d_wlin);
+            }
+            IBD_CUDA(cudaGetLastError());
         }
-        if (!vtensor) {
-            LaunchScope ls(e, K_WINDOW_LINEAR);
-            window_linear_kernel<<<(unsigned)((nWT + 127) / 128), 128, 0, e->stream>>>(v, m, d_targets, T, e->d_f, e->d_lik7, e->d_P, C, outW, d_wlin);
+        // counters
+        unsigned long long *d_cnt = nullptr;
+        if (want_counters && shared && e->shared_cnt_valid) {
+            d_cnt = e->d_shared_cnt;  // counted by site_status_kernel in prepare()
+        } else if (want_counters) {
+            if (scratch(e, SC_COUNTERS, (size_t)crows * crow * 8, (void **)&d_cnt)) return 1;
+            IBD_CUDA(cudaMemsetAsync(d_cnt, 0, (size_t)crows * crow * 8, e->stream));
+            LaunchScope ls(e, K_COUNTERS);
+            for (int r0 = 0; r0 < crows; r0 += ROW_SLICE) {
+                const int rc = std::min(ROW_SLICE, crows - r0);
+                SiteView vv = v;
+                if (vv.tgt_counts) vv.tgt_counts += (size_t)r0 * S * 2;
+                counters_kernel<<<dim3((unsigned)((S + COUNTERS_CHUNK - 1) / COUNTERS_CHUNK), rc), 256, (size_t)crow * 8, e->stream>>>(
+                    vv, shared ? nullptr : d_targets + r0, C, d_cnt + (size_t)r0 * crow);
+            }
+        }
+        // expanded per-site outputs
+        uint8_t *d_st = nullptr;
+        double *d_sl = nullptr;
+        if (out->site_status || out->site_lik) {
+            if (out->site_status && scratch(e, SC_SITE_STATUS, (size_t)T * S, (void **)&d_st)) return 1;
+            if (out->site_lik && scratch(e, SC_SITE_LIK, (size_t)T * S * 24, (void **)&d_sl)) return 1;
+            LaunchScope ls(e, K_EXPAND_SITES);
+            const int64_t n = (int64_t)T * S;
+            expand_sites_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(v, d_targets, T, e->d_f, e->d_lik7, e->d_P, C, d_st, d_sl);
         }
         IBD_CUDA(cudaGetLastError());
-    }
-    // counters
-    const bool want_counters = out->processed || out->skipped || out->final_total_cov || out->final_dist;
-    unsigned long long *d_cnt = nullptr;
-    const int crow = C + 3;
-    const int crows = shared ? 1 : T;
-    if (want_counters && shared && e->shared_cnt_valid) {
-        d_cnt = e->d_shared_cnt;  // counted by site_status_kernel in prepare()
-    } else if (want_counters) {
-        if (scratch(e, SC_COUNTERS, (size_t)crows * crow * 8, (void **)&d_cnt)) return 1;
-        IBD_CUDA(cudaMemsetAsync(d_cnt, 0, (size_t)crows * crow * 8, e->stream));
-        LaunchScope ls(e, K_COUNTERS);
-        for (int r0 = 0; r0 < crows; r0 += ROW_SLICE) {
-            const int rc = std::min(ROW_SLICE, crows - r0);
-            SiteView vv = v;
-            if (vv.tgt_counts) vv.tgt_counts += (size_t)r0 * S * 2;
-            counters_kernel<<<dim3((unsigned)((S + COUNTERS_CHUNK - 1) / COUNTERS_CHUNK), rc), 256, (size_t)crow * 8, e->stream>>>(
-                vv, shared ? nullptr : d_targets + r0, C, d_cnt + (size_t)r0 * crow);
-        }
-    }
-    // expanded per-site outputs
-    uint8_t *d_st = nullptr;
-    double *d_sl = nullptr;
-    if (out->site_status || out->site_lik) {
-        if (out->site_status && scratch(e, SC_SITE_STATUS, (size_t)T * S, (void **)&d_st)) return 1;
-        if (out->site_lik && scratch(e, SC_SITE_LIK, (size_t)T * S * 24, (void **)&d_sl)) return 1;
-        LaunchScope ls(e, K_EXPAND_SITES);
-        const int64_t n = (int64_t)T * S;
-        expand_sites_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(v, d_targets, T, e->d_f, e->d_lik7, e->d_P, C, d_st, d_sl);
-    }
-    IBD_CUDA(cudaGetLastError());
 
-    // results -> host
-    if (out->w_loglik_device && !e->wll_dev_streamed)
-        IBD_CUDA(cudaMemcpyAsync(out->w_loglik_device, d_wll, nWT * 24, cudaMemcpyDefault, e->stream));
-    if (out->w_loglik && !e->wll_streamed)
-        IBD_CUDA(cudaMemcpyAsync(out->w_loglik, d_wll, nWT * 24, cudaMemcpyDeviceToHost, e->stream));
-    if (d_wlin) IBD_CUDA(cudaMemcpyAsync(out->w_lik_linear, d_wlin, nWT * 24, cudaMemcpyDeviceToHost, e->stream));
-    if (e->t0_set) IBD_CUDA(cudaEventRecord(e->ev_wll, e->wll_streamed ? e->d2h_stream : e->stream));
-    // the bookkeeping arrays of the tensor path are final before the GEMM starts: copy them on the
-    // copy stream so the transfer overlaps it
-    cudaStream_t bs = e->stream;
-    if (e->book_ready) {
-        IBD_CUDA(cudaStreamWaitEvent(e->copy_stream, e->ev_book, 0));
-        bs = e->copy_stream;
-    }
-    if (out->w_nsites) IBD_CUDA(cudaMemcpyAsync(out->w_nsites, d_wn, nWT * 4, cudaMemcpyDeviceToHost, bs));
-    if (out->w_start) IBD_CUDA(cudaMemcpyAsync(out->w_start, d_ws, nWT * 8, cudaMemcpyDeviceToHost, bs));
-    if (out->w_end) IBD_CUDA(cudaMemcpyAsync(out->w_end, d_we, nWT * 8, cudaMemcpyDeviceToHost, bs));
-    if (e->t0_set) IBD_CUDA(cudaEventRecord(e->ev_bookdone, bs));
-    std::vector<int32_t> h_nw(T);
-    IBD_CUDA(cudaMemcpyAsync(h_nw.data(), d_nwout, (size_t)T * 4, cudaMemcpyDeviceToHost, e->stream));
-    std::vector<unsigned long long> h_cnt;
-    if (want_counters) {
-        h_cnt.resize((size_t)crows * crow);
-        IBD_CUDA(cudaMemcpyAsync(h_cnt.data(), d_cnt, h_cnt.size() * 8, cudaMemcpyDeviceToHost, e->stream));
-    }
-    if (out->site_status) IBD_CUDA(cudaMemcpyAsync(out->site_status, d_st, (size_t)T * S, cudaMemcpyDeviceToHost, e->stream));
-    if (out->site_lik) IBD_CUDA(cudaMemcpyAsync(out->site_lik, d_sl, (size_t)T * S * 24, cudaMemcpyDeviceToHost, e->stream));
-    IBD_CUDA(cudaStreamSynchronize(e->stream));
-    if (e->book_ready) IBD_CUDA(cudaStreamSynchronize(e->copy_stream));
-    if (e->wll_streamed || e->wll_dev_streamed) IBD_CUDA(cudaStreamSynchronize(e->d2h_stream));
-    e->book_ready = false;
-    settle_timers(e);
-    if (e->t0_set) {
-        if (FILE *tl = fopen(e->timeline_path, "a")) {
-            float ms = 0;
-            for (size_t k = 0; k < e->chunk_end.size(); k++)
-                if (cudaEventElapsedTime(&ms, e->ev_t0, e->chunk_ev[k]) == cudaSuccess) fprintf(tl, "chunk%d_arrived %.4f %.4f\n", (int)k, ms, ms);
-            if (cudaEventElapsedTime(&ms, e->ev_t0, e->ev_wll) == cudaSuccess) fprintf(tl, "wll_on_host %.4f %.4f\n", ms, ms);
-            if (cudaEventElapsedTime(&ms, e->ev_t0, e->ev_bookdone) == cudaSuccess) fprintf(tl, "bookkeeping_on_host %.4f %.4f\n", ms, ms);
-            fprintf(tl, "---\n");
-            fclose(tl);
-            cudaGetLastError();  // an event made before the timeline was switched on has no timestamp: not an engine error
+        // results -> host
+        if (c.w_loglik_device && !c.dev_streamed)
+            IBD_CUDA(cudaMemcpyAsync(c.w_loglik_device, c.d_wll, nWT * 24, cudaMemcpyDefault, e->stream));
+        if (c.w_loglik && !c.streamed) IBD_CUDA(cudaMemcpyAsync(c.w_loglik, c.d_wll, nWT * 24, cudaMemcpyDeviceToHost, e->stream));
+        if (d_wlin) IBD_CUDA(cudaMemcpyAsync(out->w_lik_linear, d_wlin, nWT * 24, cudaMemcpyDeviceToHost, e->stream));
+        if (e->t0_set) IBD_CUDA(cudaEventRecord(e->ev_wll, c.streamed ? e->d2h_stream : e->stream));
+        // the bookkeeping arrays of the tensor paths are final before the GEMM starts: copy them on the
+        // copy stream so the transfer overlaps it
+        cudaStream_t bs = e->stream;
+        if (c.bookkeeping_ready) {
+            IBD_CUDA(cudaStreamWaitEvent(e->copy_stream, e->ev_book, 0));
+            bs = e->copy_stream;
         }
-    }
+        if (out->w_nsites) IBD_CUDA(cudaMemcpyAsync(out->w_nsites, c.d_wn, nWT * 4, cudaMemcpyDeviceToHost, bs));
+        if (out->w_start) IBD_CUDA(cudaMemcpyAsync(out->w_start, c.d_ws, nWT * 8, cudaMemcpyDeviceToHost, bs));
+        if (out->w_end) IBD_CUDA(cudaMemcpyAsync(out->w_end, c.d_we, nWT * 8, cudaMemcpyDeviceToHost, bs));
+        if (e->t0_set) IBD_CUDA(cudaEventRecord(e->ev_bookdone, bs));
+        IBD_CUDA(cudaMemcpyAsync(h_nw.data(), c.d_nwout, (size_t)T * 4, cudaMemcpyDeviceToHost, e->stream));
+        if (want_counters) IBD_CUDA(cudaMemcpyAsync(h_cnt.data(), d_cnt, h_cnt.size() * 8, cudaMemcpyDeviceToHost, e->stream));
+        if (out->site_status) IBD_CUDA(cudaMemcpyAsync(out->site_status, d_st, (size_t)T * S, cudaMemcpyDeviceToHost, e->stream));
+        if (out->site_lik) IBD_CUDA(cudaMemcpyAsync(out->site_lik, d_sl, (size_t)T * S * 24, cudaMemcpyDeviceToHost, e->stream));
+        return 0;
+    };
+    // one way out: whatever the call queued has finished with the caller's buffers before it returns, failed or not
+    const int rc = enqueue();
+    cudaStreamSynchronize(e->stream);
+    if (c.bookkeeping_ready) cudaStreamSynchronize(e->copy_stream);
+    if (c.streamed || c.dev_streamed) cudaStreamSynchronize(e->d2h_stream);
+    if (rc) return 1;
+    IBD_CUDA(cudaGetLastError());
+    settle_timers(e);
+    timeline_step(e);
 
     for (int t = 0; t < T; t++) {
         if (want_windows && h_nw[t] > outW) {
@@ -1772,14 +1721,15 @@ static int score_common(ibdgem_engine *e, int32_t T, const int32_t *targets, int
         }
         if (out->n_windows) out->n_windows[t] = h_nw[t];
         if (want_counters) {
-            const unsigned long long *c = &h_cnt[(size_t)(shared ? 0 : t) * crow];
-            if (out->processed) out->processed[t] = c[0];
-            if (out->skipped) out->skipped[t] = c[1];
-            if (out->final_total_cov) out->final_total_cov[t] = c[2];
+            const unsigned long long *cn = &h_cnt[(size_t)(shared ? 0 : t) * crow];
+            if (out->processed) out->processed[t] = cn[0];
+            if (out->skipped) out->skipped[t] = cn[1];
+            if (out->final_total_cov) out->final_total_cov[t] = cn[2];
             if (out->final_dist)
-                for (int k = 0; k < C; k++) out->final_dist[(size_t)t * C + k] = c[3 + k];
+                for (int k = 0; k < C; k++) out->final_dist[(size_t)t * C + k] = cn[3 + k];
         }
     }
+    if (ld) e->last_ld_path = path;
     return 0;
 }
 
@@ -1802,10 +1752,7 @@ int ibdgem_engine_set_window_shard(ibdgem_engine *e, int32_t index, int32_t coun
     if (e->shard_index != index || e->shard_count != count) {
         e->shard_index = index;
         e->shard_count = count;
-        e->prepared = false;
-        e->table_from = e->table_upto = 0;
-        ld_tensor_invalidate(e);
-        ld_vtensor_invalidate(e);
+        drop_prepared(e);
     }
     return 0;
 }

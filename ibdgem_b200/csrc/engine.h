@@ -4,11 +4,13 @@
 
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdlib.h>
 
 #include <string>
 #include <vector>
 
 #include "../../include/ibdgem_b200.h"
+#include "site_math.cuh"
 
 namespace ibdgem {
 
@@ -71,7 +73,6 @@ extern const char *const *const kKernelNames;  // [K_COUNT], in enum order (engi
 
 struct LdCache;  // ld_mma.cu
 struct VCache;   // ld_vmma.cu
-struct SiteView;
 
 struct PendingTimer {
     int id;
@@ -115,13 +116,10 @@ struct ibdgem_engine {
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_order = nullptr;          // engine stream -> copy stream ordering
     cudaEvent_t ev_book = nullptr;           // window bookkeeping of the current call is final (tensor path)
-    bool book_ready = false;
     // window scores of the tensor path leave for the host range by range while later ranges are still
     // being scored: d2h_stream carries them (copy_stream is busy with the panel chunks)
     cudaStream_t d2h_stream = nullptr;
     std::vector<cudaEvent_t> range_ev;
-    double *h_wll_out = nullptr;   // the call's host destination, or nullptr
-    bool wll_streamed = false;     // ld_tensor_score has already issued the copies of d_wll
     std::vector<cudaEvent_t> chunk_ev;       // one per chunk, recorded on copy_stream
     std::vector<int64_t> chunk_end;          // exclusive site end of each chunk
     int chunks_waited = 0;                   // chunks the engine stream already depends on
@@ -130,8 +128,6 @@ struct ibdgem_engine {
     // of every target and touches only the panel rows of those windows (ibdgem_engine_set_window_shard)
     int32_t shard_index = 0, shard_count = 1;
     bool shard_compact = false;              // window shards: the host score table is [T][shard windows][3], not [T][maxW][3]
-    double *d_wll_out_device = nullptr;      // the call's optional device destination (may be peer memory)
-    bool wll_dev_streamed = false;           // ld_tensor_score has already issued the copies to it
     bool lazy_table = false;                 // status does not need the panel (no -A, AF range [0, 1])
     std::vector<int64_t> h_wlast;            // host copy of the shared window map (last site per window)
 
@@ -192,6 +188,13 @@ struct LaunchScope {
 };
 int resolve_timers(ibdgem_engine *e);
 int settle_timers(ibdgem_engine *e);
+// integer value of the environment variable `name` (read by the caller once per process), or dflt when it is unset
+inline int env_int(const char *name, int dflt) {
+    const char *s = getenv(name);
+    return s ? atoi(s) : dflt;
+}
+// columns of a per-target window map: no target has more windows than S / window_size + 2
+inline int map_windows(const ibdgem_engine *e) { return (int)(e->S / e->prm.window_size + 2); }
 // Pinned host staging of at least `bytes`.  One buffer: a caller must have synchronised the stream
 // that reads or writes it before the next caller asks (every ABI call ends with such a sync).
 int pinned_stage(ibdgem_engine *e, size_t bytes, void **out);
@@ -260,19 +263,6 @@ int ensure_table(ibdgem_engine *e, int64_t s_end);
 int dev_alloc(ibdgem_engine *e, void **p, size_t bytes);
 void dev_free(ibdgem_engine *e, void *p, size_t bytes);
 
-// tensor-path entry points (ld_mma.cu)
-bool ld_tensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t n_bg, const uint8_t *tgt_counts);
-int ld_tensor_prepare(ibdgem_engine *e);
-int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const int32_t *d_targets, int32_t n_bg,
-                    const int32_t *h_bg, int32_t pu_idx, int32_t outW, double *d_wll /*[T][outW][3]*/, int32_t *d_wn,
-                    uint64_t *d_ws, uint64_t *d_we, int32_t *d_nwout);
-void ld_tensor_release(ibdgem_engine *e);
-constexpr int PANEL_CHUNKS = 16;         // upload / scoring pipeline depth
-constexpr double PANEL_TAPER = 1.0;       // chunk k is PANEL_TAPER^k of the first chunk
-constexpr size_t PANEL_CHUNK_MIN_BYTES = (size_t)16 << 20;  // ~0.3 ms of PCIe; smaller panels use fewer chunks
-void ld_tensor_invalidate(ibdgem_engine *e);
-// site-major bits -> [block][haplotype][WP32 words] for `nwin` blocks of Wpad slots listed in `infsite` (ld_mma.cu)
-int ld_transpose_launch(ibdgem_engine *e, int w_begin, int w_end, const int32_t *infsite, int Wpad, int WP32, int H, uint32_t *tbits);
 // The call's background as both tensor paths see it (ld_mma.cu): the unique individuals in ascending order with
 // ln(multiplicity) — the pileup's own individual never contributes (src/ibdgem.c:714) — and per target its own index in
 // that list (-1: none) and nb, the background size without it, with ln nb (NaN when nb = 0: 0/0 in the reference).
@@ -280,19 +270,50 @@ struct LdBackground {
     std::vector<int32_t> bgU;
     std::vector<double> lnc;
     std::vector<int32_t> own;
-    std::vector<int64_t> nb;
+    std::vector<int32_t> nb;
     std::vector<double> lognb;
 };
 void ld_background(int32_t N, int32_t T, const int32_t *h_targets, int32_t n_bg, const int32_t *h_bg, int32_t pu_idx, LdBackground *out);
-// device alias of the caller's host table e->h_wll_out when it is page-locked and mapped, else nullptr (ld_mma.cu)
-double *host_table_alias(ibdgem_engine *e);
+
+// The scoring paths of score_ld / score_nonld; ibdgem_engine_last_ld_path reports the --LD one that ran.
+enum ScorePath { NONLD = -1, LD_GENERAL = 0, LD_TENSOR = 1, LD_VTENSOR = 2 };
+
+// One scoring call: its inputs, the window outputs in device memory, the caller's destinations of the window scores,
+// and the copies into them that a tensor path has already issued (the call's end waits for exactly those streams).
+struct ScoreCall {
+    int32_t T = 0;
+    const int32_t *d_targets = nullptr;  // [T]
+    SiteView v{};                        // v.tgt_counts: the call's -D counts in device memory, [T][S][2], or nullptr
+    LdBackground bg;                     // --LD
+    int32_t outW = 0;                    // columns of the window outputs
+    double *d_wll = nullptr;             // [T][outW][3]
+    int32_t *d_wn = nullptr;             // [T][outW]
+    uint64_t *d_ws = nullptr, *d_we = nullptr;  // [T][outW]
+    int32_t *d_nwout = nullptr;          // [T]
+    double *w_loglik = nullptr;          // the caller's host table [T][outW][3], or nullptr
+    double *w_loglik_device = nullptr;   // the caller's device table (may be peer memory), or nullptr
+    bool streamed = false;               // the copies of d_wll to w_loglik are issued on d2h_stream
+    bool dev_streamed = false;           // the copies of d_wll to w_loglik_device are issued on d2h_stream
+    bool bookkeeping_ready = false;      // ev_book is recorded: the bookkeeping copies may go on copy_stream
+};
+
+// tensor-path entry points (ld_mma.cu)
+bool ld_tensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t n_bg, const uint8_t *tgt_counts);
+int ld_tensor_prepare(ibdgem_engine *e);
+int ld_tensor_score(ibdgem_engine *e, ScoreCall &c);
+void ld_tensor_release(ibdgem_engine *e);
+constexpr int PANEL_CHUNKS = 16;         // upload / scoring pipeline depth
+constexpr size_t PANEL_CHUNK_MIN_BYTES = (size_t)16 << 20;  // ~0.3 ms of PCIe; smaller panels use fewer chunks
+void ld_tensor_invalidate(ibdgem_engine *e);
+// site-major bits -> [block][haplotype][WP32 words] for `nwin` blocks of Wpad slots listed in `infsite` (ld_mma.cu)
+int ld_transpose_launch(ibdgem_engine *e, int w_begin, int w_end, const int32_t *infsite, int Wpad, int WP32, int H, uint32_t *tbits);
+// device alias of the caller's host table c.w_loglik when it is page-locked and mapped, else nullptr (ld_mma.cu)
+double *host_table_alias(const ScoreCall &c);
 // *ev = e->range_ev[k], creating the events up to k as needed (ld_mma.cu)
 int range_event(ibdgem_engine *e, size_t k, cudaEvent_t *ev);
-// per-target-window tensor path (ld_vmma.cu): -v / -D
-bool ld_vtensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t n_bg);
-int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const int32_t *d_targets, int32_t n_bg, const int32_t *h_bg,
-                     int32_t pu_idx, const uint8_t *d_tgt_counts, int32_t outW, double *d_wll, int32_t *d_wn, uint64_t *d_ws,
-                     uint64_t *d_we, int32_t *d_nwout);  // 0 = done, 2 = not taken, 1 = error
+// per-target-window tensor path (ld_vmma.cu): -v / -D; nU is the size of the call's unique background
+bool ld_vtensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t nU);
+int ld_vtensor_score(ibdgem_engine *e, ScoreCall &c);
 void ld_vtensor_release(ibdgem_engine *e);
 void ld_vtensor_invalidate(ibdgem_engine *e);
 // window map for `rows` rows (targets == nullptr: one shared row), engine.cu

@@ -985,15 +985,15 @@ void ld_background(int32_t N, int32_t T, const int32_t *h_targets, int32_t n_bg,
         const int own = where[h_targets[t]];
         const int64_t nb = total_bg - (own >= 0 ? mult[h_targets[t]] : 0);
         out->own[t] = own;
-        out->nb[t] = nb;
+        out->nb[t] = (int32_t)nb;
         out->lognb[t] = nb > 0 ? log((double)nb) : (double)NAN;
     }
 }
 
-double *host_table_alias(ibdgem_engine *e) {
-    if (!e->h_wll_out) return nullptr;
+double *host_table_alias(const ScoreCall &c) {
+    if (!c.w_loglik) return nullptr;
     cudaPointerAttributes attr;
-    if (cudaPointerGetAttributes(&attr, e->h_wll_out) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
+    if (cudaPointerGetAttributes(&attr, c.w_loglik) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
         return static_cast<double *>(attr.devicePointer);
     cudaGetLastError();
     return nullptr;
@@ -1030,14 +1030,14 @@ int ld_tensor_prepare(ibdgem_engine *e) {
 }
 
 // Fills every window output of the call: d_wll [T][outW][3], d_wn, d_ws, d_we [T][outW], d_nwout [T].
-int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const int32_t *d_targets, int32_t n_bg,
-                    const int32_t *h_bg, int32_t pu_idx, int32_t outW, double *d_wll, int32_t *d_wn, uint64_t *d_ws,
-                    uint64_t *d_we, int32_t *d_nwout) {
+int ld_tensor_score(ibdgem_engine *e, ScoreCall &sc) {
     if (build_cache(e)) return 1;
     LdCache *c = e->ld;
-    // duplicate background entries become a ln(multiplicity) weight on one individual
-    LdBackground bg;
-    ld_background(c->N, T, h_targets, n_bg, h_bg, pu_idx, &bg);
+    // duplicate background entries are a ln(multiplicity) weight on one individual (sc.bg)
+    const LdBackground &bg = sc.bg;
+    const int T = sc.T, outW = sc.outW;
+    const int32_t *d_targets = sc.d_targets;
+    double *d_wll = sc.d_wll;
     const int nU = (int)bg.bgU.size();
     std::vector<int32_t> row_own(2 * (size_t)T);
     std::vector<double> lognb4(T);
@@ -1081,7 +1081,7 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
         const int64_t units = (int64_t)span * ((2 * T + 255) / 256);
         int parts = 1;
         if (parts_env < 0) parts = std::min(span, -parts_env);
-        else if (e->h_wll_out && parts_env > 1 && (size_t)T * span * 24 >= ((size_t)20 << 20))
+        else if (sc.w_loglik && parts_env > 1 && (size_t)T * span * 24 >= ((size_t)20 << 20))
             // (a sub-range costs ~0.1 ms in launches and GEMM ramps: measured a loss below ~20 MB of shard table — C3 over
             // 2 and 4 GPUs — and a gain above — C5 over 8)
             parts = (int)std::max<int64_t>(1, std::min<int64_t>(parts_env, units / (8 * std::max(1, e->sm_count / 2))));
@@ -1104,7 +1104,7 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
             LaunchScope ls(e, K_LD_WINDOWS);
             const int64_t n = (int64_t)T * nW;
             ld_windows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(
-                0, nW, T, nW, outW, c->W, c->K, e->d_wfirst, e->d_wlast, e->d_pos, d_wn, d_ws, d_we, d_nwout);
+                0, nW, T, nW, outW, c->W, c->K, e->d_wfirst, e->d_wlast, e->d_pos, sc.d_wn, sc.d_ws, sc.d_we, sc.d_nwout);
         }
         {
             LaunchScope ls(e, K_LD_EXPAND_TGT);
@@ -1165,12 +1165,12 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
                                                                static_cast<const uint32_t *>(h_misc), n);
     }
 
-    const bool stream_out = (range_end.size() > 1 || sharded) && e->h_wll_out != nullptr;
+    const bool stream_out = (range_end.size() > 1 || sharded) && sc.w_loglik != nullptr;
     // the optional device destination (the root's gather buffer, possibly peer memory over NVLink) is
     // filled range by range too
-    const bool stream_dev = e->d_wll_out_device != nullptr;
+    const bool stream_dev = sc.w_loglik_device != nullptr;
     // page-locked host destination: its device alias, for stores from a kernel
-    double *h_wll_mapped = host_table_alias(e);
+    double *h_wll_mapped = host_table_alias(sc);
     // direct mode: the GEMM's merge warps store finished score triples into the page-locked host table themselves
     // (not while panel chunks are still arriving: measured at C3 end to end, the 24-byte posted writes of every range
     // compete with the upload on the link — 13.3 ms against 12.6 with the per-range store kernel)
@@ -1179,8 +1179,8 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
     const bool direct = h_wll_mapped != nullptr && !by_chunk && !sharded;
     if (stream_out || stream_dev || direct) {
         if (side_streams(e)) return 1;
-        e->wll_streamed = stream_out || direct;
-        e->wll_dev_streamed = stream_dev;
+        sc.streamed = stream_out || direct;
+        sc.dev_streamed = stream_dev;
     }
     auto launch_ibd0 = [&](int wa, int wb_) -> int {
         LaunchScope ls(e, K_LD_IBD0);
@@ -1225,14 +1225,14 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
         const int b_lo = sharded ? 0 : w_lo, b_hi = sharded ? nW : w_hi;
         const int64_t n = (int64_t)T * (b_hi - b_lo);
         ld_windows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->stream>>>(
-            b_lo, b_hi, T, nW, outW, c->W, c->K, e->d_wfirst, e->d_wlast, e->d_pos, d_wn, d_ws, d_we, d_nwout);
+            b_lo, b_hi, T, nW, outW, c->W, c->K, e->d_wfirst, e->d_wlast, e->d_pos, sc.d_wn, sc.d_ws, sc.d_we, sc.d_nwout);
     }
     // START / END / NUM_SITES of every window are final: their copy to the host can overlap the GEMM (score_common).
     // Recorded ONCE: the copy waits for the event's latest record, so a record per sub-range of a shard held the
     // bookkeeping copy back until the last sub-range (200 MB at C5: it then outlasted the last GEMM on the root rank).
-    if (e->ev_book && !e->book_ready && (sharded ? rk == 0 : w_hi == nW)) {
+    if (!sc.bookkeeping_ready && (sharded ? rk == 0 : w_hi == nW)) {
         IBD_CUDA(cudaEventRecord(e->ev_book, e->stream));
-        e->book_ready = true;
+        sc.bookkeeping_ready = true;
     }
     IBD_CUDA(cudaGetLastError());
     if (w_hi == w_lo) continue;  // (an empty shard: bookkeeping only)
@@ -1295,7 +1295,7 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
     if (stream_out || stream_dev) {
         // the range's columns of d_wll [T][outW][3] are final: they leave on their own stream
         if (d2h_after(rk)) return 1;
-        if (stream_dev && export_cols(e->d_wll_out_device, e->d_wll_out_device, w_lo, w_hi - w_lo)) return 1;
+        if (stream_dev && export_cols(sc.w_loglik_device, sc.w_loglik_device, w_lo, w_hi - w_lo)) return 1;
         if (stream_out && sharded && e->shard_compact) {
             // compact host table of a window shard: pack on the device, one contiguous copy
             double *d_pack;
@@ -1303,15 +1303,15 @@ int ld_tensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const
             if (scratch(e, SC_WLL_PACK, (size_t)T * (shard_we - shard_wb) * 24, (void **)&d_pack)) return 1;
             ld_pack_cols_kernel<<<(unsigned)((n + 255) / 256), 256, 0, e->d2h_stream>>>(d_wll, d_pack + off, T, outW, w_lo, w_hi - w_lo);
             e->k_launches[K_LD_WINDOWS]++;
-            IBD_CUDA(cudaMemcpyAsync(e->h_wll_out + off, d_pack + off, (size_t)n * 8, cudaMemcpyDeviceToHost, e->d2h_stream));
+            IBD_CUDA(cudaMemcpyAsync(sc.w_loglik + off, d_pack + off, (size_t)n * 8, cudaMemcpyDeviceToHost, e->d2h_stream));
         } else if (stream_out && !direct) {
-            if (export_cols(e->h_wll_out, h_wll_mapped, w_lo, w_hi - w_lo)) return 1;
+            if (export_cols(sc.w_loglik, h_wll_mapped, w_lo, w_hi - w_lo)) return 1;
         }
     }
     w_lo = w_hi;
     }  // window ranges
     if ((stream_out || direct) && outW > nW && !sharded) {  // the unused columns nW .. outW-1 (NaN since the fill at the start of the call)
-        if (d2h_after(range_end.size()) || export_cols(e->h_wll_out, h_wll_mapped, nW, outW - nW)) return 1;
+        if (d2h_after(range_end.size()) || export_cols(sc.w_loglik, h_wll_mapped, nW, outW - nW)) return 1;
     }
     IBD_CUDA(cudaGetLastError());
     return 0;

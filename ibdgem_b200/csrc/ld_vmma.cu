@@ -865,9 +865,9 @@ void ld_vtensor_invalidate(ibdgem_engine *e) {
     if (e->vc) e->vc->valid = false;
 }
 
-bool ld_vtensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t n_bg) {
+bool ld_vtensor_eligible(ibdgem_engine *e, int32_t n_targets, int32_t nU) {
     if (!e->depth_linear || !(e->kappa < -1e-3)) return false;
-    if (e->K_shared <= 0 || n_targets <= 0 || n_bg <= 0) return false;
+    if (e->K_shared <= 0 || n_targets <= 0 || nU <= 0) return false;
     // the screen runs in fp32: |Y + kappa M| <= W * max_cov * (|alpha| + |beta| + |kappa|) must leave its ulp well under a nat
     const double mag = (double)e->prm.window_size * e->prm.max_cov * (fabs(e->alpha) + fabs(e->beta) + fabs(e->kappa));
     if (mag > 4.0e6) return false;
@@ -915,22 +915,21 @@ static int v_build_cache(ibdgem_engine *e) {
 }
 
 // Fills every window output of the call (d_wll [T][outW][3], d_wn, d_ws, d_we [T][outW], d_nwout [T]).
-// rc 0 = done; 2 = not taken (the caller falls back to the general path); 1 = error.
-int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, const int32_t *d_targets, int32_t n_bg, const int32_t *h_bg,
-                     int32_t pu_idx, const uint8_t *d_tgt_counts, int32_t outW, double *d_wll, int32_t *d_wn, uint64_t *d_ws,
-                     uint64_t *d_we, int32_t *d_nwout) {
+int ld_vtensor_score(ibdgem_engine *e, ScoreCall &sc) {
     using namespace vmma;
     if (ensure_table(e, e->S)) return 1;  // waits for the whole panel
     if (v_build_cache(e)) return 1;
     VCache *c = e->vc;
-    const int vflag = e->prm.variable_sites_only ? 1 : 0;
+    const SiteView &v = sc.v;
+    const int T = sc.T, outW = sc.outW;
+    const int32_t *d_targets = sc.d_targets;
+    const uint8_t *d_tgt_counts = v.tgt_counts;
+    double *d_wll = sc.d_wll;
     const int W = e->prm.window_size;
-    const int mapW = (int)(e->S / W + 2);
+    const int mapW = map_windows(e);
 
-    LdBackground bg;
-    ld_background(c->N, T, h_targets, n_bg, h_bg, pu_idx, &bg);
+    LdBackground &bg = sc.bg;
     const int nU = (int)bg.bgU.size();
-    if (nU == 0) return 2;
     const int NT = (nU + TILE_IND - 1) / TILE_IND;
     bg.lnc.resize((size_t)NT * TILE_IND, -INFINITY);  // padding columns of the last tile
 
@@ -979,9 +978,6 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
         scratch(e, SC_V_TWBASE, (size_t)(T + 1) * 4, (void **)&d_twbase))
         return 1;
     int64_t *d_wf = nullptr, *d_wl = nullptr;
-    SiteView v;
-    v.keep = e->d_keep; v.nref = e->d_nref; v.nalt = e->d_nalt; v.bits = e->d_bits; v.Wh = e->Wh; v.S = e->S;
-    v.tgt_counts = d_tgt_counts; v.vflag = vflag;
     if (d_tgt_counts) {
         if (scratch(e, SC_WFIRST, (size_t)T * mapW * 8, (void **)&d_wf) || scratch(e, SC_WLAST, (size_t)T * mapW * 8, (void **)&d_wl)) return 1;
         if (build_window_map(e, v, d_targets, T, mapW, d_wf, d_wl, d_nwin, d_ktot, nullptr)) return 1;
@@ -1004,7 +1000,7 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
             return 1;
         }
     if (n_tw == 0) {  // no target has a single kept site: nothing to score (n_windows = 0 everywhere)
-        IBD_CUDA(cudaMemsetAsync(d_nwout, 0, (size_t)T * 4, e->stream));
+        IBD_CUDA(cudaMemsetAsync(sc.d_nwout, 0, (size_t)T * 4, e->stream));
         return 0;
     }
     const int n_tiles = (n_tw + TW_TILE - 1) / TW_TILE;
@@ -1027,31 +1023,29 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
         if (d_tgt_counts)
             v_tw_site_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, e->stream>>>(
                 v, T, mapW, outW, d_targets, d_nwin, d_twbase, d_wf, d_wl, e->d_rank, e->d_lnP, e->C, e->d_pos, e->alpha, e->beta, e->kappa,
-                d_tw_t, d_tw_w, d_tw_ks, d_tw_ke, d_tw_C0, d_tw_R0, d_tw_R1, d_wll, d_wn, d_ws, d_we, d_nwout, d_ownT, d_tw_own);
+                d_tw_t, d_tw_w, d_tw_ks, d_tw_ke, d_tw_C0, d_tw_R0, d_tw_R1, d_wll, sc.d_wn, sc.d_ws, sc.d_we, sc.d_nwout, d_ownT, d_tw_own);
         else
             v_tw_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, e->stream>>>(
                 T, mapW, outW, d_targets, d_nwin, d_twbase, d_ks, d_ke, c->d_tbits, c->H, c->d_nr, c->d_nk, c->d_l0, c->d_slotsite, e->d_pos,
-                e->alpha, e->beta, e->kappa, d_tw_t, d_tw_w, d_tw_ks, d_tw_ke, d_tw_C0, d_tw_R0, d_tw_R1, d_wll, d_wn, d_ws, d_we, d_nwout, d_ownT, d_tw_own);
+                e->alpha, e->beta, e->kappa, d_tw_t, d_tw_w, d_tw_ks, d_tw_ke, d_tw_C0, d_tw_R0, d_tw_R1, d_wll, sc.d_wn, sc.d_ws, sc.d_we, sc.d_nwout, d_ownT,
+                d_tw_own);
     }
     // The bookkeeping arrays and LIBD2 are final here: they leave for the host now, under the rest of the preparation
     // and the GEMM (score_common copies the bookkeeping on the copy stream once ev_book has fired).  With a page-locked
     // host table the whole device table goes out once — LIBD2 in place, NaN everywhere else — and the GEMM's merge warps
     // then store LIBD0 / LIBD1 of every finished (target, window) into it themselves; the GEMM waits for that copy.
-    if (e->ev_book && e->copy_stream) {
-        IBD_CUDA(cudaEventRecord(e->ev_book, e->stream));
-        e->book_ready = true;
-    }
-    double *h_wll_mapped = host_table_alias(e);
+    IBD_CUDA(cudaEventRecord(e->ev_book, e->stream));
+    sc.bookkeeping_ready = true;
+    double *h_wll_mapped = host_table_alias(sc);
     cudaEvent_t ev_table = nullptr;  // the copy of the whole table is done
     if (h_wll_mapped) {
-        if (side_streams(e)) return 1;
         cudaEvent_t ev_ready;
         if (range_event(e, 0, &ev_ready) || range_event(e, 1, &ev_table)) return 1;
         IBD_CUDA(cudaEventRecord(ev_ready, e->stream));
         IBD_CUDA(cudaStreamWaitEvent(e->d2h_stream, ev_ready, 0));
-        IBD_CUDA(cudaMemcpyAsync(e->h_wll_out, d_wll, (size_t)T * outW * 24, cudaMemcpyDeviceToHost, e->d2h_stream));
+        sc.streamed = true;
+        IBD_CUDA(cudaMemcpyAsync(sc.w_loglik, d_wll, (size_t)T * outW * 24, cudaMemcpyDeviceToHost, e->d2h_stream));
         IBD_CUDA(cudaEventRecord(ev_table, e->d2h_stream));
-        e->wll_streamed = true;
     }
     {
         LaunchScope ls(e, K_V_SORT);
@@ -1104,7 +1098,7 @@ int ld_vtensor_score(ibdgem_engine *e, int32_t T, const int32_t *h_targets, cons
                 const int ny = std::min(65534, (b1 - b0) * 2 - y0);
                 v_expand_a_kernel<<<dim3((unsigned)max_nkb, (unsigned)ny), 128, 0, e->stream>>>(
                     b0 + y0 / 2, d_tile_kb0, d_tile_nkb, d_tile_slab, d_order, d_tw_t, d_tw_ks, d_tw_ke, d_targets, c->d_tbits, c->H, c->d_nr,
-                    c->d_nk, c->d_slotsite, d_tgt_counts, e->S, vflag, d_A);
+                    c->d_nk, c->d_slotsite, d_tgt_counts, e->S, v.vflag, d_A);
             }
         }
         IBD_CUDA(cudaGetLastError());

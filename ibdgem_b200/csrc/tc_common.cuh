@@ -296,12 +296,6 @@ __device__ __forceinline__ void unit_publish(int *uring, uint64_t *ufull, int it
 constexpr double SCREEN_NATS = 32.0;
 inline double screen_nats(int ncols) { return std::min(SCREEN_NATS, log((double)std::max(ncols, 2)) + 16.2); }
 
-// integer value of the environment variable `name` (read by the caller once per process), or dflt when it is unset
-inline int env_int(const char *name, int dflt) {
-    const char *s = getenv(name);
-    return s ? atoi(s) : dflt;
-}
-
 // TMA map of a 3-D uint8 array (dims[0] bytes contiguous; strides of dims 1 and 2 in bytes): 128-byte swizzle,
 // zero fill outside
 inline int encode_u8_3d(CUtensorMap *m, void *base, const cuuint64_t (&dims)[3], const cuuint64_t (&strides)[2],

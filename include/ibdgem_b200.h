@@ -201,7 +201,7 @@ int ibdgem_engine_score_ld(ibdgem_engine *e, int32_t n_targets, const int32_t *t
                            int32_t n_bg, const int32_t *bg, int32_t pu_idx,
                            const uint8_t *tgt_counts, ibdgem_scores *out);
 
-/* Which --LD implementation the last score_ld call used:
+/* Which --LD implementation the last successful score_ld call used:
  *   1 = tensor-core window GEMM with fused log-sum-exp (shared windows: no -v, no -D; ld_mma.cu),
  *   2 = tensor-core GEMM over per-target windows (-v, -D; rows are (target, window) pairs; ld_vmma.cu),
  *   0 = general CUDA-core path (class tables that are not depth-linear, windows above 1,024 sites without -v/-D,
