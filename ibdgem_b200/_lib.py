@@ -22,6 +22,7 @@ ABI_SYMBOLS = [
     "ibdgem_peer_close", "hiddengem_viterbi_batch_device", "hiddengem_last_flagged", "ibdgem_engine_clone_panel", "ibdgem_engine_set_shard_compact_output",
     "hiddengem_posterior_batch", "hiddengem_posterior_batch_device",
     "hiddengem_posterior_moments_batch", "hiddengem_posterior_moments_device",
+    "hiddengem_tract_counts_batch", "hiddengem_tract_counts_device",
     "hiddengem_tracts_batch", "hiddengem_tracts_device", "hiddengem_last_tracts",
 ]
 

@@ -66,6 +66,8 @@ enum KernelId {
     K_TRACT_EMIT,       // hiddengem tracts: one 64-byte record per run (likelihood sums, posterior mean / minimum)
     K_POSTERIOR_BWD_MOMENTS,  // hiddengem posterior moments: the backward pass with the covariance recursion (its
                               // forward pass is posterior_fwd; in log arithmetic both are counted under _log too)
+    K_POSTERIOR_BWD_TRACTS,   // hiddengem posterior tract counts: the backward pass with the switch sums (and, with the
+                              // covariance, its recursion on the solver lane); forward pass and _log counts as above
     K_COUNT
 };
 
@@ -250,10 +252,13 @@ int viterbi_resolve(ibdgem_engine *e, const HgCall &c, const std::vector<uint8_t
                     int is_log, double p01, double p02, double p12, uint8_t *state, double *score, int64_t *counts, bool out_on_device);
 // posterior.cu: penalty check of the posterior entries (1 and the error set when rejected), and its kernels for one
 // batch of tables in device memory (no host synchronisation).  d_cov != null runs the moment variant of the backward
-// pass: covariances into d_cov [n_tables][3][3], and d_post may then be null.
+// pass: covariances into d_cov [n_tables][3][3], and d_post may then be null.  d_sw != null runs the tract-count
+// variant instead: switches into d_sw [n_tables][3][3], tract counts into d_tr [n_tables][3], their covariance into
+// d_cov when that is not null; d_post is then not written.
 bool bad_penalties(const char *fn, double p01, double p02, double p12);
 int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
-                        int is_log, double p01, double p02, double p12, double *d_post, double *d_expected, double *d_cov = nullptr);
+                        int is_log, double p01, double p02, double p12, double *d_post, double *d_expected, double *d_cov = nullptr,
+                        double *d_sw = nullptr, double *d_tr = nullptr);
 
 // Makes the engine stream wait for the panel chunks that cover sites [0, s_end); ensure_table also
 // runs site_table on the part of [0, s_end) it has not covered yet.

@@ -8,6 +8,8 @@
 // tracts, maximal runs of one state, to FILE (hiddengem_tracts_batch); stdout is unchanged.  --share-sd (additive,
 // with --posterior) runs hiddengem_posterior_moments_batch in place of hiddengem_posterior_batch and adds the
 // standard deviations of the posterior state shares and of the kinship, per table and over all tables.
+// --tract-counts (additive, with --posterior) also runs hiddengem_tract_counts_batch and adds the posterior expected
+// number of IBD tracts per state with its sd and the expected switches between states, per table and over all tables.
 #include <getopt.h>
 
 #include <cmath>
@@ -40,6 +42,10 @@ void print_help(int code) {
           "                            of segments and the window-share kinship (N_IBD1/4 + N_IBD2/2)/n with its\n"
           "                            standard deviation, from the posterior covariance; with several -s, also\n"
           "                            these figures over all tables together\n"
+          "--tract-counts           With --posterior: also print the posterior expected number of IBD tracts\n"
+          "                            (maximal runs of segments in one state) per state with its standard\n"
+          "                            deviation, and the expected number of switches between each two states;\n"
+          "                            with several -s, also these figures over all tables together\n"
           "--tracts  FILE           Also write the IBD tracts (maximal runs of segments in one state) to FILE: per\n"
           "                            tract its summary file, state, first and last segment, START, END, number\n"
           "                            of segments and sites, LOD10 of its state against the next best (and with\n"
@@ -129,13 +135,14 @@ int read_summary(const std::string &fn, Summary *sm) {
 int main(int argc, char *argv[]) {
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
     std::vector<std::string> files;
-    bool posterior = false, share_sd = false;
+    bool posterior = false, share_sd = false, tract_counts = false;
     const char *tracts_fn = nullptr;
     static struct option longopts[] = {{"summary", required_argument, 0, 's'}, {"p01", required_argument, 0, 1},
                                        {"p02", required_argument, 0, 2},       {"p12", required_argument, 0, 3},
                                        {"posterior", no_argument, 0, 4},       // additive
                                        {"tracts", required_argument, 0, 5},    // additive
                                        {"share-sd", no_argument, 0, 6},        // additive
+                                       {"tract-counts", no_argument, 0, 7},    // additive
                                        {"help", no_argument, 0, 'h'},          {0, 0, 0, 0}};
     if (argc == 1) print_help(0);
     int option;
@@ -148,6 +155,7 @@ int main(int argc, char *argv[]) {
             case 4: posterior = true; break;
             case 5: tracts_fn = optarg; break;
             case 6: share_sd = true; break;
+            case 7: tract_counts = true; break;
             case 'h': print_help(0); break;
             case ':':
                 fprintf(stderr, "Option -%c missing required argument.\n", optopt);
@@ -164,6 +172,10 @@ int main(int argc, char *argv[]) {
     for (int i = optind; i < argc; i++) fprintf(stderr, "Given extra argument %s.\n", argv[i]);
     if (share_sd && !posterior) {
         fprintf(stderr, "[::] ERROR: --share-sd needs --posterior (the standard deviations are those of the posterior counts).\n");
+        exit(0);
+    }
+    if (tract_counts && !posterior) {
+        fprintf(stderr, "[::] ERROR: --tract-counts needs --posterior (the tract counts are those of the posterior paths).\n");
         exit(0);
     }
 
@@ -192,13 +204,17 @@ int main(int argc, char *argv[]) {
     std::vector<int64_t> counts((off.size() - 1) * 3);
     std::vector<double> post(posterior ? nb * 3 : 0), expected(posterior ? (off.size() - 1) * 3 : 0);
     std::vector<double> cov(share_sd ? (off.size() - 1) * 9 : 0);
+    const size_t ntc = tract_counts ? off.size() - 1 : 0;  // --tract-counts: expected (again), switches, tracts, tract_cov
+    std::vector<double> tc_expected(ntc * 3), tc_switches(ntc * 9), tc_tracts(ntc * 3), tc_cov(ntc * 9);
     if (ibdgem_engine_create(&prm, &e) ||
         hiddengem_viterbi_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, state.data(), score.data(),
                                 counts.data()) ||
         (posterior && !share_sd &&
          hiddengem_posterior_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, post.data(), expected.data())) ||
         (share_sd && hiddengem_posterior_moments_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, post.data(),
-                                                       expected.data(), cov.data()))) {
+                                                       expected.data(), cov.data())) ||
+        (tract_counts && hiddengem_tract_counts_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, tc_expected.data(),
+                                                      tc_switches.data(), tc_tracts.data(), tc_cov.data()))) {
         fprintf(stderr, "%s\n", ibdgem_last_error());
         exit(1);
     }
@@ -274,14 +290,21 @@ int main(int argc, char *argv[]) {
                     out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d (n = %.2f): %.2f\n", k, x, (x / n) * 100));
                 }
             if (share_sd) out += share_sd_lines(&expected[t * 3], &cov[t * 9], n);
+            if (tract_counts) out += tract_count_lines(&tc_tracts[t * 3], &tc_cov[t * 9], &tc_switches[t * 9]);
         });
         for (size_t k = 0; k < nt; k++) fwrite(text[k].data(), 1, text[k].size(), stdout);
     }
-    if (share_sd && n_tables > 1) {  // the tables are independent: their means and covariances add
+    if ((share_sd || tract_counts) && n_tables > 1) {  // the tables are independent: their means and covariances add
         double x[3] = {0, 0, 0}, c[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+        double tt[3] = {0, 0, 0}, tcv[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, sw[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
         for (size_t t = 0; t < n_tables; t++) {
             for (int k = 0; k < 3; k++) x[k] += expected[t * 3 + (size_t)k];
-            for (int k = 0; k < 9; k++) c[k] += cov[t * 9 + (size_t)k];
+            for (int k = 0; k < 9 && share_sd; k++) c[k] += cov[t * 9 + (size_t)k];
+            for (int k = 0; k < 3 && tract_counts; k++) tt[k] += tc_tracts[t * 3 + (size_t)k];
+            for (int k = 0; k < 9 && tract_counts; k++) {
+                tcv[k] += tc_cov[t * 9 + (size_t)k];
+                sw[k] += tc_switches[t * 9 + (size_t)k];
+            }
         }
         const double n = (double)off.back();
         std::string out;
@@ -289,7 +312,8 @@ int main(int argc, char *argv[]) {
         out.append(row, (size_t)snprintf(row, sizeof row, "#%% all %zu tables (n = %.0f)\n", n_tables, n));
         for (int k = 0; k < 3; k++)
             out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d (n = %.2f): %.2f\n", k, x[k], (x[k] / n) * 100));
-        out += share_sd_lines(x, c, n);
+        if (share_sd) out += share_sd_lines(x, c, n);
+        if (tract_counts) out += tract_count_lines(tt, tcv, sw);
         fwrite(out.data(), 1, out.size(), stdout);
     }
     return 0;

@@ -46,6 +46,7 @@ struct Options {
     int posterior = 0;  // --posterior (with --hiddengem): posterior state probabilities in those files
     int tracts = 0;     // --tracts (with --hiddengem): also write <pileup>.<target>.tracts.txt
     int share_sd = 0;   // --share-sd (with --posterior): sd of the posterior state shares and kinship in those files
+    int tract_counts = 0;  // --tract-counts (with --posterior): posterior tract counts and switches in those files
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
 };
 
@@ -99,6 +100,9 @@ void print_help(int code) {
         "--share-sd                      With --posterior: add the standard deviation of each state's share of\n"
         "                                   segments and the window-share kinship (N_IBD1/4 + N_IBD2/2)/n with\n"
         "                                   its standard deviation, from the posterior covariance\n"
+        "--tract-counts                  With --posterior: add the posterior expected number of IBD tracts (maximal\n"
+        "                                   runs of segments in one state) per state with its standard deviation,\n"
+        "                                   and the expected number of switches between each two states\n"
         "--tracts                        With --hiddengem: also write the IBD tracts (maximal runs of segments in\n"
         "                                   one state) to <pileup-name>.<target>.tracts.txt: state, first and last\n"
         "                                   segment, START, END, number of segments and sites, LOD10 of the state\n"
@@ -360,6 +364,7 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
         std::vector<double> hg_score;
         std::vector<int64_t> hg_counts, hg_off;
         std::vector<double> hg_post, hg_expected, hg_cov;
+        std::vector<double> tc_expected, tc_switches, tc_tracts, tc_cov;  // --tract-counts
         std::vector<int64_t> tr_off;
         std::vector<hiddengem_tract> tracts;
         if (o.hiddengem) {
@@ -386,6 +391,14 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
                 if (o.share_sd && nbins &&
                     hiddengem_posterior_moments_batch(e, (int32_t)T, hg_off.data(), packed.data(), 1, o.p01, o.p02, o.p12, hg_post.data(),
                                                       hg_expected.data(), hg_cov.data()))
+                    return fail_engine();
+                tc_expected.resize(o.tract_counts ? T * 3 : 0);
+                tc_switches.resize(o.tract_counts ? T * 9 : 0);
+                tc_tracts.resize(o.tract_counts ? T * 3 : 0);
+                tc_cov.resize(o.tract_counts ? T * 9 : 0);
+                if (o.tract_counts && nbins &&
+                    hiddengem_tract_counts_batch(e, (int32_t)T, hg_off.data(), packed.data(), 1, o.p01, o.p02, o.p12, tc_expected.data(),
+                                                 tc_switches.data(), tc_tracts.data(), tc_cov.data()))
                     return fail_engine();
             }
             if (o.tracts && nbins) {  // the same packed scores through the tract entry: only the records come back
@@ -504,6 +517,7 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
                     for (int c = 0; c < 3; c++)
                         fprintf(hg, "#%% posterior IBD%d (n = %.2f): %.2f\n", c, hg_expected[k * 3 + (size_t)c], (hg_expected[k * 3 + (size_t)c] / n) * 100);
                 if (o.share_sd) fputs(share_sd_lines(&hg_expected[k * 3], &hg_cov[k * 9], n).c_str(), hg);
+                if (o.tract_counts) fputs(tract_count_lines(&tc_tracts[k * 3], &tc_cov[k * 9], &tc_switches[k * 9]).c_str(), hg);
                 fclose(hg);
             }
             if (o.tracts && nw[k] > 0) {  // START / END / NUM_SITES from the run's own window bookkeeping
@@ -556,7 +570,7 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
 int main(int argc, char *argv[]) {
     const clock_t start = clock();
     Options o;
-    static int ld_flag = 0, no_tab_flag = 0, hg_flag = 0, post_flag = 0, tracts_flag = 0, share_sd_flag = 0;
+    static int ld_flag = 0, no_tab_flag = 0, hg_flag = 0, post_flag = 0, tracts_flag = 0, share_sd_flag = 0, tract_counts_flag = 0;
     static struct option longopts[] = {{"LD", no_argument, &ld_flag, 1},
                                        {"vcf", required_argument, 0, 'V'},
                                        {"hap", required_argument, 0, 'H'},
@@ -588,6 +602,7 @@ int main(int argc, char *argv[]) {
                                        {"posterior", no_argument, &post_flag, 1},  // additive: posteriors in the hiddengem files
                                        {"tracts", no_argument, &tracts_flag, 1},   // additive: IBD tracts beside the hiddengem files
                                        {"share-sd", no_argument, &share_sd_flag, 1},  // additive: share sd in the hiddengem files
+                                       {"tract-counts", no_argument, &tract_counts_flag, 1},  // additive: tract counts in those files
                                        {"p01", required_argument, 0, 1004},
                                        {"p02", required_argument, 0, 1005},
                                        {"p12", required_argument, 0, 1006},
@@ -645,6 +660,7 @@ int main(int argc, char *argv[]) {
     o.posterior = post_flag;
     o.tracts = tracts_flag;
     o.share_sd = share_sd_flag;
+    o.tract_counts = tract_counts_flag;
     for (int i = optind; i < argc; i++) fprintf(stderr, "Given extra argument %s.\n", argv[i]);
     // validation: the reference exits with status 0 on invalid values (src/ibdgem.c:966-989)
     if (o.opt_d && o.target_dp <= 0) {
@@ -677,6 +693,10 @@ int main(int argc, char *argv[]) {
     }
     if (o.share_sd && !o.posterior) {
         fprintf(stderr, "[::] ERROR: --share-sd needs --posterior (the standard deviations are those of the posterior counts).\n");
+        exit(0);
+    }
+    if (o.tract_counts && !o.posterior) {
+        fprintf(stderr, "[::] ERROR: --tract-counts needs --posterior (the tract counts are those of the posterior paths).\n");
         exit(0);
     }
     if (o.tracts && !o.hiddengem) {

@@ -114,4 +114,17 @@ std::string share_sd_lines(const double *expected, const double *cov, double n) 
     return out;
 }
 
+std::string tract_count_lines(const double *tracts, const double *tract_cov, const double *switches) {
+    std::string out;
+    char row[160];
+    for (int k = 0; k < 3; k++)
+        out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d tracts (sd = %.2f): %.2f\n", k, sd_of(tract_cov[k * 4]),
+                                         tracts[k]));
+    for (int k = 0; k < 3; k++)
+        for (int l = 0; l < 3; l++)
+            if (k != l)
+                out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior switches IBD%d>IBD%d: %.2f\n", k, l, switches[k * 3 + l]));
+    return out;
+}
+
 }  // namespace ibdhost

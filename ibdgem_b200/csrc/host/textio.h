@@ -52,4 +52,10 @@ std::string tract_row(const hiddengem_tract &r, int64_t k, uint64_t start, uint6
 // "#% posterior kinship (sd = <sd>): <phi>" with phi = (N_1 / 4 + N_2 / 2) / n, each ending in '\n'.
 std::string share_sd_lines(const double *expected, const double *cov, double n);
 
+// --tract-counts lines (hiddengem, ibdgem --hiddengem): from the posterior expected tract counts (tracts[3]), their
+// covariance (tract_cov[3][3]) and the expected switches (switches[3][3]), "#% posterior IBDk tracts (sd = <sd of
+// T_k>): <E[T_k]>" for k = 0, 1, 2 and "#% posterior switches IBDk>IBDl: <E[S_kl]>" for the six k != l, each ending
+// in '\n'.
+std::string tract_count_lines(const double *tracts, const double *tract_cov, const double *switches);
+
 }  // namespace ibdhost

@@ -306,6 +306,35 @@ class Engine:
             C.c_int32(1 if is_log else 0), C.c_double(p01), C.c_double(p02), C.c_double(p12),
             C.c_void_p(d_posterior_ptr or None), C.c_void_p(d_expected_ptr), C.c_void_p(d_cov_ptr)))
 
+    def tract_counts_batch(self, lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-3, cov=True):
+        """Posterior expected switches between IBD states and IBD tracts per state (hiddengem_tract_counts_batch):
+        (expected [n_tables, 3], switches [n_tables, 3, 3], tracts [n_tables, 3]), and with cov=True also the
+        covariance of the tract counts [n_tables, 3, 3]."""
+        lik = np.ascontiguousarray(lik, np.float64)
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        nt = len(off) - 1
+        expected = np.zeros((nt, 3))
+        switches = np.zeros((nt, 3, 3))
+        tracts = np.zeros((nt, 3))
+        tract_cov = np.zeros((nt, 3, 3)) if cov else None
+        self._check(self._lib.hiddengem_tract_counts_batch(self._h, C.c_int32(nt), _ptr(off), _ptr(lik),
+                                                           C.c_int32(1 if is_log else 0), C.c_double(p01),
+                                                           C.c_double(p02), C.c_double(p12), _ptr(expected),
+                                                           _ptr(switches), _ptr(tracts), _ptr(tract_cov)))
+        return (expected, switches, tracts, tract_cov) if cov else (expected, switches, tracts)
+
+    def tract_counts_device(self, d_lik_ptr: int, bin_offsets: np.ndarray, is_log: bool, d_expected_ptr: int,
+                            d_switches_ptr: int, d_tracts_ptr: int, d_tract_cov_ptr: int = 0, table_stride: int = 0,
+                            p01=1e-3, p02=1e-6, p12=1e-3):
+        """Device buffers in, device buffers out (hiddengem_tract_counts_device; d_tract_cov_ptr 0: no covariance);
+        bin_offsets stays on the host."""
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        self._check(self._lib.hiddengem_tract_counts_device(
+            self._h, C.c_int32(len(off) - 1), _ptr(off), C.c_int64(table_stride), C.c_void_p(d_lik_ptr),
+            C.c_int32(1 if is_log else 0), C.c_double(p01), C.c_double(p02), C.c_double(p12),
+            C.c_void_p(d_expected_ptr), C.c_void_p(d_switches_ptr), C.c_void_p(d_tracts_ptr),
+            C.c_void_p(d_tract_cov_ptr or None)))
+
     def tracts_batch(self, lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-3, posterior=True):
         """IBD tracts (runs of one Viterbi state) with likelihood sums and, with posterior, the mean and minimum
         posterior of their state (hiddengem_tracts_batch + hiddengem_last_tracts): (tract_offsets [n_tables + 1],

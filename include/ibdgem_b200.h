@@ -295,6 +295,37 @@ int hiddengem_posterior_moments_device(ibdgem_engine *e, int32_t n_tables, const
                                        const double *d_lik, int32_t is_log, double p01, double p02, double p12,
                                        double *d_posterior, double *d_expected, double *d_cov);
 
+/* Posterior tract counts: the posterior entries' model, emissions, uniform rule and penalties, and for one table of
+ * n bins and a path x
+ *     S_kl = #{1 <= i < n : x_{i-1} = k, x_i = l}   (all nine, diagonal included: sum_kl S_kl = n - 1)
+ *     T_s  = [x_0 = s] + #{1 <= i < n : x_i = s, x_{i-1} != s}   (the number of maximal runs of state s; on the
+ *            Viterbi path, the number of hiddengem_tract records with that state).
+ * switches[t][k][l] = E[S_kl] = sum_i xi_i(k, l), xi_i(k, l) = gamma_i(l) alpha_{i-1}(k) pen(k, l) / sum_k' alpha_{i-1}(k')
+ * pen(k', l) (0 where gamma_i(l) = 0); tracts[t][s] = E[T_s] = gamma_0(s) + sum_{k != s} E[S_ks], summed from the
+ * switches into s, never as a difference.  tract_cov[t][s][u] = Cov(T_s, T_u), exact in the model: with
+ * phi_i(s) = P(x_i = s, x_{i-1} != s) (phi_0 = gamma_0) and g_i^u[k] = E[#{j > i : x_j = u, x_{j-1} != u} | x_i = k],
+ *     Cov(T_s, T_u) = sum_i phi_i(s) (delta_su - phi_i(u)) + phi_i(s) (g_i^u[s] - G_i^u) + phi_i(u) (g_i^s[u] - G_i^s),
+ * G_i^u = sum_k gamma_i(k) g_i^u[k].  Each table's sums run over its bins in a fixed order: the same inputs give the
+ * same bits in any batch or layout, and switches and tracts are the same bits with or without tract_cov.
+ *   - expected is the posterior entries' expected, bit for bit.
+ *   - An empty table has everything 0; one bin has switches 0, tracts = gamma_0 and tract_cov = diag(gamma_0) -
+ *     gamma_0 gamma_0^T; a table of total weight 0 has NaN everywhere.
+ *   - Independent tables (e.g. the chromosomes of one pair) add: the means and covariances of the genome are the sums
+ *     of the tables'.  The sd of the number of IBD1 tracts is sqrt(tract_cov[1][1]).
+ *   expected    [n_tables][3]
+ *   switches    [n_tables][3][3]
+ *   tracts      [n_tables][3]
+ *   tract_cov   [n_tables][3][3], symmetric, or NULL: then the covariance recursion does not run
+ * Arguments, penalties and bin_offsets are checked as by hiddengem_posterior_batch. */
+int hiddengem_tract_counts_batch(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, const double *lik,
+                                 int32_t is_log, double p01, double p02, double p12,
+                                 double *expected, double *switches, double *tracts, double *tract_cov);
+/* The same on DEVICE buffers (bin_offsets a HOST array), with the layouts of hiddengem_posterior_batch_device
+ * (table_stride = max_windows takes ibdgem_scores.w_loglik_device as is); d_tract_cov may be NULL. */
+int hiddengem_tract_counts_device(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, int64_t table_stride,
+                                  const double *d_lik, int32_t is_log, double p01, double p02, double p12,
+                                  double *d_expected, double *d_switches, double *d_tracts, double *d_tract_cov);
+
 /* IBD tracts.  A tract is a maximal run [first_bin, first_bin + n_bins) of bins of one table with the same Viterbi
  * state (in IBDGem a "segment" is one window, i.e. one bin).  Tracts never cross tables; an empty table has none.
  * Records are ordered table by table, then by first_bin; table t's are records [tract_offsets[t], tract_offsets[t+1]).
