@@ -23,6 +23,7 @@ ABI_SYMBOLS = [
     "hiddengem_posterior_batch", "hiddengem_posterior_batch_device",
     "hiddengem_posterior_moments_batch", "hiddengem_posterior_moments_device",
     "hiddengem_tract_counts_batch", "hiddengem_tract_counts_device",
+    "hiddengem_tract_lengths_batch", "hiddengem_tract_lengths_device",
     "hiddengem_tracts_batch", "hiddengem_tracts_device", "hiddengem_last_tracts",
 ]
 

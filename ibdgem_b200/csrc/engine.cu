@@ -32,6 +32,7 @@ static const char *const kKernelNameList[] = {
     "v_slots",        "v_wmap",        "v_tw",          "v_sort",       "v_expand_a",  "v_expand_b",   "ld_vmma",
     "window_linear",  "posterior_fwd", "posterior_bwd", "posterior_fwd_log", "posterior_bwd_log",
     "tract_count",    "tract_emit",    "posterior_bwd_moments", "posterior_bwd_tracts",
+    "posterior_bwd_runs", "tract_lengths",
 };
 static_assert(sizeof(kKernelNameList) / sizeof(kKernelNameList[0]) == K_COUNT, "one name per KernelId, in enum order");
 const char *const *const kKernelNames = kKernelNameList;

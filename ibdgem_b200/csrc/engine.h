@@ -68,6 +68,8 @@ enum KernelId {
                               // forward pass is posterior_fwd; in log arithmetic both are counted under _log too)
     K_POSTERIOR_BWD_TRACTS,   // hiddengem posterior tract counts: the backward pass with the switch sums (and, with the
                               // covariance, its recursion on the solver lane); forward pass and _log counts as above
+    K_POSTERIOR_BWD_RUNS,     // hiddengem tract lengths: the backward pass writing per-bin run terms; as above
+    K_TRACT_LENGTHS,          // hiddengem tract lengths: windowed run products per start bin and threshold
     K_COUNT
 };
 
@@ -209,7 +211,7 @@ enum ScratchSlot {
     SC_MMA_TGT, SC_MMA_BG, SC_MMA_ROWLSE, SC_MMA_BGIDX, SC_MMA_MISC, SC_MMA_UNIT,
     SC_WLIN, SC_WLL_PACK, SC_V_KS, SC_V_KE, SC_V_TWBASE, SC_V_TWI, SC_V_TWD, SC_V_ORDER, SC_V_HIST, SC_V_TILES, SC_V_MISC, SC_HG_CKPT,
     SC_HG_TRACTS,  // the tract records of the last tract call (hiddengem_last_tracts); nothing else writes it
-    SC_HG_TOFF, SC_SLOTS
+    SC_HG_TOFF, SC_HG_RUNS, SC_HG_RUNSUM, SC_HG_COORD, SC_SLOTS
 };
 int scratch(ibdgem_engine *e, int slot, size_t bytes, void **out);
 // copy_stream with ev_order, and d2h_stream, created on first use (engine.cu)
@@ -254,11 +256,12 @@ int viterbi_resolve(ibdgem_engine *e, const HgCall &c, const std::vector<uint8_t
 // batch of tables in device memory (no host synchronisation).  d_cov != null runs the moment variant of the backward
 // pass: covariances into d_cov [n_tables][3][3], and d_post may then be null.  d_sw != null runs the tract-count
 // variant instead: switches into d_sw [n_tables][3][3], tract counts into d_tr [n_tables][3], their covariance into
-// d_cov when that is not null; d_post is then not written.
+// d_cov when that is not null; d_post is then not written.  d_runs != null runs the run-term variant instead: gamma,
+// d and ln c of every bin into d_runs [bin][9] in the layout of d_lik; d_post is then not written.
 bool bad_penalties(const char *fn, double p01, double p02, double p12);
 int posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
                         int is_log, double p01, double p02, double p12, double *d_post, double *d_expected, double *d_cov = nullptr,
-                        double *d_sw = nullptr, double *d_tr = nullptr);
+                        double *d_sw = nullptr, double *d_tr = nullptr, double *d_runs = nullptr);
 
 // Makes the engine stream wait for the panel chunks that cover sites [0, s_end); ensure_table also
 // runs site_table on the part of [0, s_end) it has not covered yet.

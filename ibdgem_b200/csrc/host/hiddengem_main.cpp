@@ -10,6 +10,9 @@
 // standard deviations of the posterior state shares and of the kinship, per table and over all tables.
 // --tract-counts (additive, with --posterior) also runs hiddengem_tract_counts_batch and adds the posterior expected
 // number of IBD tracts per state with its sd and the expected switches between states, per table and over all tables.
+// --tract-lengths X1,X2,... (additive, with --posterior) also runs hiddengem_tract_lengths_batch on the START / END
+// columns and adds the posterior expected number of IBD tracts at least X bp long per state, per table and over all
+// tables.
 #include <getopt.h>
 
 #include <cmath>
@@ -46,6 +49,11 @@ void print_help(int code) {
           "                            (maximal runs of segments in one state) per state with its standard\n"
           "                            deviation, and the expected number of switches between each two states;\n"
           "                            with several -s, also these figures over all tables together\n"
+          "--tract-lengths  X1,X2,...\n"
+          "                         With --posterior: also print the posterior expected number of IBD tracts per\n"
+          "                            state at least X bp long (END of the last segment - START of the first + 1),\n"
+          "                            for up to 16 strictly increasing positive integers X; with several -s, also\n"
+          "                            these figures over all tables together\n"
           "--tracts  FILE           Also write the IBD tracts (maximal runs of segments in one state) to FILE: per\n"
           "                            tract its summary file, state, first and last segment, START, END, number\n"
           "                            of segments and sites, LOD10 of its state against the next best (and with\n"
@@ -135,7 +143,8 @@ int read_summary(const std::string &fn, Summary *sm) {
 int main(int argc, char *argv[]) {
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
     std::vector<std::string> files;
-    bool posterior = false, share_sd = false, tract_counts = false;
+    bool posterior = false, share_sd = false, tract_counts = false, tract_lengths = false, lengths_ok = true;
+    std::vector<uint64_t> thresholds;  // --tract-lengths
     const char *tracts_fn = nullptr;
     static struct option longopts[] = {{"summary", required_argument, 0, 's'}, {"p01", required_argument, 0, 1},
                                        {"p02", required_argument, 0, 2},       {"p12", required_argument, 0, 3},
@@ -143,6 +152,7 @@ int main(int argc, char *argv[]) {
                                        {"tracts", required_argument, 0, 5},    // additive
                                        {"share-sd", no_argument, 0, 6},        // additive
                                        {"tract-counts", no_argument, 0, 7},    // additive
+                                       {"tract-lengths", required_argument, 0, 8},  // additive
                                        {"help", no_argument, 0, 'h'},          {0, 0, 0, 0}};
     if (argc == 1) print_help(0);
     int option;
@@ -156,6 +166,10 @@ int main(int argc, char *argv[]) {
             case 5: tracts_fn = optarg; break;
             case 6: share_sd = true; break;
             case 7: tract_counts = true; break;
+            case 8:
+                tract_lengths = true;
+                lengths_ok = parse_tract_lengths(optarg, &thresholds);
+                break;
             case 'h': print_help(0); break;
             case ':':
                 fprintf(stderr, "Option -%c missing required argument.\n", optopt);
@@ -176,6 +190,14 @@ int main(int argc, char *argv[]) {
     }
     if (tract_counts && !posterior) {
         fprintf(stderr, "[::] ERROR: --tract-counts needs --posterior (the tract counts are those of the posterior paths).\n");
+        exit(0);
+    }
+    if (tract_lengths && !posterior) {
+        fprintf(stderr, "[::] ERROR: --tract-lengths needs --posterior (the run lengths are those of the posterior paths).\n");
+        exit(0);
+    }
+    if (tract_lengths && !lengths_ok) {
+        fputs(kTractLengthsError, stderr);
         exit(0);
     }
 
@@ -206,6 +228,13 @@ int main(int argc, char *argv[]) {
     std::vector<double> cov(share_sd ? (off.size() - 1) * 9 : 0);
     const size_t ntc = tract_counts ? off.size() - 1 : 0;  // --tract-counts: expected (again), switches, tracts, tract_cov
     std::vector<double> tc_expected(ntc * 3), tc_switches(ntc * 9), tc_tracts(ntc * 3), tc_cov(ntc * 9);
+    const size_t nk = thresholds.size();  // --tract-lengths: the spectrum on the START / END columns
+    std::vector<double> spectrum((tract_lengths ? off.size() - 1 : 0) * nk * 3);
+    std::vector<uint64_t> bin_start, bin_end;
+    for (size_t i = 0; tract_lengths && i < files.size(); i++) {
+        bin_start.insert(bin_start.end(), per_file[i].start.begin(), per_file[i].start.end());
+        bin_end.insert(bin_end.end(), per_file[i].end.begin(), per_file[i].end.end());
+    }
     if (ibdgem_engine_create(&prm, &e) ||
         hiddengem_viterbi_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, state.data(), score.data(),
                                 counts.data()) ||
@@ -214,7 +243,9 @@ int main(int argc, char *argv[]) {
         (share_sd && hiddengem_posterior_moments_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, post.data(),
                                                        expected.data(), cov.data())) ||
         (tract_counts && hiddengem_tract_counts_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, tc_expected.data(),
-                                                      tc_switches.data(), tc_tracts.data(), tc_cov.data()))) {
+                                                      tc_switches.data(), tc_tracts.data(), tc_cov.data())) ||
+        (tract_lengths && hiddengem_tract_lengths_batch(e, (int32_t)off.size() - 1, off.data(), lik.data(), 0, p01, p02, p12, bin_start.data(),
+                                                        bin_end.data(), (int32_t)nk, thresholds.data(), spectrum.data()))) {
         fprintf(stderr, "%s\n", ibdgem_last_error());
         exit(1);
     }
@@ -291,11 +322,13 @@ int main(int argc, char *argv[]) {
                 }
             if (share_sd) out += share_sd_lines(&expected[t * 3], &cov[t * 9], n);
             if (tract_counts) out += tract_count_lines(&tc_tracts[t * 3], &tc_cov[t * 9], &tc_switches[t * 9]);
+            if (tract_lengths) out += tract_length_lines(&spectrum[t * nk * 3], thresholds);
         });
         for (size_t k = 0; k < nt; k++) fwrite(text[k].data(), 1, text[k].size(), stdout);
     }
-    if ((share_sd || tract_counts) && n_tables > 1) {  // the tables are independent: their means and covariances add
+    if ((share_sd || tract_counts || tract_lengths) && n_tables > 1) {  // the tables are independent: their means and covariances add
         double x[3] = {0, 0, 0}, c[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+        std::vector<double> sp(nk * 3, 0.0);
         double tt[3] = {0, 0, 0}, tcv[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, sw[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
         for (size_t t = 0; t < n_tables; t++) {
             for (int k = 0; k < 3; k++) x[k] += expected[t * 3 + (size_t)k];
@@ -305,6 +338,7 @@ int main(int argc, char *argv[]) {
                 tcv[k] += tc_cov[t * 9 + (size_t)k];
                 sw[k] += tc_switches[t * 9 + (size_t)k];
             }
+            for (size_t k = 0; k < nk * 3 && tract_lengths; k++) sp[k] += spectrum[t * nk * 3 + k];
         }
         const double n = (double)off.back();
         std::string out;
@@ -314,6 +348,7 @@ int main(int argc, char *argv[]) {
             out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d (n = %.2f): %.2f\n", k, x[k], (x[k] / n) * 100));
         if (share_sd) out += share_sd_lines(x, c, n);
         if (tract_counts) out += tract_count_lines(tt, tcv, sw);
+        if (tract_lengths) out += tract_length_lines(sp.data(), thresholds);
         fwrite(out.data(), 1, out.size(), stdout);
     }
     return 0;

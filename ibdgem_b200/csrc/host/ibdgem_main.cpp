@@ -47,6 +47,8 @@ struct Options {
     int tracts = 0;     // --tracts (with --hiddengem): also write <pileup>.<target>.tracts.txt
     int share_sd = 0;   // --share-sd (with --posterior): sd of the posterior state shares and kinship in those files
     int tract_counts = 0;  // --tract-counts (with --posterior): posterior tract counts and switches in those files
+    int tract_lengths = 0, tract_lengths_ok = 1;  // --tract-lengths LIST (with --posterior): tract-length spectrum in those files
+    std::vector<uint64_t> thresholds;
     double p01 = 0.001, p02 = 0.000001, p12 = 0.001;
 };
 
@@ -103,6 +105,9 @@ void print_help(int code) {
         "--tract-counts                  With --posterior: add the posterior expected number of IBD tracts (maximal\n"
         "                                   runs of segments in one state) per state with its standard deviation,\n"
         "                                   and the expected number of switches between each two states\n"
+        "--tract-lengths  X1,X2,...      With --posterior: add the posterior expected number of IBD tracts per\n"
+        "                                   state at least X bp long (END of the last window - START of the first\n"
+        "                                   + 1), for up to 16 strictly increasing positive integers X\n"
         "--tracts                        With --hiddengem: also write the IBD tracts (maximal runs of segments in\n"
         "                                   one state) to <pileup-name>.<target>.tracts.txt: state, first and last\n"
         "                                   segment, START, END, number of segments and sites, LOD10 of the state\n"
@@ -365,6 +370,7 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
         std::vector<int64_t> hg_counts, hg_off;
         std::vector<double> hg_post, hg_expected, hg_cov;
         std::vector<double> tc_expected, tc_switches, tc_tracts, tc_cov;  // --tract-counts
+        std::vector<double> spectrum;  // --tract-lengths [T][K][3]
         std::vector<int64_t> tr_off;
         std::vector<hiddengem_tract> tracts;
         if (o.hiddengem) {
@@ -400,6 +406,18 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
                     hiddengem_tract_counts_batch(e, (int32_t)T, hg_off.data(), packed.data(), 1, o.p01, o.p02, o.p12, tc_expected.data(),
                                                  tc_switches.data(), tc_tracts.data(), tc_cov.data()))
                     return fail_engine();
+                const size_t nk = o.thresholds.size();
+                spectrum.assign(o.tract_lengths ? T * nk * 3 : 0, 0.0);
+                if (o.tract_lengths && nbins) {  // the run's window coordinates, packed like the scores
+                    std::vector<uint64_t> bs, be;
+                    for (size_t k = 0; k < T; k++) {
+                        bs.insert(bs.end(), ws.begin() + (ptrdiff_t)(k * (size_t)maxW), ws.begin() + (ptrdiff_t)(k * (size_t)maxW + (size_t)nw[k]));
+                        be.insert(be.end(), we.begin() + (ptrdiff_t)(k * (size_t)maxW), we.begin() + (ptrdiff_t)(k * (size_t)maxW + (size_t)nw[k]));
+                    }
+                    if (hiddengem_tract_lengths_batch(e, (int32_t)T, hg_off.data(), packed.data(), 1, o.p01, o.p02, o.p12, bs.data(), be.data(),
+                                                      (int32_t)nk, o.thresholds.data(), spectrum.data()))
+                        return fail_engine();
+                }
             }
             if (o.tracts && nbins) {  // the same packed scores through the tract entry: only the records come back
                 tr_off.resize(T + 1);
@@ -518,6 +536,7 @@ int run_shard(Shared *sh, int device, size_t t0, size_t t1, PanelSource *psrc = 
                         fprintf(hg, "#%% posterior IBD%d (n = %.2f): %.2f\n", c, hg_expected[k * 3 + (size_t)c], (hg_expected[k * 3 + (size_t)c] / n) * 100);
                 if (o.share_sd) fputs(share_sd_lines(&hg_expected[k * 3], &hg_cov[k * 9], n).c_str(), hg);
                 if (o.tract_counts) fputs(tract_count_lines(&tc_tracts[k * 3], &tc_cov[k * 9], &tc_switches[k * 9]).c_str(), hg);
+                if (o.tract_lengths) fputs(tract_length_lines(&spectrum[k * o.thresholds.size() * 3], o.thresholds).c_str(), hg);
                 fclose(hg);
             }
             if (o.tracts && nw[k] > 0) {  // START / END / NUM_SITES from the run's own window bookkeeping
@@ -603,6 +622,7 @@ int main(int argc, char *argv[]) {
                                        {"tracts", no_argument, &tracts_flag, 1},   // additive: IBD tracts beside the hiddengem files
                                        {"share-sd", no_argument, &share_sd_flag, 1},  // additive: share sd in the hiddengem files
                                        {"tract-counts", no_argument, &tract_counts_flag, 1},  // additive: tract counts in those files
+                                       {"tract-lengths", required_argument, 0, 1007},  // additive: tract-length spectrum in those files
                                        {"p01", required_argument, 0, 1004},
                                        {"p02", required_argument, 0, 1005},
                                        {"p12", required_argument, 0, 1006},
@@ -642,6 +662,10 @@ int main(int argc, char *argv[]) {
             case 1004: o.p01 = atof(optarg); break;
             case 1005: o.p02 = atof(optarg); break;
             case 1006: o.p12 = atof(optarg); break;
+            case 1007:
+                o.tract_lengths = 1;
+                o.tract_lengths_ok = parse_tract_lengths(optarg, &o.thresholds);
+                break;
             case ':':
                 fprintf(stderr, "Option -%c missing required argument.\n", optopt);
                 exit(0);
@@ -697,6 +721,14 @@ int main(int argc, char *argv[]) {
     }
     if (o.tract_counts && !o.posterior) {
         fprintf(stderr, "[::] ERROR: --tract-counts needs --posterior (the tract counts are those of the posterior paths).\n");
+        exit(0);
+    }
+    if (o.tract_lengths && !o.posterior) {
+        fprintf(stderr, "[::] ERROR: --tract-lengths needs --posterior (the run lengths are those of the posterior paths).\n");
+        exit(0);
+    }
+    if (o.tract_lengths && !o.tract_lengths_ok) {
+        fputs(kTractLengthsError, stderr);
         exit(0);
     }
     if (o.tracts && !o.hiddengem) {

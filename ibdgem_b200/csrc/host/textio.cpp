@@ -114,6 +114,36 @@ std::string share_sd_lines(const double *expected, const double *cov, double n) 
     return out;
 }
 
+const char *const kTractLengthsError =
+    "[::] ERROR: --tract-lengths takes 1 to 16 positive integers (bp), strictly increasing, separated by commas.\n";
+
+bool parse_tract_lengths(const char *arg, std::vector<uint64_t> *thresholds) {
+    thresholds->clear();
+    const char *p = arg;
+    while (true) {
+        uint64_t x = 0;
+        const char *d = p;
+        for (; *p >= '0' && *p <= '9'; p++) {
+            if (x > 1000000000000000000ULL) return false;
+            x = x * 10 + (uint64_t)(*p - '0');
+        }
+        if (p == d || x == 0 || thresholds->size() == 16 || (!thresholds->empty() && x <= thresholds->back())) return false;
+        thresholds->push_back(x);
+        if (*p == '\0') return true;
+        if (*p++ != ',') return false;
+    }
+}
+
+std::string tract_length_lines(const double *spectrum, const std::vector<uint64_t> &thresholds) {
+    std::string out;
+    char row[160];
+    for (int s = 0; s < 3; s++)
+        for (size_t k = 0; k < thresholds.size(); k++)
+            out.append(row, (size_t)snprintf(row, sizeof row, "#%% posterior IBD%d tracts >= %" PRIu64 " bp: %.2f\n", s, thresholds[k],
+                                             spectrum[k * 3 + (size_t)s]));
+    return out;
+}
+
 std::string tract_count_lines(const double *tracts, const double *tract_cov, const double *switches) {
     std::string out;
     char row[160];

@@ -58,4 +58,13 @@ std::string share_sd_lines(const double *expected, const double *cov, double n);
 // in '\n'.
 std::string tract_count_lines(const double *tracts, const double *tract_cov, const double *switches);
 
+// The --tract-lengths list: 1 to 16 positive integers separated by commas, strictly increasing; false when malformed.
+bool parse_tract_lengths(const char *arg, std::vector<uint64_t> *thresholds);
+extern const char *const kTractLengthsError;  // the message of a malformed list, ending in '\n'
+
+// --tract-lengths lines (hiddengem, ibdgem --hiddengem): from the posterior expected number of runs at least X bp long
+// (spectrum[K][3] for the K thresholds), "#% posterior IBDs tracts >= X bp: <E[R_s(X)]>" per state s, then threshold,
+// each ending in '\n'.
+std::string tract_length_lines(const double *spectrum, const std::vector<uint64_t> &thresholds);
+
 }  // namespace ibdhost

@@ -33,6 +33,9 @@
 //             form its switch probabilities from alpha of the bin before (switch_terms) and add them per bin slot;
 //             the tract counts follow from the switches into each state.  BWD_TR_COV: the solver lane also carries
 //             the tract-count recursion (moment_step<LG, true>) for their covariance.  No posteriors are written.
+//   tract lengths (hiddengem_tract_lengths_*, tract_lengths.cu) MODE = BWD_RUNS: the workers write, per bin, gamma and
+//             the run terms d and ln c of the same ratios (run_terms) to a per-bin array (72 B per bin) that
+//             tract_lengths_kernel reads.  No posteriors are written.
 //
 // Emissions (nrm; any positive per-bin factor cancels in gamma, so only the direction is needed):
 //   is_log = 0  l_s / ((l0 + l1) + l2) as hiddengem normalises summary-file likelihoods, with the division replaced
@@ -62,8 +65,8 @@ static_assert(HG_TABLES * HG_BINS * 3 <= HG_TABLES * HG_ROW, "expected-count par
 static_assert(HG_TABLES * HG_BINS * 9 <= 3 * HG_TABLES * HG_ROW, "switch partials fit in the other three staging buffers");
 
 // Variants of the backward pass: posteriors; + the moment recursion (solver lane); + switch and tract counts
-// (workers); + both, with the tract-count covariance on the solver lane.
-enum BwdMode { BWD_POST = 0, BWD_MOM = 1, BWD_TR = 2, BWD_TR_COV = 3 };
+// (workers); + both, with the tract-count covariance on the solver lane; per-bin run terms (workers).
+enum BwdMode { BWD_POST = 0, BWD_MOM = 1, BWD_TR = 2, BWD_TR_COV = 3, BWD_RUNS = 4 };
 
 // 2^-floor(log2 s) for s >= 0: multiplying by it is exact and brings s into [1, 2) (0 stays 0)
 __device__ __forceinline__ double pow2_recip(double s) {
@@ -330,6 +333,38 @@ __device__ __forceinline__ void switch_terms(const double *A, double y0, double 
     }
 }
 
+// Run terms of bin i >= 1 (BWD_RUNS) from alpha of bin i - 1 and gamma y of bin i, with the ratios r[k] of
+// switch_terms for l = s: d[s] = P(x_{i-1} != s | x_i = s, data <= i - 1), the sum of the other two, and lc[s] =
+// ln c_i(s) = ln P(x_{i-1} = s | x_i = s, data <= i - 1), clamped at -750 (then e^lc is below every subnormal, so a
+// window holding it contributes exactly 0 however the other terms fall) and -750 where gamma_i(s) = 0.  LG: A and
+// p01 / p02 / p12 are logs, and lc is the difference of logs itself.
+template <bool LG>
+__device__ __forceinline__ void run_terms(const double *A, double y0, double y1, double y2, double p01, double p02, double p12,
+                                          double (&d)[3], double (&lc)[3]) {
+    const double a[3] = {A[0], A[1], A[2]}, y[3] = {y0, y1, y2}, one = LG ? 0.0 : 1.0;
+    const double pen[3][3] = {{one, p01, p02}, {p01, one, p12}, {p02, p12, one}};
+#pragma unroll
+    for (int l = 0; l < 3; l++) {
+        const bool ok = y[l] > 0;
+        double r[3], lr;
+        if (LG) {
+            const double w0 = a[0] + pen[0][l], w1 = a[1] + pen[1][l], w2 = a[2] + pen[2][l], D = lse3(w0, w1, w2);
+            r[0] = ok ? exp_nonpos(w0 - D) : 0.0;
+            r[1] = ok ? exp_nonpos(w1 - D) : 0.0;
+            r[2] = ok ? exp_nonpos(w2 - D) : 0.0;
+            lr = (l == 0 ? w0 : l == 1 ? w1 : w2) - D;
+        } else {
+            const double w0 = a[0] * pen[0][l], w1 = a[1] * pen[1][l], w2 = a[2] * pen[2][l], inv = recip(w0 + w1 + w2);
+            r[0] = w0 * inv;
+            r[1] = w1 * inv;
+            r[2] = w2 * inv;
+            lr = log(r[l]);
+        }
+        d[l] = l == 0 ? r[1] + r[2] : l == 1 ? r[0] + r[2] : r[0] + r[1];
+        lc[l] = ok ? fmax(lr, -750.0) : -750.0;
+    }
+}
+
 // Workers: emissions of chunk c in place, once every worker has stored its part
 template <bool LG>
 __device__ __forceinline__ void emit(const ChunkLoader &ld, int c, double (*buf)[HG_ROW], int is_log) {
@@ -401,14 +436,16 @@ posterior_fwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
 // bin down, into cov[t][3][3]; posterior may then be null (nothing per bin is written).  BWD_TR: no posterior; the
 // workers also form the switches of each bin from alpha of the bin before (switch_terms; for a chunk's first bin the
 // previous chunk's checkpoint) and sum them per bin slot like the expected counts -> switches[t][3][3], tracts[t][3];
-// BWD_TR_COV adds the tract-count covariance on the solver lane -> cov[t][3][3].  The workers' gamma, posterior and
-// expected are those of the plain pass, bit for bit, and their switches and tracts the same with or without cov.
+// BWD_TR_COV adds the tract-count covariance on the solver lane -> cov[t][3][3].  BWD_RUNS: no posterior; the
+// workers write each bin's gamma, d and ln c (run_terms; bin 0: d = 1, ln c = 0) to runs[bin][9] in the layout of
+// lik.  The workers' gamma, posterior and expected are those of the plain pass, bit for bit, and their switches and
+// tracts the same with or without cov.
 template <bool LG, int MODE = BWD_POST>
 __global__ void __launch_bounds__(HG_THREADS, 3)
 posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int64_t *__restrict__ len, const double *__restrict__ lik,
                      int is_log, double p01, double p02, double p12, const double *__restrict__ ckpt, double *__restrict__ posterior,
                      double *__restrict__ expected, double *__restrict__ cov = nullptr, double *__restrict__ switches = nullptr,
-                     double *__restrict__ tracts = nullptr) {
+                     double *__restrict__ tracts = nullptr, double *__restrict__ runs = nullptr) {
     constexpr bool MOM = MODE == BWD_MOM, TR = MODE == BWD_TR || MODE == BWD_TR_COV, SOLVE = MOM || MODE == BWD_TR_COV;
     extern __shared__ double pb_smem[];
     double (*em)[HG_TABLES][HG_ROW] = reinterpret_cast<double (*)[HG_TABLES][HG_ROW]>(pb_smem);  // emissions, then beta
@@ -469,6 +506,16 @@ posterior_bwd_kernel(int n_tables, const int64_t *__restrict__ start, const int6
                             switch_terms<LG>(A, y0, y1, y2, p01, p02, p12, xi, phi);
 #pragma unroll
                             for (int kl = 0; kl < 9; kl++) S[k][kl] += xi[kl / 3][kl % 3];
+                        }
+                        if (MODE == BWD_RUNS) {
+                            double d[3] = {1.0, 1.0, 1.0}, lc[3] = {0.0, 0.0, 0.0};
+                            if (i0 + i > 0)
+                                run_terms<LG>(i > 0 ? &al[pb][t][(i - 1) * 3] : ckpt + ((size_t)(c - 1) * n_tables + tb0 + t) * 3, y0, y1,
+                                              y2, p01, p02, p12, d, lc);
+                            double *o = runs + (s_start[t] + i0 + i) * 9;
+                            o[0] = y0; o[1] = y1; o[2] = y2;
+                            o[3] = d[0]; o[4] = d[1]; o[5] = d[2];
+                            o[6] = lc[0]; o[7] = lc[1]; o[8] = lc[2];
                         }
                     }
                 }
@@ -602,11 +649,12 @@ bool linear_penalties(double p01, double p02, double p12) {
 }
 
 // Both passes in arithmetic LG; p01 / p02 / p12 as the kernels take them (LG: their logs).  d_sw selects the tract-count
-// variant of the backward pass (with d_cov: and its covariance), d_cov alone the moment variant.
+// variant of the backward pass (with d_cov: and its covariance), d_cov alone the moment variant, d_runs the run-term
+// variant.
 template <bool LG>
 int posterior_launch(ibdgem_engine *e, int n_tables, const int64_t *d_start, const int64_t *d_len, const double *d_lik, int is_log,
                      double p01, double p02, double p12, double *d_ckpt, double *d_post, double *d_expected, double *d_cov, double *d_sw,
-                     double *d_tr) {
+                     double *d_tr, double *d_runs) {
     const unsigned grid = (unsigned)((n_tables + HG_TABLES - 1) / HG_TABLES);
     {
         LaunchScope ls(e, K_POSTERIOR_FWD);
@@ -614,14 +662,15 @@ int posterior_launch(ibdgem_engine *e, int n_tables, const int64_t *d_start, con
         posterior_fwd_kernel<LG><<<grid, HG_THREADS, PB_FWD_SMEM, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt,
                                                                                d_expected);
     }
-    LaunchScope ls(e, d_sw ? K_POSTERIOR_BWD_TRACTS : d_cov ? K_POSTERIOR_BWD_MOMENTS : K_POSTERIOR_BWD);
+    LaunchScope ls(e, d_runs ? K_POSTERIOR_BWD_RUNS : d_sw ? K_POSTERIOR_BWD_TRACTS : d_cov ? K_POSTERIOR_BWD_MOMENTS : K_POSTERIOR_BWD);
     if (LG) e->k_launches[K_POSTERIOR_BWD_LOG]++;
-    const auto bwd = d_sw ? (d_cov ? posterior_bwd_kernel<LG, BWD_TR_COV> : posterior_bwd_kernel<LG, BWD_TR>)
-                          : (d_cov ? posterior_bwd_kernel<LG, BWD_MOM> : posterior_bwd_kernel<LG, BWD_POST>);
+    const auto bwd = d_runs ? posterior_bwd_kernel<LG, BWD_RUNS>
+                     : d_sw ? (d_cov ? posterior_bwd_kernel<LG, BWD_TR_COV> : posterior_bwd_kernel<LG, BWD_TR>)
+                            : (d_cov ? posterior_bwd_kernel<LG, BWD_MOM> : posterior_bwd_kernel<LG, BWD_POST>);
     const int smem = d_sw ? PB_TR_SMEM : PB_BWD_SMEM;
     IBD_CUDA(cudaFuncSetAttribute(bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     bwd<<<grid, HG_THREADS, smem, e->stream>>>(n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt, d_post, d_expected, d_cov,
-                                               d_sw, d_tr);
+                                               d_sw, d_tr, d_runs);
     return 0;
 }
 
@@ -672,7 +721,7 @@ int posterior_call(ibdgem_engine *e, const char *fn, int n_tables, const int64_t
 // One batch of tables, everything in device memory (start / len per table); kernels only, no host synchronisation.
 int ibdgem::posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins, const int64_t *d_start, const int64_t *d_len, const double *d_lik,
                         int is_log, double p01, double p02, double p12, double *d_post, double *d_expected, double *d_cov, double *d_sw,
-                        double *d_tr) {
+                        double *d_tr, double *d_runs) {
     const int64_t nck = (maxbins + HG_BINS - 1) / HG_BINS;
     if (nck == 0) {  // only empty tables: no bins, expected occupancy 0 (and covariance, switches, tracts 0)
         IBD_CUDA(cudaMemsetAsync(d_expected, 0, (size_t)n_tables * 24, e->stream));
@@ -685,9 +734,9 @@ int ibdgem::posterior_on_device(ibdgem_engine *e, int n_tables, int64_t maxbins,
     if (scratch(e, SC_HG_CKPT, (size_t)nck * n_tables * 24, (void **)&d_ckpt)) return 1;
     // log(0) = -inf: a forbidden transition
     if (linear_penalties(p01, p02, p12) ? posterior_launch<false>(e, n_tables, d_start, d_len, d_lik, is_log, p01, p02, p12, d_ckpt, d_post,
-                                                                  d_expected, d_cov, d_sw, d_tr)
+                                                                  d_expected, d_cov, d_sw, d_tr, d_runs)
                                         : posterior_launch<true>(e, n_tables, d_start, d_len, d_lik, is_log, log(p01), log(p02), log(p12),
-                                                                 d_ckpt, d_post, d_expected, d_cov, d_sw, d_tr))
+                                                                 d_ckpt, d_post, d_expected, d_cov, d_sw, d_tr, d_runs))
         return 1;
     IBD_CUDA(cudaGetLastError());
     return 0;

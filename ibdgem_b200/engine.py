@@ -335,6 +335,37 @@ class Engine:
             C.c_void_p(d_expected_ptr), C.c_void_p(d_switches_ptr), C.c_void_p(d_tracts_ptr),
             C.c_void_p(d_tract_cov_ptr or None)))
 
+    def tract_lengths_batch(self, lik, bin_offsets, thresholds, start=None, end=None, is_log=False, p01=1e-3, p02=1e-6,
+                            p12=1e-3):
+        """Posterior expected number of runs of each IBD state at least each threshold long
+        (hiddengem_tract_lengths_batch): [n_tables, len(thresholds), 3].  With start / end (per bin, packed like lik)
+        lengths are end[J] - start[i] + 1, otherwise bins."""
+        lik = np.ascontiguousarray(lik, np.float64)
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        th = np.ascontiguousarray(thresholds, np.uint64)
+        nt = len(off) - 1
+        st = None if start is None else np.ascontiguousarray(start, np.uint64)
+        en = None if end is None else np.ascontiguousarray(end, np.uint64)
+        spectrum = np.zeros((nt, len(th), 3))
+        self._check(self._lib.hiddengem_tract_lengths_batch(self._h, C.c_int32(nt), _ptr(off), _ptr(lik),
+                                                            C.c_int32(1 if is_log else 0), C.c_double(p01),
+                                                            C.c_double(p02), C.c_double(p12), _ptr(st), _ptr(en),
+                                                            C.c_int32(len(th)), _ptr(th), _ptr(spectrum)))
+        return spectrum
+
+    def tract_lengths_device(self, d_lik_ptr: int, bin_offsets: np.ndarray, is_log: bool, thresholds, d_spectrum_ptr: int,
+                             d_start_ptr: int = 0, d_end_ptr: int = 0, table_stride: int = 0, p01=1e-3, p02=1e-6,
+                             p12=1e-3):
+        """Device buffers in, device buffers out (hiddengem_tract_lengths_device; d_start_ptr / d_end_ptr 0: lengths
+        in bins); bin_offsets and thresholds stay on the host."""
+        off = np.ascontiguousarray(bin_offsets, np.int64)
+        th = np.ascontiguousarray(thresholds, np.uint64)
+        self._check(self._lib.hiddengem_tract_lengths_device(
+            self._h, C.c_int32(len(off) - 1), _ptr(off), C.c_int64(table_stride), C.c_void_p(d_lik_ptr),
+            C.c_int32(1 if is_log else 0), C.c_double(p01), C.c_double(p02), C.c_double(p12),
+            C.c_void_p(d_start_ptr or None), C.c_void_p(d_end_ptr or None), C.c_int32(len(th)), _ptr(th),
+            C.c_void_p(d_spectrum_ptr)))
+
     def tracts_batch(self, lik, bin_offsets, is_log=False, p01=1e-3, p02=1e-6, p12=1e-3, posterior=True):
         """IBD tracts (runs of one Viterbi state) with likelihood sums and, with posterior, the mean and minimum
         posterior of their state (hiddengem_tracts_batch + hiddengem_last_tracts): (tract_offsets [n_tables + 1],

@@ -326,6 +326,40 @@ int hiddengem_tract_counts_device(ibdgem_engine *e, int32_t n_tables, const int6
                                   const double *d_lik, int32_t is_log, double p01, double p02, double p12,
                                   double *d_expected, double *d_switches, double *d_tracts, double *d_tract_cov);
 
+/* Posterior tract-length spectrum: the posterior entries' model, emissions, uniform rule and penalties, and for one
+ * table of n bins, a state s and a threshold X, R_s(X) = the number of maximal runs [i, J] of state s whose length
+ * reaches X.  The length of [i, J] is bin_end[J] - bin_start[i] + 1 with coordinates (the span hiddengem --tracts
+ * prints; START / END of the summary rows, w_start / w_end of ibdgem_scores), J - i + 1 without.
+ * spectrum[t][k][s] = E[R_s(thresholds[k])] = sum_i d_i(s) prod_{m=i+1}^{J} c_m(s) gamma_J(s), J = J(i, X) the first
+ * bin J >= i with [i, J] at least X long (no such J: start bin i adds 0), with
+ *     c_m(s) = alpha_{m-1}(s) / sum_k alpha_{m-1}(k) pen(k, s)                    (P(x_{m-1} = s | x_m = s, data < m))
+ *     d_i(s) = sum_{k != s} alpha_{i-1}(k) pen(k, s) / sum_k alpha_{i-1}(k) pen(k, s),  d_0(s) = 1;
+ * the term is P(x_{i-1} != s, x_i = ... = x_J = s | data), each run counted once, at its first bin.  The product is
+ * formed as exp of a sum of ln c_m (clamped at -750) over pieces of the window only, never as a difference of
+ * prefix sums over the table.  Differences between thresholds give the expected histogram of run lengths; X = 1 bin
+ * gives E[T_s] of hiddengem_tract_counts_batch.  Each table's sums run in a fixed order: the same table gives the
+ * same bits in any batch or layout.
+ *   - An empty table gives 0; one bin gives gamma_0(s) when its own length reaches X and 0 otherwise; a table of
+ *     total weight 0 gives NaN everywhere; where gamma_m(s) = 0, c_m(s) is taken as 0.
+ *   - Independent tables (e.g. the chromosomes of one pair) add.
+ *   bin_start, bin_end  [bins] in the layout of lik, both or neither (NULL: lengths in bins); within each table
+ *                       start <= end and both non-decreasing, else the call fails
+ *   thresholds          HOST array of 1..16 values >= 1, strictly increasing (bp, or bins without coordinates)
+ *   spectrum            [n_tables][n_thresholds][3]
+ * Arguments, penalties and bin_offsets are checked as by hiddengem_posterior_batch.  The likelihoods and coordinates
+ * go up once; only the spectrum comes back. */
+int hiddengem_tract_lengths_batch(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, const double *lik,
+                                  int32_t is_log, double p01, double p02, double p12,
+                                  const uint64_t *bin_start, const uint64_t *bin_end,
+                                  int32_t n_thresholds, const uint64_t *thresholds, double *spectrum);
+/* The same on DEVICE buffers (bin_offsets and thresholds HOST arrays), with the layouts of
+ * hiddengem_posterior_batch_device: table t at bin t * table_stride when table_stride > 0, for the coordinates too
+ * (table_stride = max_windows and is_log = 1 take ibdgem_scores.w_loglik_device as is). */
+int hiddengem_tract_lengths_device(ibdgem_engine *e, int32_t n_tables, const int64_t *bin_offsets, int64_t table_stride,
+                                   const double *d_lik, int32_t is_log, double p01, double p02, double p12,
+                                   const uint64_t *d_bin_start, const uint64_t *d_bin_end,
+                                   int32_t n_thresholds, const uint64_t *thresholds, double *d_spectrum);
+
 /* IBD tracts.  A tract is a maximal run [first_bin, first_bin + n_bins) of bins of one table with the same Viterbi
  * state (in IBDGem a "segment" is one window, i.e. one bin).  Tracts never cross tables; an empty table has none.
  * Records are ordered table by table, then by first_bin; table t's are records [tract_offsets[t], tract_offsets[t+1]).
